@@ -23,7 +23,9 @@ Content is synthetic (tools/hevc_enc closed-loop encoder + tools/heif_writer), g
   cpu_baseline : the unmodified reference (oracle/_ref: libheif + libde265, heif_decode_image -> RGB) on
                  the host cores, bounded sample of the same file
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c4|c5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c4|c5] [--dump-outputs DIR]
+Every GPU measurement times exactly K steps. The content is seeded, so the same arguments give the same inputs on every run;
+--dump-outputs DIR writes what the timed path computed in its last step, so that two builds can be compared output for output.
 Launched under torchrun for N > 1 (one rank per GPU, NCCL only for the barrier / max-over-ranks / the C5 IPC handle).
 """
 import argparse
@@ -32,6 +34,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -52,6 +55,23 @@ STREAM_DEPTH = 6     # the most batches hc_heic_decode_stream keeps in flight (3
 METRIC = "decoded MP/s HEIC->RGB (device-timed)"
 UNIT = "MP/s"
 STAGES = ("k1_transform", "k2_intra", "k3_deblock", "k4_sao", "k5_csc")
+DUMP_BYTES = 60 << 20    # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir, n, read_rgb):
+    """--dump-outputs: the n interleaved RGB images of the last timed step (read_rgb(i) -> uint8 array, all of one size) as
+    DIR/rgb.npy, float32, one row per image. Images too large for DUMP_BYTES are sampled at fixed, seeded byte positions,
+    the same in every image, which go to DIR/rgb_positions.npy."""
+    import numpy as np
+    size = read_rgb(0).size
+    per_image = min(size, DUMP_BYTES // (4 * n + 8))
+    pos = np.arange(size) if per_image == size else np.sort(np.random.default_rng(0).choice(size, per_image, replace=False))
+    out = np.empty((n, per_image), np.float32)
+    for i in range(n):
+        out[i] = read_rgb(i).reshape(-1)[pos]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rgb.npy"), out)
+    np.save(os.path.join(out_dir, "rgb_positions.npy"), pos.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------------------- content
@@ -239,8 +259,9 @@ def plugin_arm(files, threads):
 
 
 # ------------------------------------------------------------------------------------------------- GPU measurements
-def measure_list(hb, eng, files, steps, warmup, threads, images, barrier, max_over_ranks, local_rank, sample_clocks=True):
-    """Image-list workloads (c2, c4): device-timed figures and the e2e stream figure (times already max-ed over the ranks)."""
+def measure_list(hb, eng, files, steps, warmup, threads, images, barrier, max_over_ranks, local_rank, sample_clocks=True, dump_dir=None):
+    """Image-list workloads (c2, c4): device-timed figures and the e2e stream figure (times already max-ed over the ranks).
+    dump_dir: where the RGB images of the last step of the `value` loop go (dump_outputs)."""
     import numpy as np
     job = hb.HeicJob(eng, files, want_alpha=False, threads=threads)
     job.upload()
@@ -283,13 +304,15 @@ def measure_list(hb, eng, files, steps, warmup, threads, images, barrier, max_ov
         check = bool(np.array_equal(job.read_rgb(0), heic_oracle.decode_rgb(files[0], hb.OUT_RGB)))
     except Exception as e:
         check = "unchecked: %s" % e
+    if dump_dir:
+        dump_outputs(dump_dir, len(files), job.read_rgb)
     job.close()
 
     # end to end: one call of the public streaming API. The figure is the STEADY-STATE period of the pipeline: deliveries of
     # the first and the last depth - 1 batches are left out (`depth` batches are in flight: the first delivery comes late
     # relative to the ones behind it, the last batches drain without successors — over 40 batches the first-to-last figure
-    # is 6 % better than the middle of the run, tools/stream_depth_probe.py), so 4 + e2e_steps batches are decoded.
-    e2e_steps = max(12, min(steps, 32))
+    # is 6 % better than the middle of the run, tools/stream_depth_probe.py), so 2 * skip + 1 + e2e_steps batches are decoded.
+    e2e_steps = steps
     skip = STREAM_DEPTH - 1   # deliveries left out at either end: the batches in flight behind / ahead of the window
     marks, checksum = [], [0]
 
@@ -314,8 +337,9 @@ def measure_list(hb, eng, files, steps, warmup, threads, images, barrier, max_ov
             "stream": st}
 
 
-def measure_c5(hb, eng, data, steps, warmup, threads, rank, world, dist, barrier, max_over_ranks):
-    """One huge grid, tile rows split across the ranks, every K5 writing its band into rank 0's hc_shared_image."""
+def measure_c5(hb, eng, data, steps, warmup, threads, rank, world, dist, barrier, max_over_ranks, dump_dir=None):
+    """One huge grid, tile rows split across the ranks, every K5 writing its band into rank 0's hc_shared_image.
+    dump_dir: where rank 0 writes the stitched image of the last timed step (dump_outputs)."""
     import hashlib
     import torch
     from heif_b200.multigpu import BandJob, SharedImage
@@ -377,6 +401,8 @@ def measure_c5(hb, eng, data, steps, warmup, threads, rank, world, dist, barrier
         full = shared.read()
         d2h_s = time.perf_counter() - t0
         md5 = hashlib.md5(full.tobytes()).hexdigest()
+        if dump_dir:
+            dump_outputs(dump_dir, 1, lambda i: full)
         del full
     barrier()
     band_rows = job.desc.height if has else 0
@@ -419,7 +445,7 @@ def c5_report(c5, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every GPU measurement")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -436,6 +462,9 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="multi-GPU runs: do not bind a rank's threads to the CPUs next to its GPU")
     ap.add_argument("--skip-baselines", action="store_true", help="kernel experiments: leave out the cpu_baseline and plugin_dropin arms")
     ap.add_argument("--skip-extras", action="store_true", help="leave out the c4 / c5 side measurements of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the RGB images the workload's timed path computed in its last step "
+                    "(rank 0's) to DIR/rgb.npy as float32, sampled at the seeded byte positions in DIR/rgb_positions.npy when "
+                    "they exceed 60 MiB in all")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     wl = args.workload
@@ -470,7 +499,8 @@ def main():
                 numa = "%d cpus next to GPU %d" % (len(cpus), local_rank)
         except Exception as e:      # no NVML, one socket, containers without the right: run unpinned
             numa = "unpinned (%s)" % type(e).__name__
-    cache = os.path.join(ROOT, "gpurun_out", "bench_content")
+    # the synthetic content is cached outside the tree, which may be read-only; one directory per user, shared by the ranks
+    cache = os.path.join(tempfile.gettempdir(), "heif_b200_bench_content_%d" % os.getuid())
     file_mp = {"c2": GRID_W * GRID_H / 1e6, "c4": C4_W * C4_H / 1e6, "c5": C5_W * C5_H / 1e6}[wl]
 
     if args.impl == "reference":
@@ -557,7 +587,8 @@ def main():
         rec0 = hb.parse_picture(hf.coded_stream(first_item))
         rec_bytes_per_px = rec0.upload_bytes / float(rec0.pic.width * rec0.pic.height)
         hf.close()
-        m = measure_list(hb, eng, files, args.steps, args.warmup, threads, images, barrier, max_over_ranks, local_rank)
+        m = measure_list(hb, eng, files, args.steps, args.warmup, threads, images, barrier, max_over_ranks, local_rank,
+                         dump_dir=args.dump_outputs if rank == 0 else None)
         st = m["stream"]
         # ---- roofline of the dominant reconstruction kernel (algorithmic bytes for 8-bit 4:2:0: SURVEY 8d, DESIGN "kernels") ----
         px = images * file_mp * 1e6
@@ -620,7 +651,8 @@ def main():
                          "note": "k2_intra is a dependency-latency-bound CTB wavefront, not a streaming kernel (DESIGN.md)"},
         })
     else:
-        c5 = measure_c5(hb, eng, c5_file, args.steps, args.warmup, threads, rank, world, dist, barrier, max_over_ranks)
+        c5 = measure_c5(hb, eng, c5_file, args.steps, args.warmup, threads, rank, world, dist, barrier, max_over_ranks,
+                        dump_dir=args.dump_outputs)
         rep = c5_report(c5, world)
         line.update({"value": rep["value"], "ms_per_step": rep["ms_per_step"], "scaling": "strong", "value_what": rep["value_what"],
                      "config": {"workload": WORKLOADS["c5"], "tiles": 391, "parity_vs_single_gpu": c5.get("bit_exact_vs_single_gpu")},
@@ -635,7 +667,7 @@ def main():
         try:
             n4 = 384      # 1080p pictures are 17 chains each: 96 files fill a third of K0's chain slots (value 1.5 GP/s), 384 fill them (3.2)
             files4 = [c4_files[(i + rank) % len(c4_files)] for i in range(n4)]
-            m4 = measure_list(hb, eng, files4, max(3, args.steps // 3), 3, threads, n4, barrier, max_over_ranks, local_rank, sample_clocks=False)
+            m4 = measure_list(hb, eng, files4, args.steps, args.warmup, threads, n4, barrier, max_over_ranks, local_rank, sample_clocks=False)
             mp4 = n4 * C4_W * C4_H / 1e6
             line["c4"] = {"workload": WORKLOADS["c4"], "images_per_step_per_gpu": n4, "value": world * mp4 / (m4["dev_ms"] * 1e-3),
                           "value_reconstruction_only": world * mp4 / (m4["recon_ms"] * 1e-3), "e2e_value": world * mp4 / m4["e2e_dt"], "unit": UNIT,
@@ -643,7 +675,7 @@ def main():
         except Exception as e:      # a side measurement never takes the main line down
             line["c4"] = {"error": str(e)}
         try:
-            line["c5"] = c5_report(measure_c5(hb, eng, c5_file, max(3, args.steps // 3), 3, threads, rank, world, dist, barrier, max_over_ranks), world)
+            line["c5"] = c5_report(measure_c5(hb, eng, c5_file, args.steps, args.warmup, threads, rank, world, dist, barrier, max_over_ranks), world)
         except Exception as e:
             line["c5"] = {"error": str(e)}
 

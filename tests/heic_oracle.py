@@ -35,14 +35,21 @@ def _rescale_limited(plane, chroma, bit_depth):
     return np.clip(x, 0, 255).astype(np.uint16)
 
 
-def decode_planes(data, item_id=None):
-    """Returns (planes[list], alpha or None, chroma_format, bit_depth, (matrix, full_range, primaries))"""
+def _oracle_picture(stream, rec):
+    return oracle_lib.reconstruct(rec)[0]
+
+
+def decode_planes(data, item_id=None, picture=_oracle_picture):
+    """Returns (planes[list], alpha or None, chroma_format, bit_depth, (matrix, full_range, primaries)).
+    picture(coded stream, its records) -> cropped planes of one coded picture: the oracle, or another HEVC decoder in
+    the place libheif gives its decoder plugin."""
     hf = hb.HeifFile(data, host_only=True)
     iid = item_id or hf.primary_id
     info = hf.image_info(iid)
     if info.is_grid:
         ids = hf.grid_tiles(iid)
-        recs = [hb.parse_picture(hf.coded_stream(t), host_only=True) for t in ids]
+        streams = [hf.coded_stream(t) for t in ids]
+        recs = [hb.parse_picture(s, host_only=True) for s in streams]
         p0 = recs[0].pic
         cf, bd = p0.chroma_format, p0.bit_depth_y
         W, H = info.width, info.height
@@ -52,8 +59,8 @@ def decode_planes(data, item_id=None):
         if cf:
             canvas += [np.zeros(((H + sh - 1) // sh, (W + sw - 1) // sw), np.uint16) for _ in range(2)]
         tw, th = p0.crop_w, p0.crop_h
-        for i, (t, r) in enumerate(zip(ids, recs)):
-            pl, _ = oracle_lib.reconstruct(r)
+        for i, (t, s, r) in enumerate(zip(ids, streams, recs)):
+            pl = picture(s, r)
             tinfo = hf.image_info(t)
             full = tinfo.full_range if tinfo.nclx_present else r.pic.full_range
             matrix = tinfo.matrix if tinfo.nclx_present else r.pic.matrix_coeffs
@@ -67,19 +74,20 @@ def decode_planes(data, item_id=None):
         nclx = (info.matrix, info.full_range, info.primaries) if info.nclx_present else (2, 1, 2)
         planes = canvas
     else:
-        r = hb.parse_picture(hf.coded_stream(iid), host_only=True)
-        planes, _ = oracle_lib.reconstruct(r)
+        s = hf.coded_stream(iid)
+        r = hb.parse_picture(s, host_only=True)
+        planes = picture(s, r)
         cf, bd = r.pic.chroma_format, r.pic.bit_depth_y
         nclx = (info.matrix, info.full_range, info.primaries) if info.nclx_present else (r.pic.matrix_coeffs, r.pic.full_range, r.pic.colour_primaries)
     alpha = None
     if info.alpha_id:
         ainfo = hf.image_info(info.alpha_id)
         if ainfo.is_grid:     # the alpha image is decoded like any image item (context.cc:2040-2071): a grid of its own
-            apl = [decode_planes(data, info.alpha_id)[0][0]]
+            apl = [decode_planes(data, info.alpha_id, picture)[0][0]]
             alpha = apl[0]    # decode_planes applied the alpha item's own transformations already
         else:
-            a = hb.parse_picture(hf.coded_stream(info.alpha_id), host_only=True)
-            apl, _ = oracle_lib.reconstruct(a)
+            s = hf.coded_stream(info.alpha_id)
+            apl = picture(s, hb.parse_picture(s, host_only=True))
             alpha = _transform_all([apl[0]], ainfo)[0]
     planes = _transform_all(planes, info)
     if alpha is not None and alpha.shape != planes[0].shape:
@@ -171,6 +179,6 @@ def _transform_all(planes, info):
     return [np.ascontiguousarray(p) for p in planes]
 
 
-def decode_rgb(data, out_format, item_id=None, upsampling=0):
-    planes, alpha, cf, bd, (matrix, full, primaries) = decode_planes(data, item_id)
+def decode_rgb(data, out_format, item_id=None, upsampling=0, picture=_oracle_picture):
+    planes, alpha, cf, bd, (matrix, full, primaries) = decode_planes(data, item_id, picture)
     return csc(planes, cf, bd, matrix, full, out_format, alpha, primaries, upsampling)

@@ -10,17 +10,24 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 SO = os.path.join(ORACLE_DIR, "_build", "liboracle.so")
 SOURCES = ["hevc_recon_oracle.c", "csc_oracle.c"]
+# libheif's image / nclx callbacks for driving the decoder plugin without the reference libheif (oracle/plugin_host.c)
+PLUGIN_HOST_SO = os.path.join(ORACLE_DIR, "_build", "libplugin_host.so")
 
 STAGE_DEBLOCK, STAGE_SAO, STAGE_ALL = 1, 2, 3
 _lib = None
 
 
+def _compile(so, srcs, force):
+    if not force and os.path.exists(so) and all(os.path.getmtime(so) >= os.path.getmtime(s) for s in srcs):
+        return
+    os.makedirs(os.path.dirname(so), exist_ok=True)
+    subprocess.check_call(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-o", so] + srcs + ["-lm"])
+
+
 def build(force=False):
     srcs = [os.path.join(ORACLE_DIR, s) for s in SOURCES if os.path.exists(os.path.join(ORACLE_DIR, s))]
-    if not force and os.path.exists(SO) and all(os.path.getmtime(SO) >= os.path.getmtime(s) for s in srcs):
-        return SO
-    os.makedirs(os.path.dirname(SO), exist_ok=True)
-    subprocess.check_call(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-o", SO] + srcs + ["-lm"])
+    _compile(SO, srcs, force)
+    _compile(PLUGIN_HOST_SO, [os.path.join(ORACLE_DIR, "plugin_host.c")], force)
     return SO
 
 
