@@ -22,14 +22,26 @@
 #include <stddef.h>
 #include <stdint.h>
 #include <stdlib.h>
+#include "oracle_counters.h"
 
+static void count_clip(int lo, int maxi) {
+  switch (maxi) {
+    case 255: if (lo) HC_COUNT(k5_clip_lo_8); else HC_COUNT(k5_clip_hi_8); break;
+    case 1023: if (lo) HC_COUNT(k5_clip_lo_10); else HC_COUNT(k5_clip_hi_10); break;
+    case 4095: if (lo) HC_COUNT(k5_clip_lo_12); else HC_COUNT(k5_clip_hi_12); break;
+    default: break;
+  }
+}
 static uint16_t clip_f_u16(float fx, int32_t maxi) { /* common_utils.h:64-70 */
   long x = (long)(fx + 0.5f);
-  if (x < 0) return 0;
-  if (x > maxi) return (uint16_t)maxi;
+  if (x < 0) { count_clip(1, maxi); return 0; }
+  if (x > maxi) { count_clip(0, maxi); return (uint16_t)maxi; }
   return (uint16_t)x;
 }
-static uint8_t clip_int_u8(int x) { return x < 0 ? 0 : (x > 255 ? 255 : (uint8_t)x); }
+static uint8_t clip_int_u8(int x) {
+  if (x < 0 || x > 255) count_clip(x < 0, 255);
+  return x < 0 ? 0 : (x > 255 ? 255 : (uint8_t)x);
+}
 
 typedef struct { float r_cr, g_cb, g_cr, b_cb; } coeffs_t;
 

@@ -18,6 +18,22 @@
 #include <stdlib.h>
 #include <string.h>
 #include "../include/heifcuda_records.h"
+#include "oracle_counters.h"
+
+uint64_t hc_oracle_counter[HC_CNT_COUNT];
+static const char* const kCounterNames[HC_CNT_COUNT] = {
+#define X(n) #n,
+    HC_ORACLE_COUNTERS
+#undef X
+};
+
+void hc_oracle_counters_reset(void) { memset(hc_oracle_counter, 0, sizeof(hc_oracle_counter)); }
+/* Copies up to n counters to out; returns the number of counters. */
+int hc_oracle_counters(uint64_t* out, int n) {
+  for (int i = 0; i < n && i < HC_CNT_COUNT; i++) out[i] = hc_oracle_counter[i];
+  return HC_CNT_COUNT;
+}
+const char* hc_oracle_counter_name(int i) { return i >= 0 && i < HC_CNT_COUNT ? kCounterNames[i] : NULL; }
 
 static inline int clip3i(int lo, int hi, int v) { return v < lo ? lo : (v > hi ? hi : v); }
 static inline int clip_bd(int v, int bd) { return clip3i(0, (1 << bd) - 1, v); }
@@ -86,7 +102,10 @@ static void oracle_tb_residual(const hc_pic* pic, const hc_tb* tb, const hc_coef
     for (int i = 0; i < tb->ncoeff; i++) {
       int32_t c = coeffs[i].level;
       /* int32 arithmetic with wrap, as in the reference (SURVEY hazard 1) */
+      const int64_t exact = ((int64_t)c * fact + offset) >> bdShift;
       c = (int32_t)((uint32_t)c * (uint32_t)fact + (uint32_t)offset) >> bdShift;
+      if (exact != c) HC_COUNT(k1_flat_dequant_wrap);
+      if (c < -32768 || c > 32767) HC_COUNT(k1_dequant_clip16);
       coeff[coeffs[i].pos] = (int16_t)clip3i(-32768, 32767, c);
     }
   } else {
@@ -101,8 +120,10 @@ static void oracle_tb_residual(const hc_pic* pic, const hc_tb* tb, const hc_coef
     for (int i = 0; i < tb->ncoeff; i++) {
       int pos = coeffs[i].pos;
       int fact = (sc[pos] * kLevelScale[qP % 6]) << (qP / 6);
+      if (sc[pos] >= 200) HC_COUNT(k1_scaled_factor_ge200);
       int64_t c = coeffs[i].level;
       c = (c * fact + offset) >> bdShift;
+      if (c < -32768 || c > 32767) HC_COUNT(k1_dequant_clip16);
       coeff[pos] = (int16_t)(c < -32768 ? -32768 : (c > 32767 ? 32767 : c));
     }
   }
@@ -136,12 +157,14 @@ static void oracle_tb_residual(const hc_pic* pic, const hc_tb* tb, const hc_coef
       for (int i = 0; i < 4; i++) {
         int sum = 0;
         for (int j = 0; j < 4; j++) sum += kDst[j][i] * coeff[c + j * 4];
+        if (((sum + rnd1) >> 7) < -32768 || ((sum + rnd1) >> 7) > 32767) HC_COUNT(k1_dst_pass1_clip);
         g[i * 4 + c] = (int16_t)clip3i(-32768, 32767, (sum + rnd1) >> 7);
       }
     for (int y = 0; y < 4; y++)
       for (int i = 0; i < 4; i++) {
         int sum = 0;
         for (int j = 0; j < 4; j++) sum += kDst[j][i] * g[y * 4 + j];
+        if (((sum + rnd2) >> postShift) < -32768 || ((sum + rnd2) >> postShift) > 32767) HC_COUNT(k1_dst_pass2_clip);
         res[y * 4 + i] = clip3i(-32768, 32767, (sum + rnd2) >> postShift);
       }
     return;
@@ -153,6 +176,7 @@ static void oracle_tb_residual(const hc_pic* pic, const hc_tb* tb, const hc_coef
     for (int i = 0; i < nT; i++) {
       int sum = 0;
       for (int j = 0; j < nT; j++) sum += g_dct[fact * j][i] * coeff[c + j * nT];
+      if (((sum + rnd1) >> 7) < -32768 || ((sum + rnd1) >> 7) > 32767) HC_COUNT(k1_dct_pass1_clip);
       g[c + i * nT] = (int16_t)clip3i(-32768, 32767, (sum + rnd1) >> 7);
     }
   for (int y = 0; y < nT; y++)
@@ -238,18 +262,21 @@ static void oracle_predict(const hc_pic* pic, const hc_blk* b, uint16_t* plane, 
       pF[-2 * nT] = p[-2 * nT];
       pF[2 * nT] = p[2 * nT];
       if (biInt) {
+        HC_COUNT(k2_strong_smoothing);
         pF[0] = p[0];
         for (int i = 1; i <= 63; i++) {
           pF[-i] = p[0] + ((i * (p[-64] - p[0]) + 32) >> 6);
           pF[i] = p[0] + ((i * (p[64] - p[0]) + 32) >> 6);
         }
       } else {
+        HC_COUNT(k2_121_smoothing);
         for (int i = -(2 * nT - 1); i <= 2 * nT - 1; i++) pF[i] = (p[i + 1] + 2 * p[i] + p[i - 1] + 2) >> 2;
       }
       for (int i = -2 * nT; i <= 2 * nT; i++) p[i] = pF[i];
     }
   }
 
+  if (mode <= 34) hc_oracle_counter[HC_CNT_k2_mode_0 + mode]++;
   if (mode == 0) { /* planar, intrapred.h:269-293 */
     for (int y = 0; y < nT; y++)
       for (int x = 0; x < nT; x++)
@@ -315,6 +342,12 @@ static const uint8_t kBetaTab[52] = {0,  0,  0,  0,  0,  0,  0,  0,  0,  0,  0, 
 static const uint8_t kTcTab[54] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,  0,  0,  0,  0,
                                    1, 1, 1, 1, 1, 1, 1, 1, 1, 2, 2, 2, 2, 3,  3,  3,  3,  4,
                                    4, 4, 5, 5, 6, 6, 7, 8, 9, 10, 11, 13, 14, 16, 18, 20, 22, 24};
+/* clip3(0, 53, idx) of the tc table index */
+static int count_tc_idx(int idx) {
+  if (idx < 0) HC_COUNT(k3_tc_idx_clamp_lo);
+  if (idx > 53) HC_COUNT(k3_tc_idx_clamp_hi);
+  return clip3i(0, 53, idx);
+}
 static int qpc_420(int qPi) { /* H.265 Table 8-10 / transform.cc table8_22 */
   static const int8_t t[14] = {29, 30, 31, 32, 33, 33, 34, 34, 35, 35, 36, 36, 37, 37};
   if (qPi < 30) return qPi;
@@ -356,10 +389,11 @@ static void oracle_deblock_luma(const dbk_ctx* d, uint16_t* plane, int stride, i
       int QP_P = vertical ? qp_at(d, x - 1, y) : qp_at(d, x, y - 1);
       int qPL = (QP_Q + QP_P + 1) >> 1;
       const hc_ctu* ctu = ctu_at(d, x, y);
+      if (qPL + ctu->beta_offset < 0 || qPL + ctu->beta_offset > 51) HC_COUNT(k3_beta_idx_clamp);
       int beta = kBetaTab[clip3i(0, 51, qPL + ctu->beta_offset)] * (1 << (bd - 8));
       int tcs[2];
-      tcs[0] = bs0 ? kTcTab[clip3i(0, 53, qPL + 2 * (bs0 - 1) + ctu->tc_offset)] * (1 << (bd - 8)) : 0;
-      tcs[1] = bs1 ? kTcTab[clip3i(0, 53, qPL + 2 * (bs1 - 1) + ctu->tc_offset)] * (1 << (bd - 8)) : 0;
+      tcs[0] = bs0 ? kTcTab[count_tc_idx(qPL + 2 * (bs0 - 1) + ctu->tc_offset)] * (1 << (bd - 8)) : 0;
+      tcs[1] = bs1 ? kTcTab[count_tc_idx(qPL + 2 * (bs1 - 1) + ctu->tc_offset)] * (1 << (bd - 8)) : 0;
       const ptrdiff_t xs = vertical ? 1 : stride, ys = vertical ? stride : 1;
       uint16_t* pix = plane + x + (size_t)y * stride;
       for (int j = 0; j < 2; j++, pix += 4 * ys) {
@@ -386,6 +420,7 @@ static void oracle_deblock_luma(const dbk_ctx* d, uint16_t* plane, int stride, i
             iabs(PX(-4, 3) - PX(-1, 3)) + iabs(PX(3, 3) - PX(0, 3)) < beta_3 && iabs(PX(-1, 3) - PX(0, 3)) < tc25 &&
             (d0 << 1) < beta_2 && (d3 << 1) < beta_2) {
           const int tc2 = tc << 1;
+          HC_COUNT(k3_luma_strong);
           for (int k = 0; k < 4; k++) {
             const int p3 = PX(-4, k), p2 = PX(-3, k), p1 = PX(-2, k), p0 = PX(-1, k);
             const int q0 = PX(0, k), q1 = PX(1, k), q2 = PX(2, k), q3 = PX(3, k);
@@ -405,6 +440,8 @@ static void oracle_deblock_luma(const dbk_ctx* d, uint16_t* plane, int stride, i
           const int tc_2 = tc >> 1;
           if (dp0 + dp3 < ((beta + (beta >> 1)) >> 3)) nd_p = 2;
           if (dq0 + dq3 < ((beta + (beta >> 1)) >> 3)) nd_q = 2;
+          HC_COUNT(k3_luma_weak);
+          if (nd_p > 1 || nd_q > 1) HC_COUNT(k3_luma_weak_nd2);
           for (int k = 0; k < 4; k++) {
             const int p2 = PX(-3, k), p1 = PX(-2, k), p0 = PX(-1, k);
             const int q0 = PX(0, k), q1 = PX(1, k), q2 = PX(2, k);
@@ -445,9 +482,11 @@ static void oracle_deblock_chroma(const dbk_ctx* d, uint16_t* plane, int stride,
         int QP_Q = qp_at(d, qx, qy);
         int QP_P = vertical ? qp_at(d, qx - 1, qy) : qp_at(d, qx, qy - 1);
         int qPi = ((QP_Q + QP_P + 1) >> 1) + cQpPicOffset;
+        if (qPi >= 30 && qPi <= 43) HC_COUNT(k3_chroma_qpi_30_43);
+        if (qPi < 0) HC_COUNT(k3_chroma_qpi_neg);
         int QpC = pic->chroma_format == 1 ? qpc_420(qPi) : (qPi < 51 ? qPi : 51);
         int tc_offset = ctu_at(d, lx, ly)->tc_offset;
-        int tcPrime = kTcTab[clip3i(0, 53, QpC + 2 + tc_offset)];
+        int tcPrime = kTcTab[count_tc_idx(QpC + 2 + tc_offset)];
         tcv[j] = ((j ? bS1 : bS0) == 2) ? tcPrime * (1 << (bd - 8)) : 0;
       }
       const int xDi = lx / SubW, yDi = ly / SubH;
@@ -493,6 +532,11 @@ static int sao_sample_skipped(const hc_pic* pic, int e) {
   return ((pic->flags & HC_PIC_PCM_LF_DISABLED) && (e & HC_EDGE_PCM)) || (e & HC_EDGE_BYPASS);
 }
 
+static void count_sao_clip(int v, int maxv) {
+  if (v < 0) HC_COUNT(k4_clip_lo);
+  else if (v > maxv) HC_COUNT(k4_clip_hi);
+}
+
 /* sao.cc:261-488 apply_sao_internal, :552-625 driver. in = deblocked copy, out = picture. */
 static void oracle_sao_plane(const hc_pic* pic, const hc_ctu* ctus, const uint8_t* edge, int cIdx, const uint16_t* in,
                              uint16_t* out, int stride) {
@@ -525,7 +569,7 @@ static void oracle_sao_plane(const hc_pic* pic, const hc_ctu* ctus, const uint8_
         for (int j = 0; j < ctbH; j++)
           for (int i = 0; i < ctbW; i++) {
             const int x = xC + i, y = yC + j;
-            if (nofilt && sao_sample_skipped(pic, edge[((x * SubW) >> 2) + (size_t)((y * SubH) >> 2) * w4])) continue;
+            if (nofilt && sao_sample_skipped(pic, edge[((x * SubW) >> 2) + (size_t)((y * SubH) >> 2) * w4])) { HC_COUNT(k4_skip_nofilter); continue; }
             int skip = 0;
             const int on_border = (i == 0 || j == 0 || i == ctbW - 1 || j == ctbH - 1);
             for (int k = 0; k < 2 && !skip; k++) {
@@ -548,6 +592,7 @@ static void oracle_sao_plane(const hc_pic* pic, const hc_ctu* ctus, const uint8_
             const int c = in[x + (size_t)y * stride];
             const int e = isign(c - in[(x + hPos[0]) + (size_t)(y + vPos[0]) * stride]) +
                           isign(c - in[(x + hPos[1]) + (size_t)(y + vPos[1]) * stride]);
+            count_sao_clip(c + off[e + 2], maxv);
             out[x + (size_t)y * stride] = (uint16_t)clip3i(0, maxv, c + off[e + 2]);
           }
       } else {
@@ -558,10 +603,14 @@ static void oracle_sao_plane(const hc_pic* pic, const hc_ctu* ctus, const uint8_
         for (int j = 0; j < ctbH; j++)
           for (int i = 0; i < ctbW; i++) {
             const int x = xC + i, y = yC + j;
-            if (nofilt && sao_sample_skipped(pic, edge[((x * SubW) >> 2) + (size_t)((y * SubH) >> 2) * w4])) continue;
+            if (nofilt && sao_sample_skipped(pic, edge[((x * SubW) >> 2) + (size_t)((y * SubH) >> 2) * w4])) { HC_COUNT(k4_skip_nofilter); continue; }
             const int c = in[x + (size_t)y * stride];
             const int bandIdx = bandTable[c >> bandShift];
-            if (bandIdx > 0) out[x + (size_t)y * stride] = (uint16_t)clip3i(0, maxv, c + ctu->sao_offset[cIdx][bandIdx - 1]);
+            if (bandIdx > 0) {
+              if (bandIdx - 1 + ctu->sao_band_or_class[cIdx] > 31) HC_COUNT(k4_band_wrap);
+              count_sao_clip(c + ctu->sao_offset[cIdx][bandIdx - 1], maxv);
+              out[x + (size_t)y * stride] = (uint16_t)clip3i(0, maxv, c + ctu->sao_offset[cIdx][bandIdx - 1]);
+            }
           }
       }
     }
@@ -593,7 +642,14 @@ int hc_oracle_reconstruct(const hc_pic* pic, const hc_ctu* ctus, const hc_blk* b
     int32_t r[32 * 32];
     const int n = 1 << (2 * tb->log2);
     oracle_tb_residual(pic, tb, coeffs + tb->coeff_off, scaling, r);
-    for (int i = 0; i < n; i++) resid[tb->resid_off + i] = (int16_t)clip3i(-32768, 32767, r[i]);
+    for (int i = 0; i < n; i++) {
+      if (r[i] < -32768 || r[i] > 32767) {
+        if (tb->type & (HC_TB_RDPCM_H | HC_TB_RDPCM_V)) HC_COUNT(k1_rdpcm_clip);
+        else if (tb->type & HC_TB_TSKIP) HC_COUNT(k1_tskip_clip);
+        else if (!(tb->type & (HC_TB_BYPASS | HC_TB_DST))) HC_COUNT(k1_dct_store_clip);
+      }
+      resid[tb->resid_off + i] = (int16_t)clip3i(-32768, 32767, r[i]);
+    }
   }
   /* K2 equivalent: CTBs in raster order, component chains independent */
   for (int a = 0; a < pic->ctbs_w * pic->ctbs_h; a++)
@@ -615,7 +671,12 @@ int hc_oracle_reconstruct(const hc_pic* pic, const hc_ctu* ctus, const hc_blk* b
         for (int y = 0; y < nT; y++)
           for (int x = 0; x < nT; x++) {
             int v = pred[x + y * nT];
-            if (b->flags & HC_BLK_HAS_RESID) v = clip_bd(v + resid[b->resid_off + x + y * nT], bd);
+            if (b->flags & HC_BLK_HAS_RESID) {
+              const int s = v + resid[b->resid_off + x + y * nT];
+              if (s < 0) HC_COUNT(k2_add_clip_lo);
+              else if (s > (1 << bd) - 1) HC_COUNT(k2_add_clip_hi);
+              v = clip_bd(s, bd);
+            }
             pl[(b->x + x) + (size_t)(b->y + y) * st] = (uint16_t)v;
           }
       }

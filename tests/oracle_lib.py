@@ -10,6 +10,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 SO = os.path.join(ORACLE_DIR, "_build", "liboracle.so")
 SOURCES = ["hevc_recon_oracle.c", "csc_oracle.c"]
+HEADERS = ["oracle_counters.h"]
 # libheif's image / nclx callbacks for driving the decoder plugin without the reference libheif (oracle/plugin_host.c)
 PLUGIN_HOST_SO = os.path.join(ORACLE_DIR, "_build", "libplugin_host.so")
 
@@ -17,8 +18,8 @@ STAGE_DEBLOCK, STAGE_SAO, STAGE_ALL = 1, 2, 3
 _lib = None
 
 
-def _compile(so, srcs, force):
-    if not force and os.path.exists(so) and all(os.path.getmtime(so) >= os.path.getmtime(s) for s in srcs):
+def _compile(so, srcs, force, deps=()):
+    if not force and os.path.exists(so) and all(os.path.getmtime(so) >= os.path.getmtime(s) for s in list(srcs) + list(deps)):
         return
     os.makedirs(os.path.dirname(so), exist_ok=True)
     subprocess.check_call(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-o", so] + srcs + ["-lm"])
@@ -26,7 +27,7 @@ def _compile(so, srcs, force):
 
 def build(force=False):
     srcs = [os.path.join(ORACLE_DIR, s) for s in SOURCES if os.path.exists(os.path.join(ORACLE_DIR, s))]
-    _compile(SO, srcs, force)
+    _compile(SO, srcs, force, [os.path.join(ORACLE_DIR, h) for h in HEADERS])
     _compile(PLUGIN_HOST_SO, [os.path.join(ORACLE_DIR, "plugin_host.c")], force)
     return SO
 
@@ -36,7 +37,22 @@ def lib():
     if _lib is None:
         _lib = C.CDLL(build())
         _lib.hc_oracle_reconstruct.restype = C.c_int
+        _lib.hc_oracle_counters.restype = C.c_int
+        _lib.hc_oracle_counter_name.restype = C.c_char_p
     return _lib
+
+
+def counters_reset():
+    lib().hc_oracle_counters_reset()
+
+
+def counters():
+    """{name: count} of the oracle's branch counters (oracle/oracle_counters.h) since the last counters_reset()"""
+    O = lib()
+    n = O.hc_oracle_counters(None, 0)
+    out = (C.c_uint64 * n)()
+    O.hc_oracle_counters(out, n)
+    return {O.hc_oracle_counter_name(i).decode(): int(out[i]) for i in range(n)}
 
 
 def plane_dims(pic):

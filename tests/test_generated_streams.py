@@ -81,7 +81,7 @@ def test_gpu_matches_reference_and_oracle(engine, name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("stages", [0, hb.STAGE_DEBLOCK])
 def test_gpu_intermediate_stages_match_oracle(engine, stages):
-    for name in ("c422_12", "c444_10", "pcm_bypass_422", "slices_nolf_422_t", "tiles_3x2_nolf", "scaling_custom_10", "mono_12"):
+    for name in NAMES:
         rec = hb.parse_picture(stream(name))
         (got,), _ = gpu_decode(engine, [rec], stages)
         want, _ = oracle_lib.reconstruct(rec, stages)

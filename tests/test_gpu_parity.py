@@ -44,6 +44,14 @@ def pictures():
     return all_pictures()
 
 
+@pytest.fixture(scope="module")
+def generated_pictures():
+    """(label, Records) of every generated stream (tests/golden/generated/)"""
+    names = sorted(json.load(open(os.path.join(ROOT, "tests", "golden", "generated.json"))))
+    return [(n, hb.parse_picture(open(os.path.join(ROOT, "tests", "golden", "generated", n + ".hevc"), "rb").read()))
+            for n in names]
+
+
 def gpu_planes(engine, rec, stages):
     b = engine.batch()
     p = rec.pic
@@ -77,12 +85,13 @@ def test_planes_match_oracle_per_stage(engine, pictures, stages):
 
 
 @pytest.mark.parametrize("stages", [0, hb.STAGE_DEBLOCK, hb.STAGE_ALL])
-def test_fused_postfilter_matches_oracle_per_stage(engine, pictures, stages):
+def test_fused_postfilter_matches_oracle_per_stage(engine, pictures, generated_pictures, stages):
     """The fused deblock + SAO tile kernel (k34_postfilter.cu, engine option fused_postfilter; not the default — it is
-    slower than the split kernels, DESIGN.md) produces the same planes as the oracle on every bundled picture."""
+    slower than the split kernels, DESIGN.md) produces the same planes as the oracle on every bundled picture and every
+    generated stream (4:0:0 / 4:2:2 / 4:4:4, 10 and 12 bit, tiles, slices, pcm, bypass)."""
     engine.set_option("fused_postfilter", 1)
     try:
-        for label, rec in pictures:
+        for label, rec in pictures + generated_pictures:
             want, _ = oracle_lib.reconstruct(rec, stages)
             got, _ = gpu_planes(engine, rec, stages)
             for k, (g, w) in enumerate(zip(got, want)):
