@@ -223,4 +223,22 @@ hc_records* hc_parse_picture_k0(const uint8_t* data, size_t size, int stream_for
   }
 }
 
+size_t hc_image_plane_layout(const hc_image_desc* d, size_t offset[4], size_t stride[4], int32_t width[4], int32_t height[4]) {
+  if (!d || d->out_format != HC_OUT_YCBCR || d->width <= 0 || d->height <= 0 || d->chroma_format < 0 || d->chroma_format > 3 ||
+      d->bit_depth < 8 || d->bit_depth > 16)
+    return 0;
+  const size_t ps = d->bit_depth == 8 ? 1 : 2;
+  size_t total = 0;
+  for (int k = 0; k < 4; k++) {
+    const bool present = k == 3 ? d->has_alpha != 0 : hc::plane_w(d->width, d->chroma_format, k) > 0;
+    const int w = present ? hc::plane_w(d->width, d->chroma_format, k) : 0, h = present ? hc::plane_h(d->height, d->chroma_format, k) : 0;
+    if (offset) offset[k] = total;
+    if (stride) stride[k] = (size_t)w * ps;
+    if (width) width[k] = w;
+    if (height) height[k] = h;
+    total += (size_t)w * ps * h;
+  }
+  return total;
+}
+
 }  // extern "C"

@@ -22,4 +22,7 @@ struct hc_heif {
 
 namespace hc {
 void set_last_error(const std::string& s);
+// samples of plane c (0 Y, 1 Cb, 2 Cr, 3 A) of a w x h image: chroma planes round up; 0 for the chroma of monochrome
+inline int plane_w(int w, int chroma, int c) { return (c == 0 || c == 3 || chroma == 3) ? w : (chroma == 0 ? 0 : (w + 1) / 2); }
+inline int plane_h(int h, int chroma, int c) { return (c == 0 || c == 3 || chroma != 1) ? (chroma == 0 && c != 0 && c != 3 ? 0 : h) : (h + 1) / 2; }
 }

@@ -7,7 +7,7 @@
 //   residual buffer: int16, one contiguous nT*nT tile per coded transform block (K1 -> K2)
 //   plane pool     : per picture the reconstruction planes (K2 writes, K3 filters in place, K4 reads),
 //                    per canvas the final Y/Cb/Cr(/A) planes (K4 writes, K5 reads)
-//   rgb buffer     : interleaved output of K5, rows padded to 256 bytes
+//   rgb buffer     : interleaved output of K5, rows padded to 256 bytes, or the packed planes K8 writes (HC_OUT_YCBCR)
 // Device blocks come from a per-engine free list so that the plugin's one-decoder-per-tile call
 // pattern (context.cc:1799-1835) does not pay a cudaMalloc per tile.
 #include <cuda_runtime.h>
@@ -146,6 +146,11 @@ struct Canvas {
   size_t rgb_stride = 0;
   int rgb_bpp = 0;
   bool converted = false;
+  // the last convert was to HC_OUT_YCBCR: K8 packed the output view at rgb_off (poff: plane offsets, packed: total bytes;
+  // rgb_bpp: bytes per sample, rgb_stride: the Y row)
+  bool planar = false;
+  size_t poff[4] = {0, 0, 0, 0};
+  size_t packed = 0;
 };
 
 struct Placement {
@@ -211,8 +216,78 @@ struct hc_batch {
 
 namespace {
 
-int plane_w(int w, int chroma, int c) { return (c == 0 || c == 3 || chroma == 3) ? w : (chroma == 0 ? 0 : (w + 1) / 2); }
-int plane_h(int h, int chroma, int c) { return (c == 0 || c == 3 || chroma != 1) ? (chroma == 0 && c != 0 && c != 3 ? 0 : h) : (h + 1) / 2; }
+using hc::plane_w;
+using hc::plane_h;
+
+// bytes of a canvas' block in the batch's output buffer
+size_t out_block_bytes(const Canvas& c, int bpp) {
+  if (c.planar) return align_up(c.packed, 256);
+  return align_up(align_up((size_t)((c.ow + 7) & ~7) * bpp, 256) * c.oh, 256);
+}
+
+// HC_OUT_YCBCR: lays the canvas' output view out as hc_image_plane_layout does for its desc. False when the planes differ in
+// size from that layout: HeifPixelImage::crop scales a crop window to each plane by integer division, so a window at an odd
+// position can leave a chroma plane one sample larger than (w + 1) / 2.
+bool planar_layout(const Canvas& c, size_t poff[4], size_t* packed) {
+  hc_image_desc d{};
+  d.width = c.ow; d.height = c.oh; d.chroma_format = c.chroma; d.bit_depth = c.bit_depth; d.has_alpha = c.alpha;
+  d.out_format = HC_OUT_YCBCR;
+  int32_t w[4], h[4];
+  *packed = hc_image_plane_layout(&d, poff, nullptr, w, h);
+  for (int k = 0; k < 4; k++)
+    if (w[k] != c.opw[k] || (w[k] && h[k] != c.oph[k])) return false;
+  return *packed > 0;
+}
+
+// the planes of one canvas into a K8 launch (flushing it first when they do not fit)
+void add_pack_planes(hc_batch* b, hc::PackBatch& pb, const Canvas& c, const uint8_t* P, uint8_t* out) {
+  if (pb.n + 4 > hc::PACK_BATCH_MAX) {
+    hc::launch_k8_batch(pb, b->stream);
+    b->launches += 1;
+    pb.n = 0;
+  }
+  const int ps = c.bit_depth == 8 ? 1 : 2;
+  for (int k = 0; k < 4; k++) {
+    if (c.opw[k] == 0) continue;
+    hc::PackPlane& q = pb.p[pb.n++];
+    q.src = P + c.ooff[k];
+    q.dst = out + c.poff[k];
+    q.src_pitch = (unsigned)c.ostride[k] * ps;
+    q.row_bytes = (unsigned)c.opw[k] * ps;
+    q.rows = (unsigned)c.oph[k];
+    q.pad = 0;
+  }
+}
+
+const int kBppOf[6] = {3, 4, 6, 8, 6, 8};   // bytes per pixel of the interleaved HC_OUT_* formats
+
+// Can `p` convert canvas `c`? Changes nothing, so that a call over several canvases leaves them all as they were when one fails.
+int check_convert(const Canvas& c, const hc_csc_params& p) {
+  if (p.out_format < 0 || p.out_format > HC_OUT_YCBCR) { hc::set_last_error("bad output format"); return HC_ERR_ARGUMENT; }
+  if (!c.overlay && p.in_depth != c.bit_depth) { hc::set_last_error("conversion parameters were selected for another bit depth"); return HC_ERR_ARGUMENT; }
+  if (p.out_format != HC_OUT_YCBCR) {
+    if (c.ext_rgb && c.ext_stride < (size_t)((c.ow + 7) & ~7) * kBppOf[p.out_format]) { hc::set_last_error("external RGB target: rows too short for this format"); return HC_ERR_ARGUMENT; }
+    return HC_OK;
+  }
+  if (c.overlay) { hc::set_last_error("overlay canvases are composed in RGB: HC_OUT_YCBCR is not available for them"); return HC_ERR_UNSUPPORTED; }
+  if (c.ext_rgb) { hc::set_last_error("a canvas with an external RGB target cannot be converted to HC_OUT_YCBCR"); return HC_ERR_UNSUPPORTED; }
+  size_t poff[4], packed = 0;
+  if (!planar_layout(c, poff, &packed)) { hc::set_last_error("HC_OUT_YCBCR: the crop window leaves chroma planes of another size than the packed layout"); return HC_ERR_UNSUPPORTED; }
+  return HC_OK;
+}
+
+// the output format of the canvas' next convert (after check_convert): interleaved rows, or the packed planes of K8
+void apply_format(Canvas& c, const hc_csc_params& p) {
+  c.planar = p.out_format == HC_OUT_YCBCR;
+  if (c.planar) {
+    planar_layout(c, c.poff, &c.packed);
+    c.rgb_bpp = c.bit_depth == 8 ? 1 : 2;
+    c.rgb_stride = (size_t)c.ow * c.rgb_bpp;
+  } else {
+    c.rgb_bpp = kBppOf[p.out_format];
+    c.rgb_stride = align_up((size_t)((c.ow + 7) & ~7) * c.rgb_bpp, 256);
+  }
+}
 
 void release_blocks(hc_batch* b) {
   hc_engine* e = b->eng;
@@ -1037,17 +1112,16 @@ int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
   }
   if (!cuda_ok(cudaSetDevice(b->eng->device), "cudaSetDevice")) return HC_ERR_CUDA;
   Canvas& c = b->canvases[canvas];
-  static const int bpp_of[6] = {3, 4, 6, 8, 6, 8};
-  if (params->out_format < 0 || params->out_format > 5) { hc::set_last_error("bad output format"); return HC_ERR_ARGUMENT; }
+  if (params->out_format < 0 || params->out_format > HC_OUT_YCBCR) { hc::set_last_error("bad output format"); return HC_ERR_ARGUMENT; }
   if (params->in_depth != c.bit_depth) { hc::set_last_error("conversion parameters were selected for another bit depth"); return HC_ERR_ARGUMENT; }
-  c.rgb_bpp = bpp_of[params->out_format];
-  c.rgb_stride = align_up((size_t)((c.ow + 7) & ~7) * c.rgb_bpp, 256);
+  if (int rc = check_convert(c, *params)) return rc;
+  apply_format(c, *params);
   // lay all canvases' rgb buffers out in one block (grow if needed)
   size_t total = 0;
   for (auto& cv : b->canvases) {
     const int bp = &cv == &c ? c.rgb_bpp : (cv.rgb_bpp ? cv.rgb_bpp : 8);
     cv.rgb_off = total;
-    total += align_up(align_up((size_t)((cv.ow + 7) & ~7) * bp, 256) * cv.oh, 256);
+    total += out_block_bytes(cv, bp);
   }
   if (b->d_rgb.cap < total) {
     bool any = false;
@@ -1057,8 +1131,21 @@ int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
     b->d_rgb = b->eng->take(b->eng->free_dev, total, false);
     if (!b->d_rgb.p) return HC_ERR_MEMORY;
   }
-  hc::CscArgs a;
   const uint8_t* P = (const uint8_t*)b->d_planes.p;
+  if (c.planar) {   // K8, timed like K5
+    hc::PackBatch pb;
+    pb.n = 0;
+    cudaEvent_t e0 = b->eng->take_event(), e1 = b->eng->take_event();
+    cudaEventRecord(e0, b->stream);
+    add_pack_planes(b, pb, c, P, (uint8_t*)b->d_rgb.p + c.rgb_off);
+    hc::launch_k8_batch(pb, b->stream);
+    cudaEventRecord(e1, b->stream);
+    b->csc_events.push_back({e0, e1});
+    b->launches += 1;
+    c.converted = true;
+    return cuda_ok(cudaGetLastError(), "kernel launch (K8)") ? HC_OK : HC_ERR_CUDA;
+  }
+  hc::CscArgs a;
   a.y = P + c.ooff[0];
   a.cb = c.chroma ? P + c.ooff[1] : nullptr;
   a.cr = c.chroma ? P + c.ooff[2] : nullptr;
@@ -1067,7 +1154,6 @@ int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
   a.width = c.ow; a.height = c.oh; a.chroma_format = c.chroma;
   a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
   a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
-  if (c.ext_rgb && c.ext_stride < (size_t)((c.ow + 7) & ~7) * c.rgb_bpp) { hc::set_last_error("external RGB target: rows too short for this format"); return HC_ERR_ARGUMENT; }
   a.p = *params;
   cudaEvent_t e0 = b->eng->take_event(), e1 = b->eng->take_event();
   cudaEventRecord(e0, b->stream);
@@ -1085,23 +1171,16 @@ int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
 int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_params* params) {
   if (!b || n <= 0 || !canvases || !params || !b->uploaded) { hc::set_last_error("hc_batch_convert_many: bad argument"); return HC_ERR_ARGUMENT; }
   if (!cuda_ok(cudaSetDevice(b->eng->device), "cudaSetDevice")) return HC_ERR_CUDA;
-  static const int bpp_of[6] = {3, 4, 6, 8, 6, 8};
-  for (int i = 0; i < n; i++) {
-    if (canvases[i] < 0 || canvases[i] >= (int)b->canvases.size() || params[i].out_format < 0 || params[i].out_format > 5) {
-      hc::set_last_error("hc_batch_convert_many: bad canvas or output format");
-      return HC_ERR_ARGUMENT;
-    }
-    Canvas& c = b->canvases[canvases[i]];
-    if (!c.overlay && params[i].in_depth != c.bit_depth) { hc::set_last_error("conversion parameters were selected for another bit depth"); return HC_ERR_ARGUMENT; }
-    c.rgb_bpp = bpp_of[params[i].out_format];
-    c.rgb_stride = align_up((size_t)((c.ow + 7) & ~7) * c.rgb_bpp, 256);
-    if (c.ext_rgb && c.ext_stride < (size_t)((c.ow + 7) & ~7) * c.rgb_bpp) { hc::set_last_error("external RGB target: rows too short for this format"); return HC_ERR_ARGUMENT; }
+  for (int i = 0; i < n; i++) {   // every canvas is checked before any of them changes
+    if (canvases[i] < 0 || canvases[i] >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_convert_many: bad canvas"); return HC_ERR_ARGUMENT; }
+    if (int rc = check_convert(b->canvases[canvases[i]], params[i])) return rc;
   }
+  for (int i = 0; i < n; i++) apply_format(b->canvases[canvases[i]], params[i]);
   size_t total = 0;
   for (auto& cv : b->canvases) {
     const int bp = cv.rgb_bpp ? cv.rgb_bpp : 8;
     cv.rgb_off = total;
-    total += align_up(align_up((size_t)((cv.ow + 7) & ~7) * bp, 256) * cv.oh, 256);
+    total += out_block_bytes(cv, bp);
   }
   if (b->d_rgb.cap < total) {
     b->eng->give(b->eng->free_dev, b->d_rgb);
@@ -1141,7 +1220,8 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
     hc::CscBatch cb;
     cb.n = 0;
     for (int i = 0; i <= n; i++) {
-      if (i < n && !b->canvases[canvases[i]].overlay && (b->canvases[canvases[i]].bit_depth != 8) == (sixteen != 0)) {
+      if (i < n && !b->canvases[canvases[i]].overlay && !b->canvases[canvases[i]].planar &&
+          (b->canvases[canvases[i]].bit_depth != 8) == (sixteen != 0)) {
         Canvas& c = b->canvases[canvases[i]];
         hc::CscArgs& a = cb.a[cb.n++];
         a.y = P + c.ooff[0];
@@ -1162,9 +1242,23 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
       }
     }
   }
+  {   // HC_OUT_YCBCR canvases: K8 packs their planes, any sample size in one launch
+    hc::PackBatch pb;
+    pb.n = 0;
+    for (int i = 0; i < n; i++) {
+      Canvas& c = b->canvases[canvases[i]];
+      if (!c.planar) continue;
+      add_pack_planes(b, pb, c, P, (uint8_t*)b->d_rgb.p + c.rgb_off);
+      c.converted = true;
+    }
+    if (pb.n > 0) {
+      hc::launch_k8_batch(pb, b->stream);
+      b->launches += 1;
+    }
+  }
   cudaEventRecord(e1, b->stream);
   b->csc_events.push_back({e0, e1});
-  if (!cuda_ok(cudaGetLastError(), "kernel launch (K5)")) return HC_ERR_CUDA;
+  if (!cuda_ok(cudaGetLastError(), "kernel launch (K5 / K8)")) return HC_ERR_CUDA;
   return HC_OK;
 }
 
@@ -1234,12 +1328,14 @@ int hc_batch_read_rgb(hc_batch* b, int canvas, void* dst, size_t dst_stride) {
   const Canvas& c = b->canvases[canvas];
   if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
   if (c.ext_rgb) { hc::set_last_error("this image is written to an external RGB target (hc_batch_set_rgb_target): read it there"); return HC_ERR_ARGUMENT; }
+  if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are read with the stride of the Y row"); return HC_ERR_ARGUMENT; }
   cudaEvent_t e0 = b->ev_d2h[0], e1 = b->ev_d2h[1];
   cudaEventRecord(e0, b->stream);
-  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
-                                    cudaMemcpyDeviceToHost, b->stream);
+  cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream)
+                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
+                                               cudaMemcpyDeviceToHost, b->stream);
   cudaEventRecord(e1, b->stream);
-  if (!cuda_ok(e, "cudaMemcpy2DAsync(D2H rgb)")) return HC_ERR_CUDA;
+  if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2H planes)" : "cudaMemcpy2DAsync(D2H rgb)")) return HC_ERR_CUDA;
   if (int rc = batch_sync_checked(b, "cudaStreamSynchronize")) return rc;
   cudaEventElapsedTime(&b->last_d2h_ms, e0, e1);
   return HC_OK;
@@ -1250,10 +1346,12 @@ int hc_batch_copy_rgb_device(hc_batch* b, int canvas, void* dst, size_t dst_stri
   const Canvas& c = b->canvases[canvas];
   if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
   if (c.ext_rgb) { hc::set_last_error("this image is written to an external RGB target (hc_batch_set_rgb_target)"); return HC_ERR_ARGUMENT; }
+  if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are copied with the stride of the Y row"); return HC_ERR_ARGUMENT; }
   // cudaMemcpyDefault: `dst` may live on a peer device (unified addressing; a peer copy over NVLink then)
-  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
-                                    cudaMemcpyDefault, b->stream);
-  if (!cuda_ok(e, "cudaMemcpy2DAsync(D2D rgb)")) return HC_ERR_CUDA;
+  cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDefault, b->stream)
+                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
+                                               cudaMemcpyDefault, b->stream);
+  if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2D planes)" : "cudaMemcpy2DAsync(D2D rgb)")) return HC_ERR_CUDA;
   return batch_sync_checked(b, "cudaStreamSynchronize");
 }
 
@@ -1285,6 +1383,11 @@ int hc_batch_read_rgb_async(hc_batch* b, int canvas, void* dst, size_t dst_strid
   if (!b || !dst || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_read_rgb_async: bad argument"); return HC_ERR_ARGUMENT; }
   const Canvas& c = b->canvases[canvas];
   if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
+  if (c.planar) {
+    if (dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are read with the stride of the Y row"); return HC_ERR_ARGUMENT; }
+    return cuda_ok(cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream), "cudaMemcpyAsync(D2H planes)")
+               ? HC_OK : HC_ERR_CUDA;
+  }
   cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
                                     cudaMemcpyDeviceToHost, b->stream);
   return cuda_ok(e, "cudaMemcpy2DAsync(D2H rgb)") ? HC_OK : HC_ERR_CUDA;
@@ -1324,6 +1427,7 @@ int hc_batch_set_rgb_target(hc_batch* b, int canvas, void* device_dst, size_t st
     return HC_ERR_ARGUMENT;
   }
   Canvas& c = b->canvases[canvas];
+  if (c.planar) { hc::set_last_error("hc_batch_set_rgb_target: the canvas is converted to HC_OUT_YCBCR"); return HC_ERR_UNSUPPORTED; }
   c.ext_rgb = (uint8_t*)device_dst;
   c.ext_stride = device_dst ? stride_bytes : 0;
   c.converted = false;

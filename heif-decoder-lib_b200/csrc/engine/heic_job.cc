@@ -123,6 +123,12 @@ struct ImagePlan {
   std::vector<std::pair<int32_t, int32_t>> child_offsets;
 };
 
+// bytes one delivered image takes: the packed planes of HC_OUT_YCBCR, else tight interleaved rows
+size_t image_bytes(const hc_image_desc& d) {
+  if (d.out_format == HC_OUT_YCBCR) return hc_image_plane_layout(&d, nullptr, nullptr, nullptr, nullptr);
+  return (size_t)d.width * d.bytes_per_pixel * d.height;
+}
+
 int add_item(hc_batch* b, std::vector<int>& pic_file, const CodedItem& ci, int canvas, int x, int y, int role, int rescale) {
   const int pic = ci.k0 ? hc_batch_add_k0_picture(b, ci.k0.get(), canvas, x, y, role, rescale) : hc_batch_add_picture(b, &ci.rec, canvas, x, y, role, rescale);
   if (pic >= 0) {
@@ -169,9 +175,11 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
   std::unique_ptr<hc_heic_job> j(new hc_heic_job);
   j->eng = e;
   // `want_alpha` doubles as the output selector: 0 / 1 = automatic (RGB(A) for 8-bit images, RRGGBB(AA)_LE for deeper ones),
-  // HC_OUTPUT_FORMAT(fmt) = that interleaved format for every image, whatever its bit depth
+  // HC_OUTPUT_FORMAT(fmt) = that interleaved format for every image, whatever its bit depth, or the native planes (HC_OUT_YCBCR)
   j->forced_format = (want_alpha & 0x100) ? (want_alpha & 0xff) : -1;
-  if (j->forced_format > HC_OUT_RRGGBBAA_LE) { hc::set_last_error("hc_heic_job_create: unknown output format"); return nullptr; }
+  if (j->forced_format > HC_OUT_YCBCR) { hc::set_last_error("hc_heic_job_create: unknown output format"); return nullptr; }
+  const bool planar = j->forced_format == HC_OUT_YCBCR;
+  if (planar && band_end >= 0) { hc::set_last_error("banded decode: HC_OUT_YCBCR is not supported, bands are written as interleaved rows"); return nullptr; }
   j->want_alpha = j->forced_format >= 0 ? (j->forced_format == HC_OUT_RGBA || j->forced_format == HC_OUT_RRGGBBAA_BE || j->forced_format == HC_OUT_RRGGBBAA_LE)
                                         : want_alpha != 0;
   const auto t0 = std::chrono::steady_clock::now();
@@ -261,6 +269,7 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     if (hf.is_overlay(id)) {
       // 'iovl' (context.cc:2579-2675): every referenced image is decoded like a top-level image, then composed
       if (band_end >= 0) { hc::set_last_error("a tile row band needs a grid image"); return nullptr; }
+      if (planar) { hc::set_last_error("file " + std::to_string(f) + ": overlay images are composed in RGB: HC_OUT_YCBCR is not supported for them"); return nullptr; }
       hc::HeifOverlay ov;
       err = hf.overlay(id, ov);
       if (!err.empty()) { hc::set_last_error("file " + std::to_string(f) + ": " + err); return nullptr; }
@@ -447,8 +456,11 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     }
     // ---- irot / imir / clap of an image item, in ipma order (context.cc:1955-2016). Consecutive rotations and mirrors
     // are composed into one dihedral pass; a clap becomes a crop pass on the image as it is at that point. Returns
-    // false on error; `any` reports whether the item carries transformations at all. ----
-    auto apply_xforms = [&](int canvas, const hc::HeifItem* pit, int& Wc, int& Hc, int chroma_format, int bit_depth, bool& any) -> bool {
+    // false on error; `any` reports whether the item carries transformations at all. Cw x Ch follows the size of the chroma
+    // planes through the passes (HeifPixelImage::crop scales the window to each plane, pixelimage.cc:820-823, as the
+    // engine's crop pass does). ----
+    auto apply_xforms = [&](int canvas, const hc::HeifItem* pit, int& Wc, int& Hc, int& Cw, int& Ch, int chroma_format, int bit_depth,
+                            bool& any) -> bool {
       int swap = 0, fx = 0, fy = 0;
       any = false;
       size_t next_clap = 0;
@@ -469,6 +481,10 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
           const std::string e = clap_window(pit->claps[next_clap++], Wc, Hc, win);
           if (!e.empty()) { hc::set_last_error(e); return false; }
           if (hc_batch_add_canvas_pass(j->batch, canvas, HC_PASS_CROP, win[0], win[1], win[2], win[3]) != HC_OK) return false;
+          if (Cw > 0) {
+            Cw = (int)((int64_t)win[2] * Cw / Wc - (int64_t)win[0] * Cw / Wc) + 1;
+            Ch = (int)((int64_t)win[3] * Ch / Hc - (int64_t)win[1] * Ch / Hc) + 1;
+          }
           Wc = win[2] - win[0] + 1; Hc = win[3] - win[1] + 1;
           continue;
         }
@@ -482,7 +498,7 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
         // out2(x, y) = out1(x1, y1): see hc_batch_set_canvas_transform for the map of one operation
         const int nfx = swap ? (fx ^ fy2) : (fx ^ fx2), nfy = swap ? (fy ^ fx2) : (fy ^ fy2);
         swap ^= s2; fx = nfx; fy = nfy;
-        if (s2) std::swap(Wc, Hc);
+        if (s2) { std::swap(Wc, Hc); std::swap(Cw, Ch); }
       }
       return flush_dihedral();
     };
@@ -508,8 +524,17 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     }
     {
       bool any = false;
-      if (!apply_xforms(im.canvas, pit, W, H, p0.chroma_format, p0.bit_depth_y, any)) return false;
+      int Cw = hc::plane_w(W, p0.chroma_format, 1), Ch = hc::plane_h(H, p0.chroma_format, 1);
+      if (!apply_xforms(im.canvas, pit, W, H, Cw, Ch, p0.chroma_format, p0.bit_depth_y, any)) return false;
       if (any && band_end >= 0) { hc::set_last_error("banded decode of transformed images is not supported"); return false; }
+      // the packed layout (hc_image_plane_layout) has (w + 1) / 2 chroma samples per row of 4:2:0 / 4:2:2 and (h + 1) / 2 rows
+      // of 4:2:0; a clean aperture at an odd position leaves one more, and the desc cannot describe that
+      if (fmt_override < 0 && planar && (Cw != hc::plane_w(W, p0.chroma_format, 1) || Ch != hc::plane_h(H, p0.chroma_format, 1))) {
+        hc::set_last_error("file " + std::to_string(im.file) + ": HC_OUT_YCBCR: the clean aperture leaves chroma planes of " + std::to_string(Cw) +
+                           " x " + std::to_string(Ch) + " samples, not the packed layout's " + std::to_string(hc::plane_w(W, p0.chroma_format, 1)) + " x " +
+                           std::to_string(hc::plane_h(H, p0.chroma_format, 1)));
+        return false;
+      }
     }
     if (alpha_separate) {
       const hc_pic& pa = j->items[im.alpha].pic();
@@ -520,7 +545,8 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
         if (!place_tiles(im.alpha_tiles, im.alpha_cols, ac, Wa, Ha, HC_ROLE_LUMA)) return false;
       } else if (add_item(j->batch, j->pic_file, j->items[im.alpha], ac, 0, 0, HC_ROLE_LUMA, 0) < 0) return false;
       bool any = false;
-      if (!apply_xforms(ac, ait, Wa, Ha, 0, pa.bit_depth_y, any)) return false;
+      int Cwa = 0, Cha = 0;   // monochrome: no chroma planes
+      if (!apply_xforms(ac, ait, Wa, Ha, Cwa, Cha, 0, pa.bit_depth_y, any)) return false;
       if (hc_batch_link_alpha(j->batch, im.canvas, ac) != HC_OK) return false;
     }
     const bool hdr = p0.bit_depth_y != 8;
@@ -528,7 +554,8 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     if (hc_csc_select_opt(matrix, primaries, full, p0.chroma_format, p0.bit_depth_y, has_alpha, fmt, hc_engine_get_option(e, "chroma_upsampling"), &im.csc) != HC_OK) return false;
     static const int bpp_of[6] = {3, 4, 6, 8, 6, 8};
     im.desc.width = W; im.desc.height = H; im.desc.chroma_format = p0.chroma_format; im.desc.bit_depth = p0.bit_depth_y;
-    im.desc.has_alpha = has_alpha; im.desc.out_format = fmt; im.desc.bytes_per_pixel = bpp_of[fmt];
+    im.desc.has_alpha = has_alpha; im.desc.out_format = fmt;
+    im.desc.bytes_per_pixel = fmt == HC_OUT_YCBCR ? (p0.bit_depth_y == 8 ? 1 : 2) : bpp_of[fmt];
     im.desc.coded_pictures = (int)im.tiles.size() + (has_alpha ? (alpha_grid ? (int)im.alpha_tiles.size() : 1) : 0);
     // premultiplied alpha: a flag the file sets ('prem' reference, context.cc:1150-1161, :2074-2075) — or the result of
     // heif_image_rgba_premultiply_alpha (heif.cc:1444-1490), which only takes interleaved RGBA that is not premultiplied yet
@@ -612,6 +639,7 @@ extern "C" int hc_shared_image_geometry(const hc_shared_image* s, int* width, in
 int hc_heic_job_set_rgb_target(hc_heic_job* j, int image, hc_shared_image* dst, int first_row) {
   if (!j || image < 0 || image >= (int)j->images.size() || !dst || first_row < 0) { hc::set_last_error("hc_heic_job_set_rgb_target: bad argument"); return HC_ERR_ARGUMENT; }
   const ImagePlan& im = j->images[image];
+  if (im.desc.out_format == HC_OUT_YCBCR) { hc::set_last_error("hc_heic_job_set_rgb_target: HC_OUT_YCBCR images are not written to shared images"); return HC_ERR_UNSUPPORTED; }
   int w = 0, h = 0, bpp = 0;
   hc_shared_image_geometry(dst, &w, &h, &bpp);
   if (w != im.desc.width || bpp != im.desc.bytes_per_pixel || first_row + im.desc.height > h) {
@@ -819,13 +847,16 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
       // external destination (the reference's heif_decoding_options::ext_dst, heif.h:1605-1615, pixelimage.cc:221-266): the
       // final pixels land in the caller's buffer with the caller's stride when it is large enough, else in our own memory
       const hc_stream_dest* xd = dests ? &dests[(size_t)b * files_per_batch + f.map[i]] : nullptr;
-      if (xd && xd->dst && xd->stride >= row && xd->len >= xd->stride * (size_t)(d.height - 1) + row) {
+      const bool fits = d.out_format == HC_OUT_YCBCR
+                            ? xd && xd->dst && (xd->stride == 0 || xd->stride == row) && xd->len >= image_bytes(d)   // packed planes
+                            : xd && xd->dst && xd->stride >= row && xd->len >= xd->stride * (size_t)(d.height - 1) + row;
+      if (fits) {
         f.ptrs[i] = (uint8_t*)xd->dst;
-        f.strides[i] = xd->stride;
+        f.strides[i] = d.out_format == HC_OUT_YCBCR ? row : xd->stride;
         continue;
       }
       f.strides[i] = row;
-      need += (row * d.height + 255) & ~(size_t)255;
+      need += (image_bytes(d) + 255) & ~(size_t)255;
     }
     if (need > pinned_cap[f.slot]) {
       if (pinned[f.slot]) hc_engine_give_out_pinned(e, pinned[f.slot], pinned_cap[f.slot]);
@@ -911,7 +942,7 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
       for (size_t i = 0; i < j->images.size(); i++) {
         if (bad[i]) continue;
         const hc_image_desc& d = j->images[i].desc;
-        st.bytes_d2h += (uint64_t)d.width * d.bytes_per_pixel * d.height;
+        st.bytes_d2h += image_bytes(d);
         st.pixels += (int64_t)d.width * d.height;
         if (on_image) on_image(user, f.index * files_per_batch + f.map[i], &d, f.ptrs[i], f.strides[i]);
       }

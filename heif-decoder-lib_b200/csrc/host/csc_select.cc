@@ -58,10 +58,23 @@ extern "C" int hc_csc_select(int matrix, int primaries, int full_range, int chro
 
 extern "C" int hc_csc_select_opt(int matrix, int primaries, int full_range, int chroma_format, int bit_depth,
                                  int has_alpha, int out_format, int upsampling, hc_csc_params* out) {
-  if (!out || (upsampling != HC_UPSAMPLE_NEAREST && upsampling != HC_UPSAMPLE_BILINEAR) || out_format < HC_OUT_RGB || out_format > HC_OUT_RRGGBBAA_LE || bit_depth < 8 || bit_depth > 16 || chroma_format < 0 ||
+  if (!out || (upsampling != HC_UPSAMPLE_NEAREST && upsampling != HC_UPSAMPLE_BILINEAR) || out_format < HC_OUT_RGB || out_format > HC_OUT_YCBCR || bit_depth < 8 || bit_depth > 16 || chroma_format < 0 ||
       chroma_format > 3) {
     hc::set_last_error("hc_csc_select: bad argument");
     return HC_ERR_ARGUMENT;
+  }
+  if (out_format == HC_OUT_YCBCR) {
+    // the planes as decoded (heif_colorspace_undefined / heif_chroma_undefined): no op at all, so any matrix goes
+    hc_csc_params p{};
+    p.mode = HC_CSC_FLOAT;
+    p.out_format = HC_OUT_YCBCR;
+    p.full_range = full_range ? 1 : 0;
+    p.bit_depth = p.in_depth = p.out_depth = bit_depth;
+    p.pre_op = p.post_op = HC_DEPTH_NONE;
+    p.upsampling = HC_UPSAMPLE_NEAREST;
+    p.coeff_matrix = matrix;
+    *out = p;
+    return HC_OK;
   }
   // matrix 2 (unspecified) reaches the conversion ops unchanged: Kr = Kb = 0 selects the literal
   // BT.601 defaults (nclx.cc:140-149,159-169), which differ in the last ulp from the values

@@ -52,6 +52,24 @@ struct OverlayArgs {
 };
 void launch_k7(const OverlayArgs& a, cudaStream_t stream);
 
+// K8: planes copied from the plane pool (pitched rows) into packed HC_OUT_YCBCR images (tight rows, one plane after the
+// other). Plane by plane, whatever the sample size: a plane is row_bytes x rows bytes.
+struct PackPlane {
+  const uint8_t* src;        // first row of the plane in the pool
+  uint8_t* dst;              // packed destination, any alignment
+  unsigned src_pitch;        // bytes between source rows
+  unsigned row_bytes;        // plane width x sample bytes
+  unsigned rows;
+  unsigned pad;
+};
+// planes of up to 24 canvases per launch (kernel parameter space: 4 KB)
+constexpr int PACK_BATCH_MAX = 96;
+struct PackBatch {
+  PackPlane p[PACK_BATCH_MAX];
+  int n;
+};
+void launch_k8_batch(const PackBatch& b, cudaStream_t stream);
+
 namespace k0 { struct Tables; struct Pic; struct Sub; struct Chain; }
 // K0: device CABAC parse of the pictures added as bitstreams (one CTA per substream chain)
 void launch_k0(const k0::Tables* tables, const k0::Pic* pics, const k0::Sub* subs, const k0::Chain* chains, int nchains,

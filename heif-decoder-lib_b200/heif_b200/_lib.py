@@ -160,6 +160,7 @@ SYMBOLS = [
     ("hc_heic_job_destroy", None, [_vp]),
     ("hc_heic_job_image_count", _i, [_vp]),
     ("hc_heic_job_image_desc", _i, [_vp, _i, C.POINTER(ImageDesc)]),
+    ("hc_image_plane_layout", _sz, [C.POINTER(ImageDesc), C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("hc_heic_job_upload", _i, [_vp]),
     ("hc_heic_job_run", _i, [_vp]),
     ("hc_heic_job_sync", _i, [_vp]),

@@ -10,6 +10,7 @@ from ._lib import CscParams, HeifCudaError, HeifImageInfo, check
 STREAM_LENGTH_PREFIXED, STREAM_ANNEXB, STREAM_SINGLE_NAL = 0, 1, 2
 OUT_RGB, OUT_RGBA, OUT_RRGGBB_BE, OUT_RRGGBBAA_BE, OUT_RRGGBB_LE, OUT_RRGGBBAA_LE = range(6)
 OUT_BYTES_PER_PIXEL = {OUT_RGB: 3, OUT_RGBA: 4, OUT_RRGGBB_BE: 6, OUT_RRGGBBAA_BE: 8, OUT_RRGGBB_LE: 6, OUT_RRGGBBAA_LE: 8}
+OUT_YCBCR = 6    # native planes (heif_colorspace_undefined / heif_chroma_undefined), packed Y, Cb, Cr, A: see plane_layout
 STAGE_DEBLOCK, STAGE_SAO, STAGE_ALL = 1, 2, 3
 ROLE_COLOUR, ROLE_ALPHA = 0, 1
 
@@ -157,6 +158,23 @@ def csc_select(matrix, primaries, full_range, chroma_format, bit_depth, has_alph
     check(L, L.hc_csc_select_opt(matrix, primaries, int(full_range), chroma_format, bit_depth, int(has_alpha), out_format, int(upsampling),
                                  C.byref(p)), "hc_csc_select")
     return p
+
+
+def plane_layout(desc, host_only=False):
+    """hc_image_plane_layout: (total bytes, [(offset, stride, width, height) of Y, Cb, Cr, A]) of an OUT_YCBCR image; planes the
+    image lacks have width 0. total is 0 for a desc of another output format."""
+    L = _lib.load(host_only)
+    off, stride = (C.c_size_t * 4)(), (C.c_size_t * 4)()
+    w, h = (C.c_int32 * 4)(), (C.c_int32 * 4)()
+    total = L.hc_image_plane_layout(C.byref(desc), off, stride, w, h)
+    return total, [(off[k], stride[k], w[k], h[k]) for k in range(4)]
+
+
+def split_planes(desc, packed):
+    """The planes of one packed OUT_YCBCR image (1-D uint8 array) as 2-D views: uint8, or little-endian uint16 above 8 bit."""
+    total, planes = plane_layout(desc)
+    dt = np.uint8 if desc.bit_depth == 8 else np.dtype("<u2")
+    return [packed[o:o + s * h].view(dt).reshape(h, w) for o, s, w, h in planes if w]
 
 
 class Engine:
@@ -378,10 +396,22 @@ class HeicJob:
 
     def read_rgb(self, image, out=None):
         d = self.descs[image]
+        if d.out_format == OUT_YCBCR:
+            raise HeifCudaError("image %d is planar (OUT_YCBCR): read it with read_planes" % image)
         if out is None:
             out = np.empty((d.height, d.width * d.bytes_per_pixel), np.uint8)
         check(self._L, self._L.hc_heic_job_read_rgb(self._h, image, out.ctypes.data, out.strides[0]), "read_rgb")
         return out
+
+    def read_planes(self, image):
+        """OUT_YCBCR jobs: the planes of an image (Y, Cb, Cr, A as the image has them) from ONE read of its packed bytes"""
+        d = self.descs[image]
+        total, _ = plane_layout(d)
+        if not total:
+            raise HeifCudaError("image %d is not planar: create the job with out_format=OUT_YCBCR" % image)
+        buf = np.empty(total, np.uint8)
+        check(self._L, self._L.hc_heic_job_read_rgb(self._h, image, buf.ctypes.data, d.width * d.bytes_per_pixel), "read_planes")
+        return split_planes(d, buf)
 
     def read_plane(self, image, plane):
         d = self.descs[image]
@@ -433,7 +463,9 @@ def decode_stream(engine, files, on_image=None, want_alpha=False, threads=0, fil
                   isolate_errors=False):
     """Long file lists (hc_heic_decode_stream): host parse of batch b+1 overlaps upload + kernels + read-back of
     batch b. on_image(file_index, desc, rows) gets every image as a numpy view [h, w*bytes_per_pixel] of PINNED
-    host memory that is only valid inside the callback. Returns the hc_stream_stats as a dict.
+    host memory that is only valid inside the callback; with out_format=OUT_YCBCR `rows` is instead the list of the image's
+    planes (split_planes), views of the same kind. Returns the hc_stream_stats as a dict.
+    dests: per file a writable uint8 array or None; [rows, stride] for interleaved output, 1-D (the packed bytes) for OUT_YCBCR.
     isolate_errors: a file that cannot be decoded does not fail the call; the dict gains "file_status" (one HC_* code per
     file, 0 = delivered) and "first_error" (text)."""
     from ._lib import IMAGE_CALLBACK, StreamStats
@@ -453,18 +485,22 @@ def decode_stream(engine, files, on_image=None, want_alpha=False, threads=0, fil
     def _cb(_user, index, desc, pixels, stride):
         if on_image is not None:
             d = desc.contents
+            if d.out_format == OUT_YCBCR:
+                total, _ = plane_layout(d)
+                on_image(index, d, split_planes(d, np.ctypeslib.as_array((C.c_uint8 * total).from_address(pixels))))
+                return
             rows = np.ctypeslib.as_array((C.c_uint8 * (stride * d.height)).from_address(pixels)).reshape(d.height, stride)
             on_image(index, d, rows)
 
     cb = IMAGE_CALLBACK(_cb)
     st = StreamStats()
     xd = None
-    if dests is not None:    # external destinations: one writable uint8 numpy array [rows, stride] (or None) per file
+    if dests is not None:    # external destinations: one writable uint8 numpy array (or None) per file
         from ._lib import StreamDest
         xd = (StreamDest * n)()
         for k, a in enumerate(dests):
             if a is not None:
-                xd[k].dst, xd[k].len, xd[k].stride = a.ctypes.data, a.nbytes, a.strides[0]
+                xd[k].dst, xd[k].len, xd[k].stride = a.ctypes.data, a.nbytes, a.strides[0] if a.ndim > 1 else 0
     status = (C.c_int * n)() if isolate_errors else None
     check(L, L.hc_heic_decode_stream_ext(engine._h, n, ptrs, sizes, int(want_alpha), threads, files_per_batch, xd, status, cb, None,
                                          C.byref(st)), "hc_heic_decode_stream")

@@ -160,6 +160,13 @@ void hc_free(void* p);
 #define HC_OUT_RRGGBBAA_BE 3
 #define HC_OUT_RRGGBB_LE 4
 #define HC_OUT_RRGGBBAA_LE 5
+/* Native planar output, what heif_decode_image(..., heif_colorspace_undefined, heif_chroma_undefined, ...) returns: the
+ * decoded planes as they are (after grid paste, limited->full rescale, irot / imir / clap and the alpha rescale), no colour
+ * conversion, no depth change, no chroma resampling. Packed layout of one image: planes Y, Cb, Cr, A in that order, the planes
+ * the image lacks left out (monochrome: Y only; A whenever the image has alpha), each plane tight (stride = plane width x
+ * sample bytes) and right after the previous one; samples are 1 byte for 8-bit images and 2 bytes little-endian otherwise;
+ * chroma planes are (w + 1) / 2 wide for 4:2:0 / 4:2:2 and (h + 1) / 2 high for 4:2:0. See hc_image_plane_layout. */
+#define HC_OUT_YCBCR 6
 
 #define HC_CSC_INT420 0 /* Op_YCbCr420_to_RGB24 / _RGB32: 8-bit fixed point      yuv2rgb.cc:260-495 */
 #define HC_CSC_FLOAT 1  /* Op_YCbCr_to_RGB<> / Op_YCbCr420_to_RRGGBBaa: fp32     yuv2rgb.cc:28-254,498-643 */
@@ -190,6 +197,8 @@ typedef struct hc_csc_params {
                             becomes 6 behind any other op (see csc_select.cc)                     */
 } hc_csc_params;
 
+/* HC_OUT_YCBCR is accepted for every chroma format, bit depth and matrix (11 / 14 included: nothing is converted) and gives
+ * parameters that describe an identity: in_depth = out_depth = bit_depth = the image's bit depth, no pre / post op. */
 /* Chooses the conversion the reference's pipeline would run with default decoding options
  * (colorconversion.cc:266-420, table in SURVEY.md 3.5) and fills the coefficients exactly as
  * nclx.cc:82-171 computes them. `matrix`/`primaries`/`full_range` are the image's nclx values
@@ -294,9 +303,12 @@ int hc_batch_link_alpha(hc_batch* b, int canvas, int alpha_canvas);
  * (Op_YCbCr_to_RGB<uint8_t>). Children must be 8-bit 4:4:4 canvases (the reference converts nothing else) with offsets >= 0. */
 int hc_batch_add_overlay_canvas(hc_batch* b, int width, int height, const uint16_t background[4]);
 int hc_batch_overlay_add_child(hc_batch* b, int overlay_canvas, int child_canvas, int dx, int dy, const hc_csc_params* child_params);
-/* K5 for one canvas into the engine's device RGB buffer, async */
+/* K5 for one canvas into the engine's device RGB buffer, async. A canvas whose params have out_format == HC_OUT_YCBCR goes to
+ * K8 instead, which packs the canvas' output planes into the same buffer in the layout of HC_OUT_YCBCR. Overlay canvases
+ * (hc_batch_add_overlay_canvas) and canvases with an external RGB target (hc_batch_set_rgb_target) cannot be planar:
+ * HC_ERR_UNSUPPORTED. */
 int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params);
-/* K5 for n canvases (canvases[i] with params[i]) in as few launches as possible, async */
+/* K5 / K8 for n canvases (canvases[i] with params[i]) in as few launches as possible, async */
 int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_params* params);
 int hc_batch_sync(hc_batch* b);
 /* D2H reads (synchronous). plane: 0 Y, 1 Cb, 2 Cr, 3 alpha. Samples are 1 byte for 8-bit canvases,
@@ -304,6 +316,8 @@ int hc_batch_sync(hc_batch* b);
 int hc_batch_read_plane(hc_batch* b, int canvas, int plane, void* dst, size_t dst_stride_bytes);
 /* planes 0..nplanes-1 of a canvas with one synchronisation (pinned staging inside) */
 int hc_batch_read_planes(hc_batch* b, int canvas, int nplanes, void* const* dst, const size_t* dst_strides);
+/* The converted image of a canvas. For a canvas converted to HC_OUT_YCBCR these copy its packed planes with one 1-D copy
+ * (hc_image_plane_layout bytes); dst_stride_bytes must then be the tight Y row (width x sample bytes), else HC_ERR_ARGUMENT. */
 int hc_batch_read_rgb(hc_batch* b, int canvas, void* dst, size_t dst_stride_bytes);
 int hc_batch_copy_rgb_device(hc_batch* b, int canvas, void* device_dst, size_t dst_stride_bytes);
 /* same copy without the final synchronisation (dst should be pinned); pair with hc_batch_sync */
@@ -311,7 +325,7 @@ int hc_batch_read_rgb_async(hc_batch* b, int canvas, void* dst, size_t dst_strid
 /* residuals of picture `pic` as produced by K1 (resid_count int16) — used by the parity tests */
 int hc_batch_read_residual(hc_batch* b, int pic, int16_t* dst, size_t count);
 /* device time of the last run's stages in ms (CUDA events on the engine stream):
- * [0] H2D upload, [1] K1, [2] K2, [3] K3, [4] K4, [5] K5 (sum over canvases), [6] D2H of the last read,
+ * [0] H2D upload, [1] K1, [2] K2, [3] K3, [4] K4, [5] K5 / K8 (sum over convert calls), [6] D2H of the last read,
  * [7] K0 (device CABAC parse; runs once per upload, the records then stay resident) */
 int hc_batch_stage_ms(hc_batch* b, float ms[8]);
 /* CUDA-event stopwatch on the batch's stream: start records an event; stop records a second one,
@@ -339,11 +353,17 @@ typedef struct hc_image_desc {
   int32_t bit_depth;
   int32_t has_alpha;
   int32_t out_format;        /* HC_OUT_* of this image (automatic: 8-bit -> RGB/RGBA, else RRGGBB(AA)_LE) */
-  int32_t bytes_per_pixel;
+  int32_t bytes_per_pixel;   /* HC_OUT_YCBCR: bytes per sample (1 or 2), so width * bytes_per_pixel is the Y row       */
   int32_t coded_pictures;    /* HEVC pictures decoded for this image (tiles + alpha)              */
   int32_t premultiplied_alpha; /* heif_image_is_premultiplied_alpha of the result: the file says so ('prem'), or the engine option
-                                "premultiply_alpha" multiplied the RGBA output (heif_image_rgba_premultiply_alpha) */
+                                "premultiply_alpha" multiplied the RGBA output (heif_image_rgba_premultiply_alpha; never for
+                                HC_OUT_YCBCR, which that call does not take) */
 } hc_image_desc;
+
+/* Packed layout of an HC_OUT_YCBCR image (see HC_OUT_YCBCR): byte offset, stride in bytes, width and height in samples of
+ * planes 0 Y, 1 Cb, 2 Cr, 3 A; a plane the image lacks gets width, height and stride 0. Any of the arrays may be NULL.
+ * Returns the total packed bytes, or 0 for a desc of another output format. */
+size_t hc_image_plane_layout(const hc_image_desc* d, size_t offset[4], size_t stride[4], int32_t width[4], int32_t height[4]);
 
 /* Parses `nfiles` HEIC files held in host memory (the primary image of each) with `threads` host
  * threads (<=0: hardware concurrency). The buffers must stay valid until hc_heic_job_destroy.
@@ -351,7 +371,15 @@ typedef struct hc_image_desc {
  * HC_OUTPUT_FORMAT(HC_OUT_*) -> that format for every image whatever its bit depth, like the `chroma` argument of
  * heif_decode_image (heif.cc:1150): a 10-bit image to interleaved RGB goes through the reference's Op_to_sdr_planes, an
  * 8-bit image to RRGGBB through Op_to_hdr_planes (10 bit), both fused into K5. The same encoding is accepted by
- * hc_heic_job_create_band and hc_heic_decode_stream. */
+ * hc_heic_job_create_band and hc_heic_decode_stream.
+ * HC_OUTPUT_FORMAT(HC_OUT_YCBCR): every image as its native planes (heif_colorspace_undefined / heif_chroma_undefined),
+ * packed by K8; hc_heic_job_read_rgb then copies the packed planes (stride = the Y row). A is delivered whenever the image has
+ * alpha. The "premultiply_alpha" and "chroma_upsampling" options do not apply. Overlay ('iovl') images, which the reference
+ * composes in RGB, fail as unsupported images, and so does an image whose clean aperture (clap) leaves chroma planes of
+ * another size than the packed layout: the reference scales the crop window to each plane by integer division, so a 4:2:0 /
+ * 4:2:2 window at an odd column with an even width (4:2:0: or at an odd row with an even height) keeps one chroma sample
+ * more than (w + 1) / 2 (h + 1) / 2. With error isolation (hc_heic_decode_stream_ext) each such file fails alone.
+ * hc_heic_job_create_band and hc_heic_job_set_rgb_target refuse the format. */
 #define HC_OUTPUT_FORMAT(fmt) (0x100 | (fmt))
 hc_heic_job* hc_heic_job_create(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
                                 int want_alpha, int threads);
@@ -385,9 +413,10 @@ size_t hc_shared_image_stride(const hc_shared_image* s);
  * hc_heic_job_sync and whatever barrier orders the writers before the reader) */
 int hc_shared_image_read(hc_shared_image* s, int first_row, int rows, void* dst, size_t dst_stride_bytes);
 /* K5 of image `image` writes its rows to rows [first_row, ...) of `dst` instead of the job's own RGB buffer. Call before
- * hc_heic_job_run; hc_heic_job_read_rgb is not available for such an image. */
+ * hc_heic_job_run; hc_heic_job_read_rgb is not available for such an image. HC_ERR_UNSUPPORTED for HC_OUT_YCBCR images. */
 int hc_heic_job_set_rgb_target(hc_heic_job* j, int image, hc_shared_image* dst, int first_row);
-/* same at batch level: any device pointer K5 may store to (peer-mapped or local), rows `stride_bytes` apart */
+/* same at batch level: any device pointer K5 may store to (peer-mapped or local), rows `stride_bytes` apart;
+ * HC_ERR_UNSUPPORTED for a canvas converted to HC_OUT_YCBCR */
 int hc_batch_set_rgb_target(hc_batch* b, int canvas, void* device_dst, size_t stride_bytes);
 /* device-to-device copy of a converted image into caller-owned device memory (any device reachable from the job's: the copy
  * is a peer copy over NVLink then), synchronous */
@@ -440,6 +469,9 @@ int hc_heic_decode_stream(hc_engine* e, int nfiles, const uint8_t* const* data, 
  * the reference, a destination that is absent or too small (len < stride * (height - 1) + row bytes, or stride < row
  * bytes) is ignored and the image is delivered in the library's own pinned memory; the callback receives whichever pointer
  * and stride were used. dests may be NULL.
+ * HC_OUT_YCBCR: the callback gets the base of the packed planes and stride_bytes = the Y row. A destination is used when
+ * len >= hc_image_plane_layout(...) and stride is 0 or the Y row, and ignored otherwise. stats->bytes_d2h counts the packed
+ * bytes.
  * Error isolation: with file_status == NULL the first file that cannot be decoded fails the whole call (hc_heic_decode_stream).
  * With file_status != NULL (nfiles entries) such a file gets its error code there and no callback, every other file is
  * delivered, and the call returns HC_OK unless something other than the content of a file went wrong (CUDA, memory);
