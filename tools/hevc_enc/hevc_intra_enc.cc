@@ -12,7 +12,8 @@
 // pictures look like the source and every syntax path the decoder supports can be switched on:
 // chroma 4:0:0/4:2:0/4:2:2/4:4:4, 8-12 bit, CTB 16-64, TU 4-32 with RQT, NxN, SAO, deblocking
 // offsets, cu_qp_delta, sign data hiding, transform skip, WPP, tiles, (dependent) slices, PCM,
-// transquant bypass, scaling lists, strong intra smoothing, VUI.
+// transquant bypass, scaling lists, strong intra smoothing, VUI. A stress mode (hevc_enc_params::stress) pushes levels,
+// intra modes, QPs and SAO parameters to the limits of their legal ranges for the parser tests, and counts what it wrote.
 // Reconstruction inside the loop calls the CPU oracle's block functions (oracle/hevc_recon_oracle.c)
 // so that encoder-side and decoder-side arithmetic cannot drift apart.
 //
@@ -60,10 +61,39 @@ typedef struct hevc_enc_params {
   int32_t vui, full_range, matrix, primaries, transfer;
   int32_t cb_qp_offset, cr_qp_offset;
   int32_t loop_filter_across_slices, loop_filter_across_tiles;
-  int32_t amp_dummy;         // reserved
+  int32_t stress;            // HEVC_ENC_STRESS_* bit mask; 0: ordinary content
   uint32_t seed;
 } hevc_enc_params;
 }
+
+// Stress mode: syntax values at the limits of their legal ranges, for parser tests. With stress == 0 the encoder
+// makes exactly the draws of its RNG it always made, so every stream it wrote before is reproduced byte for byte.
+enum {
+  HEVC_ENC_STRESS_LEVELS = 1,   // per TB: keep the levels, or rewrite them sparse or dense with extreme values
+  HEVC_ENC_STRESS_MODES = 2,    // luma modes uniform over 0..34, NxN more often, intra_chroma_pred_mode uniform over 0..4
+  HEVC_ENC_STRESS_QP = 4,       // QG QP uniform over [-QpBdOffsetY, 51], reached through the wrap of 8.6.1
+  HEVC_ENC_STRESS_SAO = 8,      // SAO offsets uniform over 0..cMax, more merges
+  HEVC_ENC_STRESS_DENSE = 16,   // with LEVELS: every TB dense (every coefficient non-zero)
+};
+
+// Counters of what the encoder wrote (hevc_enc_encode_ex). X(name, n): n > 1 is an array, named name_0 .. name_<n-1>.
+#define HEVC_ENC_STATS(X)                                                                                               \
+  X(level_min, 1) X(level_max, 1) X(escape_long, 1) X(escape_prefix16, 1) X(rice4, 1)                                  \
+  X(sb_16_sig, 1) X(sb_beyond_8, 1) X(sign_hidden_even, 1) X(sign_hidden_odd, 1) X(sign_string_16, 1)                   \
+  X(last_suffix, 1) X(last_31, 1) X(inferred_sb_dc, 1) X(tskip_coded, 1)                                                \
+  X(ctb_coeff_full, 1) X(ctb_tb_full, 1)                                                                                \
+  X(qp_delta_ge5, 1) X(qp_delta_min, 1) X(qp_delta_max, 1) X(qp_wrap_below, 1) X(qp_wrap_above, 1) X(qp_y_neg, 1)       \
+  X(qp_y_51, 1) X(chroma_qpi_clip_lo, 1) X(chroma_qpi_clip_hi, 1)                                                       \
+  X(luma_mode, 35) X(mpm_idx, 3) X(rem_mode, 1) X(nxn_4_modes, 1) X(chroma_pred_mode, 5) X(chroma_mode_34, 1)           \
+  X(mode422, 35)                                                                                                        \
+  X(sao_offset_cmax_hbd, 1) X(sao_band_ge29, 1) X(sao_eo_class, 4) X(sao_merge_left, 1) X(sao_merge_up, 1)
+
+enum {
+#define HEVC_ENC_STAT_ENUM(name, n) ST_##name, ST_##name##_end_ = ST_##name + (n) - 1,
+  HEVC_ENC_STATS(HEVC_ENC_STAT_ENUM)
+#undef HEVC_ENC_STAT_ENUM
+  ST_COUNT
+};
 
 namespace {
 
@@ -314,10 +344,13 @@ struct Enc {
   int log2_min_cu_qp_delta = 6;
   struct Sao { uint8_t type[3], boc[3]; int8_t off[3][4]; };
   std::vector<Sao> sao;
+  uint64_t stats[ST_COUNT] = {};
+  int ctb_ntb = 0, ctb_ncoeff = 0;  // coded TBs / coefficients of the current CTB
 
   explicit Enc(const hevc_enc_params& p) : P(p), rng(p.seed) {}
 
   inline void bin(int c, int v) { cabac.bin(ctx.s[c], v); }
+  bool stress(int bit) const { return (P.stress & bit) != 0; }
 
   // ---- geometry helpers -------------------------------------------------------------------------
   int ctb_of(int x, int y) const { return (x >> log2_ctb) + (y >> log2_ctb) * ctbs_w; }
@@ -628,6 +661,7 @@ hc_blk Enc::make_blk(int cIdx, int xB, int yB, int log2, int mode, bool no_edge)
 }
 
 int Enc::choose_mode(int x0, int y0, int log2) {
+  if (stress(HEVC_ENC_STRESS_MODES)) return rng.below(35);
   int l = std::min(log2, 5);
   int nT = 1 << l;
   int cands[12] = {0, 1, 10, 26, 2, 18, 34, 6, 14, 22, 30, 2 + rng.below(33)};
@@ -719,9 +753,34 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
     }
     tu.coded = any;
     tu.tskip = tskip && any;
+    if (stress(HEVC_ENC_STRESS_LEVELS)) {
+      // 0: keep the quantised levels, 1 / 2: sparse, 3: dense; values from the ends of TransCoeffLevel's range
+      const int kind = stress(HEVC_ENC_STRESS_DENSE) ? 3 : rng.below(4);
+      if (kind) {
+        static const int kValues[8] = {1, -1, 2, -2, 3, -3, 32767, -32768};
+        any = false;
+        for (int i = 0; i < nT * nT; i++) {
+          int v = 0;
+          if (kind == 3 || rng.chance(30)) {
+            const int r = rng.below(10);
+            v = r < 8 ? kValues[r] : (int)(rng.next() & 0xffff) - 32768;
+            if (kind == 3 && v == 0) v = 1;
+          }
+          tu.levels[i] = (int16_t)v;
+          any |= v != 0;
+        }
+        tu.coded = any;
+        tu.tskip = tskip && any;
+      }
+    }
+  }
+  if (tu.coded && cIdx && !cu_bypass) {
+    const int qPi = cur_qp_y + (cIdx == 1 ? P.cb_qp_offset : P.cr_qp_offset);
+    if (qPi < -qp_bd_offset) stats[ST_chroma_qpi_clip_lo]++;
+    if (qPi > 57) stats[ST_chroma_qpi_clip_hi]++;
   }
 
-  // sign data hiding: fix the parity of every 4x4 sub-block that will hide a sign
+  // sign data hiding: fix the parity of every 4x4 sub-block that will hide a sign (never to +32768: -32768 becomes -32767)
   int scanIdx = 0;
   if (log2 == 2 || (log2 == 3 && (cIdx == 0 || cf == 3))) {
     if (mode >= 6 && mode <= 14) scanIdx = 2;
@@ -883,6 +942,13 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
   const ScanTables& st = scan_tables();
   const int nT = 1 << log2;
   if (P.transform_skip && !cu_bypass && log2 <= 2) bin(CTX_TSKIP + (cIdx ? 1 : 0), tu.tskip ? 1 : 0);
+  if (tu.tskip) stats[ST_tskip_coded]++;
+  ctb_ntb++;
+  for (int i = 0; i < nT * nT; i++) {
+    ctb_ncoeff += tu.levels[i] != 0;
+    if (tu.levels[i] == -32768) stats[ST_level_min]++;
+    if (tu.levels[i] == 32767) stats[ST_level_max]++;
+  }
   int scanIdx = 0;
   if (log2 == 2 || (log2 == 3 && (cIdx == 0 || cf == 3))) {
     if (pred_mode >= 6 && pred_mode <= 14) scanIdx = 2;
@@ -921,6 +987,8 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
   };
   code_prefix(CTX_LAST_X, px);
   code_prefix(CTX_LAST_Y, py);
+  if (px > 3 || py > 3) stats[ST_last_suffix]++;
+  if (LastX == 31 || LastY == 31) stats[ST_last_31]++;
   if (px > 3) cabac.bypass_bits((uint32_t)sx, nx);
   if (py > 3) cabac.bypass_bits((uint32_t)sy, ny);
 
@@ -981,6 +1049,7 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
       } else {
         // inferred significant: the encoder must really have a non-zero DC here
         spos[n] = 0; value[n] = v; n++;
+        stats[ST_inferred_sb_dc]++;
       }
     }
     if (n == 0) continue;
@@ -1005,6 +1074,10 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
     }
     bool signHidden = sign_hiding_possible && (spos[0] - spos[n - 1] > 3);
     int nsign = signHidden ? n - 1 : n;
+    if (n == 16) stats[ST_sb_16_sig]++;
+    if (n > 8) stats[ST_sb_beyond_8]++;
+    if (signHidden) stats[value[n - 1] < 0 ? ST_sign_hidden_odd : ST_sign_hidden_even]++;
+    if (nsign == 16) stats[ST_sign_string_16]++;
     for (int c = 0; c < nsign; c++) cabac.bypass(value[c] < 0);
     int rice = 0;
     for (int c = 0; c < n; c++) {
@@ -1022,8 +1095,10 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
         baseLevel = 1;
       }
       const int rem = a - baseLevel;
+      if (rice == 4) stats[ST_rice4]++;
       if (rem < (3 << rice)) {
         int len = rem >> rice;
+        if (len + 1 + rice > 16) stats[ST_escape_long]++;
         for (int k = 0; k < len; k++) cabac.bypass(1);
         cabac.bypass(0);
         cabac.bypass_bits((uint32_t)(rem & ((1 << rice) - 1)), rice);
@@ -1031,6 +1106,8 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
         int length = rice, code = rem - (3 << rice);
         while (code >= (1 << length)) { code -= 1 << length; length++; }
         int ones = 3 + length - rice;
+        if (ones + 1 + length > 16) stats[ST_escape_long]++;
+        if (ones >= 16) stats[ST_escape_prefix16]++;
         for (int k = 0; k < ones; k++) cabac.bypass(1);
         cabac.bypass(0);
         cabac.bypass_bits((uint32_t)code, length);
@@ -1049,7 +1126,19 @@ void Enc::write_tu(Node& n, const int* luma_modes, const int* chroma_modes) {
       int pred;
       derive_qp_pred(cu_x0, cu_y0, pred);
       int delta = qg_target_qp - pred;
-      // keep QpY = ((pred + delta + 52 + ...) % ...) in range: delta within [-26, 25] by construction
+      // CuQpDeltaVal is in [-(26 + QpBdOffsetY / 2), 25 + QpBdOffsetY / 2]; a target further away is reached through the
+      // wrap QpY = ((pred + delta + 52 + 2 * QpBdOffsetY) % (52 + QpBdOffsetY)) - QpBdOffsetY (8.6.1). Without the QP
+      // stress the target stays within +-12 of the prediction and never wraps.
+      const int dmin = -(26 + qp_bd_offset / 2), dmax = 25 + qp_bd_offset / 2;
+      if (delta > dmax) delta -= 52 + qp_bd_offset;
+      if (delta < dmin) delta += 52 + qp_bd_offset;
+      if (std::abs(delta) >= 5) stats[ST_qp_delta_ge5]++;
+      if (delta == dmin) stats[ST_qp_delta_min]++;
+      if (delta == dmax) stats[ST_qp_delta_max]++;
+      if (pred + delta < -qp_bd_offset) stats[ST_qp_wrap_below]++;
+      if (pred + delta > 51) stats[ST_qp_wrap_above]++;
+      if (qg_target_qp < 0) stats[ST_qp_y_neg]++;
+      if (qg_target_qp == 51) stats[ST_qp_y_51]++;
       int a = std::abs(delta);
       bin(CTX_CU_QP_DELTA, a > 0);
       if (a > 0) {
@@ -1135,7 +1224,7 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
 
   bool nxn = false;
   if (log2 == log2_min_cb) {
-    nxn = log2 > log2_min_tb && (variance(x0, y0, nCbS) > 200 ? rng.chance(60) : rng.chance(10));
+    nxn = log2 > log2_min_tb && (stress(HEVC_ENC_STRESS_MODES) ? rng.chance(50) : variance(x0, y0, nCbS) > 200 ? rng.chance(60) : rng.chance(10));
     bin(CTX_PART_MODE, nxn ? 0 : 1);
   }
   bool pcm = false;
@@ -1176,11 +1265,13 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
   Node root;
   root.x0 = x0; root.y0 = y0; root.xBase = x0; root.yBase = y0; root.log2 = log2; root.depth = 0; root.blkIdx = 0;
   auto derive_chroma = [&](int idx) {
-    int ic = rng.chance(65) ? 4 : rng.below(4);
+    int ic = stress(HEVC_ENC_STRESS_MODES) ? rng.below(5) : rng.chance(65) ? 4 : rng.below(4);
     icpm[idx] = ic;
     static const int cands[4] = {0, 26, 10, 1};
     int m = ic == 4 ? luma_modes[idx] : (cands[ic] == luma_modes[idx] ? 34 : cands[ic]);
-    if (cf == 2) m = kMode422[m];
+    stats[ST_chroma_pred_mode + ic]++;
+    if (ic != 4 && cands[ic] == luma_modes[idx]) stats[ST_chroma_mode_34]++;
+    if (cf == 2) { stats[ST_mode422 + m]++; m = kMode422[m]; }
     chroma_modes[idx] = m;
   };
   if (!nxn) {
@@ -1241,8 +1332,16 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
       for (int k = 2; k >= 0; k--) if (r > cand[k]) r--;
       rem[idx] = r;
     }
+    stats[ST_luma_mode + mode]++;
+    if (prev_flag[idx]) stats[ST_mpm_idx + mpm_idx[idx]]++;
+    else stats[ST_rem_mode]++;
     int n4 = pb >> 2;
     for (int yy = 0; yy < n4; yy++) for (int xx = 0; xx < n4; xx++) ipm[((x >> 2) + xx) + (size_t)((y >> 2) + yy) * w4] = (uint8_t)mode;
+  }
+  if (nparts == 4) {
+    bool distinct = true;
+    for (int i = 0; i < 4; i++) for (int j = 0; j < i; j++) distinct &= luma_modes[i] != luma_modes[j];
+    if (distinct) stats[ST_nxn_4_modes]++;
   }
   for (int idx = 0; idx < nparts; idx++) bin(CTX_PREV_INTRA_LUMA, prev_flag[idx]);
   for (int idx = 0; idx < nparts; idx++) {
@@ -1278,6 +1377,7 @@ void Enc::coding_quadtree(int x0, int y0, int log2, int depth) {
     CuQpDeltaVal = 0;
     // target QP of this quantisation group (kept within +-6 of the slice QP and the legal range)
     qg_target_qp = clip3(std::max(0, slice_qp - 6), std::min(51, slice_qp + 6), slice_qp + rng.below(7) - 3);
+    if (stress(HEVC_ENC_STRESS_QP)) qg_target_qp = -qp_bd_offset + rng.below(52 + qp_bd_offset);
   }
   if (split) {
     int h = size >> 1, x1 = x0 + h, y1 = y0 + h;
@@ -1296,14 +1396,14 @@ void Enc::code_sao(int rx, int ry) {
   bool merge_left = false, merge_up = false;
   if (rx > 0) {
     int left = ctb_addr_rs - 1;
-    if (ctb_slice[left] == slice_addr_rs && tile_id[left] == tile_id[ctb_addr_rs]) { merge_left = rng.chance(20); bin(CTX_SAO_MERGE, merge_left); }
+    if (ctb_slice[left] == slice_addr_rs && tile_id[left] == tile_id[ctb_addr_rs]) { merge_left = rng.chance(stress(HEVC_ENC_STRESS_SAO) ? 35 : 20); bin(CTX_SAO_MERGE, merge_left); }
   }
   if (ry > 0 && !merge_left) {
     int up = ctb_addr_rs - ctbs_w;
-    if (ctb_slice[up] == slice_addr_rs && tile_id[up] == tile_id[ctb_addr_rs]) { merge_up = rng.chance(20); bin(CTX_SAO_MERGE, merge_up); }
+    if (ctb_slice[up] == slice_addr_rs && tile_id[up] == tile_id[ctb_addr_rs]) { merge_up = rng.chance(stress(HEVC_ENC_STRESS_SAO) ? 35 : 20); bin(CTX_SAO_MERGE, merge_up); }
   }
-  if (merge_left) { s = sao[ctb_addr_rs - 1]; return; }
-  if (merge_up) { s = sao[ctb_addr_rs - ctbs_w]; return; }
+  if (merge_left) { stats[ST_sao_merge_left]++; s = sao[ctb_addr_rs - 1]; return; }
+  if (merge_up) { stats[ST_sao_merge_up]++; s = sao[ctb_addr_rs - ctbs_w]; return; }
   int ncomp = cf ? 3 : 1;
   for (int c = 0; c < ncomp; c++) {
     if (!((slice_sao_luma && c == 0) || (slice_sao_chroma && c > 0))) continue;
@@ -1319,7 +1419,8 @@ void Enc::code_sao(int rx, int ry) {
     int cMax = (1 << (std::min(bd, 10) - 5)) - 1;
     int absv[4];
     for (int i = 0; i < 4; i++) {
-      absv[i] = rng.below(std::min(cMax, 4) + 1);
+      absv[i] = rng.below((stress(HEVC_ENC_STRESS_SAO) ? cMax : std::min(cMax, 4)) + 1);
+      if (absv[i] == cMax && bd >= 10) stats[ST_sao_offset_cmax_hbd]++;
       for (int k = 0; k < absv[i]; k++) cabac.bypass(1);
       if (absv[i] < cMax) cabac.bypass(0);
     }
@@ -1328,9 +1429,10 @@ void Enc::code_sao(int rx, int ry) {
       for (int i = 0; i < 4; i++) { sign[i] = 0; if (absv[i]) { sign[i] = rng.below(2); cabac.bypass(sign[i]); } }
       s.boc[c] = (uint8_t)rng.below(32);
       cabac.bypass_bits(s.boc[c], 5);
+      if (s.boc[c] >= 29) stats[ST_sao_band_ge29]++;
       for (int i = 0; i < 4; i++) s.off[c][i] = (int8_t)(sign[i] ? -absv[i] : absv[i]);
     } else {
-      if (c < 2) { s.boc[c] = (uint8_t)rng.below(4); cabac.bypass_bits(s.boc[c], 2); }
+      if (c < 2) { s.boc[c] = (uint8_t)rng.below(4); cabac.bypass_bits(s.boc[c], 2); stats[ST_sao_eo_class + s.boc[c]]++; }
       else s.boc[2] = s.boc[1];
     }
   }
@@ -1339,7 +1441,12 @@ void Enc::code_sao(int rx, int ry) {
 void Enc::encode_ctu() {
   int rx = ctb_addr_rs % ctbs_w, ry = ctb_addr_rs / ctbs_w;
   if (slice_sao_luma || slice_sao_chroma) code_sao(rx, ry);
+  ctb_ntb = ctb_ncoeff = 0;
   coding_quadtree(rx * ctb, ry * ctb, log2_ctb, 0);
+  // the records' per-CTB capacities: every sample a coefficient, every 4x4 block of every component a TB
+  const int csamples = cf ? 2 * (ctb / SubW) * (ctb / SubH) : 0;
+  if (ctb_ncoeff == ctb * ctb + csamples) stats[ST_ctb_coeff_full]++;
+  if (ctb_ntb == (ctb * ctb + csamples) / 16) stats[ST_ctb_tb_full]++;
 }
 
 void Enc::encode_picture(std::vector<uint8_t>& out) {
@@ -1468,15 +1575,17 @@ extern "C" {
 
 // planes: uint16 samples of the visible picture (width x height, chroma subsampled), tightly
 // packed strides given in samples. Output: 4-byte-length-prefixed NAL units (VPS, SPS, PPS, slices).
-// If recon_out is not NULL it receives the encoder's reconstruction before the in-loop filters
-// (coded size), for debugging.
-int hevc_enc_encode(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
-                    size_t* out_size) {
+// recon (optional): per component a buffer of the coded size (width and height rounded up to a multiple of 8,
+// chroma subsampled, tightly packed) that receives the encoder's reconstruction before the in-loop filters.
+// stats (optional): hevc_enc_stat_count() counters of what was written (names: hevc_enc_stat_name).
+int hevc_enc_encode_ex(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
+                       size_t* out_size, uint16_t* const recon[3], uint64_t* stats) {
   if (!params || !planes || !out || !out_size) return -1;
   hevc_enc_params P = *params;
   if (P.width <= 0 || P.height <= 0 || P.chroma_format < 0 || P.chroma_format > 3 || P.bit_depth < 8 || P.bit_depth > 12) return -2;
   if (P.log2_ctb < 4 || P.log2_ctb > 6 || P.log2_min_tb < 2 || P.log2_max_tb > 5 || P.log2_min_tb > P.log2_max_tb) return -2;
   if (P.log2_min_tb >= 3) return -2;  // min CB is fixed at 8x8 here
+  if (P.qp < -6 * (P.bit_depth - 8) || P.qp > 51) return -2;
   Enc enc(P);
   enc.setup();
   const int ncomp = enc.cf ? 3 : 1;
@@ -1496,7 +1605,30 @@ int hevc_enc_encode(const hevc_enc_params* params, const uint16_t* const planes[
   memcpy(p, bytes.data(), bytes.size());
   *out = p;
   *out_size = bytes.size();
+  if (recon)
+    for (int c = 0; c < ncomp; c++)
+      if (recon[c]) memcpy(recon[c], enc.rec[c].data(), enc.rec[c].size() * sizeof(uint16_t));
+  if (stats) memcpy(stats, enc.stats, sizeof(enc.stats));
   return 0;
+}
+
+int hevc_enc_encode(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
+                    size_t* out_size) {
+  return hevc_enc_encode_ex(params, planes, strides, out, out_size, nullptr, nullptr);
+}
+
+int hevc_enc_stat_count(void) { return ST_COUNT; }
+
+const char* hevc_enc_stat_name(int i) {
+  static const std::vector<std::string> names = [] {
+    std::vector<std::string> v;
+#define HEVC_ENC_STAT_NAME(name, n) \
+  for (int k = 0; k < (n); k++) v.push_back((n) == 1 ? std::string(#name) : std::string(#name) + "_" + std::to_string(k));
+    HEVC_ENC_STATS(HEVC_ENC_STAT_NAME)
+#undef HEVC_ENC_STAT_NAME
+    return v;
+  }();
+  return i >= 0 && i < (int)names.size() ? names[(size_t)i].c_str() : nullptr;
 }
 
 void hevc_enc_free(void* p) { free(p); }

@@ -13,7 +13,11 @@ FIELDS = ["width", "height", "chroma_format", "bit_depth", "qp", "log2_ctb", "lo
           "sao", "deblock_disable", "beta_offset_div2", "tc_offset_div2", "sign_hiding", "cu_qp_delta", "transform_skip",
           "wpp", "tile_cols", "tile_rows", "slice_ctbs", "dependent_slices", "strong_intra", "scaling_list", "pcm",
           "transquant_bypass", "vui", "full_range", "matrix", "primaries", "transfer", "cb_qp_offset", "cr_qp_offset",
-          "loop_filter_across_slices", "loop_filter_across_tiles", "amp_dummy"]
+          "loop_filter_across_slices", "loop_filter_across_tiles", "stress"]
+
+# stress bits (hevc_enc_params::stress): syntax values at the limits of their legal ranges, for parser tests
+STRESS_LEVELS, STRESS_MODES, STRESS_QP, STRESS_SAO, STRESS_DENSE = 1, 2, 4, 8, 16
+STRESS_ALL = STRESS_LEVELS | STRESS_MODES | STRESS_QP | STRESS_SAO
 
 
 class Params(C.Structure):
@@ -39,13 +43,23 @@ def lib():
     if _lib is None:
         _lib = C.CDLL(build())
         _lib.hevc_enc_encode.restype = C.c_int
+        _lib.hevc_enc_encode_ex.restype = C.c_int
+        _lib.hevc_enc_stat_name.restype = C.c_char_p
         _lib.hevc_enc_free.argtypes = [C.c_void_p]
     return _lib
 
 
-def encode(planes, **kw):
+def stat_names():
+    L = lib()
+    return [L.hevc_enc_stat_name(i).decode() for i in range(L.hevc_enc_stat_count())]
+
+
+def encode(planes, want=(), **kw):
     """planes: list of 2-D integer arrays (Y[,Cb,Cr]) of the visible picture. Returns bytes:
-    4-byte-length-prefixed NAL units (VPS, SPS, PPS, slice segments)."""
+    4-byte-length-prefixed NAL units (VPS, SPS, PPS, slice segments).
+    want: any of "recon" (the encoder's reconstruction before the in-loop filters: uint16 planes of the coded size,
+    width and height rounded up to a multiple of 8) and "stats" ({counter name: count} of what was written). With a
+    non-empty want the result is (bytes, {name: value})."""
     L = lib()
     opts = dict(DEFAULTS)
     opts.update(kw)
@@ -57,12 +71,28 @@ def encode(planes, **kw):
     pp = (C.c_void_p * 3)(*([a.ctypes.data for a in pl] + [None] * (3 - len(pl))))
     st = (C.c_int * 3)(*([a.shape[1] for a in pl] + [0] * (3 - len(pl))))
     out, size = C.c_void_p(), C.c_size_t()
-    rc = L.hevc_enc_encode(C.byref(p), pp, st, C.byref(out), C.byref(size))
+    recon = rp = stats = None
+    if "recon" in want:
+        cf = p.chroma_format
+        w8, h8 = (p.width + 7) & ~7, (p.height + 7) & ~7
+        sw, sh = (2 if cf in (1, 2) else 1), (2 if cf == 1 else 1)
+        recon = [np.zeros(d, np.uint16) for d in [(h8, w8)] + ([(h8 // sh, w8 // sw)] * 2 if cf else [])]
+        rp = (C.c_void_p * 3)(*([a.ctypes.data for a in recon] + [None] * (3 - len(recon))))
+    if "stats" in want:
+        stats = (C.c_uint64 * L.hevc_enc_stat_count())()
+    rc = L.hevc_enc_encode_ex(C.byref(p), pp, st, C.byref(out), C.byref(size), rp, stats)
     if rc != 0:
         raise RuntimeError("hevc_enc_encode failed: %d" % rc)
     data = C.string_at(out, size.value)
     L.hevc_enc_free(out)
-    return data
+    if not want:
+        return data
+    extra = {}
+    if recon is not None:
+        extra["recon"] = recon
+    if stats is not None:
+        extra["stats"] = dict(zip(stat_names(), (int(v) for v in stats)))
+    return data, extra
 
 
 def split_nals(stream):
