@@ -56,7 +56,6 @@ struct hc_engine {
   int k0_max_critical = 160;               // hc_heic_job: pictures whose parse critical path exceeds this many CTBs stay with the host parser
   int premultiply_alpha = 0;               // hc_heic_job: RGBA output multiplied by alpha in K5
   int chroma_upsampling = 0;               // HC_UPSAMPLE_*: colour conversion of hc_heic_job / hc_heic_decode_stream
-  bool fused_postfilter = false;           // HEIFCUDA_POSTFILTER=fused: K3+K4 as one shared-memory tile kernel (measured slower: both forms are bound by instruction issue, not HBM — DESIGN.md)
   int stream_depth = 0;                    // hc_heic_decode_stream: batches in flight; 0 = automatic (3 or 6 by the measured read-back time), 2..6 fixed
   int stream_depth_learned = 0;            // what the last automatic call ended with: the next call starts there
   cudaEvent_t origin = nullptr;            // HEIFCUDA_TRACE: time zero of hc_batch_timeline_ms
@@ -176,11 +175,10 @@ struct hc_batch {
   const uint32_t* d_tb_index[4] = {nullptr, nullptr, nullptr, nullptr};
   int tb_counts[4] = {0, 0, 0, 0};
   const hc::RowTask* d_tasks = nullptr;
-  const hc::WarpWork* d_work = nullptr;   // packed K2 mapping (k2_packed == 3): 3 lists per CTA
+  const hc::WarpWork* d_work = nullptr;   // K2 task lists: 3 per CTA
   int k2_ctas = 0;
   int ntasks = 0;
   int k2_smem = 0;   // dynamic shared memory per K2 CTA
-  int k2_packed = 0;        // 0: six warps per CTA; 1: Y, Y, CbCr, CbCr; 2: Y, Y, 4 x chroma (all 4:2:0, HEIFCUDA_K2_PACKED); 3: lists (default)
   // K0 (device CABAC parse) of the pictures added as bitstreams
   int nk0 = 0, nchains = 0;
   bool k0_done = false;
@@ -201,8 +199,7 @@ struct hc_batch {
   cudaEvent_t ev_k0[2] = {};
   cudaEvent_t ev_d2h[2] = {};
   size_t k0_input_bytes = 0;
-  long long max_dbk_units = 0, max_sao_quads = 0, max_pf_tiles = 0;
-  bool any_16bit = false;   // some picture has samples of more than 8 bits (sizes the fused post-filter's tile)
+  long long max_dbk_units = 0, max_sao_quads = 0;
   int max_planes = 1;
   bool uploaded = false;
   cudaEvent_t ev[8] = {};
@@ -326,7 +323,6 @@ hc_engine* hc_engine_create(int device) {
   cudaDeviceGetAttribute(&eng->sm_count, cudaDevAttrMultiProcessorCount, device);
   cudaDeviceGetStreamPriorityRange(&eng->prio_lo, &eng->prio_hi);   // (least, greatest): greatest is numerically lowest
   if (const char* m = getenv("HEIFCUDA_PARSER")) eng->device_parse = strcmp(m, "host") != 0;
-  if (const char* m = getenv("HEIFCUDA_POSTFILTER")) eng->fused_postfilter = strcmp(m, "fused") == 0;
   if (const char* m = getenv("HEIFCUDA_HOST_SHARE")) eng->host_share_pct = std::max(-1, std::min(100, atoi(m)));
   if (!cuda_ok(cudaMalloc(&eng->d_k0_tables, sizeof(hc::k0::Tables)), "cudaMalloc(K0 tables)") ||
       !cuda_ok(cudaMemcpy(eng->d_k0_tables, &hc::k0_tables(), sizeof(hc::k0::Tables), cudaMemcpyHostToDevice), "cudaMemcpy(K0 tables)")) {
@@ -353,7 +349,6 @@ int hc_engine_set_option(hc_engine* e, const char* name, int value) {
   if (!e || !name) return HC_ERR_ARGUMENT;
   if (!strcmp(name, "device_parse")) { e->device_parse = value; return HC_OK; }
   if (!strcmp(name, "k0_max_critical_ctbs")) { e->k0_max_critical = value < 1 ? 1 : value; return HC_OK; }
-  if (!strcmp(name, "fused_postfilter")) { e->fused_postfilter = value != 0; return HC_OK; }
   if (!strcmp(name, "stream_depth")) { e->stream_depth = value <= 0 ? 0 : (value < 2 ? 2 : (value > 6 ? 6 : value)); return HC_OK; }
   if (!strcmp(name, "stream_depth_learned")) { e->stream_depth_learned = value; return HC_OK; }
   if (!strcmp(name, "host_share_pct")) { e->host_share_pct = value < 0 ? -1 : (value > 100 ? 100 : value); return HC_OK; }
@@ -369,7 +364,6 @@ int hc_engine_set_option(hc_engine* e, const char* name, int value) {
 int hc_engine_get_option(const hc_engine* e, const char* name) {
   if (!e || !name) return 0;
   if (!strcmp(name, "device_parse")) return e->device_parse;
-  if (!strcmp(name, "fused_postfilter")) return e->fused_postfilter ? 1 : 0;
   if (!strcmp(name, "stream_depth")) return e->stream_depth;
   if (!strcmp(name, "stream_depth_learned")) return e->stream_depth_learned;
   if (!strcmp(name, "host_share_pct")) return e->host_share_pct;
@@ -573,8 +567,7 @@ int hc_batch_upload(hc_batch* b) {
   std::vector<int> idx_base((size_t)np * 4);   // first slot of picture i in the size-l launch list
   int max_rows = 0;
   size_t n_tasks = 0;
-  b->max_dbk_units = b->max_sao_quads = b->max_pf_tiles = 0;
-  b->any_16bit = false;
+  b->max_dbk_units = b->max_sao_quads = 0;
   b->max_planes = 1;
   b->nk0 = 0;
   b->k0_pic_of.clear();
@@ -610,8 +603,6 @@ int hc_batch_upload(hc_batch* b) {
     b->max_planes = std::max(b->max_planes, ncomp);
     b->max_dbk_units = std::max(b->max_dbk_units, (long long)(p.width >> 3) * (p.height >> 2));
     b->max_sao_quads = std::max(b->max_sao_quads, (long long)p.ctbs_w * p.ctbs_h);   // CTBs: K4 runs one warp per CTB
-    b->max_pf_tiles = std::max(b->max_pf_tiles, (long long)((p.width + 127) / 128) * ((p.height + 63) / 64));
-    if (p.bit_depth_y != 8 || p.bit_depth_c != 8) b->any_16bit = true;
     // reconstruction planes
     const int ps = (p.bit_depth_y == 8 && p.bit_depth_c == 8) ? 1 : 2;
     const int SubW = (p.chroma_format == 1 || p.chroma_format == 2) ? 2 : 1, SubH = p.chroma_format == 1 ? 2 : 1;
@@ -646,7 +637,7 @@ int hc_batch_upload(hc_batch* b) {
   size_t o_idx[4];
   for (int l = 0; l < 4; l++) o_idx[l] = place(sizeof(uint32_t) * counts[l]);
   const size_t o_tasks = place(sizeof(hc::RowTask) * n_tasks);
-  const size_t o_work = place(sizeof(hc::WarpWork) * 3 * n_tasks);   // packed K2 mapping: at most one CTA per task
+  const size_t o_work = place(sizeof(hc::WarpWork) * 3 * n_tasks);   // K2 task lists: at most one CTA per task
   // K0 inputs (uploaded): picture descriptors, slices, per-CTB tables, substreams, chains, RBSP bytes
   const int nk0 = b->nk0;
   size_t k_slices = 0, k_ctbs = 0, k_subs = 0, k_chains = 0, k_bytes = 0;
@@ -832,8 +823,7 @@ int hc_batch_upload(hc_batch* b) {
   {
     hc::RowTask* tasks = (hc::RowTask*)(H + o_tasks);
     std::vector<int> first_of_row((size_t)np * 3, -1), prev((size_t)np * 3, -1);
-    int t = 0, cta_smem = 0;
-    b->k2_smem = 0;
+    int t = 0;
     for (int row = 0; row < max_rows; row++)
       for (int i = 0; i < np; i++) {
         const hc_pic& p = b->hpics[i];
@@ -844,92 +834,54 @@ int hc_batch_upload(hc_batch* b) {
           k.pic = (uint32_t)i; k.row = (uint16_t)row; k.comp = (uint8_t)c; k.pad = 0;
           k.dep = prev[(size_t)i * 3 + c];
           prev[(size_t)i * 3 + c] = t;
-          // this warp's slice of its CTA's shared memory
-          const int ps = (p.bit_depth_y == 8 && p.bit_depth_c == 8) ? 1 : 2;
-          const int cw = (1 << p.log2_ctb) >> ((c && (p.chroma_format == 1 || p.chroma_format == 2)) ? 1 : 0);
-          const int ch = (1 << p.log2_ctb) >> ((c && p.chroma_format == 1) ? 1 : 0);
-          if (t % hc::K2_WARPS == 0) cta_smem = 0;
-          k.smem_off = (uint32_t)cta_smem;
-          cta_smem += hc::k2_task_smem_bytes(cw, ch, ps);
-          b->k2_smem = std::max(b->k2_smem, cta_smem);
           t++;
         }
       }
     b->ntasks = t;
-    // Packed mapping (kernels/k2_intra.cu): when every picture is 4:2:0, a CTA is three warps — the two luma rows of its
-    // six tasks on a warp each, the four chroma rows one after the other on the third (a chroma row takes about a quarter
-    // of a luma row) — so that all warps of a CTA run for about the same time and 12 instead of 8 luma rows are resident
-    // per SM. The chroma rows share one region of shared memory. HEIFCUDA_K2_PACKED = 0 / 1 / 2 overrides.
-    bool all420 = t > 0;
-    for (int i = 0; i < np; i++) all420 = all420 && b->hpics[i].chroma_format == 1;
-    b->k2_packed = all420 ? 2 : 0;   // measured per 32 x 12 MP: six-warp CTAs 6.48 ms, mode 1 5.35 ms, mode 2 5.04 ms
-    if (const char* m = getenv("HEIFCUDA_K2_PACKED")) b->k2_packed = all420 ? atoi(m) : 0;
-    // Default for every batch: explicit per-warp lists (mode 3). A luma-class row (luma, or chroma that is not subsampled)
-    // takes a warp of its own, subsampled chroma rows share the third warp up to four units (4:2:0 row = 1, 4:2:2 row = 2).
-    if (!getenv("HEIFCUDA_K2_PACKED") && t > 0) {
-      b->k2_packed = 3;
-      hc::WarpWork* work = (hc::WarpWork*)(H + o_work);
-      auto task_bytes = [&](int idx, int& units) {
-        const hc_pic& p = b->hpics[tasks[idx].pic];
-        const int ps = (p.bit_depth_y == 8 && p.bit_depth_c == 8) ? 1 : 2;
-        const int c = tasks[idx].comp;
-        const int sw = (c && (p.chroma_format == 1 || p.chroma_format == 2)) ? 1 : 0, sh = (c && p.chroma_format == 1) ? 1 : 0;
-        units = (sw + sh == 2) ? 1 : (sw + sh == 1 ? 2 : 0);   // 0: luma class
-        return hc::k2_task_smem_bytes((1 << p.log2_ctb) >> sw, (1 << p.log2_ctb) >> sh, ps);
-      };
-      int ncta = 0;
-      b->k2_smem = 0;
-      int luma[2], nl = 0, chroma[4], nc = 0, cunits = 0;
-      auto flush = [&]() {
-        if (nl == 0 && nc == 0) return;
-        hc::WarpWork* w = work + 3 * (size_t)ncta;
-        memset(w, 0, 3 * sizeof(hc::WarpWork));
-        int off = 0, u;
-        for (int k = 0; k < nl; k++) { w[k].task[0] = (uint32_t)luma[k]; w[k].n = 1; tasks[luma[k]].smem_off = (uint32_t)off; off += task_bytes(luma[k], u); }
-        int cmax = 0;
-        for (int k = 0; k < nc; k++) { w[2].task[k] = (uint32_t)chroma[k]; tasks[chroma[k]].smem_off = (uint32_t)off; cmax = std::max(cmax, task_bytes(chroma[k], u)); }
-        w[2].n = (uint32_t)nc;
-        b->k2_smem = std::max(b->k2_smem, off + cmax);
-        ncta++;
-        nl = nc = cunits = 0;
-      };
-      for (int idx = 0; idx < t; idx++) {
-        int units;
-        task_bytes(idx, units);
-        if (units == 0) {
-          if (nl == 2) flush();
-          luma[nl++] = idx;
-        } else {
-          if (cunits + units > 4 || nc == 4) flush();
-          chroma[nc++] = idx;
-          cunits += units;
-        }
-      }
-      flush();
-      b->k2_ctas = ncta;
-    } else if (b->k2_packed) {
-      b->k2_smem = 0;
-      for (int base = 0; base < t; base += 6) {
-        auto bytes = [&](int idx) {
-          if (idx >= t) return 0;
-          const hc_pic& p = b->hpics[tasks[idx].pic];
-          const int ps = (p.bit_depth_y == 8 && p.bit_depth_c == 8) ? 1 : 2;
-          const int c = tasks[idx].comp;
-          return hc::k2_task_smem_bytes((1 << p.log2_ctb) >> (c ? 1 : 0), (1 << p.log2_ctb) >> (c ? 1 : 0), ps);
-        };
-        const int ya = bytes(base), yb = bytes(base + 3);
-        const int ca = std::max(bytes(base + 1), bytes(base + 2)), cb = std::max(bytes(base + 4), bytes(base + 5));
-        const int off_b = b->k2_packed == 1 ? ya + yb + ca : ya + yb;           // mode 2: all four chroma rows share one region
-        const int total = b->k2_packed == 1 ? ya + yb + ca + cb : ya + yb + std::max(ca, cb);
-        tasks[base].smem_off = 0;
-        if (base + 3 < t) tasks[base + 3].smem_off = (uint32_t)ya;
-        for (int k : {1, 2})
-          if (base + k < t) tasks[base + k].smem_off = (uint32_t)(ya + yb);
-        for (int k : {4, 5})
-          if (base + k < t) tasks[base + k].smem_off = (uint32_t)off_b;
-        b->k2_smem = std::max(b->k2_smem, total);
+    // Per-warp task lists of the K2 CTAs (kernels/k2_intra.cu: k2_intra_lists_kernel) and each task's slice of its CTA's
+    // shared memory. A CTA is three warps: a luma-class row (luma, or chroma that is not subsampled) takes a warp of its
+    // own, subsampled chroma rows share the third warp up to four units (4:2:0 row = 1, 4:2:2 row = 2; a 4:2:0 chroma row
+    // takes about a quarter of a luma row), so that all warps of a CTA run for about the same time. The chroma rows of a
+    // CTA run one after the other and share one region of shared memory.
+    hc::WarpWork* work = (hc::WarpWork*)(H + o_work);
+    auto task_bytes = [&](int idx, int& units) {
+      const hc_pic& p = b->hpics[tasks[idx].pic];
+      const int ps = (p.bit_depth_y == 8 && p.bit_depth_c == 8) ? 1 : 2;
+      const int c = tasks[idx].comp;
+      const int sw = (c && (p.chroma_format == 1 || p.chroma_format == 2)) ? 1 : 0, sh = (c && p.chroma_format == 1) ? 1 : 0;
+      units = (sw + sh == 2) ? 1 : (sw + sh == 1 ? 2 : 0);   // 0: luma class
+      return hc::k2_task_smem_bytes((1 << p.log2_ctb) >> sw, (1 << p.log2_ctb) >> sh, ps);
+    };
+    int ncta = 0;
+    b->k2_smem = 0;
+    int luma[2], nl = 0, chroma[4], nc = 0, cunits = 0;
+    auto flush = [&]() {
+      if (nl == 0 && nc == 0) return;
+      hc::WarpWork* w = work + 3 * (size_t)ncta;
+      memset(w, 0, 3 * sizeof(hc::WarpWork));
+      int off = 0, u;
+      for (int k = 0; k < nl; k++) { w[k].task[0] = (uint32_t)luma[k]; w[k].n = 1; tasks[luma[k]].smem_off = (uint32_t)off; off += task_bytes(luma[k], u); }
+      int cmax = 0;
+      for (int k = 0; k < nc; k++) { w[2].task[k] = (uint32_t)chroma[k]; tasks[chroma[k]].smem_off = (uint32_t)off; cmax = std::max(cmax, task_bytes(chroma[k], u)); }
+      w[2].n = (uint32_t)nc;
+      b->k2_smem = std::max(b->k2_smem, off + cmax);
+      ncta++;
+      nl = nc = cunits = 0;
+    };
+    for (int idx = 0; idx < t; idx++) {
+      int units;
+      task_bytes(idx, units);
+      if (units == 0) {
+        if (nl == 2) flush();
+        luma[nl++] = idx;
+      } else {
+        if (cunits + units > 4 || nc == 4) flush();
+        chroma[nc++] = idx;
+        cunits += units;
       }
     }
+    flush();
+    b->k2_ctas = ncta;
   }
 
   // ---- device view ----
@@ -1033,29 +985,19 @@ int hc_batch_reconstruct_async(hc_batch* b, int stages) {
   if (b->nk0)
     hc::launch_k1_indirect(b->view, b->d_k0_tb_index, b->k0_list_cap, (const unsigned*)(D + b->k0_status_off) + b->nk0, b->eng->sm_count, s);
   cudaEventRecord(b->ev[3], s);
-  if (b->k2_packed == 3) hc::launch_k2_lists(b->view, b->d_tasks, b->d_work, b->k2_ctas, b->k2_smem, (int*)b->d_progress.p, s);
-  else hc::launch_k2(b->view, b->d_tasks, b->ntasks, b->k2_smem, (int*)b->d_progress.p, b->k2_packed, s);
+  hc::launch_k2(b->view, b->d_tasks, b->d_work, b->k2_ctas, b->k2_smem, (int*)b->d_progress.p, s);
   b->launches += 1;
   cudaEventRecord(b->ev[4], s);
-  // K4 (or the fused K3+K4) always runs: it is also the crop + paste pass; SAO parameters are ignored when disabled
+  // K4 always runs: it is also the crop + paste pass; SAO parameters are ignored when disabled
   hc::BatchView v = b->view;
   v.flags = (stages & HC_STAGE_SAO) ? 0 : hc::HC_VIEW_NO_SAO;
-  if (b->eng->fused_postfilter) {
-    // one tile kernel: deblocking + SAO + crop + paste with the tile in shared memory (k34_postfilter.cu); its time is
-    // reported as the K4 stage, the K3 stage is empty
-    cudaEventRecord(b->ev[5], s);
-    if (!(stages & HC_STAGE_DEBLOCK)) v.flags |= hc::HC_VIEW_NO_DEBLOCK;
-    hc::launch_k34(v, b->max_pf_tiles, b->max_planes, b->any_16bit, s);
-    b->launches += 1;
-  } else {
-    if (stages & HC_STAGE_DEBLOCK) {
-      hc::launch_k3(b->view, b->max_dbk_units, b->max_planes, s);
-      b->launches += 2;
-    }
-    cudaEventRecord(b->ev[5], s);
-    hc::launch_k4(v, b->max_sao_quads, b->max_planes, s);
-    b->launches += 1;
+  if (stages & HC_STAGE_DEBLOCK) {
+    hc::launch_k3(b->view, b->max_dbk_units, b->max_planes, s);
+    b->launches += 2;
   }
+  cudaEventRecord(b->ev[5], s);
+  hc::launch_k4(v, b->max_sao_quads, b->max_planes, s);
+  b->launches += 1;
   // K6: irot / imir / clap passes of the canvases that carry any, plane by plane (rare; timed with K4)
   for (const Canvas& c : b->canvases) {
     if (!c.transformed()) continue;

@@ -34,7 +34,6 @@ struct BatchView {
   int flags;               // HC_VIEW_*
 };
 constexpr int HC_VIEW_NO_SAO = 1;  // K4 only crops + pastes (parity tests of the earlier stages)
-constexpr int HC_VIEW_NO_DEBLOCK = 2;  // fused post-filter: skip the two deblocking phases
 
 // One wavefront task of K2: a CTB row of one colour component of one picture.
 struct RowTask {
@@ -45,9 +44,8 @@ struct RowTask {
   int32_t dep;   // task index of the row above (same picture / component), -1 for row 0
   uint32_t smem_off;  // byte offset of this warp's slice of the CTA's dynamic shared memory
 };
-constexpr int K2_WARPS = 6;   // row tasks per CTA (two Y/Cb/Cr triples of a 4:2:0 picture) — six-warp mapping
-// Packed mapping of K2: the row tasks one warp runs one after the other (a CTA is three warps: two luma-class rows and one
-// list of up to four subsampled chroma rows; see k2_intra_lists_kernel)
+// The row tasks one warp of K2 runs one after the other (a CTA is three warps: two luma-class rows and one list of up to
+// four subsampled chroma rows; see k2_intra_lists_kernel)
 struct WarpWork {
   uint32_t task[4];
   uint32_t n;

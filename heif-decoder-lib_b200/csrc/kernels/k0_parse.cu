@@ -6,7 +6,6 @@
 // chains in flight. Chains are ordered row-major across all pictures so that a chain only ever waits for a chain
 // with a smaller index (scheduled no later than itself). Tables, context states and the picture / slice descriptors
 // of a chain live in shared memory (k0_core.cuh: Scratch).
-#include <cstdlib>
 #include "launch.h"
 #include "k0_core.cuh"
 
@@ -17,15 +16,17 @@ namespace hc {
 // consecutive pictures, so the warps of a CTA run for about the same time.
 constexpr int K0_WARPS = 4;
 
-// MIN_CTAS: CTAs per SM the register allocation must allow (5 -> 96 registers, 6 -> 80, 8 -> 64). A chain uses one
-// lane, so resident chains per SM = 4 * MIN_CTAS is limited by registers x 32 lanes; HEIFCUDA_K0_OCC picks the trade-off
-// between spills in a chain and chains in flight. Measured per 32 x 12 MP (DESIGN.md), v6 (one lane per chain): 5 -> 114 ms,
-// 6 -> 109 ms, 8 -> 109 ms, 10 -> 116 ms, 12 -> 129 ms; v7 (warp-uniform chains): 5 -> 102.8, 6 -> 103.2, 7 -> 100.2,
-// 8 -> 97.7 (default), 9 -> 97.4, 10 -> 110.2, 12 -> 115.0, 16 -> 126.2 ms.
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(32 * K0_WARPS, MIN_CTAS) k0_parse_kernel(const k0::Tables* __restrict__ tables, const k0::Pic* __restrict__ pics,
-                                                                          const k0::Sub* __restrict__ subs, const k0::Chain* __restrict__ chains,
-                                                                          int nchains) {
+// K0_MIN_CTAS: CTAs per SM the register allocation must allow (5 -> 96 registers, 6 -> 80, 8 -> 64). A chain uses one
+// lane, so resident chains per SM = 4 * K0_MIN_CTAS is limited by registers x 32 lanes: the value trades spills in a chain
+// against chains in flight. Measured per 32 x 12 MP (DESIGN.md), v6 (one lane per chain): 5 -> 114 ms, 6 -> 109 ms,
+// 8 -> 109 ms, 10 -> 116 ms, 12 -> 129 ms; v7 (warp-uniform chains): 5 -> 102.8, 6 -> 103.2, 7 -> 100.2, 8 -> 97.7,
+// 9 -> 97.4, 10 -> 110.2, 12 -> 115.0, 16 -> 126.2 ms: 8 is the fastest up to noise. Ten or more CTAs per SM would also
+// need more shared memory than the default carve-out offers (12.4 KB per CTA).
+constexpr int K0_MIN_CTAS = 8;
+
+__global__ void __launch_bounds__(32 * K0_WARPS, K0_MIN_CTAS) k0_parse_kernel(const k0::Tables* __restrict__ tables, const k0::Pic* __restrict__ pics,
+                                                                             const k0::Sub* __restrict__ subs, const k0::Chain* __restrict__ chains,
+                                                                             int nchains) {
   {
     const uint32_t* src = reinterpret_cast<const uint32_t*>(tables);
     uint32_t* dst = reinterpret_cast<uint32_t*>(k0::k0_smem);
@@ -74,25 +75,9 @@ void launch_k0(const k0::Tables* tables, const k0::Pic* pics, const k0::Sub* sub
                cudaStream_t stream) {
   if (nchains <= 0) return;
   static_assert(sizeof(k0::Tables) % 4 == 0, "tables are copied word-wise");
-  static const int occ = []() { const char* e = getenv("HEIFCUDA_K0_OCC"); return e ? atoi(e) : 8; }();
   const int smem = k0::TABLE_BYTES + K0_WARPS * k0::SCRATCH_BYTES;
   const int grid = (nchains + K0_WARPS - 1) / K0_WARPS;
-  // more than ten CTAs per SM need more shared memory than the default carve-out offers (12.4 KB per CTA)
-  static const bool carve = [&]() {
-    if (occ >= 16) cudaFuncSetAttribute(k0_parse_kernel<16>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    else if (occ >= 12) cudaFuncSetAttribute(k0_parse_kernel<12>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    else if (occ >= 10) cudaFuncSetAttribute(k0_parse_kernel<10>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    return true;
-  }();
-  (void)carve;
-  if (occ >= 16) k0_parse_kernel<16><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ >= 12) k0_parse_kernel<12><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ >= 10) k0_parse_kernel<10><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ >= 9) k0_parse_kernel<9><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ >= 8) k0_parse_kernel<8><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ == 7) k0_parse_kernel<7><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else if (occ <= 5) k0_parse_kernel<5><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
-  else k0_parse_kernel<6><<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
+  k0_parse_kernel<<<grid, 32 * K0_WARPS, smem, stream>>>(tables, pics, subs, chains, nchains);
 }
 
 }  // namespace hc

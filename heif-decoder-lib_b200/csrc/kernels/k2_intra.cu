@@ -567,8 +567,8 @@ __device__ void run_row(const BatchView& bv, const hc_pic& pic, const RowTask ta
     off_cur = off_nxt; total_cur = total_nxt;
     buf ^= 1;
   }
-  // the packed mapping runs several rows one after the other in the same shared memory: the mbarriers are re-initialised
-  // by the next row, which requires them to be invalidated first
+  // a warp may run several chroma rows one after the other in the same shared memory (k2_intra_lists_kernel): the
+  // mbarriers are re-initialised by the next row, which requires them to be invalidated first
   __syncwarp();
   if (lane == 0) {
     asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(bar0) : "memory");
@@ -577,53 +577,12 @@ __device__ void run_row(const BatchView& bv, const hc_pic& pic, const RowTask ta
   __syncwarp();
 }
 
-__global__ void __launch_bounds__(K2_WARPS * 32, 4)
-k2_intra_kernel(BatchView bv, const RowTask* __restrict__ tasks, int ntasks, int* progress) {
-  extern __shared__ __align__(16) uint8_t k2_smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int index = blockIdx.x * K2_WARPS + warp;
-  if (index >= ntasks) return;
-  const RowTask task = tasks[index];
-  const hc_pic& pic = bv.pics[task.pic];
-  // planes of a picture share one sample type: 8-bit pictures use bytes, everything else uint16
-  if (pic.bit_depth_y == 8 && pic.bit_depth_c == 8)
-    run_row<uint8_t>(bv, pic, task, progress, index, k2_smem + task.smem_off, lane);
-  else
-    run_row<uint16_t>(bv, pic, task, progress, index, k2_smem + task.smem_off, lane);
-}
-
-// Packed mapping for batches of 4:2:0 pictures: tasks 6c .. 6c+5 are (picture A: Y, Cb, Cr; picture B: Y, Cb, Cr) of one CTB
-// row each. A luma row takes about as long as the four chroma rows together, so the CTA is three warps: Y_A, Y_B, and
-// Cb_A, Cr_A, Cb_B, Cr_B one after the other. Every task still only waits for a task with a smaller index (the row above),
-// which lives in an earlier CTA or earlier in the same warp's list, so the forward-progress argument is unchanged.
-// MODE 1: four warps (Y_A, Y_B, Cb_A + Cr_A, Cb_B + Cr_B); MODE 2: three warps (Y_A, Y_B, all four chroma rows).
-template <int MODE>
-__global__ void __launch_bounds__(MODE == 1 ? 128 : 96, MODE == 1 ? 5 : 6)
-k2_intra_packed_kernel(BatchView bv, const RowTask* __restrict__ tasks, int ntasks, int* progress) {
-  extern __shared__ __align__(16) uint8_t k2_smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int base = blockIdx.x * 6;
-  // first task of the warp inside the group of six, and how many it runs
-  const int first = warp == 0 ? 0 : (warp == 1 ? 3 : (warp == 2 ? 1 : 4));
-  const int count = warp < 2 ? 1 : (MODE == 1 ? 2 : 4);
-#pragma unroll 1
-  for (int k = 0; k < count; k++) {
-    const int index = base + first + k + ((MODE == 2 && k >= 2) ? 1 : 0);   // MODE 2, warp 2: 1, 2, 4, 5
-    if (index >= ntasks) break;
-    const RowTask task = tasks[index];
-    const hc_pic& pic = bv.pics[task.pic];
-    if (pic.bit_depth_y == 8 && pic.bit_depth_c == 8)
-      run_row<uint8_t>(bv, pic, task, progress, index, k2_smem + task.smem_off, lane);
-    else
-      run_row<uint16_t>(bv, pic, task, progress, index, k2_smem + task.smem_off, lane);
-    __syncwarp();
-  }
-}
-
-// General form of the packed mapping (any mix of chroma formats, monochrome alpha pictures): the host builds the three task
-// lists of every CTA (engine.cu: two luma-class rows on a warp each, up to four units of subsampled chroma rows on the
-// third). Lists are filled in task order, a luma-class list holds one task and all chroma rows of a CTA share one warp, so
-// a task still only waits for a task in an earlier CTA, in another warp's single-task list, or earlier in its own list.
+// A CTA is three warps, each running the row tasks of its list one after the other. The host builds the lists (engine.cu):
+// a luma-class row takes a warp of its own, and up to four units of subsampled chroma rows (a 4:2:0 row is one unit, a
+// 4:2:2 row two) share the third warp, since a luma row takes about as long as the four chroma rows of 4:2:0 together.
+// Lists are filled in task order, a luma-class list holds one task and all chroma rows of a CTA share one warp, so a task
+// only waits for a task in an earlier CTA, in another warp's single-task list, or earlier in its own list: forward progress
+// holds as for one task per warp.
 __global__ void __launch_bounds__(96, 6)
 k2_intra_lists_kernel(BatchView bv, const RowTask* __restrict__ tasks, const WarpWork* __restrict__ work, int* progress) {
   extern __shared__ __align__(16) uint8_t k2_smem[];
@@ -642,8 +601,10 @@ k2_intra_lists_kernel(BatchView bv, const RowTask* __restrict__ tasks, const War
   }
 }
 
-void launch_k2_lists(const BatchView& bv, const RowTask* tasks, const WarpWork* work, int nctas, int smem_bytes, int* progress, cudaStream_t stream) {
+void launch_k2(const BatchView& bv, const RowTask* tasks, const WarpWork* work, int nctas, int smem_bytes, int* progress, cudaStream_t stream) {
   if (nctas <= 0) return;
+  // per device attribute: raised only when a launch needs more than any earlier one on this device (the plugin launches
+  // K2 once per tile from many threads, and every CUDA call serialises on the context)
   {
     static std::atomic<int> max_set[64];
     int dev = 0;
@@ -656,29 +617,6 @@ void launch_k2_lists(const BatchView& bv, const RowTask* tasks, const WarpWork* 
     }
   }
   k2_intra_lists_kernel<<<nctas, 96, smem_bytes, stream>>>(bv, tasks, work, progress);
-}
-
-void launch_k2(const BatchView& bv, const RowTask* tasks, int ntasks, int smem_bytes, int* progress, int packed, cudaStream_t stream) {
-  if (ntasks <= 0) return;
-  // per device attribute: raised only when a launch needs more than any earlier one on this device (the plugin launches
-  // K2 once per tile from many threads, and every CUDA call serialises on the context)
-  {
-    static std::atomic<int> max_set[64];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    dev &= 63;
-    if (smem_bytes > max_set[dev].load(std::memory_order_relaxed)) {
-      cudaFuncSetAttribute(k2_intra_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-      cudaFuncSetAttribute(k2_intra_packed_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-      cudaFuncSetAttribute(k2_intra_packed_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-      int cur = max_set[dev].load();
-      while (smem_bytes > cur && !max_set[dev].compare_exchange_weak(cur, smem_bytes)) {}
-    }
-  }
-  const int grid = (ntasks + K2_WARPS - 1) / K2_WARPS;
-  if (packed == 1) k2_intra_packed_kernel<1><<<(ntasks + 5) / 6, 128, smem_bytes, stream>>>(bv, tasks, ntasks, progress);
-  else if (packed == 2) k2_intra_packed_kernel<2><<<(ntasks + 5) / 6, 96, smem_bytes, stream>>>(bv, tasks, ntasks, progress);
-  else k2_intra_kernel<<<grid, K2_WARPS * 32, smem_bytes, stream>>>(bv, tasks, ntasks, progress);
 }
 
 }  // namespace hc

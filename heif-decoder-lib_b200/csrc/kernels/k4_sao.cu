@@ -36,7 +36,7 @@ __device__ __forceinline__ void sao_ctb(const BatchView& bv, const hc_pic& pic, 
   const int sstride = (int)pic.rec_stride[c];
   const int y_end = min(P.height, (ctby + 1) << P.log2h);
   for (int y = (ctby << P.log2h) + (lane >> lu); y < y_end; y += rows)
-    sao_unit<Pixel, false>(bv, pic, P, x0, y, src + (size_t)y * sstride + x0, sstride);
+    sao_unit<Pixel>(bv, pic, P, x0, y, src + (size_t)y * sstride + x0, sstride);
 }
 
 // One warp per CTB (it walks the CTB's row groups), 8 CTBs per CTA, the picture descriptor staged in shared memory:

@@ -81,14 +81,11 @@ void launch_k1_indirect(const BatchView& bv, const uint32_t* const tb_index[4], 
                         int sm_count, cudaStream_t stream);
 // shared-memory bytes one K2 row task needs (CTB of ctb_w x ctb_h samples of this component)
 int k2_task_smem_bytes(int ctb_w, int ctb_h, int pixel_bytes);
-// smem_bytes: dynamic shared memory per CTA = max over CTAs of the sum of its K2_WARPS tasks
-void launch_k2(const BatchView& bv, const RowTask* tasks, int ntasks, int smem_bytes, int* progress, int packed, cudaStream_t stream);
-// packed mapping with explicit per-warp task lists: `work` holds 3 entries per CTA
-void launch_k2_lists(const BatchView& bv, const RowTask* tasks, const WarpWork* work, int nctas, int smem_bytes, int* progress, cudaStream_t stream);
+// per-warp task lists: `work` holds 3 entries per CTA; smem_bytes: dynamic shared memory per CTA = max over CTAs of the
+// bytes its lists need
+void launch_k2(const BatchView& bv, const RowTask* tasks, const WarpWork* work, int nctas, int smem_bytes, int* progress, cudaStream_t stream);
 void launch_k3(const BatchView& bv, long long max_units, int planes, cudaStream_t stream);
 void launch_k4(const BatchView& bv, long long max_ctbs, int planes, cudaStream_t stream);
-// K3 + K4 fused, one shared-memory tile at a time (k34_postfilter.cu); bv.flags: HC_VIEW_NO_DEBLOCK / HC_VIEW_NO_SAO
-void launch_k34(const BatchView& bv, long long max_tiles, int planes, bool sixteen_bit, cudaStream_t stream);
 void launch_k5(const CscArgs& a, bool sixteen_bit, cudaStream_t stream);
 void launch_k5_batch(const CscBatch& b, bool sixteen_bit, cudaStream_t stream);
 void launch_k6(const XformArgs& a, bool sixteen_bit, cudaStream_t stream);

@@ -1,5 +1,5 @@
-// postfilter_core.cuh — the per-unit arithmetic of the in-loop filters, shared by the split kernels (k3_deblock.cu,
-// k4_sao.cu: one pass over global memory each) and the fused tile kernel (k34_postfilter.cu: the tile in shared memory).
+// postfilter_core.cuh — the per-unit arithmetic of the in-loop filters: deblocking (k3_deblock.cu) and SAO + crop + paste
+// (k4_sao.cu), one pass over global memory each.
 //
 // Deblocking replaces edge_filtering_luma_internal (deblock.cc:708-792) + loop_filter_luma (fallback-postfilter.h:31-135)
 // and edge_filtering_chroma_internal (:1607-1772) + loop_filter_chroma (:138-179); SAO replaces apply_sao_internal
@@ -88,9 +88,9 @@ __device__ void deblock_luma_unit(Pixel* __restrict__ pix, ptrdiff_t xs, ptrdiff
   }
 }
 
-// One 4-line unit of one edge. (x, y): plane position of the unit's first q0 sample; `pix` points at that sample in whichever
-// memory holds the plane (global: the split kernel filters in place; shared: the fused kernel's tile), `stride` is the
-// pitch of that memory in samples. Edge flags / QP / slice offsets are looked up by picture position.
+// One 4-line unit of one edge. (x, y): plane position of the unit's first q0 sample; `pix` points at that sample (K3 filters
+// the plane in place), `stride` is the plane's pitch in samples. Edge flags / QP / slice offsets are looked up by picture
+// position.
 template <typename Pixel>
 __device__ __forceinline__ void deblock_unit_at(const BatchView& bv, const hc_pic& pic, int plane_idx, bool vertical, int x, int y, Pixel* pix,
                                                 int stride) {
@@ -213,23 +213,6 @@ HC_D void store8(uint16_t* p, const int v[8]) {
   *reinterpret_cast<uint4*>(p) = w;
 }
 
-// the same eight samples from a row that is only aligned to four samples (the fused kernel's shared-memory tile starts
-// four samples left of an 8-aligned column)
-template <typename Pixel>
-HC_D void load8_half(const Pixel* p, int v[8]);
-template <>
-HC_D void load8_half<uint8_t>(const uint8_t* p, int v[8]) {
-  const uint32_t a = *reinterpret_cast<const uint32_t*>(p), b = *reinterpret_cast<const uint32_t*>(p + 4);
-#pragma unroll
-  for (int k = 0; k < 4; k++) { v[k] = (a >> (8 * k)) & 0xff; v[4 + k] = (b >> (8 * k)) & 0xff; }
-}
-template <>
-HC_D void load8_half<uint16_t>(const uint16_t* p, int v[8]) {
-  const uint2 a = *reinterpret_cast<const uint2*>(p), b = *reinterpret_cast<const uint2*>(p + 4);
-  v[0] = a.x & 0xffff; v[1] = a.x >> 16; v[2] = a.y & 0xffff; v[3] = a.y >> 16;
-  v[4] = b.x & 0xffff; v[5] = b.x >> 16; v[6] = b.y & 0xffff; v[7] = b.y >> 16;
-}
-
 // Geometry of one colour plane of one picture for the SAO + crop + paste step (context.cc:2467-2497 for the windows)
 template <typename Pixel>
 struct SaoPlane {
@@ -257,8 +240,8 @@ struct SaoPlane {
 };
 
 // One unit: 8 horizontally adjacent samples (x0 8-aligned, so inside one CTB) of row y. `row` points at sample (x0, y) of
-// the deblocked plane in whichever memory holds it, `sstride` is that memory's pitch; HALF: rows are only 4-sample aligned.
-template <typename Pixel, bool HALF>
+// the deblocked plane, `sstride` is its pitch in samples.
+template <typename Pixel>
 __device__ __forceinline__ void sao_unit(const BatchView& bv, const hc_pic& pic, const SaoPlane<Pixel>& P, int x0, int y, const Pixel* row,
                                          int sstride) {
   const int c = P.c, width = P.width, height = P.height, log2w = P.log2w, log2h = P.log2h, bit_depth = P.bit_depth, maxv = P.maxv;
@@ -272,7 +255,7 @@ __device__ __forceinline__ void sao_unit(const BatchView& bv, const hc_pic& pic,
   const hc_ctu& ctu = bv.ctus[pic.ctu_base + ctbx + ctby * pic.ctbs_w];
   const int nvalid = min(8, width - x0);            // 4 or 8
   int v[8];
-  if (nvalid == 8) { if (HALF) load8_half<Pixel>(row, v); else load8<Pixel>(row, v); }
+  if (nvalid == 8) load8<Pixel>(row, v);
   else {
 #pragma unroll
     for (int k = 0; k < 8; k++) v[k] = k < nvalid ? (int)row[k] : 0;
@@ -321,11 +304,11 @@ __device__ __forceinline__ void sao_unit(const BatchView& bv, const hc_pic& pic,
         for (int k = 0; k < 8; k++) { ra[k + 1] = v[k]; rb[k + 1] = v[k]; }
       } else {
         if (oka) {
-          if (nvalid == 8) { if (HALF) load8_half<Pixel>(rowa, ra + 1); else load8<Pixel>(rowa, ra + 1); }
+          if (nvalid == 8) load8<Pixel>(rowa, ra + 1);
           else for (int k = 0; k < nvalid; k++) ra[k + 1] = rowa[k];
         }
         if (okb) {
-          if (nvalid == 8) { if (HALF) load8_half<Pixel>(rowb, rb + 1); else load8<Pixel>(rowb, rb + 1); }
+          if (nvalid == 8) load8<Pixel>(rowb, rb + 1);
           else for (int k = 0; k < nvalid; k++) rb[k + 1] = rowb[k];
         }
       }

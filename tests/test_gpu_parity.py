@@ -44,14 +44,6 @@ def pictures():
     return all_pictures()
 
 
-@pytest.fixture(scope="module")
-def generated_pictures():
-    """(label, Records) of every generated stream (tests/golden/generated/)"""
-    names = sorted(json.load(open(os.path.join(ROOT, "tests", "golden", "generated.json"))))
-    return [(n, hb.parse_picture(open(os.path.join(ROOT, "tests", "golden", "generated", n + ".hevc"), "rb").read()))
-            for n in names]
-
-
 def gpu_planes(engine, rec, stages):
     b = engine.batch()
     p = rec.pic
@@ -82,22 +74,6 @@ def test_planes_match_oracle_per_stage(engine, pictures, stages):
             bad = np.argwhere(g.astype(np.uint16) != w)
             assert bad.size == 0, "%s stages=%d plane %d: %d samples differ, first at (y,x)=%s" % (
                 label, stages, k, len(bad), tuple(bad[0]))
-
-
-@pytest.mark.parametrize("stages", [0, hb.STAGE_DEBLOCK, hb.STAGE_ALL])
-def test_fused_postfilter_matches_oracle_per_stage(engine, pictures, generated_pictures, stages):
-    """The fused deblock + SAO tile kernel (k34_postfilter.cu, engine option fused_postfilter; not the default — it is
-    slower than the split kernels, DESIGN.md) produces the same planes as the oracle on every bundled picture and every
-    generated stream (4:0:0 / 4:2:2 / 4:4:4, 10 and 12 bit, tiles, slices, pcm, bypass)."""
-    engine.set_option("fused_postfilter", 1)
-    try:
-        for label, rec in pictures + generated_pictures:
-            want, _ = oracle_lib.reconstruct(rec, stages)
-            got, _ = gpu_planes(engine, rec, stages)
-            for k, (g, w) in enumerate(zip(got, want)):
-                assert np.array_equal(g.astype(np.uint16), w), (label, stages, k)
-    finally:
-        engine.set_option("fused_postfilter", 0)
 
 
 def test_full_decode_matches_reference_golden(engine, pictures):

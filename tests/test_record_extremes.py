@@ -211,26 +211,6 @@ def test_gpu_single_picture_batches_match_oracle(engine):
         check_corpus(engine, "all", 1, (hb.STAGE_ALL,), [label])
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("family,seed", CASES)
-def test_gpu_fused_postfilter_matches_oracle_on_mutated_records(engine, family, seed):
-    engine.set_option("fused_postfilter", 1)
-    try:
-        check_corpus(engine, family, seed, (hb.STAGE_DEBLOCK, hb.STAGE_ALL), residuals=False)
-    finally:
-        engine.set_option("fused_postfilter", 0)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("packed", ["0", "1", "2"])
-@pytest.mark.parametrize("family", ["modes", "flat", "all"])
-def test_gpu_k2_mappings_match_oracle(engine, monkeypatch, packed, family):
-    """The K2 warp mappings HEIFCUDA_K2_PACKED selects for batches that are all 4:2:0 (read by hc_batch_upload)."""
-    labels = [label for label in FIXTURES if load(label, True).pic.chroma_format == 1]
-    monkeypatch.setenv("HEIFCUDA_K2_PACKED", packed)
-    check_corpus(engine, family, 1, (0, hb.STAGE_ALL), labels)
-
-
 def k5_batch(engine, name, with_alpha):
     """A batch with one mutated K5 picture on a canvas (and a mutated monochrome alpha picture of its size)."""
     rec = mutated("gen:" + name, "all", 1)
