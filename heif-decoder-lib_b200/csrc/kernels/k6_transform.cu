@@ -9,6 +9,8 @@
 //
 // Mapping: one thread per output sample through a 32 x 32 shared tile when the map swaps the axes (reads and writes
 // both coalesced), a plain gather otherwise. Algorithmic bytes: read s + write s per sample.
+#include <algorithm>
+
 #include "launch.h"
 
 namespace hc {
@@ -60,19 +62,22 @@ __global__ void __launch_bounds__(256) k6_scale_kernel(const Pixel* __restrict__
   const int x = blockIdx.x * 32 + (threadIdx.x & 31);
   if (x >= dw) return;
   const int ix = (int)((long long)x * sw / dw);
+  // gridDim.y is at most 65,535: taller planes are covered by striding over 32-row blocks
+  for (int y0 = blockIdx.y * 32; y0 < dh; y0 += gridDim.y * 32) {
 #pragma unroll
-  for (int r = 0; r < 4; r++) {
-    const int y = blockIdx.y * 32 + (threadIdx.x >> 5) + 8 * r;
-    if (y >= dh) continue;
-    const int iy = (int)((long long)y * sh / dh);
-    dst[(size_t)y * dst_stride + x] = src[(size_t)iy * src_stride + ix];
+    for (int r = 0; r < 4; r++) {
+      const int y = y0 + (threadIdx.x >> 5) + 8 * r;
+      if (y >= dh) continue;
+      const int iy = (int)((long long)y * sh / dh);
+      dst[(size_t)y * dst_stride + x] = src[(size_t)iy * src_stride + ix];
+    }
   }
 }
 
 void launch_k6_scale(const uint8_t* src, int sw, int sh, int src_stride, uint8_t* dst, int dw, int dh, int dst_stride, bool sixteen_bit,
                      cudaStream_t stream) {
   if (sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0) return;
-  dim3 grid((unsigned)((dw + 31) / 32), (unsigned)((dh + 31) / 32));
+  dim3 grid((unsigned)((dw + 31) / 32), (unsigned)std::min((dh + 31) / 32, kMaxGridY));
   if (sixteen_bit)
     k6_scale_kernel<uint16_t><<<grid, 256, 0, stream>>>(reinterpret_cast<const uint16_t*>(src), sw, sh, src_stride, reinterpret_cast<uint16_t*>(dst), dw, dh, dst_stride);
   else
@@ -82,9 +87,25 @@ void launch_k6_scale(const uint8_t* src, int sw, int sh, int src_stride, uint8_t
 void launch_k6(const XformArgs& a, bool sixteen_bit, cudaStream_t stream) {
   if (a.w <= 0 || a.h <= 0) return;
   const int ow = a.swap ? a.h : a.w, oh = a.swap ? a.w : a.h;
-  dim3 grid((unsigned)((ow + 31) / 32), (unsigned)((oh + 31) / 32));
-  if (sixteen_bit) k6_transform_kernel<uint16_t><<<grid, 256, 0, stream>>>(a);
-  else k6_transform_kernel<uint8_t><<<grid, 256, 0, stream>>>(a);
+  // gridDim.y is at most 65,535 blocks of 32 output rows. A taller output is transformed in bands of output rows; a band
+  // is the same map on a sub-image of the input: rows of the input without swap, columns with swap (from the far end when
+  // that axis is flipped).
+  const size_t ps = sixteen_bit ? 2 : 1;
+  for (int r0 = 0; r0 < oh; r0 += kMaxGridY * 32) {
+    const int n = std::min(oh - r0, kMaxGridY * 32);
+    XformArgs b = a;
+    b.dst = a.dst + (size_t)r0 * a.dst_stride * ps;
+    if (!a.swap) {
+      b.h = n;
+      b.src = a.src + (size_t)(a.flip_y ? a.h - r0 - n : r0) * a.src_stride * ps;
+    } else {
+      b.w = n;
+      b.src = a.src + (size_t)(a.flip_x ? a.w - r0 - n : r0) * ps;
+    }
+    dim3 grid((unsigned)((ow + 31) / 32), (unsigned)((n + 31) / 32));
+    if (sixteen_bit) k6_transform_kernel<uint16_t><<<grid, 256, 0, stream>>>(b);
+    else k6_transform_kernel<uint8_t><<<grid, 256, 0, stream>>>(b);
+  }
 }
 
 }  // namespace hc

@@ -8,6 +8,8 @@
 // interleaves the canvas (Op_RGB_to_RGB24_32, rgb2rgb.cc:28-143; Op_to_hdr_planes + Op_RGB_HDR_to_RRGGBBaa_BE [+ swap] for the
 // RRGGBB(AA) targets). Here one thread owns one output pixel and walks the child list in the same order, so no planar
 // canvas, no per-child pass and no extra allocation exist. Children are canvases of the batch after K4 / K6.
+#include <algorithm>
+
 #include "launch.h"
 
 namespace hc {
@@ -79,7 +81,15 @@ __global__ void __launch_bounds__(256) k7_overlay_kernel(OverlayArgs a) {
 
 void launch_k7(const OverlayArgs& a, cudaStream_t stream) {
   if (a.width <= 0 || a.height <= 0) return;
-  k7_overlay_kernel<<<dim3((unsigned)((a.width + 31) / 32), (unsigned)((a.height + 7) / 8)), 256, 0, stream>>>(a);
+  // gridDim.y is at most 65,535 blocks of 8 rows: a taller canvas is composed in bands of rows, each with its output rows
+  // and the children's offsets shifted up by the band's first row
+  for (int r0 = 0; r0 < a.height; r0 += kMaxGridY * 8) {
+    OverlayArgs b = a;
+    b.height = std::min(a.height - r0, kMaxGridY * 8);
+    b.out = a.out + r0 * a.out_stride;
+    for (int k = 0; k < a.n; k++) b.child[k].dy = a.child[k].dy - r0;
+    k7_overlay_kernel<<<dim3((unsigned)((a.width + 31) / 32), (unsigned)((b.height + 7) / 8)), 256, 0, stream>>>(b);
+  }
 }
 
 }  // namespace hc

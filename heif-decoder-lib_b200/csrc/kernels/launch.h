@@ -6,6 +6,9 @@
 
 namespace hc {
 
+// largest gridDim.y (and gridDim.z) of a launch
+constexpr int kMaxGridY = 65535;
+
 struct CscArgs {
   const uint8_t* y;  const uint8_t* cb;  const uint8_t* cr;  const uint8_t* a;   // plane bases (bytes)
   int y_stride, c_stride, a_stride;   // in samples

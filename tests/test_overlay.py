@@ -6,7 +6,6 @@ import hashlib
 import json
 import os
 
-import numpy as np
 import pytest
 
 import heif_b200 as hb
@@ -29,44 +28,18 @@ def md5(b):
 
 
 def compose(data, out_format):
-    """decode_overlay_image restated: 8-bit planar RGB canvas filled with the high bytes of the background colour; every
-    child converted like Op_YCbCr_to_RGB<uint8_t> (the csc oracle's general path) and overlaid in order — copied, or
-    (child * a + canvas * (255 - a)) / 255 with an alpha plane; then the interleaver of the requested format."""
+    """decode_overlay_image restated: every child converted like Op_YCbCr_to_RGB<uint8_t> (the csc oracle's general path),
+    then heic_oracle.compose_overlay"""
     hf = hb.HeifFile(data, host_only=True)
     ov = hf.overlay(hf.primary_id)
-    W, H = ov.canvas_w, ov.canvas_h
-    canvas = np.empty((H, W, 3), np.int64)
-    for k in range(3):
-        canvas[:, :, k] = ov.background[k] >> 8
+    children, alphas = [], []
     for k in range(ov.n):
         rgba = heic_oracle.decode_rgb(data, hb.OUT_RGBA, item_id=int(ov.children[k]))       # 4:4:4 8 bit: the general fp32 op, alpha copied
-        h, w = rgba.shape[0], rgba.shape[1] // 4
-        px = rgba.reshape(h, w, 4).astype(np.int64)
-        dx, dy = ov.dx[k], ov.dy[k]
-        if dx >= W or dy >= H:
-            continue
-        ww, hh = min(w, W - dx), min(h, H - dy)
-        src = px[:hh, :ww]
-        dst = canvas[dy:dy + hh, dx:dx + ww]
-        has_alpha = bool(hf.image_info(int(ov.children[k])).alpha_id)
-        if has_alpha:
-            a = src[:, :, 3:4]
-            canvas[dy:dy + hh, dx:dx + ww] = (src[:, :, :3] * a + dst * (255 - a)) // 255
-        else:
-            canvas[dy:dy + hh, dx:dx + ww] = src[:, :, :3]
-    rgb = canvas.astype(np.uint16)
-    if out_format == hb.OUT_RGB:
-        return rgb.astype(np.uint8).reshape(H, W * 3)
-    if out_format == hb.OUT_RGBA:
-        out = np.full((H, W, 4), 255, np.uint8)
-        out[:, :, :3] = rgb
-        return out.reshape(H, W * 4)
-    v = (rgb << 2) | (rgb >> 6)                                  # Op_to_hdr_planes, 8 -> 10 bit
-    alpha = out_format in (hb.OUT_RRGGBBAA_BE, hb.OUT_RRGGBBAA_LE)
-    if alpha:
-        v = np.concatenate([v, np.full((H, W, 1), 1023, np.uint16)], axis=2)
-    dt = "<u2" if out_format in (hb.OUT_RRGGBB_LE, hb.OUT_RRGGBBAA_LE) else ">u2"
-    return np.frombuffer(v.astype(dt).tobytes(), np.uint8).reshape(H, -1)
+        px = rgba.reshape(rgba.shape[0], -1, 4)
+        children.append(px[:, :, :3])
+        alphas.append(px[:, :, 3] if hf.image_info(int(ov.children[k])).alpha_id else None)
+    offsets = [(ov.dx[k], ov.dy[k]) for k in range(ov.n)]
+    return heic_oracle.compose_overlay(children, alphas, offsets, ov.background, ov.canvas_w, ov.canvas_h, out_format)
 
 
 @pytest.mark.parametrize("name", NAMES)
