@@ -19,6 +19,7 @@ int hc_batch_k0_pictures(const hc_batch*) { return 0; }
 int hc_batch_set_canvas_transform(hc_batch*, int, int, int, int) { return NO_ENGINE(); }
 int hc_batch_add_canvas_pass(hc_batch*, int, int, int, int, int, int) { return NO_ENGINE(); }
 int hc_batch_link_alpha(hc_batch*, int, int) { return NO_ENGINE(); }
+int hc_batch_set_canvas_output_size(hc_batch*, int, int, int) { return NO_ENGINE(); }
 int hc_batch_upload(hc_batch*) { return NO_ENGINE(); }
 int hc_batch_reconstruct(hc_batch*, int) { return NO_ENGINE(); }
 int hc_batch_reconstruct_async(hc_batch*, int) { return NO_ENGINE(); }

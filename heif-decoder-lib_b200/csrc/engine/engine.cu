@@ -60,6 +60,7 @@ struct hc_engine {
   int stream_depth_learned = 0;            // what the last automatic call ended with: the next call starts there
   cudaEvent_t origin = nullptr;            // HEIFCUDA_TRACE: time zero of hc_batch_timeline_ms
   int host_share_pct = -1;                 // hc_heic_job with device_parse: percentage of the coded items the host threads parse meanwhile
+  int scale_max_side = 0;                  // hc_heic_job / stream: images larger than this on their longer side are delivered scaled (0: off)
 
   Block take(std::vector<Block>& list, size_t size, bool pinned) {
     std::lock_guard<std::mutex> lk(mu);
@@ -129,6 +130,11 @@ struct Canvas {
   std::vector<Pass> passes;
   bool transformed() const { return !passes.empty(); }
   int ow = 0, oh = 0;               // output image size
+  // delivered image size (hc_batch_set_canvas_output_size; 0 = not set): K5 / K7 sample the output view by nearest neighbour.
+  // dw x dh is what the conversion writes and the read-backs copy; filled at upload (ow x oh when no size is set).
+  int req_w = 0, req_h = 0;
+  int dw = 0, dh = 0;
+  bool scaled() const { return dw != ow || dh != oh; }
   size_t ooff[4] = {0, 0, 0, 0};
   int ostride[4] = {0, 0, 0, 0}, opw[4] = {0, 0, 0, 0}, oph[4] = {0, 0, 0, 0};
   // 'iovl' derived image (hc_batch_add_overlay_canvas): no planes of its own; K7 composes the child canvases into its RGB output
@@ -219,7 +225,7 @@ using hc::plane_h;
 // bytes of a canvas' block in the batch's output buffer
 size_t out_block_bytes(const Canvas& c, int bpp) {
   if (c.planar) return align_up(c.packed, 256);
-  return align_up(align_up((size_t)((c.ow + 7) & ~7) * bpp, 256) * c.oh, 256);
+  return align_up(align_up((size_t)((c.dw + 7) & ~7) * bpp, 256) * c.dh, 256);
 }
 
 // HC_OUT_YCBCR: lays the canvas' output view out as hc_image_plane_layout does for its desc. False when the planes differ in
@@ -263,11 +269,12 @@ int check_convert(const Canvas& c, const hc_csc_params& p) {
   if (p.out_format < 0 || p.out_format > HC_OUT_YCBCR) { hc::set_last_error("bad output format"); return HC_ERR_ARGUMENT; }
   if (!c.overlay && p.in_depth != c.bit_depth) { hc::set_last_error("conversion parameters were selected for another bit depth"); return HC_ERR_ARGUMENT; }
   if (p.out_format != HC_OUT_YCBCR) {
-    if (c.ext_rgb && c.ext_stride < (size_t)((c.ow + 7) & ~7) * kBppOf[p.out_format]) { hc::set_last_error("external RGB target: rows too short for this format"); return HC_ERR_ARGUMENT; }
+    if (c.ext_rgb && c.ext_stride < (size_t)((c.dw + 7) & ~7) * kBppOf[p.out_format]) { hc::set_last_error("external RGB target: rows too short for this format"); return HC_ERR_ARGUMENT; }
     return HC_OK;
   }
   if (c.overlay) { hc::set_last_error("overlay canvases are composed in RGB: HC_OUT_YCBCR is not available for them"); return HC_ERR_UNSUPPORTED; }
   if (c.ext_rgb) { hc::set_last_error("a canvas with an external RGB target cannot be converted to HC_OUT_YCBCR"); return HC_ERR_UNSUPPORTED; }
+  if (c.scaled()) { hc::set_last_error("a scaled canvas cannot be converted to HC_OUT_YCBCR"); return HC_ERR_UNSUPPORTED; }
   size_t poff[4], packed = 0;
   if (!planar_layout(c, poff, &packed)) { hc::set_last_error("HC_OUT_YCBCR: the crop window leaves chroma planes of another size than the packed layout"); return HC_ERR_UNSUPPORTED; }
   return HC_OK;
@@ -282,7 +289,7 @@ void apply_format(Canvas& c, const hc_csc_params& p) {
     c.rgb_stride = (size_t)c.ow * c.rgb_bpp;
   } else {
     c.rgb_bpp = kBppOf[p.out_format];
-    c.rgb_stride = align_up((size_t)((c.ow + 7) & ~7) * c.rgb_bpp, 256);
+    c.rgb_stride = align_up((size_t)((c.dw + 7) & ~7) * c.rgb_bpp, 256);
   }
 }
 
@@ -353,6 +360,11 @@ int hc_engine_set_option(hc_engine* e, const char* name, int value) {
   if (!strcmp(name, "stream_depth_learned")) { e->stream_depth_learned = value; return HC_OK; }
   if (!strcmp(name, "host_share_pct")) { e->host_share_pct = value < 0 ? -1 : (value > 100 ? 100 : value); return HC_OK; }
   if (!strcmp(name, "premultiply_alpha")) { e->premultiply_alpha = value != 0; return HC_OK; }
+  if (!strcmp(name, "scale_max_side")) {
+    if (value < 0) { hc::set_last_error("scale_max_side: 0 (off) or the longest side in pixels"); return HC_ERR_ARGUMENT; }
+    e->scale_max_side = value;
+    return HC_OK;
+  }
   if (!strcmp(name, "chroma_upsampling")) {
     if (value != HC_UPSAMPLE_NEAREST && value != HC_UPSAMPLE_BILINEAR) { hc::set_last_error("chroma_upsampling: HC_UPSAMPLE_NEAREST or HC_UPSAMPLE_BILINEAR"); return HC_ERR_ARGUMENT; }
     e->chroma_upsampling = value;
@@ -369,6 +381,7 @@ int hc_engine_get_option(const hc_engine* e, const char* name) {
   if (!strcmp(name, "host_share_pct")) return e->host_share_pct;
   if (!strcmp(name, "chroma_upsampling")) return e->chroma_upsampling;
   if (!strcmp(name, "premultiply_alpha")) return e->premultiply_alpha;
+  if (!strcmp(name, "scale_max_side")) return e->scale_max_side;
   if (!strcmp(name, "k0_max_critical_ctbs")) return e->k0_max_critical;
   return 0;
 }
@@ -447,6 +460,18 @@ int hc_batch_add_canvas_pass(hc_batch* b, int canvas, int kind, int a0, int a1, 
   Canvas::Pass p;
   p.kind = kind; p.a = a0; p.b = a1; p.c = a2; p.d = a3;
   c.passes.push_back(p);
+  b->uploaded = false;
+  return HC_OK;
+}
+
+int hc_batch_set_canvas_output_size(hc_batch* b, int canvas, int width, int height) {
+  if (!b || canvas < 0 || canvas >= (int)b->canvases.size() || width < 1 || height < 1) {
+    hc::set_last_error("hc_batch_set_canvas_output_size: bad argument");
+    return HC_ERR_ARGUMENT;
+  }
+  Canvas& c = b->canvases[canvas];
+  if (c.ext_rgb) { hc::set_last_error("hc_batch_set_canvas_output_size: the canvas has an external RGB target"); return HC_ERR_UNSUPPORTED; }
+  c.req_w = width; c.req_h = height;
   b->uploaded = false;
   return HC_OK;
 }
@@ -554,6 +579,7 @@ int hc_batch_upload(hc_batch* b) {
         iw = nw; ih = nh; ipw = ps_.pw; iph = ps_.ph;
       }
       c.ow = iw; c.oh = ih;
+      c.dw = c.req_w ? c.req_w : iw; c.dh = c.req_h ? c.req_h : ih;
       for (int k = 0; k < 4; k++) {
         if (c.passes.empty()) { c.ooff[k] = c.off[k]; c.ostride[k] = c.stride[k]; c.opw[k] = c.pw[k]; c.oph[k] = c.ph[k]; }
         else { const Canvas::Pass& l = c.passes.back(); c.ooff[k] = l.off[k]; c.ostride[k] = l.stride[k]; c.opw[k] = l.pw[k]; c.oph[k] = l.ph[k]; }
@@ -1093,7 +1119,8 @@ int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
   a.cr = c.chroma ? P + c.ooff[2] : nullptr;
   a.a = c.alpha ? P + c.ooff[3] : nullptr;
   a.y_stride = c.ostride[0]; a.c_stride = c.ostride[1]; a.a_stride = c.ostride[3];
-  a.width = c.ow; a.height = c.oh; a.chroma_format = c.chroma;
+  a.width = c.dw; a.height = c.dh; a.chroma_format = c.chroma;
+  a.src_w = c.ow; a.src_h = c.oh; a.gather = c.scaled();
   a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
   a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
   a.p = *params;
@@ -1149,7 +1176,8 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
       oc.mode = cp.mode; oc.full_range = cp.full_range;
       oc.r_cr = cp.r_cr; oc.g_cb = cp.g_cb; oc.g_cr = cp.g_cr; oc.b_cb = cp.b_cb;
     }
-    oa.width = c.w; oa.height = c.h;
+    oa.width = c.dw; oa.height = c.dh;
+    oa.src_w = c.ow; oa.src_h = c.oh;
     for (int k = 0; k < 3; k++) oa.bkg[k] = c.bkg[k];
     oa.out_format = params[i].out_format;
     oa.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
@@ -1171,7 +1199,8 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
         a.cr = c.chroma ? P + c.ooff[2] : nullptr;
         a.a = c.alpha ? P + c.ooff[3] : nullptr;
         a.y_stride = c.ostride[0]; a.c_stride = c.ostride[1]; a.a_stride = c.ostride[3];
-        a.width = c.ow; a.height = c.oh; a.chroma_format = c.chroma;
+        a.width = c.dw; a.height = c.dh; a.chroma_format = c.chroma;
+        a.src_w = c.ow; a.src_h = c.oh; a.gather = c.scaled();
         a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
         a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
         a.p = params[i];
@@ -1274,7 +1303,7 @@ int hc_batch_read_rgb(hc_batch* b, int canvas, void* dst, size_t dst_stride) {
   cudaEvent_t e0 = b->ev_d2h[0], e1 = b->ev_d2h[1];
   cudaEventRecord(e0, b->stream);
   cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream)
-                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
+                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
                                                cudaMemcpyDeviceToHost, b->stream);
   cudaEventRecord(e1, b->stream);
   if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2H planes)" : "cudaMemcpy2DAsync(D2H rgb)")) return HC_ERR_CUDA;
@@ -1291,7 +1320,7 @@ int hc_batch_copy_rgb_device(hc_batch* b, int canvas, void* dst, size_t dst_stri
   if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are copied with the stride of the Y row"); return HC_ERR_ARGUMENT; }
   // cudaMemcpyDefault: `dst` may live on a peer device (unified addressing; a peer copy over NVLink then)
   cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDefault, b->stream)
-                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
+                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
                                                cudaMemcpyDefault, b->stream);
   if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2D planes)" : "cudaMemcpy2DAsync(D2D rgb)")) return HC_ERR_CUDA;
   return batch_sync_checked(b, "cudaStreamSynchronize");
@@ -1330,7 +1359,7 @@ int hc_batch_read_rgb_async(hc_batch* b, int canvas, void* dst, size_t dst_strid
     return cuda_ok(cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream), "cudaMemcpyAsync(D2H planes)")
                ? HC_OK : HC_ERR_CUDA;
   }
-  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.ow * c.rgb_bpp, c.oh,
+  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
                                     cudaMemcpyDeviceToHost, b->stream);
   return cuda_ok(e, "cudaMemcpy2DAsync(D2H rgb)") ? HC_OK : HC_ERR_CUDA;
 }
@@ -1370,6 +1399,7 @@ int hc_batch_set_rgb_target(hc_batch* b, int canvas, void* device_dst, size_t st
   }
   Canvas& c = b->canvases[canvas];
   if (c.planar) { hc::set_last_error("hc_batch_set_rgb_target: the canvas is converted to HC_OUT_YCBCR"); return HC_ERR_UNSUPPORTED; }
+  if (device_dst && c.req_w) { hc::set_last_error("hc_batch_set_rgb_target: the canvas has an output size of its own"); return HC_ERR_UNSUPPORTED; }
   c.ext_rgb = (uint8_t*)device_dst;
   c.ext_stride = device_dst ? stride_bytes : 0;
   c.converted = false;

@@ -121,7 +121,16 @@ struct ImagePlan {
   uint16_t background[4] = {0, 0, 0, 0};
   std::vector<int> child_plans;                          // indices into hc_heic_job::children
   std::vector<std::pair<int32_t, int32_t>> child_offsets;
+  bool scaled = false;      // delivered smaller than its full-size output (engine option "scale_max_side")
 };
+
+// the fit rule of "scale_max_side" (include/heifcuda.h): the delivered size of a W x H image, S > 0
+void fit_within(int W, int H, int S, int* w, int* h) {
+  *w = W; *h = H;
+  if (std::max(W, H) <= S) return;
+  if (W >= H) { *w = S; *h = (int)std::max<int64_t>(1, (int64_t)H * S / W); }
+  else { *w = (int)std::max<int64_t>(1, (int64_t)W * S / H); *h = S; }
+}
 
 // bytes one delivered image takes: the packed planes of HC_OUT_YCBCR, else tight interleaved rows
 size_t image_bytes(const hc_image_desc& d) {
@@ -180,6 +189,9 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
   if (j->forced_format > HC_OUT_YCBCR) { hc::set_last_error("hc_heic_job_create: unknown output format"); return nullptr; }
   const bool planar = j->forced_format == HC_OUT_YCBCR;
   if (planar && band_end >= 0) { hc::set_last_error("banded decode: HC_OUT_YCBCR is not supported, bands are written as interleaved rows"); return nullptr; }
+  const int scale_max = hc_engine_get_option(e, "scale_max_side");
+  if (scale_max > 0 && planar) { hc::set_last_error("scale_max_side: HC_OUT_YCBCR images are not delivered scaled"); return nullptr; }
+  if (scale_max > 0 && band_end >= 0) { hc::set_last_error("scale_max_side: band jobs are not delivered scaled"); return nullptr; }
   j->want_alpha = j->forced_format >= 0 ? (j->forced_format == HC_OUT_RGBA || j->forced_format == HC_OUT_RRGGBBAA_BE || j->forced_format == HC_OUT_RRGGBBAA_LE)
                                         : want_alpha != 0;
   const auto t0 = std::chrono::steady_clock::now();
@@ -598,6 +610,17 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     im.desc.coded_pictures = 0;
     for (int ci : im.child_plans) im.desc.coded_pictures += j->children[ci].desc.coded_pictures;
   }
+  if (scale_max > 0) {
+    // overlay children stay full size: K7 samples the composed image
+    for (ImagePlan& im : j->images) {
+      int w, h;
+      fit_within(im.desc.width, im.desc.height, scale_max, &w, &h);
+      if (w == im.desc.width && h == im.desc.height) continue;
+      if (hc_batch_set_canvas_output_size(j->batch, im.canvas, w, h) != HC_OK) return nullptr;
+      im.desc.width = w; im.desc.height = h;
+      im.scaled = true;
+    }
+  }
   if (trace_on())
     fprintf(stderr, "[heifcuda] job_create: %d files, %zu items: containers %.2f ms, parse/prepare %.2f ms (%d threads), placement %.2f ms\n", nfiles,
             j->items.size(), (t_containers - std::chrono::duration<double>(t0.time_since_epoch()).count()) * 1e3, (t_parsed - t_containers) * 1e3, nthreads,
@@ -640,6 +663,7 @@ int hc_heic_job_set_rgb_target(hc_heic_job* j, int image, hc_shared_image* dst, 
   if (!j || image < 0 || image >= (int)j->images.size() || !dst || first_row < 0) { hc::set_last_error("hc_heic_job_set_rgb_target: bad argument"); return HC_ERR_ARGUMENT; }
   const ImagePlan& im = j->images[image];
   if (im.desc.out_format == HC_OUT_YCBCR) { hc::set_last_error("hc_heic_job_set_rgb_target: HC_OUT_YCBCR images are not written to shared images"); return HC_ERR_UNSUPPORTED; }
+  if (im.scaled) { hc::set_last_error("hc_heic_job_set_rgb_target: scaled images are not written to shared images"); return HC_ERR_UNSUPPORTED; }
   int w = 0, h = 0, bpp = 0;
   hc_shared_image_geometry(dst, &w, &h, &bpp);
   if (w != im.desc.width || bpp != im.desc.bytes_per_pixel || first_row + im.desc.height > h) {
@@ -683,6 +707,8 @@ int hc_heic_job_read_rgb(hc_heic_job* j, int image, void* dst, size_t stride) {
 
 int hc_heic_job_read_plane(hc_heic_job* j, int image, int plane, void* dst, size_t stride) {
   if (!j || image < 0 || image >= (int)j->images.size()) { hc::set_last_error("hc_heic_job_read_plane: bad argument"); return HC_ERR_ARGUMENT; }
+  // the planes are full size, the desc (which sizes the caller's destination) is the delivered size
+  if (j->images[image].scaled) { hc::set_last_error("hc_heic_job_read_plane: the image is delivered scaled"); return HC_ERR_UNSUPPORTED; }
   return hc_batch_read_plane(j->batch, j->images[image].canvas, plane, dst, stride);
 }
 
@@ -723,6 +749,11 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
   if (!e || nfiles <= 0 || !data || !sizes || files_per_batch <= 0) {
     hc::set_last_error("hc_heic_decode_stream: bad argument");
     return HC_ERR_ARGUMENT;
+  }
+  if ((want_alpha & 0x100) && (want_alpha & 0xff) == HC_OUT_YCBCR && hc_engine_get_option(e, "scale_max_side") > 0) {
+    // a property of the call, not of a file: error isolation would otherwise fail every file on its own
+    hc::set_last_error("scale_max_side: HC_OUT_YCBCR images are not delivered scaled");
+    return HC_ERR_UNSUPPORTED;
   }
   using clock = std::chrono::steady_clock;
   auto secs = [](clock::time_point a, clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };

@@ -19,13 +19,21 @@ HC_D int k7_clip_f(float fx, int maxi) {
   return x < 0 ? 0 : (x > maxi ? maxi : (int)x);
 }
 
+// SCALED: output pixel (x, y) of a band is the composition at canvas pixel (x * src_w / width, (row0 + y) * src_h / full_h)
+// (HeifPixelImage::scale_nearest_neighbor of the composed image, pixelimage.cc:1156-1253); otherwise at (x, y) itself.
+template <bool SCALED>
 __global__ void __launch_bounds__(256) k7_overlay_kernel(OverlayArgs a) {
   const int x = blockIdx.x * 32 + (threadIdx.x & 31), y = blockIdx.y * 8 + (threadIdx.x >> 5);
   if (x >= a.width || y >= a.height) return;
+  int sx = x, sy = y;
+  if (SCALED) {
+    sx = (int)((long long)x * a.src_w / a.width);
+    sy = (int)((long long)(a.row0 + y) * a.src_h / a.full_h);
+  }
   int R = a.bkg[0], G = a.bkg[1], B = a.bkg[2];
   for (int k = 0; k < a.n; k++) {
     const OverlayChild& c = a.child[k];
-    const int cx = x - c.dx, cy = y - c.dy;
+    const int cx = sx - c.dx, cy = sy - c.dy;
     if (cx < 0 || cy < 0 || cx >= c.w || cy >= c.h) continue;
     const int yv = c.y[(size_t)cy * c.y_stride + cx], cbv = c.cb[(size_t)cy * c.c_stride + cx], crv = c.cr[(size_t)cy * c.c_stride + cx];
     int r, g, b;
@@ -81,14 +89,22 @@ __global__ void __launch_bounds__(256) k7_overlay_kernel(OverlayArgs a) {
 
 void launch_k7(const OverlayArgs& a, cudaStream_t stream) {
   if (a.width <= 0 || a.height <= 0) return;
-  // gridDim.y is at most 65,535 blocks of 8 rows: a taller canvas is composed in bands of rows, each with its output rows
-  // and the children's offsets shifted up by the band's first row
+  // gridDim.y is at most 65,535 blocks of 8 rows: a taller image is composed in bands of delivered rows, each with its output
+  // rows and the children's offsets shifted up by the band's first row (scaled: the band's first row is passed instead)
+  const bool scaled = a.src_w != a.width || a.src_h != a.height;
   for (int r0 = 0; r0 < a.height; r0 += kMaxGridY * 8) {
     OverlayArgs b = a;
     b.height = std::min(a.height - r0, kMaxGridY * 8);
     b.out = a.out + r0 * a.out_stride;
-    for (int k = 0; k < a.n; k++) b.child[k].dy = a.child[k].dy - r0;
-    k7_overlay_kernel<<<dim3((unsigned)((a.width + 31) / 32), (unsigned)((b.height + 7) / 8)), 256, 0, stream>>>(b);
+    b.row0 = r0;
+    b.full_h = a.height;
+    const dim3 grid((unsigned)((a.width + 31) / 32), (unsigned)((b.height + 7) / 8));
+    if (scaled) {
+      k7_overlay_kernel<true><<<grid, 256, 0, stream>>>(b);
+    } else {
+      for (int k = 0; k < a.n; k++) b.child[k].dy = a.child[k].dy - r0;
+      k7_overlay_kernel<false><<<grid, 256, 0, stream>>>(b);
+    }
   }
 }
 

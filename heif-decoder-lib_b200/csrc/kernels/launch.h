@@ -12,11 +12,14 @@ constexpr int kMaxGridY = 65535;
 struct CscArgs {
   const uint8_t* y;  const uint8_t* cb;  const uint8_t* cr;  const uint8_t* a;   // plane bases (bytes)
   int y_stride, c_stride, a_stride;   // in samples
-  int width, height;
+  int width, height;                  // written (delivered) image
   int chroma_format;                  // 0..3
   uint8_t* out;
   long long out_stride;               // bytes
   hc_csc_params p;
+  // gather != 0: the planes are src_w x src_h and output pixel (x, y) is converted from source pixel
+  // (x * src_w / width, y * src_h / height), nearest neighbour like HeifPixelImage::scale_nearest_neighbor
+  int src_w, src_h, gather;
 };
 
 // up to CSC_BATCH_MAX canvases of one sample size converted by one launch (kernel parameter space: 4 KB)
@@ -47,11 +50,15 @@ struct OverlayChild {
 struct OverlayArgs {
   OverlayChild child[OVERLAY_MAX];
   int n;
-  int width, height;
+  int width, height;               // written (delivered) image
   int bkg[3];                      // background colour, already reduced to 8 bit
   int out_format;
   uint8_t* out;
   long long out_stride;
+  // canvas size; when it differs from width x height, output pixel (x, y) is the composition at canvas pixel
+  // (x * src_w / width, y * src_h / height)
+  int src_w, src_h;
+  int row0, full_h;                // set by launch_k7 for each band of a scaled image: its first row, all delivered rows
 };
 void launch_k7(const OverlayArgs& a, cudaStream_t stream);
 

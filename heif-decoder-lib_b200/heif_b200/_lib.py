@@ -125,6 +125,7 @@ SYMBOLS = [
     ("hc_batch_set_canvas_transform", _i, [_vp, _i, _i, _i, _i]),
     ("hc_batch_add_canvas_pass", _i, [_vp, _i, _i, _i, _i, _i, _i]),
     ("hc_batch_link_alpha", _i, [_vp, _i, _i]),
+    ("hc_batch_set_canvas_output_size", _i, [_vp, _i, _i, _i]),
     ("hc_batch_upload", _i, [_vp]),
     ("hc_batch_reconstruct", _i, [_vp, _i]),
     ("hc_batch_reconstruct_async", _i, [_vp, _i]),

@@ -190,7 +190,8 @@ class Engine:
         return Batch(self)
 
     def set_option(self, name, value):
-        """"device_parse": 1 = K0 parses the slice data on the GPU (default), 0 = host CABAC parser"""
+        """"device_parse": 1 = K0 parses the slice data on the GPU (default), 0 = host CABAC parser; "scale_max_side": S > 0
+        delivers HeicJob / decode_stream images whose longer side exceeds S scaled to fit S (include/heifcuda.h)"""
         check(self._L, self._L.hc_engine_set_option(self._h, name.encode(), int(value)), "set_option")
 
     def get_option(self, name):
@@ -211,6 +212,7 @@ class Batch:
         if not self._h:
             raise HeifCudaError("batch: " + (self._L.hc_last_error() or b"").decode())
         self._canvases = []
+        self._out_size = {}      # canvas -> delivered (width, height) set by set_output_size
         self._keep = []
 
     def add_canvas(self, width, height, chroma_format, bit_depth, with_alpha=False):
@@ -226,6 +228,12 @@ class Batch:
         """a picture whose slice data the GPU parses (K0)"""
         self._keep.append(k0pic)
         return check(self._L, self._L.hc_batch_add_k0_picture(self._h, k0pic._h, canvas, x, y, role, int(rescale_limited)), "add_k0_picture")
+
+    def set_output_size(self, canvas, width, height):
+        """hc_batch_set_canvas_output_size: deliver the canvas as width x height pixels sampled by nearest neighbour from its
+        full-size converted image (heif_image_scale_image); read_plane keeps returning the full-size planes"""
+        check(self._L, self._L.hc_batch_set_canvas_output_size(self._h, canvas, width, height), "set_output_size")
+        self._out_size[canvas] = (width, height)
 
     def upload(self):
         check(self._L, self._L.hc_batch_upload(self._h), "upload")
@@ -256,7 +264,7 @@ class Batch:
         return out
 
     def read_rgb(self, canvas, out_format):
-        w, h = self._canvases[canvas][:2]
+        w, h = self._out_size.get(canvas, self._canvases[canvas][:2])
         out = np.empty((h, w * OUT_BYTES_PER_PIXEL[out_format]), np.uint8)
         check(self._L, self._L.hc_batch_read_rgb(self._h, canvas, out.ctypes.data, out.strides[0]), "read_rgb")
         return out

@@ -244,7 +244,17 @@ void hc_engine_destroy(hc_engine* e);
  * images the file already marks premultiplied ('prem') are left alone, as that call refuses them.
  * "k0_max_critical_ctbs" (default 160): K0 is serial per substream, so hc_heic_job only hands it pictures whose parse
  * critical path is at most this many CTBs (WPP: CTB columns + 2 x (CTB rows - 1); no WPP: all CTBs of the picture);
- * the others stay with the host parser. */
+ * the others stay with the host parser.
+ * "scale_max_side" (default 0 = off; negative: HC_ERR_ARGUMENT): hc_heic_job / hc_heic_decode_stream deliver every image
+ * whose full-size output W x H (after irot / imir / clap and the alpha link: what hc_image_desc reported without the option)
+ * has max(W, H) > S as a smaller image that fits S: W >= H -> S x max(1, H * S / W), else max(1, W * S / H) x S (integer
+ * division). Images within S are delivered unchanged; the option never enlarges. This is the library's fit rule (no claim of
+ * parity with any thumbnailer). The pixels are those of heif_image_scale_image (nearest neighbour, see
+ * hc_batch_set_canvas_output_size) applied to the full-size output, which is never written: K5 / K7 convert only the
+ * sampled pixels. hc_image_desc then reports the delivered size, and the stream's buffers, external-destination check and
+ * stats follow it. Read when a job is created. Not available with HC_OUT_YCBCR (a job fails at creation,
+ * hc_heic_decode_stream(_ext) fails the call with HC_ERR_UNSUPPORTED) nor for band jobs (hc_heic_job_create_band fails);
+ * hc_heic_job_set_rgb_target and hc_heic_job_read_plane refuse a scaled image (HC_ERR_UNSUPPORTED). */
 int hc_engine_set_option(hc_engine* e, const char* name, int value);
 int hc_engine_get_option(const hc_engine* e, const char* name);
 
@@ -295,6 +305,14 @@ int hc_batch_add_canvas_pass(hc_batch* b, int canvas, int kind, int a0, int a1, 
  * iy = y * in_h / out_h) as HeifContext::decode_image_planar does for an alpha image whose size differs from the colour
  * image's (context.cc:2064-2071). Both canvases are taken after their own geometric passes. Call before hc_batch_upload. */
 int hc_batch_link_alpha(hc_batch* b, int canvas, int alpha_canvas);
+/* Delivered size of a canvas (any width, height >= 1, smaller or larger): pixel (x, y) of the delivered image is pixel
+ * (x * W / width, y * H / height) of the full-size interleaved image (W x H: the canvas after its passes; 64-bit products,
+ * integer division) — HeifPixelImage::scale_nearest_neighbor (pixelimage.cc:1156-1253), i.e. heif_image_scale_image on the
+ * converted image. Every per-pixel step of K5 / K7 runs at the source pixel as without it. Call before hc_batch_upload;
+ * overlay canvases included. hc_batch_convert(_many), hc_batch_read_rgb(_async) and hc_batch_copy_rgb_device then see the
+ * delivered size; hc_batch_read_plane(s) keep returning the full-size planes. HC_ERR_UNSUPPORTED for a canvas with an
+ * external RGB target; a scaled canvas cannot be converted to HC_OUT_YCBCR nor take an external target either. */
+int hc_batch_set_canvas_output_size(hc_batch* b, int canvas, int width, int height);
 /* 'iovl' derived image (libheif context.cc:2579-2675): an output canvas without planes of its own. K7 fills it with the
  * background colour (16-bit R, G, B, A as stored in the item; the reference keeps the high byte of R, G, B) and overlays
  * the child canvases in the order they are added at (dx, dy) — copied, or alpha-blended when the child canvas has an alpha
@@ -348,7 +366,7 @@ size_t hc_batch_upload_bytes(const hc_batch* b);
 typedef struct hc_heic_job hc_heic_job;
 
 typedef struct hc_image_desc {
-  int32_t width, height;     /* output size in pixels                                             */
+  int32_t width, height;     /* output size in pixels (the delivered size under "scale_max_side") */
   int32_t chroma_format;     /* of the decoded YCbCr image                                        */
   int32_t bit_depth;
   int32_t has_alpha;
