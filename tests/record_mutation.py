@@ -25,8 +25,10 @@ assert (COEFF.itemsize, TB.itemsize, BLK.itemsize, CTU.itemsize) == (4, 16, 16, 
 assert TB.fields["qp"][1] == 13 and BLK.fields["mode"][1] == 5 and CTU.fields["sao_type"][1] == 18
 assert CTU.fields["sao_offset"][1] == 24 and CTU.fields["beta_offset"][1] == 36 and CTU.fields["tc_offset"][1] == 37
 
-TB_CIDX, TB_BYPASS, TB_RDPCM = 0x03, 0x10, 0x60
-BLK_HAS_RESID, BLK_PCM = 0x02, 0x08
+TB_CIDX, TB_DST, TB_TSKIP, TB_BYPASS, TB_RDPCM_H, TB_RDPCM_V, TB_ROTATE = 0x03, 0x04, 0x08, 0x10, 0x20, 0x40, 0x80
+TB_RDPCM = TB_RDPCM_H | TB_RDPCM_V
+BLK_HAS_RESID, BLK_NO_EDGE_FLT, BLK_PCM = 0x02, 0x04, 0x08
+PIC_NO_INTRA_SMOOTH = 0x0002
 EDGE_V, EDGE_H = 0x01, 0x02
 PIC_HAS_DEBLOCK, PIC_HAS_SAO, PIC_SCALING_LIST = 0x0004, 0x0008, 0x0010
 # host/hevc_parse.cc kMode422: 4:2:2 chroma intra modes after the remapping of H.265 Table 8-3
@@ -34,7 +36,7 @@ MODE_422 = (0, 1, 2, 2, 2, 2, 3, 5, 7, 8, 10, 12, 13, 15, 17, 18, 19, 20, 21, 22
             29, 29, 30, 31)
 MODES_422 = np.array(sorted(set(MODE_422)), np.uint8)
 FLAT_MODES = np.array([0, 1, 10, 26], np.uint8)   # planar, DC, pure horizontal, pure vertical: all in the 4:2:2 image
-FAMILIES = ("levels", "modes", "flat", "filters", "all")
+FAMILIES = ("levels", "modes", "flat", "filters", "all", "rext")
 
 
 def views(rec):
@@ -174,6 +176,36 @@ def _edge_allowed(w4, h4):
     return (v | h).astype(np.uint8)
 
 
+def _rext(v, pic, rng):
+    """The range-extension residual and prediction tools: transform skip on blocks of every size (log2_max_transform_
+    skip_block_size up to 32), implicit RDPCM with the block's mode forced to 10 (horizontal) or 26 (vertical), rotation
+    of 4x4 transform-skipped and bypass blocks, intra_smoothing_disabled and disableIntraBoundaryFilter. Levels and qP'
+    of the transform-skipped blocks are pushed to their extremes, so that RDPCM accumulation leaves the int16 range."""
+    tbs, b = v["tbs"], v["blks"]
+    coded = ~_pcm_tbs(v)
+    tskip = coded & ((tbs["type"] & TB_BYPASS) == 0) & (rng.random(len(tbs)) < 0.5)
+    tbs["type"][tskip] = (tbs["type"][tskip] & np.uint8(0xff ^ TB_DST)) | TB_TSKIP
+    _levels(v, pic, rng, tskip & (rng.random(len(tbs)) < 0.5))
+    ts_or_bypass = coded & ((tbs["type"] & (TB_TSKIP | TB_BYPASS)) != 0)
+    tbs["type"][ts_or_bypass] &= np.uint8(0xff ^ (TB_RDPCM | TB_ROTATE))
+    rot = ts_or_bypass & (tbs["log2"] == 2) & (rng.random(len(tbs)) < 0.5)
+    tbs["type"][rot] |= TB_ROTATE
+    # RDPCM: the block that adds the residual takes mode 10 or 26
+    blk_of = {int(o): i for i, o in enumerate(b["resid_off"]) if b["flags"][i] & BLK_HAS_RESID and not b["flags"][i] & BLK_PCM}
+    for t in np.flatnonzero(ts_or_bypass & (rng.random(len(tbs)) < 0.6)):
+        i = blk_of.get(int(tbs["resid_off"][t]))
+        if i is None:
+            continue
+        vertical = rng.random() < 0.5
+        b["mode"][i] = 26 if vertical else 10
+        tbs["type"][t] |= TB_RDPCM_V if vertical else TB_RDPCM_H
+    nopcm = (b["flags"] & BLK_PCM) == 0
+    edge = nopcm & (rng.random(len(b)) < 0.3)
+    b["flags"][edge] ^= BLK_NO_EDGE_FLT
+    if rng.random() < 0.5:
+        pic.flags = pic.flags ^ PIC_NO_INTRA_SMOOTH
+
+
 def _update_pic_flags(v, pic):
     ncomp = 3 if pic.chroma_format else 1
     flags = pic.flags & ~(PIC_HAS_DEBLOCK | PIC_HAS_SAO)
@@ -200,12 +232,14 @@ def mutate(rec, family, seed):
         _flat(v, pic, rng, np.ones(ntb, bool), np.ones(nblk, bool))
     elif family == "filters":
         _filters(v, pic, rng)
-    else:   # every family at once: each block and transform block is either extreme or flat
+    elif family == "all":   # every family at once: each block and transform block is either extreme or flat
         flat_tb, flat_blk = rng.random(ntb) < 0.3, rng.random(nblk) < 0.3
         _levels(v, pic, rng, ~flat_tb)
         _modes(v, pic, rng, ~flat_blk)
         _flat(v, pic, rng, flat_tb, flat_blk)
         _filters(v, pic, rng)
+    else:
+        _rext(v, pic, rng)
     _update_pic_flags(v, pic)
 
 
@@ -225,6 +259,18 @@ def check_legal(rec):
     lv = v["coeffs"]["level"][in_pcm].astype(np.int64)
     assert np.all((lv >= 0) & (lv < (1 << bd_of[owner[in_pcm]]))), "PCM sample outside the sample range"
     assert np.all(blks["mode"] <= 34), "intra mode above 34"
+    t = tbs["type"]
+    assert not np.any((t & TB_TSKIP) & ((t & (TB_BYPASS | TB_DST)) != 0)), "transform skip with bypass or DST"
+    skipped = (t & (TB_TSKIP | TB_BYPASS)) != 0
+    assert np.all(skipped | ((t & (TB_RDPCM | TB_ROTATE)) == 0)), "RDPCM / rotation on a transformed block"
+    assert np.all(((t & TB_ROTATE) == 0) | (tbs["log2"] == 2)), "rotation of a block larger than 4x4"
+    assert not np.any(((t & TB_RDPCM_H) != 0) & ((t & TB_RDPCM_V) != 0)), "RDPCM in both directions"
+    rdpcm = (t & TB_RDPCM) != 0
+    if rdpcm.any():   # implicit RDPCM: mode 10 accumulates horizontally, 26 vertically (8.6.2)
+        mode_of = dict(zip(blks["resid_off"][(blks["flags"] & BLK_HAS_RESID) != 0].tolist(),
+                           blks["mode"][(blks["flags"] & BLK_HAS_RESID) != 0].tolist()))
+        for typ, off in zip(t[rdpcm].tolist(), tbs["resid_off"][rdpcm].tolist()):
+            assert mode_of[off] == (26 if typ & TB_RDPCM_V else 10), "RDPCM direction and intra mode disagree"
     if pic.chroma_format == 2:
         assert np.all(np.isin(blks["mode"][blks["cidx"] != 0], MODES_422)), "4:2:2 chroma mode outside the image of Table 8-3"
     if (pic.flags & PIC_SCALING_LIST) and len(v["scaling"]):

@@ -34,9 +34,6 @@ STAGES = (0, hb.STAGE_DEBLOCK, hb.STAGE_ALL)
 UNREACHABLE = {
     # |second-pass sum| <= 32768 * 242 (largest column sum of |DST|), shifted right by 20 - bitDepth >= 8: below 2^15
     "k1_dst_pass2_clip": "the DST second pass cannot leave int16 at bit depths up to 12",
-    # transform skip is 4x4 in every fixture: |level << 7| >> (20 - bitDepth) <= 2^14 at 12 bit
-    "k1_tskip_clip": "a 4x4 transform-skip residual cannot leave int16 at bit depths up to 12",
-    "k1_rdpcm_clip": "no fixture uses RDPCM (range-extension implicit or explicit RDPCM)",
 }
 
 # one picture per (chroma format, bit depth) the fixtures have, for K5

@@ -12,13 +12,16 @@
 // pictures look like the source and every syntax path the decoder supports can be switched on:
 // chroma 4:0:0/4:2:0/4:2:2/4:4:4, 8-12 bit, CTB 16-64, TU 4-32 with RQT, NxN, SAO, deblocking
 // offsets, cu_qp_delta, sign data hiding, transform skip, WPP, tiles, (dependent) slices, PCM,
-// transquant bypass, scaling lists, strong intra smoothing, VUI. A stress mode (hevc_enc_params::stress) pushes levels,
+// transquant bypass, scaling lists, strong intra smoothing, VUI, the SPS / PPS range extensions (transform skip up
+// to 32x32, implicit RDPCM, rotation, transform-skip contexts, intra smoothing disabled, persistent Rice adaptation,
+// CU chroma QP offset lists, SAO offset scale). A stress mode (hevc_enc_params::stress) pushes levels,
 // intra modes, QPs and SAO parameters to the limits of their legal ranges for the parser tests, and counts what it wrote.
 // Reconstruction inside the loop calls the CPU oracle's block functions (oracle/hevc_recon_oracle.c)
 // so that encoder-side and decoder-side arithmetic cannot drift apart.
 //
 // Written from ITU-T H.265 §7.3 (syntax), §9.3 (CABAC encoding, §9.3.4.5 flush).
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
@@ -62,6 +65,15 @@ typedef struct hevc_enc_params {
   int32_t cb_qp_offset, cr_qp_offset;
   int32_t loop_filter_across_slices, loop_filter_across_tiles;
   int32_t stress;            // HEVC_ENC_STRESS_* bit mask; 0: ordinary content
+  // range extensions (SPS / PPS range extension syntax); all 0: no extension is written
+  int32_t transform_skip_rotation, transform_skip_context, implicit_rdpcm, intra_smoothing_disabled;
+  int32_t persistent_rice_adaptation;
+  int32_t extended_precision, cabac_bypass_alignment;  // flags only: the slice data ignores them (refused streams)
+  int32_t log2_max_transform_skip_minus2;               // 0..3
+  int32_t cross_component_prediction;                   // flag only (refused streams)
+  int32_t chroma_qp_offset_list_len;                    // 0 off, else 1..6 entries with offsets drawn in -12..12
+  int32_t diff_cu_chroma_qp_offset_depth;
+  int32_t log2_sao_offset_scale_luma, log2_sao_offset_scale_chroma;
   uint32_t seed;
 } hevc_enc_params;
 }
@@ -77,6 +89,8 @@ enum {
 };
 
 // Counters of what the encoder wrote (hevc_enc_encode_ex). X(name, n): n > 1 is an array, named name_0 .. name_<n-1>.
+// Two groups: the syntax extremes of the stress mode, then the range-extension tools (from hevc_enc_rext_stat_first()
+// on), which only streams with those tools switched on reach.
 #define HEVC_ENC_STATS(X)                                                                                               \
   X(level_min, 1) X(level_max, 1) X(escape_long, 1) X(escape_prefix16, 1) X(rice4, 1)                                  \
   X(sb_16_sig, 1) X(sb_beyond_8, 1) X(sign_hidden_even, 1) X(sign_hidden_odd, 1) X(sign_string_16, 1)                   \
@@ -88,9 +102,19 @@ enum {
   X(mode422, 35)                                                                                                        \
   X(sao_offset_cmax_hbd, 1) X(sao_band_ge29, 1) X(sao_eo_class, 4) X(sao_merge_left, 1) X(sao_merge_up, 1)
 
+#define HEVC_ENC_REXT_STATS(X)                                                                                          \
+  X(rdpcm_h_tskip, 1) X(rdpcm_v_tskip, 1) X(rdpcm_h_bypass, 1) X(rdpcm_v_bypass, 1)                                     \
+  X(rotate_tskip, 1) X(rotate_bypass, 1) X(tskip_log2, 4) X(sig_ctx_42, 1) X(sig_ctx_43, 1) X(sdh_off_rdpcm, 1)          \
+  X(rice_init_gt0, 1) X(rice_gt4, 1) X(wpp_stat_coeff_restored, 1)                                                      \
+  X(cu_chroma_qp_offset_off, 1) X(cu_chroma_qp_offset_idx, 6)                                                            \
+  X(sao_offset_scaled_cmax, 1) X(no_edge_flt, 1) X(smoothing_skipped, 1) X(smoothing_skipped_strong, 1)
+
 enum {
 #define HEVC_ENC_STAT_ENUM(name, n) ST_##name, ST_##name##_end_ = ST_##name + (n) - 1,
   HEVC_ENC_STATS(HEVC_ENC_STAT_ENUM)
+  ST_REXT_FIRST_,
+  ST_REXT_BEFORE_ = ST_REXT_FIRST_ - 1,
+  HEVC_ENC_REXT_STATS(HEVC_ENC_STAT_ENUM)
 #undef HEVC_ENC_STAT_ENUM
   ST_COUNT
 };
@@ -283,6 +307,8 @@ const int kDst[4][4] = {{29, 55, 74, 84}, {74, 74, 0, -74}, {84, -29, -74, 55}, 
 struct TuData {
   bool coded = false;
   bool tskip = false;
+  int rdpcm = 0;                // implicit RDPCM: 0 none, 1 horizontal, 2 vertical
+  bool rotate = false;
   std::vector<int16_t> levels;  // nT*nT, raster
 };
 
@@ -328,6 +354,10 @@ struct Enc {
   CtxSet ctx;
   std::vector<CtxSet> wpp_ctx;
   CtxSet dep_ctx;
+  // StatCoeff (9.3.2.2 persistent Rice adaptation), stored and synchronised together with the context variables
+  uint8_t stat_coeff[4] = {0, 0, 0, 0};
+  std::vector<std::array<uint8_t, 4>> wpp_stat;
+  std::array<uint8_t, 4> dep_stat = {{0, 0, 0, 0}};
   std::vector<uint8_t> slice_data;
   std::vector<uint32_t> entry_points;
   size_t substream_start = 0;
@@ -342,6 +372,15 @@ struct Enc {
   bool cu_bypass = false;
   int cu_x0 = 0, cu_y0 = 0, cu_log2 = 0;
   int log2_min_cu_qp_delta = 6;
+  // cu_chroma_qp_offset: the decision of a chroma quantisation group is drawn when the group starts, takes effect at its
+  // first TU with a coded chroma block (pass A) and is written there (pass B, in the same order)
+  int log2_min_cu_chroma_qp_offset = 6, max_tskip_log2 = 2;
+  int cqo_cb[6] = {}, cqo_cr[6] = {};
+  bool cqo_coded_a = false, cqo_coded_b = false;
+  int cqo_next = 0;                 // drawn for the current group: 0 flag off, k > 0 list entry k - 1
+  int cqo_cur_cb = 0, cqo_cur_cr = 0;
+  std::vector<int> cqo_queue;
+  size_t cqo_read = 0;
   struct Sao { uint8_t type[3], boc[3]; int8_t off[3][4]; };
   std::vector<Sao> sao;
   uint64_t stats[ST_COUNT] = {};
@@ -371,7 +410,15 @@ struct Enc {
   void write_parameter_sets(std::vector<uint8_t>& out);
   void write_scaling_list_data(BitWriter& bw);
   void encode_picture(std::vector<uint8_t>& out);
-  void init_contexts() { ctx_init_all(ctx, slice_qp); }
+  void init_contexts() { ctx_init_all(ctx, slice_qp); memset(stat_coeff, 0, sizeof(stat_coeff)); }
+  bool rext_sps() const {
+    return P.transform_skip_rotation || P.transform_skip_context || P.implicit_rdpcm || P.intra_smoothing_disabled ||
+           P.persistent_rice_adaptation || P.extended_precision || P.cabac_bypass_alignment;
+  }
+  bool rext_pps() const {
+    return P.log2_max_transform_skip_minus2 || P.cross_component_prediction || P.chroma_qp_offset_list_len ||
+           P.log2_sao_offset_scale_luma || P.log2_sao_offset_scale_chroma;
+  }
   void encode_ctu();
   void code_sao(int rx, int ry);
   void coding_quadtree(int x0, int y0, int log2, int depth);
@@ -387,7 +434,8 @@ struct Enc {
   void residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode);
   void derive_qp_pred(int xCU, int yCU, int& pred);
   void set_cu_qp(int qpy);
-  int chroma_qp(int qpy, int c) const;
+  int chroma_qp(int qpy, int c, int cu_off) const;
+  int cu_chroma_offset(int c) const;
   int mode_for(const int* modes, int x, int y) const;
 };
 
@@ -438,6 +486,11 @@ void Enc::setup() {
   pic.width = W; pic.height = H; pic.chroma_format = (uint8_t)cf; pic.bit_depth_y = pic.bit_depth_c = (uint8_t)bd;
   pic.log2_ctb = (uint8_t)log2_ctb; pic.ctbs_w = (uint16_t)ctbs_w; pic.ctbs_h = (uint16_t)ctbs_h;
   if (P.strong_intra) pic.flags |= HC_PIC_STRONG_INTRA;
+  if (P.intra_smoothing_disabled) pic.flags |= HC_PIC_NO_INTRA_SMOOTH;
+  wpp_stat.assign(ctbs_h, std::array<uint8_t, 4>{{0, 0, 0, 0}});
+  max_tskip_log2 = P.transform_skip ? 2 + P.log2_max_transform_skip_minus2 : 2;
+  log2_min_cu_chroma_qp_offset = log2_ctb - P.diff_cu_chroma_qp_offset_depth;
+  for (int i = 0; i < P.chroma_qp_offset_list_len; i++) { cqo_cb[i] = rng.below(25) - 12; cqo_cr[i] = rng.below(25) - 12; }
   log2_min_cu_qp_delta = P.cu_qp_delta ? log2_ctb - std::min(P.cu_qp_delta - 1, log2_ctb - 3) : log2_ctb;
 
   // scaling lists
@@ -516,7 +569,7 @@ void Enc::write_scaling_list_data(BitWriter& bw) {
 }
 
 void Enc::write_parameter_sets(std::vector<uint8_t>& out) {
-  int profile = (cf == 1 && bd == 8) ? 1 : (cf == 1 && bd <= 10) ? 2 : 4;
+  int profile = rext_sps() || rext_pps() ? 4 : (cf == 1 && bd == 8) ? 1 : (cf == 1 && bd <= 10) ? 2 : 4;
   {  // VPS
     BitWriter bw;
     bw.put(0, 4); bw.put(1, 1); bw.put(1, 1); bw.put(0, 6); bw.put(0, 3); bw.put(1, 1); bw.put(0xffff, 16);
@@ -566,7 +619,19 @@ void Enc::write_parameter_sets(std::vector<uint8_t>& out) {
       bw.put((uint32_t)P.primaries, 8); bw.put((uint32_t)P.transfer, 8); bw.put((uint32_t)P.matrix, 8);
       bw.put(0, 1); bw.put(0, 3); bw.put(0, 1); bw.put(0, 1); bw.put(0, 1);
     }
-    bw.put(0, 1);                    // sps_extension_present
+    bw.put(rext_sps(), 1);           // sps_extension_present
+    if (rext_sps()) {
+      bw.put(1, 1); bw.put(0, 7);    // sps_range_extension_flag, no multilayer / 3d / scc / 4 bits
+      bw.put(P.transform_skip_rotation ? 1 : 0, 1);
+      bw.put(P.transform_skip_context ? 1 : 0, 1);
+      bw.put(P.implicit_rdpcm ? 1 : 0, 1);
+      bw.put(0, 1);                  // explicit_rdpcm (inter only)
+      bw.put(P.extended_precision ? 1 : 0, 1);
+      bw.put(P.intra_smoothing_disabled ? 1 : 0, 1);
+      bw.put(0, 1);                  // high_precision_offsets (inter only)
+      bw.put(P.persistent_rice_adaptation ? 1 : 0, 1);
+      bw.put(P.cabac_bypass_alignment ? 1 : 0, 1);
+    }
     bw.trailing();
     append_nal(out, 33, bw.bytes);
   }
@@ -607,7 +672,20 @@ void Enc::write_parameter_sets(std::vector<uint8_t>& out) {
     bw.put(0, 1);
     bw.ue(0);
     bw.put(0, 1);
-    bw.put(0, 1);
+    bw.put(rext_pps(), 1);           // pps_extension_present
+    if (rext_pps()) {
+      bw.put(1, 1); bw.put(0, 7);    // pps_range_extension_flag, no multilayer / 3d / scc / 4 bits
+      if (P.transform_skip) bw.ue((uint32_t)P.log2_max_transform_skip_minus2);
+      bw.put(P.cross_component_prediction ? 1 : 0, 1);
+      bw.put(P.chroma_qp_offset_list_len ? 1 : 0, 1);
+      if (P.chroma_qp_offset_list_len) {
+        bw.ue((uint32_t)P.diff_cu_chroma_qp_offset_depth);
+        bw.ue((uint32_t)(P.chroma_qp_offset_list_len - 1));
+        for (int i = 0; i < P.chroma_qp_offset_list_len; i++) { bw.se(cqo_cb[i]); bw.se(cqo_cr[i]); }
+      }
+      bw.ue((uint32_t)P.log2_sao_offset_scale_luma);
+      bw.ue((uint32_t)P.log2_sao_offset_scale_chroma);
+    }
     bw.trailing();
     append_nal(out, 34, bw.bytes);
   }
@@ -680,11 +758,20 @@ int Enc::choose_mode(int x0, int y0, int log2) {
   return best;
 }
 
-int Enc::chroma_qp(int qpy, int c) const {
-  int off = c == 1 ? P.cb_qp_offset : P.cr_qp_offset;
+int Enc::chroma_qp(int qpy, int c, int cu_off) const {
+  int off = (c == 1 ? P.cb_qp_offset : P.cr_qp_offset) + cu_off;
   int qPi = clip3(-qp_bd_offset, 57, qpy + off);
   int q = cf == 1 ? qpc_table_420(qPi) : qPi;
   return std::max(0, q + qp_bd_offset);
+}
+
+// CuQpOffsetCb / Cr a coded chroma block of the current TU is quantised with: the group's decision once it took effect,
+// else the one drawn for the group (a TU with a coded chroma block is where it takes effect)
+int Enc::cu_chroma_offset(int c) const {
+  if (!P.chroma_qp_offset_list_len) return 0;
+  if (cqo_coded_a) return c == 1 ? cqo_cur_cb : cqo_cur_cr;
+  if (!cqo_next) return 0;
+  return c == 1 ? cqo_cb[cqo_next - 1] : cqo_cr[cqo_next - 1];
 }
 
 // forward transform + quantisation of one block, then the decoder-exact reconstruction
@@ -693,27 +780,60 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
   uint16_t* plane = rec[cIdx].data();
   const int stride = pw[cIdx];
   uint16_t pred[32 * 32];
-  bool no_edge = false;
+  // disableIntraBoundaryFilter as the decoder derives it: the bypass flag at the block's component coordinates
+  const bool no_edge = P.implicit_rdpcm &&
+                       (cu_flags[(std::min(xB, W - 1) >> 3) + (size_t)(std::min(yB, H - 1) >> 3) * w8] & 2);
+  if (no_edge && cIdx == 0 && (mode == 10 || mode == 26) && nT < 32) stats[ST_no_edge_flt]++;
+  if (P.intra_smoothing_disabled && (cIdx == 0 || cf == 3) && mode != 1 && nT != 4) {
+    const int minDist = std::min(std::abs(mode - 26), std::abs(mode - 10));
+    if (nT == 8 ? minDist > 7 : nT == 16 ? minDist > 1 : minDist > 0) {
+      stats[ST_smoothing_skipped]++;
+      if (cIdx == 0 && nT == 32 && P.strong_intra) stats[ST_smoothing_skipped_strong]++;
+    }
+  }
   hc_blk blk = make_blk(cIdx, xB, yB, log2, mode, no_edge);
   hc_oracle_predict_block(&pic, &blk, plane, stride, pred);
   int res[32 * 32];
   for (int y = 0; y < nT; y++)
     for (int x = 0; x < nT; x++) res[x + y * nT] = (int)orig[cIdx][(xB + x) + (size_t)(yB + y) * stride] - (int)pred[x + y * nT];
 
-  const int qpP = cIdx == 0 ? cur_qp_y + qp_bd_offset : chroma_qp(cur_qp_y, cIdx);
+  const int cu_off = cIdx ? cu_chroma_offset(cIdx) : 0;
+  const int qpP = cIdx == 0 ? cur_qp_y + qp_bd_offset : chroma_qp(cur_qp_y, cIdx, cu_off);
   tu.levels.assign((size_t)nT * nT, 0);
   tu.tskip = false;
   tu.coded = false;
+  tu.rdpcm = 0;
+  tu.rotate = false;
+  // implicit RDPCM (8.6.2: intra, transform-skipped or bypass, mode 10 or 26) codes the differences along the
+  // accumulation direction; rotation (nTbS = 4) codes the block turned by 180 degrees, i.e. in reversed raster order
+  const int rdpcm = P.implicit_rdpcm && (mode == 10 || mode == 26) ? (mode == 26 ? 2 : 1) : 0;
+  auto differences = [&](const int* r, int* d) {
+    for (int y = 0; y < nT; y++)
+      for (int x = 0; x < nT; x++) {
+        const int i = x + y * nT;
+        d[i] = r[i] - (rdpcm == 1 && x ? r[i - 1] : rdpcm == 2 && y ? r[i - nT] : 0);
+      }
+  };
+  const bool rotate = P.transform_skip_rotation && log2 == 2;
   if (cu_bypass) {
+    int d[32 * 32];
+    differences(res, d);
     bool any = false;
-    for (int i = 0; i < nT * nT; i++) { tu.levels[i] = (int16_t)res[i]; any |= res[i] != 0; }
+    for (int i = 0; i < nT * nT; i++) { tu.levels[i] = (int16_t)d[rotate ? nT * nT - 1 - i : i]; any |= res[i] != 0; }
     tu.coded = any;
+    tu.rdpcm = rdpcm;
+    tu.rotate = rotate;
   } else {
-    bool tskip = P.transform_skip && log2 == 2 && rng.chance(25);
+    bool tskip = P.transform_skip && log2 <= max_tskip_log2 && rng.chance(25);
     long long coef[32 * 32];
     const int tshift = 15 - bd - log2;
     if (tskip) {
-      for (int i = 0; i < nT * nT; i++) coef[i] = tshift >= 0 ? ((long long)res[i] << tshift) : ((long long)res[i] >> -tshift);
+      int d[32 * 32];
+      differences(res, d);
+      for (int i = 0; i < nT * nT; i++) {
+        const int v = d[rotate ? nT * nT - 1 - i : i];
+        coef[i] = tshift >= 0 ? ((long long)v << tshift) : ((long long)v >> -tshift);
+      }
     } else {
       const bool dst = log2 == 2 && cIdx == 0;
       const int fact = 1 << (5 - log2);
@@ -753,6 +873,7 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
     }
     tu.coded = any;
     tu.tskip = tskip && any;
+    if (tskip) { tu.rdpcm = rdpcm; tu.rotate = rotate; }
     if (stress(HEVC_ENC_STRESS_LEVELS)) {
       // 0: keep the quantised levels, 1 / 2: sparse, 3: dense; values from the ends of TransCoeffLevel's range
       const int kind = stress(HEVC_ENC_STRESS_DENSE) ? 3 : rng.below(4);
@@ -774,8 +895,9 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
       }
     }
   }
+  if (!tu.tskip && !cu_bypass) { tu.rdpcm = 0; tu.rotate = false; }
   if (tu.coded && cIdx && !cu_bypass) {
-    const int qPi = cur_qp_y + (cIdx == 1 ? P.cb_qp_offset : P.cr_qp_offset);
+    const int qPi = cur_qp_y + (cIdx == 1 ? P.cb_qp_offset : P.cr_qp_offset) + cu_off;
     if (qPi < -qp_bd_offset) stats[ST_chroma_qpi_clip_lo]++;
     if (qPi > 57) stats[ST_chroma_qpi_clip_hi]++;
   }
@@ -786,7 +908,7 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
     if (mode >= 6 && mode <= 14) scanIdx = 2;
     else if (mode >= 22 && mode <= 30) scanIdx = 1;
   }
-  if (tu.coded && P.sign_hiding && !cu_bypass) {
+  if (tu.coded && P.sign_hiding && !cu_bypass && !(tu.tskip && tu.rdpcm)) {
     const ScanTables& st = scan_tables();
     const ScanPos* sp = st.order[2][scanIdx];
     for (int sy = 0; sy < nT / 4; sy++)
@@ -823,6 +945,8 @@ void Enc::process_tb(int cIdx, int xB, int yB, int log2, int mode, TuData& tu) {
     if (cu_bypass) type |= HC_TB_BYPASS;
     else if (tu.tskip) type |= HC_TB_TSKIP;
     else if (log2 == 2 && cIdx == 0) type |= HC_TB_DST;
+    if (tu.rdpcm) type |= tu.rdpcm == 2 ? HC_TB_RDPCM_V : HC_TB_RDPCM_H;
+    if (tu.rotate) type |= HC_TB_ROTATE;
     tb.type = type;
     int32_t r[32 * 32];
     hc_oracle_residual_block(&pic, &tb, co.data(), scaling.empty() ? nullptr : scaling.data(), r);
@@ -897,6 +1021,16 @@ void Enc::build_tree(Node& n, int max_depth, int intra_split, const int* luma_mo
   int modeC = mode_for(chroma_modes, n.nchroma && log2 == 2 && cf != 3 ? n.xBase : n.x0, n.nchroma && log2 == 2 && cf != 3 ? n.yBase : n.y0);
   for (int c = 1; c <= 2; c++)
     for (int t = 0; t < n.nchroma; t++) process_tb(c, n.cxB, n.cyB + t * (1 << n.log2C), n.log2C, modeC, n.chroma[c - 1][t]);
+  if (P.chroma_qp_offset_list_len && !cu_bypass && !cqo_coded_a) {
+    bool any = false;
+    for (int c = 0; c < 2; c++) for (int t = 0; t < n.nchroma; t++) any |= n.chroma[c][t].coded;
+    if (any) {
+      cqo_cur_cb = cu_chroma_offset(1);
+      cqo_cur_cr = cu_chroma_offset(2);
+      cqo_coded_a = true;
+      cqo_queue.push_back(cqo_next);
+    }
+  }
   if (log2 > 2 || cf == 3) {
     n.cbf_cb = n.cbf_cr = 0;
     for (int t = 0; t < n.nchroma; t++) {
@@ -941,8 +1075,12 @@ void Enc::set_cu_qp(int qpy) {
 void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
   const ScanTables& st = scan_tables();
   const int nT = 1 << log2;
-  if (P.transform_skip && !cu_bypass && log2 <= 2) bin(CTX_TSKIP + (cIdx ? 1 : 0), tu.tskip ? 1 : 0);
-  if (tu.tskip) stats[ST_tskip_coded]++;
+  if (P.transform_skip && !cu_bypass && log2 <= max_tskip_log2) bin(CTX_TSKIP + (cIdx ? 1 : 0), tu.tskip ? 1 : 0);
+  if (tu.tskip) { stats[ST_tskip_coded]++; stats[ST_tskip_log2 + log2 - 2]++; }
+  if (tu.rdpcm) stats[cu_bypass ? (tu.rdpcm == 1 ? ST_rdpcm_h_bypass : ST_rdpcm_v_bypass) : (tu.rdpcm == 1 ? ST_rdpcm_h_tskip : ST_rdpcm_v_tskip)]++;
+  if (tu.rotate) stats[cu_bypass ? ST_rotate_bypass : ST_rotate_tskip]++;
+  const bool ts_ctx = P.transform_skip_context && (cu_bypass || tu.tskip);   // sig_coeff_flag contexts 42 / 43 (9.3.4.2.5)
+  const int sbType = (cIdx == 0 ? 2 : 0) + (cu_bypass || tu.tskip ? 1 : 0);
   ctb_ntb++;
   for (int i = 0; i < nT * nT; i++) {
     ctb_ncoeff += tu.levels[i] != 0;
@@ -994,7 +1132,7 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
 
   uint8_t csbf_nb[64];
   memset(csbf_nb, 0, sizeof(csbf_nb));
-  const bool sign_hiding_possible = P.sign_hiding && !cu_bypass;
+  const bool sign_hiding_possible = P.sign_hiding && !cu_bypass && !(tu.tskip && tu.rdpcm);
   int c1 = 1;
   for (int i = lastSub; i >= 0; i--) {
     const int Sx = scanSub[i].x, Sy = scanSub[i].y, xS0 = Sx << 2, yS0 = Sy << 2;
@@ -1016,6 +1154,7 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
     if (!coded) continue;
     const int prevCsbf = csbf_nb[Sx + Sy * sbW];
     auto sig_ctx = [&](int xC, int yC) -> int {
+      if (ts_ctx) { stats[cIdx ? ST_sig_ctx_43 : ST_sig_ctx_42]++; return cIdx ? 43 : 42; }
       int sigCtx;
       if (log2 == 2) sigCtx = kSigCtx4x4[(yC << 2) + xC];
       else if (xC + yC == 0) sigCtx = 0;
@@ -1073,13 +1212,18 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
       if (g2) base[firstG1] = 3;
     }
     bool signHidden = sign_hiding_possible && (spos[0] - spos[n - 1] > 3);
+    if (P.sign_hiding && tu.tskip && tu.rdpcm && spos[0] - spos[n - 1] > 3) stats[ST_sdh_off_rdpcm]++;
     int nsign = signHidden ? n - 1 : n;
     if (n == 16) stats[ST_sb_16_sig]++;
     if (n > 8) stats[ST_sb_beyond_8]++;
     if (signHidden) stats[value[n - 1] < 0 ? ST_sign_hidden_odd : ST_sign_hidden_even]++;
     if (nsign == 16) stats[ST_sign_string_16]++;
     for (int c = 0; c < nsign; c++) cabac.bypass(value[c] < 0);
-    int rice = 0;
+    // persistent Rice adaptation (9.3.3.11): the sub-block starts at StatCoeff / 4, which its first
+    // coeff_abs_level_remaining updates; the parameter then rises without the cap at 4
+    int rice = P.persistent_rice_adaptation ? stat_coeff[sbType] / 4 : 0;
+    if (rice > 0) stats[ST_rice_init_gt0]++;
+    bool first_remaining = true;
     for (int c = 0; c < n; c++) {
       const int a = std::abs(value[c]);
       // which coefficients carry coeff_abs_level_remaining (mirror of the decoder's base levels):
@@ -1112,7 +1256,14 @@ void Enc::residual_coding(const TuData& tu, int log2, int cIdx, int pred_mode) {
         cabac.bypass(0);
         cabac.bypass_bits((uint32_t)code, length);
       }
-      if (baseLevel + rem > 3 * (1 << rice)) rice = std::min(rice + 1, 4);
+      if (P.persistent_rice_adaptation && first_remaining) {
+        uint8_t& sc = stat_coeff[sbType];
+        if (rem >= (3 << (sc / 4))) sc++;
+        else if (2 * rem < (1 << (sc / 4)) && sc > 0) sc--;
+      }
+      first_remaining = false;
+      if (baseLevel + rem > 3 * (1 << rice)) rice = P.persistent_rice_adaptation ? rice + 1 : std::min(rice + 1, 4);
+      if (rice > 4) stats[ST_rice_gt4]++;
     }
   }
 }
@@ -1157,6 +1308,18 @@ void Enc::write_tu(Node& n, const int* luma_modes, const int* chroma_modes) {
       CuQpDeltaVal = delta;
       set_cu_qp(qg_target_qp);
     }
+    if (P.chroma_qp_offset_list_len && cbfChroma && !cu_bypass && !cqo_coded_b) {
+      // cu_chroma_qp_offset_flag, cu_chroma_qp_offset_idx: TR with cMax = chroma_qp_offset_list_len_minus1, one context
+      const int k = cqo_queue.at(cqo_read++);
+      bin(CTX_CHROMA_QP_OFFSET_FLAG, k > 0);
+      if (k > 0 && P.chroma_qp_offset_list_len > 1) {
+        const int idx = k - 1, cmax = P.chroma_qp_offset_list_len - 1;
+        for (int i = 0; i < idx; i++) bin(CTX_CHROMA_QP_OFFSET_IDX, 1);
+        if (idx < cmax) bin(CTX_CHROMA_QP_OFFSET_IDX, 0);
+      }
+      stats[k > 0 ? ST_cu_chroma_qp_offset_idx + k - 1 : ST_cu_chroma_qp_offset_off]++;
+      cqo_coded_b = true;
+    }
   }
   int modeY = mode_for(luma_modes, n.x0, n.y0);
   if (n.cbf_luma) residual_coding(n.luma, log2, 0, modeY);
@@ -1200,6 +1363,8 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
   const int nCbS = 1 << log2;
   cu_x0 = x0; cu_y0 = y0; cu_log2 = log2;
   cu_bypass = P.transquant_bypass && rng.chance(10);
+  cqo_queue.clear();
+  cqo_read = 0;
   if (P.transquant_bypass) bin(CTX_TQ_BYPASS, cu_bypass);
   {
     int n8 = nCbS >> 3;
@@ -1379,6 +1544,10 @@ void Enc::coding_quadtree(int x0, int y0, int log2, int depth) {
     qg_target_qp = clip3(std::max(0, slice_qp - 6), std::min(51, slice_qp + 6), slice_qp + rng.below(7) - 3);
     if (stress(HEVC_ENC_STRESS_QP)) qg_target_qp = -qp_bd_offset + rng.below(52 + qp_bd_offset);
   }
+  if (P.chroma_qp_offset_list_len && log2 >= log2_min_cu_chroma_qp_offset) {
+    cqo_coded_a = cqo_coded_b = false;
+    cqo_next = rng.chance(80) ? 1 + rng.below(P.chroma_qp_offset_list_len) : 0;
+  }
   if (split) {
     int h = size >> 1, x1 = x0 + h, y1 = y0 + h;
     coding_quadtree(x0, y0, log2 - 1, depth + 1);
@@ -1421,6 +1590,7 @@ void Enc::code_sao(int rx, int ry) {
     for (int i = 0; i < 4; i++) {
       absv[i] = rng.below((stress(HEVC_ENC_STRESS_SAO) ? cMax : std::min(cMax, 4)) + 1);
       if (absv[i] == cMax && bd >= 10) stats[ST_sao_offset_cmax_hbd]++;
+      if (absv[i] == cMax && (c ? P.log2_sao_offset_scale_chroma : P.log2_sao_offset_scale_luma)) stats[ST_sao_offset_scaled_cmax]++;
       for (int k = 0; k < absv[i]; k++) cabac.bypass(1);
       if (absv[i] < cMax) cabac.bypass(0);
     }
@@ -1477,7 +1647,7 @@ void Enc::encode_picture(std::vector<uint8_t>& out) {
       int x = std::min((((prev % ctbs_w) + 1) << log2_ctb) - 1, W - 1), y = std::min((((prev / ctbs_w) + 1) << log2_ctb) - 1, H - 1);
       currentQPY = qp_y[(x >> 3) + (size_t)(y >> 3) * w8];
     }
-    if (dependent && !tile_start[seg_addr]) ctx = dep_ctx;
+    if (dependent && !tile_start[seg_addr]) { ctx = dep_ctx; memcpy(stat_coeff, dep_stat.data(), 4); }
     else init_contexts();
     bool first_substream_of_independent = !dependent;
     for (int k = 0; k < seg_len; k++) {
@@ -1485,16 +1655,22 @@ void Enc::encode_picture(std::vector<uint8_t>& out) {
       ctb_addr_rs = ts2rs[ctb_addr_ts];
       int cxr = ctb_addr_rs % ctbs_w, cyr = ctb_addr_rs / ctbs_w;
       if (P.wpp && cxr == 0 && cyr >= 1 && !(first_substream_of_independent && ctb_addr_rs == seg_addr)) {
-        if (ctbs_w > 1) ctx = wpp_ctx[cyr - 1];
-        else init_contexts();
+        if (ctbs_w > 1) {
+          ctx = wpp_ctx[cyr - 1];
+          if (memcmp(stat_coeff, wpp_stat[cyr - 1].data(), 4)) stats[ST_wpp_stat_coeff_restored]++;
+          memcpy(stat_coeff, wpp_stat[cyr - 1].data(), 4);
+        } else {
+          init_contexts();
+        }
       }
       ctb_slice[ctb_addr_rs] = slice_addr_rs;
       encode_ctu();
-      if (P.wpp && cxr == 1 && cyr < ctbs_h - 1) wpp_ctx[cyr] = ctx;
+      if (P.wpp && cxr == 1 && cyr < ctbs_h - 1) { wpp_ctx[cyr] = ctx; memcpy(wpp_stat[cyr].data(), stat_coeff, 4); }
       bool last = k == seg_len - 1;
       cabac.terminate(last ? 1 : 0);
       if (last) {
         dep_ctx = ctx;
+        memcpy(dep_stat.data(), stat_coeff, 4);
         cabac.finish();
         break;
       }
@@ -1543,6 +1719,7 @@ void Enc::encode_picture(std::vector<uint8_t>& out) {
       bw.ue(2);  // I slice
       if (P.sao) { bw.put(slice_sao_luma, 1); if (cf) bw.put(slice_sao_chroma, 1); }
       bw.se(slice_qp - 26);
+      if (P.chroma_qp_offset_list_len) bw.put(1, 1);  // cu_chroma_qp_offset_enabled_flag
       if (P.loop_filter_across_slices && (slice_sao_luma || slice_sao_chroma || !P.deblock_disable)) bw.put(1, 1);
     }
     std::vector<uint8_t> payload;
@@ -1577,7 +1754,8 @@ extern "C" {
 // packed strides given in samples. Output: 4-byte-length-prefixed NAL units (VPS, SPS, PPS, slices).
 // recon (optional): per component a buffer of the coded size (width and height rounded up to a multiple of 8,
 // chroma subsampled, tightly packed) that receives the encoder's reconstruction before the in-loop filters.
-// stats (optional): hevc_enc_stat_count() counters of what was written (names: hevc_enc_stat_name).
+// stats (optional): hevc_enc_stat_count() counters of what was written (names: hevc_enc_stat_name; the range-extension
+// group starts at hevc_enc_rext_stat_first()).
 int hevc_enc_encode_ex(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
                        size_t* out_size, uint16_t* const recon[3], uint64_t* stats) {
   if (!params || !planes || !out || !out_size) return -1;
@@ -1586,6 +1764,12 @@ int hevc_enc_encode_ex(const hevc_enc_params* params, const uint16_t* const plan
   if (P.log2_ctb < 4 || P.log2_ctb > 6 || P.log2_min_tb < 2 || P.log2_max_tb > 5 || P.log2_min_tb > P.log2_max_tb) return -2;
   if (P.log2_min_tb >= 3) return -2;  // min CB is fixed at 8x8 here
   if (P.qp < -6 * (P.bit_depth - 8) || P.qp > 51) return -2;
+  if (P.log2_max_transform_skip_minus2 < 0 || P.log2_max_transform_skip_minus2 > 3) return -2;
+  if (P.chroma_qp_offset_list_len < 0 || P.chroma_qp_offset_list_len > 6) return -2;
+  if (P.diff_cu_chroma_qp_offset_depth < 0 || P.diff_cu_chroma_qp_offset_depth > P.log2_ctb - 3) return -2;
+  const int max_sao_scale = std::max(0, P.bit_depth - 10);
+  if (P.log2_sao_offset_scale_luma < 0 || P.log2_sao_offset_scale_luma > max_sao_scale) return -2;
+  if (P.log2_sao_offset_scale_chroma < 0 || P.log2_sao_offset_scale_chroma > max_sao_scale) return -2;
   Enc enc(P);
   enc.setup();
   const int ncomp = enc.cf ? 3 : 1;
@@ -1619,12 +1803,15 @@ int hevc_enc_encode(const hevc_enc_params* params, const uint16_t* const planes[
 
 int hevc_enc_stat_count(void) { return ST_COUNT; }
 
+int hevc_enc_rext_stat_first(void) { return ST_REXT_FIRST_; }
+
 const char* hevc_enc_stat_name(int i) {
   static const std::vector<std::string> names = [] {
     std::vector<std::string> v;
 #define HEVC_ENC_STAT_NAME(name, n) \
   for (int k = 0; k < (n); k++) v.push_back((n) == 1 ? std::string(#name) : std::string(#name) + "_" + std::to_string(k));
     HEVC_ENC_STATS(HEVC_ENC_STAT_NAME)
+    HEVC_ENC_REXT_STATS(HEVC_ENC_STAT_NAME)
 #undef HEVC_ENC_STAT_NAME
     return v;
   }();

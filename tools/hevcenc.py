@@ -13,7 +13,12 @@ FIELDS = ["width", "height", "chroma_format", "bit_depth", "qp", "log2_ctb", "lo
           "sao", "deblock_disable", "beta_offset_div2", "tc_offset_div2", "sign_hiding", "cu_qp_delta", "transform_skip",
           "wpp", "tile_cols", "tile_rows", "slice_ctbs", "dependent_slices", "strong_intra", "scaling_list", "pcm",
           "transquant_bypass", "vui", "full_range", "matrix", "primaries", "transfer", "cb_qp_offset", "cr_qp_offset",
-          "loop_filter_across_slices", "loop_filter_across_tiles", "stress"]
+          "loop_filter_across_slices", "loop_filter_across_tiles", "stress",
+          # range extensions (SPS / PPS range extension syntax); all 0: no extension is written
+          "transform_skip_rotation", "transform_skip_context", "implicit_rdpcm", "intra_smoothing_disabled",
+          "persistent_rice_adaptation", "extended_precision", "cabac_bypass_alignment", "log2_max_transform_skip_minus2",
+          "cross_component_prediction", "chroma_qp_offset_list_len", "diff_cu_chroma_qp_offset_depth",
+          "log2_sao_offset_scale_luma", "log2_sao_offset_scale_chroma"]
 
 # stress bits (hevc_enc_params::stress): syntax values at the limits of their legal ranges, for parser tests
 STRESS_LEVELS, STRESS_MODES, STRESS_QP, STRESS_SAO, STRESS_DENSE = 1, 2, 4, 8, 16
@@ -49,16 +54,27 @@ def lib():
     return _lib
 
 
-def stat_names():
+def _all_stat_names():
     L = lib()
     return [L.hevc_enc_stat_name(i).decode() for i in range(L.hevc_enc_stat_count())]
+
+
+def stat_names():
+    """Counters of the syntax extremes the stress mode writes."""
+    return _all_stat_names()[:lib().hevc_enc_rext_stat_first()]
+
+
+def rext_stat_names():
+    """Counters of the range-extension coding tools (the range-extension fields of the encoder options)."""
+    return _all_stat_names()[lib().hevc_enc_rext_stat_first():]
 
 
 def encode(planes, want=(), **kw):
     """planes: list of 2-D integer arrays (Y[,Cb,Cr]) of the visible picture. Returns bytes:
     4-byte-length-prefixed NAL units (VPS, SPS, PPS, slice segments).
     want: any of "recon" (the encoder's reconstruction before the in-loop filters: uint16 planes of the coded size,
-    width and height rounded up to a multiple of 8) and "stats" ({counter name: count} of what was written). With a
+    width and height rounded up to a multiple of 8) and "stats" ({counter name: count} of what was written: the stress
+    counters under "stats", the range-extension ones under "rext_stats"). With a
     non-empty want the result is (bytes, {name: value})."""
     L = lib()
     opts = dict(DEFAULTS)
@@ -91,7 +107,10 @@ def encode(planes, want=(), **kw):
     if recon is not None:
         extra["recon"] = recon
     if stats is not None:
-        extra["stats"] = dict(zip(stat_names(), (int(v) for v in stats)))
+        first = L.hevc_enc_rext_stat_first()
+        counts = dict(zip(_all_stat_names(), (int(v) for v in stats)))
+        extra["stats"] = {k: counts[k] for k in _all_stat_names()[:first]}
+        extra["rext_stats"] = {k: counts[k] for k in _all_stat_names()[first:]}
     return data, extra
 
 
