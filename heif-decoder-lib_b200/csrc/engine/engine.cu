@@ -111,21 +111,32 @@ struct hc_engine {
 
 namespace {
 
+// Y, Cb, Cr and alpha planes in the plane pool; w == 0: no such plane
+struct Planes {
+  size_t off[4] = {0, 0, 0, 0};     // byte offsets in the plane pool
+  int stride[4] = {0, 0, 0, 0};     // samples
+  int w[4] = {0, 0, 0, 0}, h[4] = {0, 0, 0, 0};
+  // plane k at the end of the pool: rows of at least w + 4 samples of ps bytes padded to 128 bytes, the plane 256-byte aligned
+  void place(int k, int pw, int ph, int ps, size_t& pool) {
+    w[k] = pw; h[k] = ph;
+    stride[k] = (int)(align_up((size_t)(pw + 4) * ps, 128) / ps);
+    off[k] = pool;
+    pool += align_up((size_t)stride[k] * ph * ps, 256);
+  }
+};
+
 struct Canvas {
   int w = 0, h = 0, chroma = 1, bit_depth = 8;
   bool alpha = false;
-  size_t off[4] = {0, 0, 0, 0};     // byte offsets in the plane pool
-  int stride[4] = {0, 0, 0, 0};     // samples
-  int pw[4] = {0, 0, 0, 0}, ph[4] = {0, 0, 0, 0};
-  // geometric passes between K4 and K5 (irot / imir / clap of the reference, in the order they are given); the "output
-  // view" below is what K5 and the read-backs use; without passes it is the canvas itself
+  Planes planes;                    // K4 writes them
+  // geometric passes between K4 and K5 (irot / imir / clap of the reference, in the order they are given); the output
+  // view below is what K5 and the read-backs use; without passes it is the canvas itself
   struct Pass {
     int kind;                        // 0: dihedral map (a = swap, b = flip_x, c = flip_y), 1: crop (a..d = left, top, right, bottom)
     int a, b, c, d;
-    // filled at upload: the planes this pass writes
-    int w = 0, h = 0;                // image size after the pass
-    size_t off[4] = {0, 0, 0, 0};
-    int stride[4] = {0, 0, 0, 0}, pw[4] = {0, 0, 0, 0}, ph[4] = {0, 0, 0, 0};
+    // filled at upload: the image size after the pass and the planes this pass writes
+    int w = 0, h = 0;
+    Planes planes;
   };
   std::vector<Pass> passes;
   bool transformed() const { return !passes.empty(); }
@@ -135,8 +146,7 @@ struct Canvas {
   int req_w = 0, req_h = 0;
   int dw = 0, dh = 0;
   bool scaled() const { return dw != ow || dh != oh; }
-  size_t ooff[4] = {0, 0, 0, 0};
-  int ostride[4] = {0, 0, 0, 0}, opw[4] = {0, 0, 0, 0}, oph[4] = {0, 0, 0, 0};
+  Planes view;                      // output view: the planes of the last pass, or the canvas' own (filled at upload)
   // 'iovl' derived image (hc_batch_add_overlay_canvas): no planes of its own; K7 composes the child canvases into its RGB output
   bool overlay = false;
   int bkg[3] = {0, 0, 0};
@@ -222,9 +232,8 @@ namespace {
 using hc::plane_w;
 using hc::plane_h;
 
-// bytes of a canvas' block in the batch's output buffer
-size_t out_block_bytes(const Canvas& c, int bpp) {
-  if (c.planar) return align_up(c.packed, 256);
+// bytes of a canvas' block in the batch's output buffer for interleaved rows of bpp bytes per pixel
+size_t interleaved_block_bytes(const Canvas& c, int bpp) {
   return align_up(align_up((size_t)((c.dw + 7) & ~7) * bpp, 256) * c.dh, 256);
 }
 
@@ -238,7 +247,7 @@ bool planar_layout(const Canvas& c, size_t poff[4], size_t* packed) {
   int32_t w[4], h[4];
   *packed = hc_image_plane_layout(&d, poff, nullptr, w, h);
   for (int k = 0; k < 4; k++)
-    if (w[k] != c.opw[k] || (w[k] && h[k] != c.oph[k])) return false;
+    if (w[k] != c.view.w[k] || (w[k] && h[k] != c.view.h[k])) return false;
   return *packed > 0;
 }
 
@@ -251,13 +260,13 @@ void add_pack_planes(hc_batch* b, hc::PackBatch& pb, const Canvas& c, const uint
   }
   const int ps = c.bit_depth == 8 ? 1 : 2;
   for (int k = 0; k < 4; k++) {
-    if (c.opw[k] == 0) continue;
+    if (c.view.w[k] == 0) continue;
     hc::PackPlane& q = pb.p[pb.n++];
-    q.src = P + c.ooff[k];
+    q.src = P + c.view.off[k];
     q.dst = out + c.poff[k];
-    q.src_pitch = (unsigned)c.ostride[k] * ps;
-    q.row_bytes = (unsigned)c.opw[k] * ps;
-    q.rows = (unsigned)c.oph[k];
+    q.src_pitch = (unsigned)c.view.stride[k] * ps;
+    q.row_bytes = (unsigned)c.view.w[k] * ps;
+    q.rows = (unsigned)c.view.h[k];
     q.pad = 0;
   }
 }
@@ -291,6 +300,79 @@ void apply_format(Canvas& c, const hc_csc_params& p) {
     c.rgb_bpp = kBppOf[p.out_format];
     c.rgb_stride = align_up((size_t)((c.dw + 7) & ~7) * c.rgb_bpp, 256);
   }
+}
+
+// Where every canvas' output lies after a convert of canvases[0..n) with params[0..n) (after check_convert), decided without
+// changing anything: one block per canvas in canvas order, in the new format for the canvases the call names and as it is for
+// the others (8 bytes per pixel for a canvas never converted). A converted canvas the call does not name keeps its offset and
+// its bytes, so the call fails when the layout would move one, or would make the buffer grow while one exists.
+int plan_output(const hc_batch* b, int n, const int* canvases, const hc_csc_params* params, std::vector<size_t>& off, size_t& total) {
+  std::vector<const hc_csc_params*> named(b->canvases.size(), nullptr);
+  for (int i = 0; i < n; i++) named[canvases[i]] = &params[i];
+  off.resize(b->canvases.size());
+  total = 0;
+  bool kept = false;
+  for (size_t k = 0; k < b->canvases.size(); k++) {
+    const Canvas& c = b->canvases[k];
+    const hc_csc_params* p = named[k];
+    if (!p && c.converted) {
+      if (c.rgb_off != total) {
+        hc::set_last_error("convert: the output of a converted canvas the call does not name would move; convert it in the same call");
+        return HC_ERR_ARGUMENT;
+      }
+      kept = true;
+    }
+    off[k] = total;
+    const bool planar = p ? p->out_format == HC_OUT_YCBCR : c.planar;
+    size_t poff[4], packed = c.packed;
+    if (p && planar) planar_layout(c, poff, &packed);
+    total += planar ? align_up(packed, 256) : interleaved_block_bytes(c, p ? kBppOf[p->out_format] : (c.rgb_bpp ? c.rgb_bpp : 8));
+  }
+  if (kept && total > b->d_rgb.cap) {
+    hc::set_last_error("convert: the output buffer would have to grow under a converted canvas the call does not name; convert it in the same call");
+    return HC_ERR_ARGUMENT;
+  }
+  return HC_OK;
+}
+
+// K5's arguments for canvas c: its output view into its block of the output buffer, or into its external target
+hc::CscArgs csc_args(const hc_batch* b, const Canvas& c, const hc_csc_params& p) {
+  const uint8_t* P = (const uint8_t*)b->d_planes.p;
+  hc::CscArgs a;
+  a.y = P + c.view.off[0];
+  a.cb = c.chroma ? P + c.view.off[1] : nullptr;
+  a.cr = c.chroma ? P + c.view.off[2] : nullptr;
+  a.a = c.alpha ? P + c.view.off[3] : nullptr;
+  a.y_stride = c.view.stride[0]; a.c_stride = c.view.stride[1]; a.a_stride = c.view.stride[3];
+  a.width = c.dw; a.height = c.dh; a.chroma_format = c.chroma;
+  a.src_w = c.ow; a.src_h = c.oh; a.gather = c.scaled();
+  a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
+  a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
+  a.p = p;
+  return a;
+}
+
+// Enqueues the copy of a converted canvas' output to dst: the packed planes in one 1-D copy (HC_OUT_YCBCR: dst_stride must be
+// the Y row), else dh rows of dw interleaved pixels. `timed`: between the events ev_d2h.
+int enqueue_output_copy(hc_batch* b, const char* fn, int canvas, void* dst, size_t dst_stride, cudaMemcpyKind kind, bool timed) {
+  if (!b || !dst || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error(std::string(fn) + ": bad argument"); return HC_ERR_ARGUMENT; }
+  const Canvas& c = b->canvases[canvas];
+  if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
+  if (c.ext_rgb) { hc::set_last_error("this image is written to an external RGB target (hc_batch_set_rgb_target): read it there"); return HC_ERR_ARGUMENT; }
+  if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are read with the stride of the Y row"); return HC_ERR_ARGUMENT; }
+  const uint8_t* src = (const uint8_t*)b->d_rgb.p + c.rgb_off;
+  if (timed) cudaEventRecord(b->ev_d2h[0], b->stream);
+  const cudaError_t e = c.planar ? cudaMemcpyAsync(dst, src, c.packed, kind, b->stream)
+                                 : cudaMemcpy2DAsync(dst, dst_stride, src, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh, kind, b->stream);
+  if (timed) cudaEventRecord(b->ev_d2h[1], b->stream);
+  return cuda_ok(e, c.planar ? "cudaMemcpyAsync(packed planes)" : "cudaMemcpy2DAsync(rgb)") ? HC_OK : HC_ERR_CUDA;
+}
+
+// plane k of a canvas' output view, which the plane read-backs copy
+int check_view_plane(const Canvas& c, int k) {
+  if (c.view.w[k] != 0) return HC_OK;
+  hc::set_last_error("canvas has no such plane");
+  return HC_ERR_ARGUMENT;
 }
 
 void release_blocks(hc_batch* b) {
@@ -541,50 +623,37 @@ int hc_batch_upload(hc_batch* b) {
   b->hpics.resize(np);
   for (auto& c : b->canvases) {
     const int ps = c.bit_depth == 8 ? 1 : 2;
-    for (int k = 0; k < 4; k++) {
-      if (k == 3 && !c.alpha) continue;
-      c.pw[k] = c.overlay ? 0 : plane_w(c.w, c.chroma, k);
-      c.ph[k] = c.overlay ? 0 : plane_h(c.h, c.chroma, k);
-      if (c.pw[k] == 0) continue;
-      c.stride[k] = (int)(align_up((size_t)(c.pw[k] + 4) * ps, 128) / ps);
-      c.off[k] = pool;
-      pool += align_up((size_t)c.stride[k] * c.ph[k] * ps, 256);
-    }
+    c.planes = Planes();
+    for (int k = 0; k < (c.alpha ? 4 : 3); k++)
+      if (!c.overlay && plane_w(c.w, c.chroma, k)) c.planes.place(k, plane_w(c.w, c.chroma, k), plane_h(c.h, c.chroma, k), ps, pool);
     c.converted = false;
     // pass outputs: every pass writes its own set of planes (passes are rare; the chain stays simple and exact)
-    {
-      int iw = c.w, ih = c.h;
-      const int* ipw = c.pw; const int* iph = c.ph;
-      for (Canvas::Pass& ps_ : c.passes) {
-        int nw, nh;
-        if (ps_.kind == HC_PASS_DIHEDRAL) { nw = ps_.a ? ih : iw; nh = ps_.a ? iw : ih; }
-        else {
-          if (ps_.c >= iw || ps_.d >= ih) { hc::set_last_error("crop window outside the image"); return HC_ERR_ARGUMENT; }
-          nw = ps_.c - ps_.a + 1; nh = ps_.d - ps_.b + 1;
-        }
-        for (int k = 0; k < 4; k++) {
-          ps_.pw[k] = ps_.ph[k] = 0;
-          if (ipw[k] == 0 || (k == 3 && !c.alpha)) continue;
-          if (ps_.kind == HC_PASS_DIHEDRAL) { ps_.pw[k] = ps_.a ? iph[k] : ipw[k]; ps_.ph[k] = ps_.a ? ipw[k] : iph[k]; }
-          else {
-            // HeifPixelImage::crop (pixelimage.cc:820-823): the window is scaled to every plane by integer division
-            const int pl = ps_.a * ipw[k] / iw, pr = ps_.c * ipw[k] / iw, pt = ps_.b * iph[k] / ih, pb = ps_.d * iph[k] / ih;
-            ps_.pw[k] = pr - pl + 1; ps_.ph[k] = pb - pt + 1;
-          }
-          ps_.stride[k] = (int)(align_up((size_t)(ps_.pw[k] + 4) * ps, 128) / ps);
-          ps_.off[k] = pool;
-          pool += align_up((size_t)ps_.stride[k] * ps_.ph[k] * ps, 256);
-        }
-        ps_.w = nw; ps_.h = nh;
-        iw = nw; ih = nh; ipw = ps_.pw; iph = ps_.ph;
+    int iw = c.w, ih = c.h;
+    const Planes* in = &c.planes;
+    for (Canvas::Pass& pass : c.passes) {
+      int nw, nh;
+      if (pass.kind == HC_PASS_DIHEDRAL) { nw = pass.a ? ih : iw; nh = pass.a ? iw : ih; }
+      else {
+        if (pass.c >= iw || pass.d >= ih) { hc::set_last_error("crop window outside the image"); return HC_ERR_ARGUMENT; }
+        nw = pass.c - pass.a + 1; nh = pass.d - pass.b + 1;
       }
-      c.ow = iw; c.oh = ih;
-      c.dw = c.req_w ? c.req_w : iw; c.dh = c.req_h ? c.req_h : ih;
+      pass.planes = Planes();
       for (int k = 0; k < 4; k++) {
-        if (c.passes.empty()) { c.ooff[k] = c.off[k]; c.ostride[k] = c.stride[k]; c.opw[k] = c.pw[k]; c.oph[k] = c.ph[k]; }
-        else { const Canvas::Pass& l = c.passes.back(); c.ooff[k] = l.off[k]; c.ostride[k] = l.stride[k]; c.opw[k] = l.pw[k]; c.oph[k] = l.ph[k]; }
+        const int w = in->w[k], h = in->h[k];
+        if (w == 0) continue;
+        if (pass.kind == HC_PASS_DIHEDRAL) pass.planes.place(k, pass.a ? h : w, pass.a ? w : h, ps, pool);
+        else {
+          // HeifPixelImage::crop (pixelimage.cc:820-823): the window is scaled to every plane by integer division
+          const int pl = pass.a * w / iw, pr = pass.c * w / iw, pt = pass.b * h / ih, pb = pass.d * h / ih;
+          pass.planes.place(k, pr - pl + 1, pb - pt + 1, ps, pool);
+        }
       }
+      pass.w = iw = nw; pass.h = ih = nh;
+      in = &pass.planes;
     }
+    c.ow = iw; c.oh = ih;
+    c.dw = c.req_w ? c.req_w : iw; c.dh = c.req_h ? c.req_h : ih;
+    c.view = c.passes.empty() ? c.planes : c.passes.back().planes;
   }
   // ---- record bases ----
   size_t n_ctu = 0, n_blk = 0, n_tb = 0, n_coeff = 0, n_edge = 0, n_qp = 0, n_scal = 0;
@@ -644,13 +713,13 @@ int hc_batch_upload(hc_batch* b) {
     p.dst_flags = 0;
     if (b->pics[i].rescale) p.dst_flags |= HC_DST_RESCALE_LIMITED;
     if (b->pics[i].role == HC_ROLE_ALPHA) {
-      p.dst_off[0] = cv.off[3]; p.dst_stride[0] = (uint32_t)cv.stride[3];
+      p.dst_off[0] = cv.planes.off[3]; p.dst_stride[0] = (uint32_t)cv.planes.stride[3];
       p.dst_flags |= HC_DST_SKIP_CB | HC_DST_SKIP_CR;
     } else if (b->pics[i].role == HC_ROLE_LUMA) {
-      p.dst_off[0] = cv.off[0]; p.dst_stride[0] = (uint32_t)cv.stride[0];
+      p.dst_off[0] = cv.planes.off[0]; p.dst_stride[0] = (uint32_t)cv.planes.stride[0];
       p.dst_flags |= HC_DST_SKIP_CB | HC_DST_SKIP_CR;
     } else {
-      for (int c = 0; c < ncomp; c++) { p.dst_off[c] = cv.off[c]; p.dst_stride[c] = (uint32_t)cv.stride[c]; }
+      for (int c = 0; c < ncomp; c++) { p.dst_off[c] = cv.planes.off[c]; p.dst_stride[c] = (uint32_t)cv.planes.stride[c]; }
     }
   }
 
@@ -1029,35 +1098,36 @@ int hc_batch_reconstruct_async(hc_batch* b, int stages) {
     if (!c.transformed()) continue;
     const int ps = c.bit_depth == 8 ? 1 : 2;
     int iw = c.w, ih = c.h;
-    const size_t* ioff = c.off; const int* istride = c.stride; const int* ipw = c.pw; const int* iph = c.ph;
+    const Planes* in = &c.planes;
     for (const Canvas::Pass& p : c.passes) {
+      const Planes& out = p.planes;
       for (int k = 0; k < 4; k++) {
-        if (p.pw[k] == 0) continue;
-        const uint8_t* src = (const uint8_t*)b->d_planes.p + ioff[k];
-        uint8_t* dst = (uint8_t*)b->d_planes.p + p.off[k];
+        if (out.w[k] == 0) continue;
+        const uint8_t* src = (const uint8_t*)b->d_planes.p + in->off[k];
+        uint8_t* dst = (uint8_t*)b->d_planes.p + out.off[k];
         if (p.kind == HC_PASS_DIHEDRAL) {
           hc::XformArgs a;
           a.src = src; a.dst = dst;
-          a.w = ipw[k]; a.h = iph[k]; a.src_stride = istride[k]; a.dst_stride = p.stride[k];
+          a.w = in->w[k]; a.h = in->h[k]; a.src_stride = in->stride[k]; a.dst_stride = out.stride[k];
           a.swap = p.a; a.flip_x = p.b; a.flip_y = p.c;
           hc::launch_k6(a, c.bit_depth != 8, s);
         } else {
-          const int pl = p.a * ipw[k] / iw, pt = p.b * iph[k] / ih;
-          cudaMemcpy2DAsync(dst, (size_t)p.stride[k] * ps, src + ((size_t)pt * istride[k] + pl) * ps, (size_t)istride[k] * ps,
-                            (size_t)p.pw[k] * ps, p.ph[k], cudaMemcpyDeviceToDevice, s);
+          const int pl = p.a * in->w[k] / iw, pt = p.b * in->h[k] / ih;
+          cudaMemcpy2DAsync(dst, (size_t)out.stride[k] * ps, src + ((size_t)pt * in->stride[k] + pl) * ps, (size_t)in->stride[k] * ps,
+                            (size_t)out.w[k] * ps, out.h[k], cudaMemcpyDeviceToDevice, s);
         }
         b->launches += 1;
       }
-      iw = p.w; ih = p.h; ioff = p.off; istride = p.stride; ipw = p.pw; iph = p.ph;
+      iw = p.w; ih = p.h; in = &out;
     }
   }
   // alpha planes that come from an alpha image of another size (hc_batch_link_alpha): nearest-neighbour rescale of the
   // alpha canvas' output view into the alpha plane of the colour canvas' output view
   for (const auto& l : b->alpha_links) {
     const Canvas& c = b->canvases[l.first];
-    const Canvas& a = b->canvases[l.second];
-    hc::launch_k6_scale((const uint8_t*)b->d_planes.p + a.ooff[0], a.opw[0], a.oph[0], a.ostride[0], (uint8_t*)b->d_planes.p + c.ooff[3], c.opw[3],
-                        c.oph[3], c.ostride[3], c.bit_depth != 8, s);
+    const Planes& a = b->canvases[l.second].view;
+    hc::launch_k6_scale((const uint8_t*)b->d_planes.p + a.off[0], a.w[0], a.h[0], a.stride[0], (uint8_t*)b->d_planes.p + c.view.off[3],
+                        c.view.w[3], c.view.h[3], c.view.stride[3], c.bit_depth != 8, s);
     b->launches += 1;
   }
   cudaEventRecord(b->ev[6], s);
@@ -1074,69 +1144,12 @@ int hc_batch_reconstruct(hc_batch* b, int stages) {
 }
 
 int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params) {
-  if (!b || !params || canvas < 0 || canvas >= (int)b->canvases.size() || !b->uploaded) {
-    hc::set_last_error("hc_batch_convert: bad argument");
-    return HC_ERR_ARGUMENT;
-  }
-  if (!cuda_ok(cudaSetDevice(b->eng->device), "cudaSetDevice")) return HC_ERR_CUDA;
-  Canvas& c = b->canvases[canvas];
-  if (params->out_format < 0 || params->out_format > HC_OUT_YCBCR) { hc::set_last_error("bad output format"); return HC_ERR_ARGUMENT; }
-  if (params->in_depth != c.bit_depth) { hc::set_last_error("conversion parameters were selected for another bit depth"); return HC_ERR_ARGUMENT; }
-  if (int rc = check_convert(c, *params)) return rc;
-  apply_format(c, *params);
-  // lay all canvases' rgb buffers out in one block (grow if needed)
-  size_t total = 0;
-  for (auto& cv : b->canvases) {
-    const int bp = &cv == &c ? c.rgb_bpp : (cv.rgb_bpp ? cv.rgb_bpp : 8);
-    cv.rgb_off = total;
-    total += out_block_bytes(cv, bp);
-  }
-  if (b->d_rgb.cap < total) {
-    bool any = false;
-    for (auto& cv : b->canvases) any |= cv.converted;
-    if (any) { hc::set_last_error("hc_batch_convert: convert all canvases with the same format class"); return HC_ERR_ARGUMENT; }
-    b->eng->give(b->eng->free_dev, b->d_rgb);
-    b->d_rgb = b->eng->take(b->eng->free_dev, total, false);
-    if (!b->d_rgb.p) return HC_ERR_MEMORY;
-  }
-  const uint8_t* P = (const uint8_t*)b->d_planes.p;
-  if (c.planar) {   // K8, timed like K5
-    hc::PackBatch pb;
-    pb.n = 0;
-    cudaEvent_t e0 = b->eng->take_event(), e1 = b->eng->take_event();
-    cudaEventRecord(e0, b->stream);
-    add_pack_planes(b, pb, c, P, (uint8_t*)b->d_rgb.p + c.rgb_off);
-    hc::launch_k8_batch(pb, b->stream);
-    cudaEventRecord(e1, b->stream);
-    b->csc_events.push_back({e0, e1});
-    b->launches += 1;
-    c.converted = true;
-    return cuda_ok(cudaGetLastError(), "kernel launch (K8)") ? HC_OK : HC_ERR_CUDA;
-  }
-  hc::CscArgs a;
-  a.y = P + c.ooff[0];
-  a.cb = c.chroma ? P + c.ooff[1] : nullptr;
-  a.cr = c.chroma ? P + c.ooff[2] : nullptr;
-  a.a = c.alpha ? P + c.ooff[3] : nullptr;
-  a.y_stride = c.ostride[0]; a.c_stride = c.ostride[1]; a.a_stride = c.ostride[3];
-  a.width = c.dw; a.height = c.dh; a.chroma_format = c.chroma;
-  a.src_w = c.ow; a.src_h = c.oh; a.gather = c.scaled();
-  a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
-  a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
-  a.p = *params;
-  cudaEvent_t e0 = b->eng->take_event(), e1 = b->eng->take_event();
-  cudaEventRecord(e0, b->stream);
-  hc::launch_k5(a, c.bit_depth != 8, b->stream);
-  cudaEventRecord(e1, b->stream);
-  b->csc_events.push_back({e0, e1});
-  b->launches += 1;
-  c.converted = true;
-  if (!cuda_ok(cudaGetLastError(), "kernel launch (K5)")) return HC_ERR_CUDA;
-  return HC_OK;
+  if (!b || !params || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_convert: bad argument"); return HC_ERR_ARGUMENT; }
+  return hc_batch_convert_many(b, 1, &canvas, params);
 }
 
-// K5 for several canvases with as few launches as possible (one per group of up to CSC_BATCH_MAX canvases of the
-// same sample size). Same result as calling hc_batch_convert for each of them.
+// K5 / K7 / K8 for several canvases with as few launches as possible (K5: one per group of up to CSC_BATCH_MAX canvases of
+// the same sample size).
 int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_params* params) {
   if (!b || n <= 0 || !canvases || !params || !b->uploaded) { hc::set_last_error("hc_batch_convert_many: bad argument"); return HC_ERR_ARGUMENT; }
   if (!cuda_ok(cudaSetDevice(b->eng->device), "cudaSetDevice")) return HC_ERR_CUDA;
@@ -1144,19 +1157,17 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
     if (canvases[i] < 0 || canvases[i] >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_convert_many: bad canvas"); return HC_ERR_ARGUMENT; }
     if (int rc = check_convert(b->canvases[canvases[i]], params[i])) return rc;
   }
-  for (int i = 0; i < n; i++) apply_format(b->canvases[canvases[i]], params[i]);
+  std::vector<size_t> off;
   size_t total = 0;
-  for (auto& cv : b->canvases) {
-    const int bp = cv.rgb_bpp ? cv.rgb_bpp : 8;
-    cv.rgb_off = total;
-    total += out_block_bytes(cv, bp);
-  }
-  if (b->d_rgb.cap < total) {
+  if (int rc = plan_output(b, n, canvases, params, off, total)) return rc;
+  if (b->d_rgb.cap < total) {   // no converted canvas outside the call (plan_output): nothing in the old buffer is kept
+    Block grown = b->eng->take(b->eng->free_dev, total, false);
+    if (!grown.p) return HC_ERR_MEMORY;
     b->eng->give(b->eng->free_dev, b->d_rgb);
-    b->d_rgb = b->eng->take(b->eng->free_dev, total, false);
-    if (!b->d_rgb.p) return HC_ERR_MEMORY;
-    for (auto& cv : b->canvases) cv.converted = false;
+    b->d_rgb = grown;
   }
+  for (size_t k = 0; k < b->canvases.size(); k++) b->canvases[k].rgb_off = off[k];
+  for (int i = 0; i < n; i++) apply_format(b->canvases[canvases[i]], params[i]);
   const uint8_t* P = (const uint8_t*)b->d_planes.p;
   cudaEvent_t e0 = b->eng->take_event(), e1 = b->eng->take_event();
   cudaEventRecord(e0, b->stream);
@@ -1169,8 +1180,8 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
     for (int k = 0; k < oa.n; k++) {
       const Canvas& ch = b->canvases[c.children[k].canvas];
       hc::OverlayChild& oc = oa.child[k];
-      oc.y = P + ch.ooff[0]; oc.cb = P + ch.ooff[1]; oc.cr = P + ch.ooff[2]; oc.a = ch.alpha ? P + ch.ooff[3] : nullptr;
-      oc.y_stride = ch.ostride[0]; oc.c_stride = ch.ostride[1]; oc.a_stride = ch.ostride[3];
+      oc.y = P + ch.view.off[0]; oc.cb = P + ch.view.off[1]; oc.cr = P + ch.view.off[2]; oc.a = ch.alpha ? P + ch.view.off[3] : nullptr;
+      oc.y_stride = ch.view.stride[0]; oc.c_stride = ch.view.stride[1]; oc.a_stride = ch.view.stride[3];
       oc.w = ch.ow; oc.h = ch.oh; oc.dx = c.children[k].dx; oc.dy = c.children[k].dy;
       const hc_csc_params& cp = c.children[k].p;
       oc.mode = cp.mode; oc.full_range = cp.full_range;
@@ -1193,17 +1204,7 @@ int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_
       if (i < n && !b->canvases[canvases[i]].overlay && !b->canvases[canvases[i]].planar &&
           (b->canvases[canvases[i]].bit_depth != 8) == (sixteen != 0)) {
         Canvas& c = b->canvases[canvases[i]];
-        hc::CscArgs& a = cb.a[cb.n++];
-        a.y = P + c.ooff[0];
-        a.cb = c.chroma ? P + c.ooff[1] : nullptr;
-        a.cr = c.chroma ? P + c.ooff[2] : nullptr;
-        a.a = c.alpha ? P + c.ooff[3] : nullptr;
-        a.y_stride = c.ostride[0]; a.c_stride = c.ostride[1]; a.a_stride = c.ostride[3];
-        a.width = c.dw; a.height = c.dh; a.chroma_format = c.chroma;
-        a.src_w = c.ow; a.src_h = c.oh; a.gather = c.scaled();
-        a.out = c.ext_rgb ? c.ext_rgb : (uint8_t*)b->d_rgb.p + c.rgb_off;
-        a.out_stride = (long long)(c.ext_rgb ? c.ext_stride : c.rgb_stride);
-        a.p = params[i];
+        cb.a[cb.n++] = csc_args(b, c, params[i]);
         c.converted = true;
       }
       if (cb.n == hc::CSC_BATCH_MAX || (i == n && cb.n > 0)) {
@@ -1244,12 +1245,12 @@ int hc_batch_read_plane(hc_batch* b, int canvas, int plane, void* dst, size_t ds
     return HC_ERR_ARGUMENT;
   }
   const Canvas& c = b->canvases[canvas];
-  if (c.pw[plane] == 0 || (plane == 3 && !c.alpha)) { hc::set_last_error("canvas has no such plane"); return HC_ERR_ARGUMENT; }
+  if (int rc = check_view_plane(c, plane)) return rc;
   const int ps = c.bit_depth == 8 ? 1 : 2;
   cudaEvent_t e0 = b->ev_d2h[0], e1 = b->ev_d2h[1];
   cudaEventRecord(e0, b->stream);
-  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_planes.p + c.ooff[plane], (size_t)c.ostride[plane] * ps,
-                                    (size_t)c.opw[plane] * ps, c.oph[plane], cudaMemcpyDeviceToHost, b->stream);
+  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_planes.p + c.view.off[plane], (size_t)c.view.stride[plane] * ps,
+                                    (size_t)c.view.w[plane] * ps, c.view.h[plane], cudaMemcpyDeviceToHost, b->stream);
   cudaEventRecord(e1, b->stream);
   if (!cuda_ok(e, "cudaMemcpy2DAsync(D2H plane)")) return HC_ERR_CUDA;
   if (int rc = batch_sync_checked(b, "cudaStreamSynchronize")) return rc;
@@ -1266,27 +1267,29 @@ int hc_batch_read_planes(hc_batch* b, int canvas, int nplanes, void* const* dst,
     return HC_ERR_ARGUMENT;
   }
   const Canvas& c = b->canvases[canvas];
+  const Planes& v = c.view;
   const int ps = c.bit_depth == 8 ? 1 : 2;
   size_t off[4] = {0, 0, 0, 0}, total = 0;
   for (int k = 0; k < nplanes; k++) {
-    if (c.opw[k] == 0 || (k == 3 && !c.alpha) || !dst[k]) { hc::set_last_error("canvas has no such plane"); return HC_ERR_ARGUMENT; }
+    if (!dst[k]) { hc::set_last_error("hc_batch_read_planes: bad argument"); return HC_ERR_ARGUMENT; }
+    if (int rc = check_view_plane(c, k)) return rc;
     off[k] = total;
-    total += align_up((size_t)c.opw[k] * ps * c.oph[k], 256);
+    total += align_up((size_t)v.w[k] * ps * v.h[k], 256);
   }
   Block stage = b->eng->take(b->eng->free_pin, total, true);
   if (!stage.p) return HC_ERR_MEMORY;
   cudaEventRecord(b->ev_d2h[0], b->stream);
   cudaError_t e = cudaSuccess;
   for (int k = 0; k < nplanes && e == cudaSuccess; k++)
-    e = cudaMemcpy2DAsync((uint8_t*)stage.p + off[k], (size_t)c.opw[k] * ps, (const uint8_t*)b->d_planes.p + c.ooff[k], (size_t)c.ostride[k] * ps,
-                          (size_t)c.opw[k] * ps, c.oph[k], cudaMemcpyDeviceToHost, b->stream);
+    e = cudaMemcpy2DAsync((uint8_t*)stage.p + off[k], (size_t)v.w[k] * ps, (const uint8_t*)b->d_planes.p + v.off[k], (size_t)v.stride[k] * ps,
+                          (size_t)v.w[k] * ps, v.h[k], cudaMemcpyDeviceToHost, b->stream);
   cudaEventRecord(b->ev_d2h[1], b->stream);
   int rc = cuda_ok(e, "cudaMemcpy2DAsync(D2H planes)") ? batch_sync_checked(b, "cudaStreamSynchronize") : HC_ERR_CUDA;
   if (rc == HC_OK) {
     for (int k = 0; k < nplanes; k++) {
-      const size_t row = (size_t)c.opw[k] * ps;
+      const size_t row = (size_t)v.w[k] * ps;
       const uint8_t* src = (const uint8_t*)stage.p + off[k];
-      for (int y = 0; y < c.oph[k]; y++) memcpy((uint8_t*)dst[k] + (size_t)y * dst_strides[k], src + (size_t)y * row, row);
+      for (int y = 0; y < v.h[k]; y++) memcpy((uint8_t*)dst[k] + (size_t)y * dst_strides[k], src + (size_t)y * row, row);
     }
     cudaEventElapsedTime(&b->last_d2h_ms, b->ev_d2h[0], b->ev_d2h[1]);
   }
@@ -1295,34 +1298,15 @@ int hc_batch_read_planes(hc_batch* b, int canvas, int nplanes, void* const* dst,
 }
 
 int hc_batch_read_rgb(hc_batch* b, int canvas, void* dst, size_t dst_stride) {
-  if (!b || !dst || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_read_rgb: bad argument"); return HC_ERR_ARGUMENT; }
-  const Canvas& c = b->canvases[canvas];
-  if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
-  if (c.ext_rgb) { hc::set_last_error("this image is written to an external RGB target (hc_batch_set_rgb_target): read it there"); return HC_ERR_ARGUMENT; }
-  if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are read with the stride of the Y row"); return HC_ERR_ARGUMENT; }
-  cudaEvent_t e0 = b->ev_d2h[0], e1 = b->ev_d2h[1];
-  cudaEventRecord(e0, b->stream);
-  cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream)
-                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
-                                               cudaMemcpyDeviceToHost, b->stream);
-  cudaEventRecord(e1, b->stream);
-  if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2H planes)" : "cudaMemcpy2DAsync(D2H rgb)")) return HC_ERR_CUDA;
+  if (int rc = enqueue_output_copy(b, "hc_batch_read_rgb", canvas, dst, dst_stride, cudaMemcpyDeviceToHost, true)) return rc;
   if (int rc = batch_sync_checked(b, "cudaStreamSynchronize")) return rc;
-  cudaEventElapsedTime(&b->last_d2h_ms, e0, e1);
+  cudaEventElapsedTime(&b->last_d2h_ms, b->ev_d2h[0], b->ev_d2h[1]);
   return HC_OK;
 }
 
 int hc_batch_copy_rgb_device(hc_batch* b, int canvas, void* dst, size_t dst_stride) {
-  if (!b || !dst || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_copy_rgb_device: bad argument"); return HC_ERR_ARGUMENT; }
-  const Canvas& c = b->canvases[canvas];
-  if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
-  if (c.ext_rgb) { hc::set_last_error("this image is written to an external RGB target (hc_batch_set_rgb_target)"); return HC_ERR_ARGUMENT; }
-  if (c.planar && dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are copied with the stride of the Y row"); return HC_ERR_ARGUMENT; }
   // cudaMemcpyDefault: `dst` may live on a peer device (unified addressing; a peer copy over NVLink then)
-  cudaError_t e = c.planar ? cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDefault, b->stream)
-                           : cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
-                                               cudaMemcpyDefault, b->stream);
-  if (!cuda_ok(e, c.planar ? "cudaMemcpyAsync(D2D planes)" : "cudaMemcpy2DAsync(D2D rgb)")) return HC_ERR_CUDA;
+  if (int rc = enqueue_output_copy(b, "hc_batch_copy_rgb_device", canvas, dst, dst_stride, cudaMemcpyDefault, false)) return rc;
   return batch_sync_checked(b, "cudaStreamSynchronize");
 }
 
@@ -1351,17 +1335,7 @@ extern "C" float hc_batch_async_d2h_ms(hc_batch* b) {
 }
 
 int hc_batch_read_rgb_async(hc_batch* b, int canvas, void* dst, size_t dst_stride) {
-  if (!b || !dst || canvas < 0 || canvas >= (int)b->canvases.size()) { hc::set_last_error("hc_batch_read_rgb_async: bad argument"); return HC_ERR_ARGUMENT; }
-  const Canvas& c = b->canvases[canvas];
-  if (!c.converted) { hc::set_last_error("canvas was not converted"); return HC_ERR_ARGUMENT; }
-  if (c.planar) {
-    if (dst_stride != c.rgb_stride) { hc::set_last_error("HC_OUT_YCBCR: the packed planes are read with the stride of the Y row"); return HC_ERR_ARGUMENT; }
-    return cuda_ok(cudaMemcpyAsync(dst, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.packed, cudaMemcpyDeviceToHost, b->stream), "cudaMemcpyAsync(D2H planes)")
-               ? HC_OK : HC_ERR_CUDA;
-  }
-  cudaError_t e = cudaMemcpy2DAsync(dst, dst_stride, (const uint8_t*)b->d_rgb.p + c.rgb_off, c.rgb_stride, (size_t)c.dw * c.rgb_bpp, c.dh,
-                                    cudaMemcpyDeviceToHost, b->stream);
-  return cuda_ok(e, "cudaMemcpy2DAsync(D2H rgb)") ? HC_OK : HC_ERR_CUDA;
+  return enqueue_output_copy(b, "hc_batch_read_rgb_async", canvas, dst, dst_stride, cudaMemcpyDeviceToHost, false);
 }
 
 int hc_batch_add_overlay_canvas(hc_batch* b, int width, int height, const uint16_t background[4]) {

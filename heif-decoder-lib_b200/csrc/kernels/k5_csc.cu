@@ -341,11 +341,6 @@ __device__ __forceinline__ void csc_unit(const CscArgs& a, unsigned tid) {
   }
 }
 
-template <typename Pixel, bool GATHER>
-__global__ void __launch_bounds__(256) k5_csc_kernel(CscArgs a) {
-  csc_unit<Pixel, GATHER>(a, blockIdx.x * blockDim.x + threadIdx.x);
-}
-
 // All canvases of a batch in one launch (blockIdx.y = canvas): a 12 MP canvas is a ~10 us kernel at HBM speed, so
 // per-canvas launches are dominated by launch gaps and tails.
 template <typename Pixel, bool GATHER>
@@ -419,19 +414,6 @@ static bool k5_fast_path(const CscArgs& a, bool sixteen_bit) {
          (a.width & 7) == 0 && (a.height & 1) == 0 && (a.y_stride & 7) == 0 && (a.c_stride & 3) == 0 &&
          (reinterpret_cast<uintptr_t>(a.y) & 7) == 0 && (reinterpret_cast<uintptr_t>(a.cb) & 3) == 0 && (reinterpret_cast<uintptr_t>(a.cr) & 3) == 0 &&
          (a.out_stride & 7) == 0 && (reinterpret_cast<uintptr_t>(a.out) & 7) == 0;
-}
-
-void launch_k5(const CscArgs& a, bool sixteen_bit, cudaStream_t stream) {
-  const long long n = (long long)((a.width + 7) >> 3) * a.height;
-  if (n <= 0) return;
-  const unsigned grid = (unsigned)((n + 255) / 256);
-  if (a.gather) {
-    if (sixteen_bit) k5_csc_kernel<uint16_t, true><<<grid, 256, 0, stream>>>(a);
-    else k5_csc_kernel<uint8_t, true><<<grid, 256, 0, stream>>>(a);
-  } else {
-    if (sixteen_bit) k5_csc_kernel<uint16_t, false><<<grid, 256, 0, stream>>>(a);
-    else k5_csc_kernel<uint8_t, false><<<grid, 256, 0, stream>>>(a);
-  }
 }
 
 void launch_k5_batch(const CscBatch& b, bool sixteen_bit, cudaStream_t stream) {

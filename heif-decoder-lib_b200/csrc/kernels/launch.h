@@ -96,7 +96,6 @@ int k2_task_smem_bytes(int ctb_w, int ctb_h, int pixel_bytes);
 void launch_k2(const BatchView& bv, const RowTask* tasks, const WarpWork* work, int nctas, int smem_bytes, int* progress, cudaStream_t stream);
 void launch_k3(const BatchView& bv, long long max_units, int planes, cudaStream_t stream);
 void launch_k4(const BatchView& bv, long long max_ctbs, int planes, cudaStream_t stream);
-void launch_k5(const CscArgs& a, bool sixteen_bit, cudaStream_t stream);
 void launch_k5_batch(const CscBatch& b, bool sixteen_bit, cudaStream_t stream);
 void launch_k6(const XformArgs& a, bool sixteen_bit, cudaStream_t stream);
 // nearest-neighbour rescale of one plane (strides in samples): dst(x, y) = src(x * sw / dw, y * sh / dh)

@@ -321,13 +321,18 @@ int hc_batch_set_canvas_output_size(hc_batch* b, int canvas, int width, int heig
  * (Op_YCbCr_to_RGB<uint8_t>). Children must be 8-bit 4:4:4 canvases (the reference converts nothing else) with offsets >= 0. */
 int hc_batch_add_overlay_canvas(hc_batch* b, int width, int height, const uint16_t background[4]);
 int hc_batch_overlay_add_child(hc_batch* b, int overlay_canvas, int child_canvas, int dx, int dy, const hc_csc_params* child_params);
-/* K5 for one canvas into the engine's device RGB buffer, async. A canvas whose params have out_format == HC_OUT_YCBCR goes to
- * K8 instead, which packs the canvas' output planes into the same buffer in the layout of HC_OUT_YCBCR. Overlay canvases
- * (hc_batch_add_overlay_canvas) and canvases with an external RGB target (hc_batch_set_rgb_target) cannot be planar:
- * HC_ERR_UNSUPPORTED. */
-int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params);
-/* K5 / K8 for n canvases (canvases[i] with params[i]) in as few launches as possible, async */
+/* K5 / K7 / K8 for n canvases (canvases[i] with params[i]) in as few launches as possible, async. K5 converts a canvas into
+ * the batch's device RGB buffer, K7 composes an overlay canvas (hc_batch_add_overlay_canvas) there; a canvas whose params have
+ * out_format == HC_OUT_YCBCR goes to K8 instead, which packs the canvas' output planes into the same buffer in the layout of
+ * HC_OUT_YCBCR. Overlay canvases and canvases with an external RGB target (hc_batch_set_rgb_target) cannot be planar:
+ * HC_ERR_UNSUPPORTED.
+ * The buffer holds one block per canvas in canvas order, sized by the canvas' output format (8 bytes per pixel before its
+ * first conversion). A call lays out anew the canvases it names and those not converted yet; a converted canvas it does not
+ * name keeps its block and its bytes. When the new layout would move such a canvas, or the buffer would have to grow while one
+ * exists, the call fails with HC_ERR_ARGUMENT and changes nothing: convert it again in the same call. */
 int hc_batch_convert_many(hc_batch* b, int n, const int* canvases, const hc_csc_params* params);
+/* hc_batch_convert_many for one canvas */
+int hc_batch_convert(hc_batch* b, int canvas, const hc_csc_params* params);
 int hc_batch_sync(hc_batch* b);
 /* D2H reads (synchronous). plane: 0 Y, 1 Cb, 2 Cr, 3 alpha. Samples are 1 byte for 8-bit canvases,
  * 2 bytes little-endian otherwise. */

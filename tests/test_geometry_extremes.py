@@ -502,7 +502,7 @@ def test_gpu_overlay_geometry_and_blending(engine):
     """K7: children clipped at the right / bottom edge with 1 and 0 samples left, a 1 x 1 child, children wholly outside,
     16 overlapping children in order, alpha children (mutated alpha: 0, 255 and between), GBR / YCgCo / matrix children in
     full and limited range, background words whose low bytes are dropped, 1 x N and N x 1 canvases, every interleaved
-    output format."""
+    output format; through hc_batch_convert_many and hc_batch_convert."""
     rec, planes = picture(3, 8, seed=12)
     arec, aplanes = picture(0, 8, seed=13)
     assert aplanes[0].min() == 0 and aplanes[0].max() == 255
@@ -533,12 +533,15 @@ def test_gpu_overlay_geometry_and_blending(engine):
         params = [hb.csc_select(2, 2, 1, 3, 8, False, j[1]) for j in jobs]
         api.check(b._L, b._L.hc_batch_convert_many(b._h, n, (C.c_int * n)(*[j[0] for j in jobs]), (CscParams * n)(*params)),
                   "hc_batch_convert_many")
-        for o, fmt, W, H, want, kids in jobs:
-            got = np.empty_like(want)
-            api.check(b._L, b._L.hc_batch_read_rgb(b._h, o, got.ctypes.data, got.strides[0]), "read_rgb")
-            nd, at = first_diff(got, want)
-            assert nd == 0, "overlay %dx%d format %d children (dx, dy, conversion)=%s: %d bytes differ, first at %s" % (
-                W, H, fmt, kids, nd, at)
+        for single in (False, True):      # then each canvas again through hc_batch_convert
+            for (o, fmt, W, H, want, kids), p in zip(jobs, params):
+                if single:
+                    b.convert(o, p)
+                got = np.empty_like(want)
+                api.check(b._L, b._L.hc_batch_read_rgb(b._h, o, got.ctypes.data, got.strides[0]), "read_rgb")
+                nd, at = first_diff(got, want)
+                assert nd == 0, "overlay %dx%d format %d children (dx, dy, conversion)=%s single=%s: %d bytes differ, first at %s" % (
+                    W, H, fmt, kids, single, nd, at)
     finally:
         b.close()
 

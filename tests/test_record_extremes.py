@@ -41,7 +41,7 @@ K5_PICTURES = ("mono_8", "mono_12", "base_420_8", "c420_10", "c420_12", "c422_8"
                "c444_10")
 # (matrix_coefficients, colour_primaries): the primaries only matter to matrices 12 and 13
 K5_MATRICES = ((0, 1), (1, 1), (2, 1), (5, 1), (6, 1), (9, 1), (10, 1), (12, 1), (12, 9), (13, 1), (13, 9))
-# widest output first: hc_batch_convert may only grow the RGB buffer before any canvas of the batch was converted
+# in any order: the K5 batch below has one canvas, and a convert lays out anew the block of the canvas it names
 K5_OUT_FORMATS = (hb.OUT_RRGGBBAA_BE, hb.OUT_RRGGBBAA_LE, hb.OUT_RRGGBB_BE, hb.OUT_RRGGBB_LE, hb.OUT_RGBA, hb.OUT_RGB)
 
 
@@ -251,12 +251,20 @@ def test_gpu_k5_every_conversion_matches_oracle(engine, name, with_alpha):
         b.close()
 
 
+def first_conversion(cases, planes, cf, out):
+    """(params, oracle bytes) of the first of an 8-bit canvas' csc_cases to `out` that the oracle converts"""
+    for case, params in cases:
+        want = oracle_rgb(planes, None, cf, 8, case) if case[3] == out else None
+        if want is not None:
+            return params, want
+
+
 @pytest.mark.gpu
 def test_gpu_k5_convert_many_mixed_canvases(engine):
     """One hc_batch_convert_many call (the form hc_heic_job uses) over canvases of every format, depth and alpha, each
-    with its own conversion."""
+    with its own conversion; before it, single converts whose layout would move a canvas converted earlier."""
     b = engine.batch()
-    jobs = []
+    jobs, seq = [], []
     for i, name in enumerate(K5_PICTURES):
         rec = mutated("gen:" + name, "all", 2)
         p = rec.pic
@@ -279,9 +287,21 @@ def test_gpu_k5_convert_many_mixed_canvases(engine):
                 break
             k += 1
         jobs.append((name, c, case, params, want))
+        if i in (0, 2):   # 8-bit canvases without alpha for the convert sequence below
+            seq.append((c, {out: first_conversion(cases, planes, p.chroma_format, out) for out in (hb.OUT_RGBA, hb.OUT_RGB)}))
     try:
         b.upload()
         b.reconstruct(hb.STAGE_ALL)
+        # convert c0 to RGBA, c1 to RGB, c0 to RGB: the narrower c0 would move c1's block, so the last call either fails and
+        # changes nothing or leaves c1 where it was
+        (c0, f0), (c1, f1) = seq
+        b.convert(c0, f0[hb.OUT_RGBA][0])
+        b.convert(c1, f1[hb.OUT_RGB][0])
+        rc = engine._L.hc_batch_convert(b._h, c0, C.byref(f0[hb.OUT_RGB][0]))
+        assert rc in (0, -2), rc      # HC_OK, HC_ERR_ARGUMENT
+        assert np.array_equal(b.read_rgb(c1, hb.OUT_RGB), f1[hb.OUT_RGB][1])
+        fmt0 = hb.OUT_RGB if rc == 0 else hb.OUT_RGBA
+        assert np.array_equal(b.read_rgb(c0, fmt0), f0[fmt0][1])
         canv = (C.c_int * len(jobs))(*[j[1] for j in jobs])
         params = (hb.CscParams * len(jobs))(*[j[3] for j in jobs])
         api.check(engine._L, engine._L.hc_batch_convert_many(b._h, len(jobs), canv, params), "hc_batch_convert_many")
