@@ -20,6 +20,7 @@
 // Layout of a K0 picture: every CTB owns fixed-capacity slices of the picture's blk / tb / coeff / residual
 // regions (worst case of a CTB), so chains never allocate.
 #pragma once
+#include <cstring>
 #include "common.cuh"
 
 // functions that must stay real calls: the syntax tree recursion is unrolled by templates and would otherwise
@@ -135,14 +136,6 @@ HC_D void progress_store(int* p, int v) {
   __syncwarp();
   if ((threadIdx.x & 31) == 0) st_release_s32(p, v);
 }
-// the lanes of a warp that run the same chain (warp-uniform execution) reserve once
-HC_D unsigned list_reserve(unsigned int* counter, unsigned n) {
-  const unsigned m = __activemask();
-  const int leader = __ffs((int)m) - 1;
-  unsigned r = 0;
-  if ((int)(threadIdx.x & 31) == leader) r = atomicAdd(counter, n);
-  return __shfl_sync(m, r, leader);
-}
 // A waiting chain polls a progress word of the row above. A CTB takes milliseconds to parse, so the poll interval grows
 // to ~16 us: the first version polled every ~80 ns (__nanosleep(400) returns much earlier than asked), and the wait loops
 // of the chains that cannot start yet issued as many instructions — and L2 requests on a handful of hot words — as all
@@ -155,7 +148,6 @@ HC_HD int k0_popc(unsigned v) { return __builtin_popcount(v); }
 HC_HD int k0_ctz(unsigned v) { return __builtin_ctz(v); }
 HC_HD int progress_load(const int* p) { return *p; }
 HC_HD void progress_store(int* p, int v) { *p = v; }
-HC_HD unsigned list_reserve(unsigned int* counter, unsigned n) { const unsigned r = *counter; *counter += n; return r; }
 HC_HD void backoff(unsigned&) {}
 HC_HD void far_wait() {}
 #endif
@@ -174,8 +166,23 @@ struct alignas(16) CabState {
   const uint8_t* end;
   uint32_t pad[2];
 };
+// The parse state of the chain: CTB position, record counters of the current CTB, QG / QP and CU state. It lives in the
+// Scratch rather than in the parser object: the parser's syntax functions are real calls, and a stack object reached
+// through `this` turns every access into a local- or generic-memory one (run_chain zeroes it).
+struct ChainState {
+  int err;
+  int ctb_rs, ctb_x, ctb_y;
+  uint32_t nblk[3], ntb, ncoeff, nresid;       // used inside the current CTB
+  int IsCuQpDeltaCoded, CuQpDeltaVal;
+  int currentQG_x, currentQG_y, lastQPYinPreviousQG, currentQPY;
+  int qPYPrime, qPCbPrime, qPCrPrime;
+  int cu_x0, cu_y0, cu_log2;
+  int cu_max_trafo_depth, cu_intra_split;      // of the current CU, read by every level of its transform tree
+  int filterLeftCbEdge, filterTopCbEdge;
+};
 struct Scratch {
   CabState cab;
+  ChainState cs;
   uint8_t ctx[CTX_BYTES];            // CABAC context states
   Pic pic;                           // copy of the picture descriptor
   Slice slice;                       // copy of the current slice segment descriptor
@@ -186,6 +193,10 @@ constexpr int TABLE_BYTES = (int)((sizeof(Tables) + 15) & ~(size_t)15);
 constexpr int SCRATCH_BYTES = (int)((sizeof(Scratch) + 15) & ~(size_t)15);
 #if defined(__CUDACC__)
 extern __shared__ __align__(16) uint8_t k0_smem[];   // [Tables][Scratch x warps of the CTA]
+// Byte offset of the calling warp's Scratch in k0_smem. The device parser derives every address from it instead of
+// keeping one in the parser object: that object is a stack variable of the kernel, so each syntax function (a real call)
+// had to read it back from local memory and keep `this` live across its calls.
+HC_D uint32_t scratch_offset() { return (uint32_t)TABLE_BYTES + (threadIdx.x >> 5) * (uint32_t)SCRATCH_BYTES; }
 #endif
 
 // ---- arithmetic decoder: same design as host/hevc_cabac.h (offset + look-ahead in one 64-bit register) --------
@@ -463,16 +474,17 @@ static __device__ __noinline__ int cab_terminate(uint32_t sa) {
 #undef K0_CAB_REFILL
 #undef K0_CAB_STORE
 
-// Same interface as Cabac; its only state are the two shared-space addresses (set once per chain, k0_parse.cu), so
-// copying it in and out of the hot functions is free.
+// Same interface as Cabac, without state of its own: `sa` = shared-space address of the warp's CabState (the Scratch
+// starts with it), `ta` = of the CTA's Tables. Copying it in and out of the hot functions is free.
 struct CabacDev {
-  uint32_t sa, ta;
-  HC_D CabState& state() const { return *reinterpret_cast<CabState*>(__cvta_shared_to_generic(sa)); }
+  HC_D static uint32_t ta() { return (uint32_t)__cvta_generic_to_shared(k0_smem); }
+  HC_D static uint32_t sa() { return ta() + scratch_offset(); }
+  HC_D CabState& state() const { return *reinterpret_cast<CabState*>(k0_smem + scratch_offset()); }
   HC_D void init(const uint8_t* p, const uint8_t* e) {
     CabState& c = state();
     c.start = p; c.end = e; c.next = p;
     c.range = 510;
-    c.value = cab_next32(sa);
+    c.value = cab_next32(sa());
     c.avail = 32 - 9;
   }
   HC_D const uint8_t* position() const {
@@ -481,12 +493,12 @@ struct CabacDev {
     return c.start + 2 + (shifts >> 3);
   }
   HC_D bool overrun() const { return position() > state().end; }
-  HC_D int bin(const Tables&, uint8_t*, int i) { return cab_bin(sa, ta, i); }
-  HC_D int bypass() { return cab_bypass(sa); }
-  HC_D uint32_t bypass_bits(const Tables&, int n) { return cab_bypass_bits(sa, ta, n); }
-  HC_D uint32_t peek16(const Tables&) const { return cab_peek16(sa, ta); }
-  HC_D void consume(int n, uint32_t bins) { cab_consume(sa, n, bins); }
-  HC_D int terminate() { return cab_terminate(sa); }
+  HC_D int bin(const Tables&, uint8_t*, int i) { return cab_bin(sa(), ta(), i); }
+  HC_D int bypass() { return cab_bypass(sa()); }
+  HC_D uint32_t bypass_bits(const Tables&, int n) { return cab_bypass_bits(sa(), ta(), n); }
+  HC_D uint32_t peek16(const Tables&) const { return cab_peek16(sa(), ta()); }
+  HC_D void consume(int n, uint32_t bins) { cab_consume(sa(), n, bins); }
+  HC_D int terminate() { return cab_terminate(sa()); }
 };
 #endif
 #if defined(__CUDA_ARCH__)
@@ -565,28 +577,25 @@ HC_HD void finish_ctb(const Pic& p, int ctb, int lane, int stride) {
     for (int k = lane; k < (int)ctu.blk_count[c]; k += stride) finish_blk(p, p.blks[ctu.blk_first[c] + k]);
 }
 
+// One 16-byte record (hc_tb, hc_blk) from four words held in registers: one vector store on the device.
+HC_HD void store_rec16(void* dst, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+#if defined(__CUDA_ARCH__)
+  *reinterpret_cast<uint4*>(dst) = make_uint4(w0, w1, w2, w3);   // the record arrays are 16-byte aligned
+#else
+  const uint32_t w[4] = {w0, w1, w2, w3};
+  memcpy(dst, w, 16);
+#endif
+}
+static_assert(sizeof(hc_tb) == 16 && sizeof(hc_blk) == 16, "records are stored as four words");
+
 // ---- the parser of one chain ---------------------------------------------------------------------------------
+// All parse state is in the chain's Scratch (cs()).
 struct Parser {
-  // host build: the tables, picture, slice segment and scratch are reached through these pointers; the device build
-  // reaches its copies in shared memory through `wbase` (tab() / pic() / slice() / scratch() below)
+  // host build: the tables and the scratch are reached through these pointers and the decoder is a member; the device
+  // build finds its copies in shared memory from the warp index (scratch_offset()), and CabacDev is empty
   const Tables* T;
-  const Pic* P;
-  const Slice* sh;
   Scratch* S;
-  uint32_t wbase;          // device: byte offset of this chain's Scratch in k0_smem
   CabacT cabac;
-  int err;
-  // CTB state
-  int ctb_rs, ctb_x, ctb_y;
-  int slice_addr;          // slice_addr_rs of the current slice
-  uint32_t nblk[3], ntb, ncoeff, nresid;       // used inside the current CTB
-  // CU / QG state
-  bool IsCuQpDeltaCoded;
-  int CuQpDeltaVal;
-  int currentQG_x, currentQG_y, lastQPYinPreviousQG, currentQPY;
-  int qPYPrime, qPCbPrime, qPCrPrime;
-  int cu_x0, cu_y0, cu_log2;
-  int filterLeftCbEdge, filterTopCbEdge;
 
   // Device: the 32 lanes of a warp execute the parser with identical data (warp-uniform: one instruction issue serves all
   // of them) and share out the data-parallel loops: `for (i = lane(); i < n; i += K0_LANES)`. After such a loop whose
@@ -596,7 +605,7 @@ struct Parser {
   HC_HD int lane() const { return (int)(threadIdx.x & 31); }
   HC_HD void lanes_sync() const { __syncwarp(); }
   HC_HD const Tables& tab() const { return *reinterpret_cast<const Tables*>(k0_smem); }
-  HC_HD Scratch& scratch() const { return *reinterpret_cast<Scratch*>(k0_smem + wbase); }
+  HC_HD Scratch& scratch() const { return *reinterpret_cast<Scratch*>(k0_smem + scratch_offset()); }
 #else
   static constexpr int K0_LANES = 1;
   HC_HD int lane() const { return 0; }
@@ -607,9 +616,11 @@ struct Parser {
   HC_HD const Pic& pic() const { return scratch().pic; }
   HC_HD const Slice& slice() const { return scratch().slice; }
   HC_HD uint8_t* ctxs() const { return scratch().ctx; }
+  HC_HD ChainState& cs() const { return scratch().cs; }
 
   HC_HD int bin(int c) { return cabac.bin(tab(), ctxs(), c); }
-  HC_HD void fail(int code) { if (!err) err = code; }
+  HC_HD int err() const { return cs().err; }
+  HC_HD void fail(int code) { ChainState& c = cs(); if (!c.err) c.err = code; }
   HC_HD void init_contexts() {
     const Tables& t = tab();
     uint8_t* ctx = ctxs();
@@ -641,14 +652,16 @@ struct Parser {
   }
 
   // ---- 7.3.8.3 SAO ----
-  K0_FN void read_sao(hc_ctu& ctu) {
+  K0_FN void read_sao() {
     const Pic& p = pic();
     const Tables& t = tab();
     uint8_t* const ctx = ctxs();
     CabacT cb = cabac;
+    const int ctb_rs = cs().ctb_rs;
+    hc_ctu& ctu = p.ctus[ctb_rs];
     bool merge_left = false, merge_up = false;
-    if (ctb_x > 0 && slice_addr_of_ctb(ctb_rs - 1) == slice().slice_addr_rs) merge_left = cb.bin(t, ctx, CX_SAO_MERGE);
-    if (ctb_y > 0 && !merge_left && slice_addr_of_ctb(ctb_rs - p.ctbs_w) == slice().slice_addr_rs) merge_up = cb.bin(t, ctx, CX_SAO_MERGE);
+    if (cs().ctb_x > 0 && slice_addr_of_ctb(ctb_rs - 1) == slice().slice_addr_rs) merge_left = cb.bin(t, ctx, CX_SAO_MERGE);
+    if (cs().ctb_y > 0 && !merge_left && slice_addr_of_ctb(ctb_rs - p.ctbs_w) == slice().slice_addr_rs) merge_up = cb.bin(t, ctx, CX_SAO_MERGE);
     if (merge_left || merge_up) {
       const hc_ctu& src = p.ctus[merge_left ? ctb_rs - 1 : ctb_rs - p.ctbs_w];
       K0_LOOP for (int c = 0; c < 3; c++) {
@@ -674,26 +687,29 @@ struct Parser {
       if (ctu.sao_type[c] == 0) continue;
       const int bitDepth = c == 0 ? p.bit_depth_y : p.bit_depth_c;
       const int cMax = (1 << ((bitDepth < 10 ? bitDepth : 10) - 5)) - 1;
-      int absv[4];
+      uint32_t absv = 0;   // the four magnitudes (<= 31), 8 bits each
       K0_LOOP for (int i = 0; i < 4; i++) {
         int v = 0;
         K0_LOOP while (v < cMax && cb.bypass()) v++;
-        absv[i] = v;
+        absv |= (uint32_t)v << (8 * i);
       }
       const int scale = c == 0 ? p.log2_sao_offset_scale_luma : p.log2_sao_offset_scale_chroma;
       if (ctu.sao_type[c] == 1) {
-        int sign[4] = {0, 0, 0, 0};
+        uint32_t sign = 0;   // bit i: offset i is negative
         K0_LOOP for (int i = 0; i < 4; i++)
-          if (absv[i]) sign[i] = cb.bypass();
+          if ((absv >> (8 * i)) & 0xffu) sign |= (uint32_t)cb.bypass() << i;
         ctu.sao_band_or_class[c] = (uint8_t)cb.bypass_bits(t, 5);
-        K0_LOOP for (int i = 0; i < 4; i++) ctu.sao_offset[c][i] = (int8_t)((sign[i] ? -absv[i] : absv[i]) * (1 << scale));
+        K0_LOOP for (int i = 0; i < 4; i++) {
+          const int a = (int)((absv >> (8 * i)) & 0xffu);
+          ctu.sao_offset[c][i] = (int8_t)((((sign >> i) & 1u) ? -a : a) * (1 << scale));
+        }
       } else {
         if (c < 2) ctu.sao_band_or_class[c] = (uint8_t)cb.bypass_bits(t, 2);
         else ctu.sao_band_or_class[2] = ctu.sao_band_or_class[1];
-        ctu.sao_offset[c][0] = (int8_t)(absv[0] * (1 << scale));
-        ctu.sao_offset[c][1] = (int8_t)(absv[1] * (1 << scale));
-        ctu.sao_offset[c][2] = (int8_t)(-absv[2] * (1 << scale));
-        ctu.sao_offset[c][3] = (int8_t)(-absv[3] * (1 << scale));
+        K0_LOOP for (int i = 0; i < 4; i++) {
+          const int a = (int)((absv >> (8 * i)) & 0xffu);
+          ctu.sao_offset[c][i] = (int8_t)((i < 2 ? a : -a) * (1 << scale));
+        }
       }
     }
     cabac = cb;
@@ -702,24 +718,25 @@ struct Parser {
   // ---- 8.6.1 QP derivation (transform.cc:31-210 bookkeeping) ----
   K0_FN void derive_qp(int xCU, int yCU) {
     const Pic& p = pic();
+    ChainState& s = cs();
     const int qgmask = (1 << p.log2_min_cu_qp_delta_size) - 1;
     const int xQG = xCU - (xCU & qgmask), yQG = yCU - (yCU & qgmask);
-    if (xQG != currentQG_x || yQG != currentQG_y) {
-      lastQPYinPreviousQG = currentQPY;
-      currentQG_x = xQG;
-      currentQG_y = yQG;
+    if (xQG != s.currentQG_x || yQG != s.currentQG_y) {
+      s.lastQPYinPreviousQG = s.currentQPY;
+      s.currentQG_x = xQG;
+      s.currentQG_y = yQG;
     }
     const int ctbmask = (1 << p.log2_ctb) - 1;
     const bool firstInCTBRow = (xQG == 0 && (yQG & ctbmask) == 0);
     const int sx = (slice().slice_addr_rs % p.ctbs_w) << p.log2_ctb, sy = (slice().slice_addr_rs / p.ctbs_w) << p.log2_ctb;
     const bool firstQGInSlice = (sx == xQG && sy == yQG);
-    int pred = (firstQGInSlice || (firstInCTBRow && p.entropy_coding_sync)) ? slice().slice_qp_y : lastQPYinPreviousQG;
+    int pred = (firstQGInSlice || (firstInCTBRow && p.entropy_coding_sync)) ? slice().slice_qp_y : s.lastQPYinPreviousQG;
     int qA = pred, qB = pred;
-    if (available_zscan(xQG, yQG, xQG - 1, yQG) && ctb_of(xQG - 1, yQG) == ctb_rs) qA = p.qp_map[((xQG - 1) >> 3) + (yQG >> 3) * p.w8];
-    if (available_zscan(xQG, yQG, xQG, yQG - 1) && ctb_of(xQG, yQG - 1) == ctb_rs) qB = p.qp_map[(xQG >> 3) + ((yQG - 1) >> 3) * p.w8];
+    if (available_zscan(xQG, yQG, xQG - 1, yQG) && ctb_of(xQG - 1, yQG) == s.ctb_rs) qA = p.qp_map[((xQG - 1) >> 3) + (yQG >> 3) * p.w8];
+    if (available_zscan(xQG, yQG, xQG, yQG - 1) && ctb_of(xQG, yQG - 1) == s.ctb_rs) qB = p.qp_map[(xQG >> 3) + ((yQG - 1) >> 3) * p.w8];
     pred = (qA + qB + 1) >> 1;
-    const int QPY = ((pred + CuQpDeltaVal + 52 + 2 * p.qp_bd_offset_y) % (52 + p.qp_bd_offset_y)) - p.qp_bd_offset_y;
-    qPYPrime = QPY + p.qp_bd_offset_y < 0 ? 0 : QPY + p.qp_bd_offset_y;
+    const int QPY = ((pred + s.CuQpDeltaVal + 52 + 2 * p.qp_bd_offset_y) % (52 + p.qp_bd_offset_y)) - p.qp_bd_offset_y;
+    s.qPYPrime = QPY + p.qp_bd_offset_y < 0 ? 0 : QPY + p.qp_bd_offset_y;
     const int qPiCb = clip3i(-p.qp_bd_offset_c, 57, QPY + p.pps_cb_qp_offset + slice().cb_qp_offset);
     const int qPiCr = clip3i(-p.qp_bd_offset_c, 57, QPY + p.pps_cr_qp_offset + slice().cr_qp_offset);
     int qPCb = qPiCb, qPCr = qPiCr;   // the reference does not cap non-4:2:0 at 51 (transform.cc:175-178)
@@ -727,23 +744,24 @@ struct Parser {
       qPCb = qPiCb < 30 ? qPiCb : (qPiCb >= 44 ? qPiCb - 6 : tab().qpc420[qPiCb - 30]);
       qPCr = qPiCr < 30 ? qPiCr : (qPiCr >= 44 ? qPiCr - 6 : tab().qpc420[qPiCr - 30]);
     }
-    qPCbPrime = qPCb + p.qp_bd_offset_c < 0 ? 0 : qPCb + p.qp_bd_offset_c;
-    qPCrPrime = qPCr + p.qp_bd_offset_c < 0 ? 0 : qPCr + p.qp_bd_offset_c;
-    const int l8 = cu_log2 > 3 ? cu_log2 - 3 : 0, n8 = 1 << l8;
+    s.qPCbPrime = qPCb + p.qp_bd_offset_c < 0 ? 0 : qPCb + p.qp_bd_offset_c;
+    s.qPCrPrime = qPCr + p.qp_bd_offset_c < 0 ? 0 : qPCr + p.qp_bd_offset_c;
+    const int l8 = s.cu_log2 > 3 ? s.cu_log2 - 3 : 0, n8 = 1 << l8;
     K0_LOOP for (int i = lane(); i < n8 * n8; i += K0_LANES) {
-      const int xx = (cu_x0 >> 3) + (i & (n8 - 1)), yy = (cu_y0 >> 3) + (i >> l8);
+      const int xx = (s.cu_x0 >> 3) + (i & (n8 - 1)), yy = (s.cu_y0 >> 3) + (i >> l8);
       if (xx < p.w8 && yy < p.h8) p.qp_map[xx + yy * p.w8] = (int8_t)QPY;
     }
     lanes_sync();
-    currentQPY = QPY;
+    s.currentQPY = QPY;
   }
 
   // every 4x4 unit belongs to exactly one transform unit and the map starts zeroed, so plain stores suffice
   HC_HD void mark_tu_edges(int x0, int y0, int log2) {
     if (slice().deblocking_disabled) return;
     const Pic& p = pic();
+    const ChainState& s = cs();
     const int n4 = (1 << log2) >> 2;
-    const int left = (x0 == cu_x0) ? filterLeftCbEdge : 1, top = (y0 == cu_y0) ? filterTopCbEdge : 1;
+    const int left = (x0 == s.cu_x0) ? s.filterLeftCbEdge : 1, top = (y0 == s.cu_y0) ? s.filterTopCbEdge : 1;
     uint8_t* e = p.edge_map + (x0 >> 2) + (y0 >> 2) * p.w4;
     const uint8_t fl = left ? HC_EDGE_V : 0, ft = top ? HC_EDGE_H : 0;
     if (fl | ft) e[0] = (uint8_t)(fl | ft);
@@ -760,21 +778,17 @@ struct Parser {
   // massively parallel pass (finish_blk below: k0_finish_kernel on the device) instead of by the serial chain.
   HC_HD void emit_blk(int cIdx, int xB, int yB, int log2, int mode, bool has_resid, uint32_t resid_off) {
     const Pic& p = pic();
-    if (nblk[cIdx] >= p.blk_cap[cIdx]) { fail(ERR_CAPACITY); return; }
-    uint32_t base = (uint32_t)ctb_rs * p.blk_cap_ctb;
+    ChainState& s = cs();
+    const uint32_t n = s.nblk[cIdx];
+    if (n >= p.blk_cap[cIdx]) { fail(ERR_CAPACITY); return; }
+    s.nblk[cIdx] = n + 1;
+    uint32_t base = (uint32_t)s.ctb_rs * p.blk_cap_ctb;
     if (cIdx > 0) base += p.blk_cap[0];
     if (cIdx > 1) base += p.blk_cap[1];
-    hc_blk b;
-    b.x = (uint16_t)xB;
-    b.y = (uint16_t)yB;
-    b.log2 = (uint8_t)log2;
-    b.mode = (uint8_t)mode;
-    b.flags = (uint8_t)(has_resid ? HC_BLK_HAS_RESID : 0);
-    b.cidx = (uint8_t)cIdx;
-    b.avail_left = 0;
-    b.avail_top = 0;
-    b.resid_off = has_resid ? resid_off : 0;
-    p.blks[base + nblk[cIdx]++] = b;
+    // hc_blk: x, y | log2, mode, flags, cidx | avail_left = avail_top = 0 | resid_off
+    store_rec16(p.blks + base + n, ((uint32_t)xB & 0xffffu) | ((uint32_t)yB << 16),
+                ((uint32_t)log2 & 0xffu) | (((uint32_t)mode & 0xffu) << 8) | ((has_resid ? HC_BLK_HAS_RESID : 0u) << 16) | ((uint32_t)cIdx << 24),
+                0u, has_resid ? resid_off : 0u);
   }
 
   // ---- 7.3.8.11 residual_coding ----
@@ -790,7 +804,7 @@ struct Parser {
     if (p.transform_skip_enabled && log2 <= p.log2_max_transform_skip_size) tskip = cb.bin(t, ctx, CX_TSKIP + (cIdx ? 1 : 0));
 
     // last significant coefficient position
-    int last[2];
+    int last_x = 0, last_y = 0;
     {
       const int cMax = (log2 << 1) - 1;
       int offset, shift;
@@ -800,12 +814,13 @@ struct Parser {
         int v = 0;
         const int base = (d ? CX_LAST_Y : CX_LAST_X) + offset;
         K0_LOOP while (v < cMax && cb.bin(t, ctx, base + (v >> shift))) v++;
-        last[d] = v;
+        if (d) last_y = v;
+        else last_x = v;
       }
     }
-    int LastX = last[0], LastY = last[1];
-    if (last[0] > 3) { const int nb = (last[0] >> 1) - 1; LastX = ((2 + (last[0] & 1)) << nb) + (int)cb.bypass_bits(t, nb); }
-    if (last[1] > 3) { const int nb = (last[1] >> 1) - 1; LastY = ((2 + (last[1] & 1)) << nb) + (int)cb.bypass_bits(t, nb); }
+    int LastX = last_x, LastY = last_y;
+    if (last_x > 3) { const int nb = (last_x >> 1) - 1; LastX = ((2 + (last_x & 1)) << nb) + (int)cb.bypass_bits(t, nb); }
+    if (last_y > 3) { const int nb = (last_y >> 1) - 1; LastY = ((2 + (last_y & 1)) << nb) + (int)cb.bypass_bits(t, nb); }
 
     int scanIdx = 0;
     if (log2 == 2 || (log2 == 3 && (cIdx == 0 || p.chroma_array_type == 3))) {
@@ -825,24 +840,18 @@ struct Parser {
     // coded_sub_block_flag of the right / lower neighbour, one bit per sub-block at Sx + 8 * Sy
     unsigned long long csbf_right = 0, csbf_below = 0;
 
-    if (ntb >= p.tb_cap_ctb || nresid + (uint32_t)(nT * nT) > p.resid_cap_ctb) { fail(ERR_CAPACITY); return 0; }
-    const uint32_t coeff_first = (uint32_t)ctb_rs * p.coeff_cap_ctb + ncoeff;
-    hc_coeff* out = p.coeffs + coeff_first;
-    const uint32_t coeff_room = p.coeff_cap_ctb - ncoeff;
+    {
+      const ChainState& s = cs();
+      if (s.ntb >= p.tb_cap_ctb || s.nresid + (uint32_t)(nT * nT) > p.resid_cap_ctb) { fail(ERR_CAPACITY); return 0; }
+    }
+    // the coefficient records of this block start at cs().ncoeff, which stays put until the block's record is written
+    hc_coeff* out = p.coeffs + ((uint32_t)cs().ctb_rs * p.coeff_cap_ctb + cs().ncoeff);
 
-    hc_tb tb;
-    tb.coeff_off = coeff_first;
-    tb.resid_off = (uint32_t)ctb_rs * p.resid_cap_ctb + nresid;
-    tb.pic = (uint16_t)p.pic_index;
-    tb.log2 = (uint8_t)log2;
-    tb.qp = (uint8_t)(cIdx == 0 ? qPYPrime : (cIdx == 1 ? qPCbPrime : qPCrPrime));
-    tb.matrix_id = (uint8_t)(log2 == 5 ? 0 : cIdx);
-    uint8_t type = (uint8_t)cIdx;
+    uint32_t type = (uint32_t)cIdx;
     if (tskip) type |= HC_TB_TSKIP;
     else if (log2 == 2 && cIdx == 0) type |= HC_TB_DST;
     if (p.implicit_rdpcm && tskip && (pred_mode == 10 || pred_mode == 26)) type |= (pred_mode == 26) ? HC_TB_RDPCM_V : HC_TB_RDPCM_H;
     if (p.tskip_rotation && log2 == 2 && tskip) type |= HC_TB_ROTATE;
-    tb.type = type;
 
     const bool ts_ctx = p.tskip_context && tskip;
     const bool sign_hiding_possible = p.sign_data_hiding && !(p.implicit_rdpcm && tskip && (pred_mode == 10 || pred_mode == 26));
@@ -875,7 +884,7 @@ struct Parser {
       const int last_coeff = (i == lastSubBlock) ? lastScanPos - 1 : 15;
       if (i == lastSubBlock) sig = 1u << lastScanPos;
 #if defined(__CUDA_ARCH__)
-      if (last_coeff > 0) sig |= cab_sig_run(cb.sa, cb.ta, (uint32_t)(CX_SIG + (ts_ctx ? ts_c : sigtab[lane() & 15])), last_coeff);
+      if (last_coeff > 0) sig |= cab_sig_run(cb.sa(), cb.ta(), (uint32_t)(CX_SIG + (ts_ctx ? ts_c : sigtab[lane() & 15])), last_coeff);
 #else
       if (ts_ctx) {
         K0_LOOP for (int k = last_coeff; k > 0; k--) sig |= (uint32_t)cb.bin(t, ctx, CX_SIG + ts_c) << k;
@@ -921,7 +930,7 @@ struct Parser {
       const int nsign = signHidden ? n - 1 : n;
       const uint32_t signs = cb.bypass_bits(t, nsign) << (16 - nsign);
 
-      if (ncoeff_total + (uint32_t)n > coeff_room) { fail(ERR_CAPACITY); return 0; }
+      if (cs().ncoeff + ncoeff_total + (uint32_t)n > p.coeff_cap_ctb) { fail(ERR_CAPACITY); return 0; }
       // (1) serial: coeff_abs_level_remaining of the coefficients that have one, in coding order (Rice adaptation)
       int32_t* remv = scratch().rem;
       int sumRem = 0, rice = 0;
@@ -972,22 +981,28 @@ struct Parser {
       ncoeff_total += (uint32_t)n;
     }
     cabac = cb;
-    tb.ncoeff = (uint16_t)ncoeff_total;
-    const uint32_t tb_local = (uint32_t)ctb_rs * p.tb_cap_ctb + ntb;
-    p.tbs[tb_local] = tb;
+    ChainState& s = cs();
+    const uint32_t ctb = (uint32_t)s.ctb_rs, ntb = s.ntb;
+    const uint32_t resid_off = ctb * p.resid_cap_ctb + s.nresid;
+    const uint32_t qp = (uint32_t)(cIdx == 0 ? s.qPYPrime : (cIdx == 1 ? s.qPCbPrime : s.qPCrPrime));
+    // hc_tb: coeff_off | resid_off | ncoeff, pic | log2, qp, type, matrix_id
+    store_rec16(p.tbs + (ctb * p.tb_cap_ctb + ntb), ctb * p.coeff_cap_ctb + s.ncoeff, resid_off,
+                (ncoeff_total & 0xffffu) | (p.pic_index << 16),
+                (uint32_t)log2 | ((qp & 0xffu) << 8) | (type << 16) | ((log2 == 5 ? 0u : (uint32_t)cIdx) << 24));
     scratch().tb_size[ntb] = (uint8_t)(log2 - 2);
-    ntb++;
-    ncoeff += ncoeff_total;
-    nresid += (uint32_t)(nT * nT);
-    return tb.resid_off;
+    s.ntb = ntb + 1;
+    s.ncoeff += ncoeff_total;
+    s.nresid += (uint32_t)(nT * nT);
+    return resid_off;
   }
 
   // ---- 7.3.8.10 transform_unit (record emission in the reference's reconstruction order, slice.cc:3979-4118) ----
-  K0_FN void transform_unit(int x0, int y0, int xBase, int yBase, int log2, int blkIdx, int cbf_luma, int cbf_cb, int cbf_cr) {
+  // `f`: the flags of transform_tree_flags
+  K0_FN void transform_unit(int x0, int y0, int xBase, int yBase, int log2, int blkIdx, int f) {
     const Pic& p = pic();
     const int cat = p.chroma_array_type;
     const int log2C = cat == 3 ? log2 : (log2 - 1 < 2 ? 2 : log2 - 1);
-    if ((cbf_luma || cbf_cb || cbf_cr) && p.cu_qp_delta_enabled && !IsCuQpDeltaCoded) {
+    if ((f & 0x3e) && p.cu_qp_delta_enabled && !cs().IsCuQpDeltaCoded) {
       int v = 0;
       if (bin(CX_CU_QP_DELTA)) {
         v = 1;
@@ -1001,17 +1016,19 @@ struct Parser {
       }
       int sign = 0;
       if (v) sign = cabac.bypass();
-      IsCuQpDeltaCoded = true;
-      CuQpDeltaVal = sign ? -v : v;
-      derive_qp(cu_x0, cu_y0);
+      ChainState& s = cs();
+      s.IsCuQpDeltaCoded = 1;
+      s.CuQpDeltaVal = sign ? -v : v;
+      derive_qp(s.cu_x0, s.cu_y0);
     }
     mark_tu_edges(x0, y0, log2);
 
     const int modeY = p.ipm[(x0 >> 2) + (y0 >> 2) * p.w4];
+    const bool cbf_luma = (f >> 5) & 1;
     uint32_t roff = 0;
     if (cbf_luma) roff = residual_coding(log2, 0, modeY);
-    if (err) return;
-    emit_blk(0, x0, y0, log2, modeY, cbf_luma != 0, roff);
+    if (err()) return;
+    emit_blk(0, x0, y0, log2, modeY, cbf_luma, roff);
     if (cat == 0) return;
     const int SubW = p.sub_w, SubH = p.sub_h;
     const bool own = log2 > 2 || cat == 3;     // chroma of this TU; else the parent's chroma with the 4th 4x4 luma block
@@ -1019,7 +1036,7 @@ struct Parser {
     const int bx = own ? x0 : xBase, by = own ? y0 : yBase;
     const int l2 = own ? log2C : 2, nTC = 1 << l2;
     K0_LOOP for (int c = 1; c <= 2; c++) {
-      const int cbf = c == 1 ? cbf_cb : cbf_cr;
+      const int cbf = (f >> (2 * c - 1)) & 3;
       const int nblk2 = cat == 2 ? 2 : 1;
       K0_LOOP for (int t = 0; t < nblk2; t++) {
         const int xB = bx / SubW, yB = by / SubH + t * nTC;
@@ -1028,7 +1045,7 @@ struct Parser {
         uint32_t ro = 0;
         const bool coded = (cbf >> t) & 1;
         if (coded) ro = residual_coding(l2, c, m);
-        if (err) return;
+        if (err()) return;
         emit_blk(c, xB, yB, l2, m, coded, ro);
       }
     }
@@ -1036,11 +1053,13 @@ struct Parser {
 
   // ---- 7.3.8.8 transform_tree: the flags are read by one size-independent function, the compile-time recursion
   // over the block size is a thin shell around it (code size: the parser is instruction-fetch bound) ----
-  // returns split | cbf_cb << 1 | cbf_cr << 3 | cbf_luma << 5
-  K0_FN int transform_tree_flags(int log2, int depth, int max_depth, int intra_split, int parent_cbf_cb, int parent_cbf_cr) {
+  // `parent_cbf`: cbf_cb | cbf_cr << 2 of the parent; returns split | cbf_cb << 1 | cbf_cr << 3 | cbf_luma << 5
+  K0_FN int transform_tree_flags(int log2, int depth, int parent_cbf) {
     const Pic& p = pic();
     const Tables& t = tab();
     uint8_t* const ctx = ctxs();
+    const int max_depth = cs().cu_max_trafo_depth, intra_split = cs().cu_intra_split;
+    const int parent_cbf_cb = parent_cbf & 3, parent_cbf_cr = parent_cbf >> 2;
     CabacT cb = cabac;
     int split;
     if (log2 <= p.log2_max_tb && log2 > p.log2_min_tb && depth < max_depth && !(intra_split && depth == 0)) split = cb.bin(t, ctx, CX_SPLIT_TRANSFORM + 5 - log2);
@@ -1065,34 +1084,37 @@ struct Parser {
     return split | (cbf_cb << 1) | (cbf_cr << 3) | (cbf_luma << 5);
   }
 
+  // the transform depth limit and the intra split of the CU are in cs(); `parent_cbf` as for transform_tree_flags
   template <int LOG2>
-  K0_FN void transform_tree(int x0, int y0, int xBase, int yBase, int depth, int blkIdx, int max_depth, int intra_split,
-                            int parent_cbf_cb, int parent_cbf_cr) {
-    if (err) return;
-    const int f = transform_tree_flags(LOG2, depth, max_depth, intra_split, parent_cbf_cb, parent_cbf_cr);
-    const int cbf_cb = (f >> 1) & 3, cbf_cr = (f >> 3) & 3;
+  K0_FN void transform_tree(int x0, int y0, int xBase, int yBase, int depth, int blkIdx, int parent_cbf) {
+    if (err()) return;
+    const int f = transform_tree_flags(LOG2, depth, parent_cbf);
     if (f & 1) {
       if (LOG2 > 2) {
         constexpr int L = LOG2 > 2 ? LOG2 - 1 : 2;
         constexpr int h = 1 << L;
-        transform_tree<L>(x0, y0, x0, y0, depth + 1, 0, max_depth, intra_split, cbf_cb, cbf_cr);
-        transform_tree<L>(x0 + h, y0, x0, y0, depth + 1, 1, max_depth, intra_split, cbf_cb, cbf_cr);
-        transform_tree<L>(x0, y0 + h, x0, y0, depth + 1, 2, max_depth, intra_split, cbf_cb, cbf_cr);
-        transform_tree<L>(x0 + h, y0 + h, x0, y0, depth + 1, 3, max_depth, intra_split, cbf_cb, cbf_cr);
+        const int cbf = (f >> 1) & 15;
+        transform_tree<L>(x0, y0, x0, y0, depth + 1, 0, cbf);
+        transform_tree<L>(x0 + h, y0, x0, y0, depth + 1, 1, cbf);
+        transform_tree<L>(x0, y0 + h, x0, y0, depth + 1, 2, cbf);
+        transform_tree<L>(x0 + h, y0 + h, x0, y0, depth + 1, 3, cbf);
       } else {
         fail(ERR_BITSTREAM);
       }
     } else {
-      transform_unit(x0, y0, xBase, yBase, LOG2, blkIdx, (f >> 5) & 1, cbf_cb, cbf_cr);
+      transform_unit(x0, y0, xBase, yBase, LOG2, blkIdx, f);
     }
   }
 
   // ---- 7.3.8.5 coding_unit (I slices) ----
-  // size-independent part: everything up to the transform tree; returns max transform depth | intra_split << 4
-  K0_FN int coding_unit_modes(int LOG2, int x0, int y0, int depth) {
+  // size-independent part: everything up to the transform tree; leaves the CU's transform depth limit and intra split in cs()
+  K0_FN void coding_unit_modes(int LOG2, int x0, int y0, int depth) {
     const Pic& p = pic();
     const int nCbS = 1 << LOG2;
-    cu_x0 = x0; cu_y0 = y0; cu_log2 = LOG2;
+    {
+      ChainState& s = cs();
+      s.cu_x0 = x0; s.cu_y0 = y0; s.cu_log2 = LOG2;
+    }
     {
       const int l8 = LOG2 - 3, n8 = nCbS >> 3;     // CUs are at least 8 x 8
       K0_LOOP for (int i = lane(); i < n8 * n8; i += K0_LANES)
@@ -1100,12 +1122,14 @@ struct Parser {
       lanes_sync();
     }
     // deblocking: which CU edges may be filtered (deblock.cc:165-215)
-    filterLeftCbEdge = x0 != 0;
-    filterTopCbEdge = y0 != 0;
     {
+      int filterLeftCbEdge = x0 != 0, filterTopCbEdge = y0 != 0;
       const int ctbmask = (1 << p.log2_ctb) - 1;
       if (x0 && (x0 & ctbmask) == 0 && !slice().loop_filter_across_slices && slice_addr_of_ctb(ctb_of(x0 - 1, y0)) != slice().slice_addr_rs) filterLeftCbEdge = 0;
       if (y0 && (y0 & ctbmask) == 0 && !slice().loop_filter_across_slices && slice_addr_of_ctb(ctb_of(x0, y0 - 1)) != slice().slice_addr_rs) filterTopCbEdge = 0;
+      ChainState& s = cs();
+      s.filterLeftCbEdge = filterLeftCbEdge;
+      s.filterTopCbEdge = filterTopCbEdge;
     }
     derive_qp(x0, y0);
 
@@ -1115,24 +1139,25 @@ struct Parser {
     bool nxn = false;
     if (LOG2 == p.log2_min_cb) {
       nxn = !cb.bin(t, ctx, CX_PART_MODE);
-      if (nxn && LOG2 <= p.log2_min_tb) { fail(ERR_BITSTREAM); return 0; }
+      if (nxn && LOG2 <= p.log2_min_tb) { fail(ERR_BITSTREAM); return; }
     }
     // ---- intra prediction modes ----
     const int pbOffset = nxn ? nCbS / 2 : nCbS;
     const int nparts = nxn ? 4 : 1;
-    int prev_flag[4], mpm_idx[4] = {0, 0, 0, 0}, rem[4] = {0, 0, 0, 0};
-    K0_LOOP for (int i = 0; i < nparts; i++) prev_flag[i] = cb.bin(t, ctx, CX_PREV_INTRA_LUMA);
+    uint32_t prev_flag = 0;   // bit i: prev_intra_luma_pred_flag of partition i
+    uint32_t idx_rem = 0;     // bits 8i..8i+7: mpm_idx or rem_intra_luma_pred_mode of partition i
+    K0_LOOP for (int i = 0; i < nparts; i++) prev_flag |= (uint32_t)cb.bin(t, ctx, CX_PREV_INTRA_LUMA) << i;
     K0_LOOP for (int i = 0; i < nparts; i++) {
-      if (prev_flag[i]) {
-        int v = 0;
+      uint32_t v = 0;
+      if ((prev_flag >> i) & 1u) {
         K0_LOOP while (v < 2 && cb.bypass()) v++;
-        mpm_idx[i] = v;
       } else {
-        rem[i] = (int)cb.bypass_bits(t, 5);
+        v = cb.bypass_bits(t, 5);
       }
+      idx_rem |= v << (8 * i);
     }
     const bool availA0 = ctb_available(x0, y0, x0 - 1, y0), availB0 = ctb_available(x0, y0, x0, y0 - 1);
-    int luma_modes[4];
+    uint32_t luma_modes = 0;  // bits 8i..8i+7: IntraPredModeY of partition i
     K0_LOOP for (int idx = 0; idx < nparts; idx++) {
       const int i = (idx & 1) * pbOffset, j = (idx >> 1) * pbOffset;
       const int x = x0 + i, y = y0 + j;
@@ -1140,29 +1165,31 @@ struct Parser {
       int candA = 1, candB = 1;
       if (availA) candA = p.ipm[((x - 1) >> 2) + (y >> 2) * p.w4];
       if (availB && !(y - 1 < ((y >> p.log2_ctb) << p.log2_ctb))) candB = p.ipm[(x >> 2) + ((y - 1) >> 2) * p.w4];
-      int cand[3];
+      int cand0, cand1, cand2;
       if (candA == candB) {
-        if (candA < 2) { cand[0] = 0; cand[1] = 1; cand[2] = 26; }
-        else { cand[0] = candA; cand[1] = 2 + ((candA - 2 - 1 + 32) % 32); cand[2] = 2 + ((candA - 2 + 1) % 32); }
+        if (candA < 2) { cand0 = 0; cand1 = 1; cand2 = 26; }
+        else { cand0 = candA; cand1 = 2 + ((candA - 2 - 1 + 32) % 32); cand2 = 2 + ((candA - 2 + 1) % 32); }
       } else {
-        cand[0] = candA; cand[1] = candB;
-        if (candA != 0 && candB != 0) cand[2] = 0;
-        else if (candA != 1 && candB != 1) cand[2] = 1;
-        else cand[2] = 26;
+        cand0 = candA; cand1 = candB;
+        if (candA != 0 && candB != 0) cand2 = 0;
+        else if (candA != 1 && candB != 1) cand2 = 1;
+        else cand2 = 26;
       }
+      const int v = (int)((idx_rem >> (8 * idx)) & 0xffu);
       int mode;
-      if (prev_flag[idx]) {
-        mode = cand[mpm_idx[idx]];
+      if ((prev_flag >> idx) & 1u) {
+        mode = v == 0 ? cand0 : (v == 1 ? cand1 : cand2);
       } else {
         int t;
-        if (cand[0] > cand[1]) { t = cand[0]; cand[0] = cand[1]; cand[1] = t; }
-        if (cand[0] > cand[2]) { t = cand[0]; cand[0] = cand[2]; cand[2] = t; }
-        if (cand[1] > cand[2]) { t = cand[1]; cand[1] = cand[2]; cand[2] = t; }
-        mode = rem[idx];
-        K0_LOOP for (int n = 0; n < 3; n++)
-          if (mode >= cand[n]) mode++;
+        if (cand0 > cand1) { t = cand0; cand0 = cand1; cand1 = t; }
+        if (cand0 > cand2) { t = cand0; cand0 = cand2; cand2 = t; }
+        if (cand1 > cand2) { t = cand1; cand1 = cand2; cand2 = t; }
+        mode = v;
+        if (mode >= cand0) mode++;
+        if (mode >= cand1) mode++;
+        if (mode >= cand2) mode++;
       }
-      luma_modes[idx] = mode;
+      luma_modes |= (uint32_t)mode << (8 * idx);
       const int n4 = pbOffset >> 2, l4 = k0_ctz((unsigned)n4);
       K0_LOOP for (int i = lane(); i < n4 * n4; i += K0_LANES)
         p.ipm[((x >> 2) + (i & (n4 - 1))) + ((y >> 2) + (i >> l4)) * p.w4] = (uint8_t)mode;
@@ -1174,7 +1201,7 @@ struct Parser {
       K0_LOOP for (int idx = 0; idx < nchroma; idx++) {
         int icpm = 4;
         if (cb.bin(t, ctx, CX_INTRA_CHROMA)) icpm = (int)cb.bypass_bits(t, 2);
-        const int luma = luma_modes[idx];
+        const int luma = (int)((luma_modes >> (8 * idx)) & 0xffu);
         int m = luma;
         if (icpm != 4) {
           m = icpm == 0 ? 0 : (icpm == 1 ? 26 : (icpm == 2 ? 10 : 1));
@@ -1189,14 +1216,16 @@ struct Parser {
       lanes_sync();     // transform_unit reads the chroma mode of its position
     }
     cabac = cb;
-    return (p.max_th_depth_intra + (nxn ? 1 : 0)) | (nxn ? 16 : 0);
+    ChainState& s = cs();
+    s.cu_max_trafo_depth = p.max_th_depth_intra + (nxn ? 1 : 0);
+    s.cu_intra_split = nxn ? 1 : 0;
   }
 
   template <int LOG2>
   HC_HD void coding_unit(int x0, int y0, int depth) {
-    const int r = coding_unit_modes(LOG2, x0, y0, depth);
-    if (err) return;
-    transform_tree<LOG2>(x0, y0, x0, y0, 0, 0, r & 15, r >> 4, 1, 1);
+    coding_unit_modes(LOG2, x0, y0, depth);
+    if (err()) return;
+    transform_tree<LOG2>(x0, y0, x0, y0, 0, 0, 1 | (1 << 2));
   }
 
   // ---- 7.3.8.4 coding_quadtree ----
@@ -1212,13 +1241,13 @@ struct Parser {
     } else {
       split = log2 > p.log2_min_cb;
     }
-    if (p.cu_qp_delta_enabled && log2 >= p.log2_min_cu_qp_delta_size) { IsCuQpDeltaCoded = false; CuQpDeltaVal = 0; }
+    if (p.cu_qp_delta_enabled && log2 >= p.log2_min_cu_qp_delta_size) { ChainState& s = cs(); s.IsCuQpDeltaCoded = 0; s.CuQpDeltaVal = 0; }
     return split;
   }
 
   template <int LOG2>
   K0_FN void coding_quadtree(int x0, int y0, int depth) {
-    if (err || cabac.overrun()) { fail(ERR_BITSTREAM); return; }
+    if (err() || cabac.overrun()) { fail(ERR_BITSTREAM); return; }
     if (coding_quadtree_split(LOG2, x0, y0, depth)) {
       if (LOG2 > 3) {
         const Pic& p = pic();
@@ -1240,32 +1269,43 @@ struct Parser {
   // ---- one CTU ----
   K0_FN void decode_ctu() {
     const Pic& p = pic();
+    {
+      ChainState& s = cs();
+      s.nblk[0] = s.nblk[1] = s.nblk[2] = 0;
+      s.ntb = s.ncoeff = s.nresid = 0;
+      hc_ctu& ctu = p.ctus[s.ctb_rs];
+      K0_LOOP for (int c = 0; c < 3; c++) { ctu.sao_type[c] = 0; ctu.sao_band_or_class[c] = 0; for (int i = 0; i < 4; i++) ctu.sao_offset[c][i] = 0; }
+    }
+    if (slice().sao_luma || slice().sao_chroma) read_sao();
+    {
+      const int x0 = cs().ctb_x << p.log2_ctb, y0 = cs().ctb_y << p.log2_ctb;
+      if (p.log2_ctb == 6) coding_quadtree<6>(x0, y0, 0);
+      else if (p.log2_ctb == 5) coding_quadtree<5>(x0, y0, 0);
+      else if (p.log2_ctb == 4) coding_quadtree<4>(x0, y0, 0);
+      else coding_quadtree<3>(x0, y0, 0);
+    }
+    const ChainState& s = cs();
+    const int ctb_rs = s.ctb_rs;
+    const uint32_t ntb = s.ntb;
     hc_ctu& ctu = p.ctus[ctb_rs];
-    nblk[0] = nblk[1] = nblk[2] = 0;
-    ntb = ncoeff = nresid = 0;
-    K0_LOOP for (int c = 0; c < 3; c++) { ctu.sao_type[c] = 0; ctu.sao_band_or_class[c] = 0; for (int i = 0; i < 4; i++) ctu.sao_offset[c][i] = 0; }
-    if (slice().sao_luma || slice().sao_chroma) read_sao(ctu);
-    const int x0 = ctb_x << p.log2_ctb, y0 = ctb_y << p.log2_ctb;
-    if (p.log2_ctb == 6) coding_quadtree<6>(x0, y0, 0);
-    else if (p.log2_ctb == 5) coding_quadtree<5>(x0, y0, 0);
-    else if (p.log2_ctb == 4) coding_quadtree<4>(x0, y0, 0);
-    else coding_quadtree<3>(x0, y0, 0);
     // K1 launch lists: one reservation per size class and CTB instead of one atomic per transform block
     if (ntb) {
       const uint8_t* ts = scratch().tb_size;
       const uint32_t tb0 = p.tb_global_base + (uint32_t)ctb_rs * p.tb_cap_ctb;
       unsigned long long packed = 0;   // four 16-bit counters
-      unsigned slot[4];
-      uint32_t* dst[4];
 #if defined(__CUDA_ARCH__)
-      // lane-parallel: count, reserve once per size class, then an order-preserving compaction 32 blocks at a time
+      // lane-parallel: count, lane l < 4 reserves the entries of size class l, then an order-preserving compaction 32
+      // blocks at a time
       K0_LOOP for (uint32_t t = (uint32_t)lane(); t < ntb; t += K0_LANES) packed += 1ull << (16 * ts[t]);
       K0_LOOP for (int o = 16; o > 0; o >>= 1) packed += __shfl_xor_sync(0xffffffffu, packed, o);
-      K0_LOOP for (int l = 0; l < 4; l++) {
-        const unsigned n = (unsigned)(packed >> (16 * l)) & 0xffffu;
-        slot[l] = n ? list_reserve(p.tb_counts + l, n) : 0u;
-        dst[l] = p.tb_lists[l];
+      unsigned mine = 0;
+      if (lane() < 4) {
+        const unsigned n = (unsigned)(packed >> (16 * lane())) & 0xffffu;
+        if (n) mine = atomicAdd(p.tb_counts + lane(), n);
       }
+      unsigned slot[4];
+#pragma unroll
+      for (int l = 0; l < 4; l++) slot[l] = __shfl_sync(0xffffffffu, mine, l);
       const unsigned below = (1u << lane()) - 1u;
       K0_LOOP for (uint32_t t0 = 0; t0 < ntb; t0 += K0_LANES) {
         const uint32_t t = t0 + (uint32_t)lane();
@@ -1273,7 +1313,7 @@ struct Parser {
 #pragma unroll
         for (int l = 0; l < 4; l++) {
           const unsigned m = __ballot_sync(0xffffffffu, sz == l);
-          if (sz == l) dst[l][slot[l] + (unsigned)__popc(m & below)] = tb0 + t;
+          if (sz == l) p.tb_lists[l][slot[l] + (unsigned)__popc(m & below)] = tb0 + t;
           slot[l] += (unsigned)__popc(m);
         }
       }
@@ -1282,17 +1322,17 @@ struct Parser {
       K0_LOOP for (int l = 0; l < 4; l++) {
         const unsigned n = (unsigned)(packed >> (16 * l)) & 0xffffu;
         if (!n) continue;
-        slot[l] = list_reserve(p.tb_counts + l, n);
-        dst[l] = p.tb_lists[l];
+        unsigned slot = p.tb_counts[l];
+        p.tb_counts[l] += n;
         K0_LOOP for (uint32_t t = 0; t < ntb; t++)
-          if (ts[t] == l) dst[l][slot[l]++] = tb0 + t;
+          if (ts[t] == l) p.tb_lists[l][slot++] = tb0 + t;
       }
 #endif
     }
     uint32_t base = (uint32_t)ctb_rs * p.blk_cap_ctb;
     K0_LOOP for (int c = 0; c < 3; c++) {
       ctu.blk_first[c] = base;
-      ctu.blk_count[c] = (uint16_t)nblk[c];
+      ctu.blk_count[c] = (uint16_t)s.nblk[c];
       base += p.blk_cap[c];
     }
     ctu.beta_offset = slice().beta_offset;
@@ -1306,29 +1346,33 @@ struct Parser {
 
   // ---- a chain of substreams (decode_slice_segment loop of the host parser) ----
   K0_FN void run_chain(const Pic* pics, const Sub* subs, uint32_t first_sub, uint32_t nsubs) {
-    err = ERR_NONE;
+    ChainState& c = cs();
+    {
+      uint32_t* w = reinterpret_cast<uint32_t*>(&c);   // CuQpDeltaVal & co. are read even when the stream never codes them
+      K0_LOOP for (int i = lane(); i < (int)(sizeof(ChainState) / 4); i += K0_LANES) w[i] = 0;
+      lanes_sync();
+    }
     uint32_t loaded_pic = 0xffffffffu;
     uint8_t* const ctx = ctxs();
-    K0_LOOP for (uint32_t s = 0; s < nsubs && !err; s++) {
+    K0_LOOP for (uint32_t s = 0; s < nsubs && !c.err; s++) {
       const Sub sub = subs[first_sub + s];
       if (sub.pic != loaded_pic) { scratch().pic = pics[sub.pic]; loaded_pic = sub.pic; }
       const Pic& p = pic();
       scratch().slice = p.slices[sub.slice];
-      slice_addr = slice().slice_addr_rs;
       const uint8_t* seg_end = p.bytes + slice().data_end;
       if (sub.byte_begin != 0xffffffffu) cabac.init(p.bytes + sub.byte_begin, seg_end);
       const bool row_chain = sub.flags & SUB_ROW_CHAIN;
-      ctb_rs = sub.first_ctb;
-      currentQG_x = currentQG_y = -1;
-      currentQPY = 0;
-      if (s == 0) { IsCuQpDeltaCoded = false; CuQpDeltaVal = 0; lastQPYinPreviousQG = 0; }
+      c.ctb_rs = sub.first_ctb;
+      c.currentQG_x = c.currentQG_y = -1;
+      c.currentQPY = 0;
+      if (s == 0) { c.IsCuQpDeltaCoded = 0; c.CuQpDeltaVal = 0; c.lastQPYinPreviousQG = 0; }
       if (!row_chain && sub.first_ctb == slice().segment_address && slice().segment_address > 0) {
         // thread-context initialisation of the reference (decctx.cc:467-506)
         const int prev = slice().segment_address - 1;
         int x = (((prev % p.ctbs_w) + 1) << p.log2_ctb) - 1, y = (((prev / p.ctbs_w) + 1) << p.log2_ctb) - 1;
         if (x > p.W - 1) x = p.W - 1;
         if (y > p.H - 1) y = p.H - 1;
-        currentQPY = p.qp_map[(x >> 3) + (y >> 3) * p.w8];
+        c.currentQPY = p.qp_map[(x >> 3) + (y >> 3) * p.w8];
       }
       // 9.3.1: context initialisation at the start of the slice segment (dependent segments of a serial chain keep
       // the table of the previous segment; rows of a WPP picture synchronise below)
@@ -1336,9 +1380,10 @@ struct Parser {
       if (segment_start && !slice().dependent) init_contexts();
       bool first_of_independent = segment_start && !slice().dependent;
 
-      ctb_x = ctb_rs % p.ctbs_w;
-      ctb_y = ctb_rs / p.ctbs_w;
-      K0_LOOP while (ctb_rs < sub.end_ctb && !err) {
+      c.ctb_x = c.ctb_rs % p.ctbs_w;
+      c.ctb_y = c.ctb_rs / p.ctbs_w;
+      K0_LOOP while (c.ctb_rs < sub.end_ctb && !c.err) {
+        const int ctb_x = c.ctb_x, ctb_y = c.ctb_y;
         if (row_chain && ctb_y > 0) {
           // wavefront: the row above must be two CTBs ahead (its context table, split depths and SAO parameters)
           const int need = ctb_x + 2 < p.ctbs_w ? ctb_x + 2 : p.ctbs_w;
@@ -1353,7 +1398,7 @@ struct Parser {
             if (need - have >= 2) far_wait(); else backoff(ns);
           }
         }
-        if (p.entropy_coding_sync && ctb_x == 0 && ctb_y >= 1 && !(first_of_independent && ctb_rs == slice().segment_address)) {
+        if (p.entropy_coding_sync && ctb_x == 0 && ctb_y >= 1 && !(first_of_independent && c.ctb_rs == slice().segment_address)) {
           if (p.ctbs_w > 1) {
             const uint32_t* src = reinterpret_cast<const uint32_t*>(p.wpp_ctx + (size_t)(ctb_y - 1) * CTX_BYTES);
             uint32_t* dst = reinterpret_cast<uint32_t*>(ctx);
@@ -1364,7 +1409,7 @@ struct Parser {
           }
         }
         decode_ctu();
-        if (err) break;
+        if (c.err) break;
         if (cabac.overrun()) { fail(ERR_BITSTREAM); break; }
         if (p.entropy_coding_sync && ctb_x == 1 && ctb_y < p.ctbs_h - 1) {
           uint32_t* dst = reinterpret_cast<uint32_t*>(p.wpp_ctx + (size_t)ctb_y * CTX_BYTES);
@@ -1373,11 +1418,12 @@ struct Parser {
         }
         if (row_chain) progress_store(p.progress + ctb_y, ctb_x + 1);
         const int end_of_slice_segment = cabac.terminate();
-        ctb_rs++;
-        if (++ctb_x == p.ctbs_w) { ctb_x = 0; ctb_y++; }
+        const int next_rs = ++c.ctb_rs;
+        if (ctb_x + 1 == p.ctbs_w) { c.ctb_x = 0; c.ctb_y = ctb_y + 1; }
+        else c.ctb_x = ctb_x + 1;
         if (end_of_slice_segment) break;
-        if (ctb_rs >= p.ctbs_w * p.ctbs_h) { fail(ERR_BITSTREAM); break; }
-        if (p.entropy_coding_sync && ctb_x == 0) {
+        if (next_rs >= p.ctbs_w * p.ctbs_h) { fail(ERR_BITSTREAM); break; }
+        if (p.entropy_coding_sync && c.ctb_x == 0) {
           if (!cabac.terminate()) { fail(ERR_BITSTREAM); break; }   // end_of_subset_one_bit
           if (row_chain) break;                                       // the next row is another chain
           const uint8_t* np = cabac.position();
@@ -1386,14 +1432,14 @@ struct Parser {
           first_of_independent = false;
         }
       }
-      if (!err && row_chain && ctb_rs != sub.end_ctb) fail(ERR_BITSTREAM);
+      if (!c.err && row_chain && c.ctb_rs != sub.end_ctb) fail(ERR_BITSTREAM);
     }
-    if (err) {
+    if (c.err) {
       // unblock every waiter of this picture, then report
       if (loaded_pic == 0xffffffffu) scratch().pic = pics[subs[first_sub].pic];
       const Pic& p = pic();
       K0_LOOP for (int r = 0; r < p.ctbs_h; r++) progress_store(p.progress + r, 1 << 30);
-      *p.error = err;
+      *p.error = c.err;
     }
   }
 };

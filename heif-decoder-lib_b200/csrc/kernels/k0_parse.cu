@@ -21,7 +21,7 @@ constexpr int K0_WARPS = 4;
 // against chains in flight. Measured per 32 x 12 MP (DESIGN.md), v6 (one lane per chain): 5 -> 114 ms, 6 -> 109 ms,
 // 8 -> 109 ms, 10 -> 116 ms, 12 -> 129 ms; v7 (warp-uniform chains): 5 -> 102.8, 6 -> 103.2, 7 -> 100.2, 8 -> 97.7,
 // 9 -> 97.4, 10 -> 110.2, 12 -> 115.0, 16 -> 126.2 ms: 8 is the fastest up to noise. Ten or more CTAs per SM would also
-// need more shared memory than the default carve-out offers (12.4 KB per CTA).
+// need more shared memory than the default carve-out offers (12.8 KB per CTA).
 constexpr int K0_MIN_CTAS = 8;
 
 __global__ void __launch_bounds__(32 * K0_WARPS, K0_MIN_CTAS) k0_parse_kernel(const k0::Tables* __restrict__ tables, const k0::Pic* __restrict__ pics,
@@ -40,13 +40,7 @@ __global__ void __launch_bounds__(32 * K0_WARPS, K0_MIN_CTAS) k0_parse_kernel(co
   // map fills, context tables, K1 lists — are spread over the lanes (k0_core.cuh: K0_LANES / lane())
   if (chain >= nchains) return;
   const k0::Chain ch = chains[chain];
-  k0::Parser ps;
-  memset(&ps, 0, sizeof(ps));   // CuQpDeltaVal & co. are read even when the stream never codes them
-  ps.wbase = (uint32_t)(k0::TABLE_BYTES + warp * k0::SCRATCH_BYTES);
-#if defined(__CUDA_ARCH__)
-  ps.cabac.ta = (uint32_t)__cvta_generic_to_shared(k0::k0_smem);
-  ps.cabac.sa = ps.cabac.ta + ps.wbase;   // the Scratch starts with the decoder state
-#endif
+  k0::Parser ps;   // finds the warp's Scratch by itself (k0::scratch_offset)
   ps.run_chain(pics, subs, ch.first_sub, ch.nsubs);
 }
 
