@@ -23,8 +23,8 @@
 #include <cstring>
 #include "common.cuh"
 
-// functions that must stay real calls: the syntax tree recursion is unrolled by templates and would otherwise
-// be inlined 4^depth times
+// functions that stay real calls: those with several call sites (the parser is instruction-fetch bound, so each has one
+// copy), and the per-CTB / per-CU steps of the syntax walk
 #if defined(__CUDACC__)
 #define K0_FN __host__ __device__ __noinline__
 #else
@@ -176,9 +176,13 @@ struct ChainState {
   int IsCuQpDeltaCoded, CuQpDeltaVal;
   int currentQG_x, currentQG_y, lastQPYinPreviousQG, currentQPY;
   int qPYPrime, qPCbPrime, qPCrPrime;
-  int cu_x0, cu_y0, cu_log2;
-  int cu_max_trafo_depth, cu_intra_split;      // of the current CU, read by every level of its transform tree
-  int filterLeftCbEdge, filterTopCbEdge;
+  int cu_x0, cu_y0;
+  int tt_x, tt_y;                              // the transform-tree node being parsed
+  uint32_t tt_cbf;                             // nibble l: cbf_cb | cbf_cr << 2 the open level above hands to nodes of log2 l
+  uint8_t cu_log2, tt_log2;
+  uint8_t cu_max_trafo_depth, cu_intra_split;  // of the current CU, read by every level of its transform tree
+  uint8_t filterLeftCbEdge, filterTopCbEdge;
+  uint8_t tt_flags, tt_mode;                  // of the transform unit being parsed: transform_tree_flags, intra mode of the block
 };
 struct Scratch {
   CabState cab;
@@ -997,12 +1001,12 @@ struct Parser {
   }
 
   // ---- 7.3.8.10 transform_unit (record emission in the reference's reconstruction order, slice.cc:3979-4118) ----
-  // `f`: the flags of transform_tree_flags
-  K0_FN void transform_unit(int x0, int y0, int xBase, int yBase, int log2, int blkIdx, int f) {
+  // The unit is the transform-tree node in cs(): tt_x, tt_y, tt_log2, and tt_flags from transform_tree_flags. Inlined into
+  // the transform-tree walk, its only caller. residual_coding needs nearly all registers, so across its calls this keeps
+  // only the chroma block index; the rest is read again from cs() and pic().
+  HC_HD void transform_unit() {
     const Pic& p = pic();
-    const int cat = p.chroma_array_type;
-    const int log2C = cat == 3 ? log2 : (log2 - 1 < 2 ? 2 : log2 - 1);
-    if ((f & 0x3e) && p.cu_qp_delta_enabled && !cs().IsCuQpDeltaCoded) {
+    if ((cs().tt_flags & 0x3e) && p.cu_qp_delta_enabled && !cs().IsCuQpDeltaCoded) {
       int v = 0;
       if (bin(CX_CU_QP_DELTA)) {
         v = 1;
@@ -1021,40 +1025,51 @@ struct Parser {
       s.CuQpDeltaVal = sign ? -v : v;
       derive_qp(s.cu_x0, s.cu_y0);
     }
-    mark_tu_edges(x0, y0, log2);
-
-    const int modeY = p.ipm[(x0 >> 2) + (y0 >> 2) * p.w4];
-    const bool cbf_luma = (f >> 5) & 1;
+    ChainState& s = cs();
+    mark_tu_edges(s.tt_x, s.tt_y, s.tt_log2);
+    s.tt_mode = p.ipm[(s.tt_x >> 2) + (s.tt_y >> 2) * p.w4];
     uint32_t roff = 0;
-    if (cbf_luma) roff = residual_coding(log2, 0, modeY);
+    if (s.tt_flags & 0x20) roff = residual_coding(s.tt_log2, 0, s.tt_mode);
     if (err()) return;
-    emit_blk(0, x0, y0, log2, modeY, cbf_luma, roff);
+    emit_blk(0, s.tt_x, s.tt_y, s.tt_log2, s.tt_mode, (s.tt_flags & 0x20) != 0, roff);
+    const int cat = p.chroma_array_type;
     if (cat == 0) return;
-    const int SubW = p.sub_w, SubH = p.sub_h;
-    const bool own = log2 > 2 || cat == 3;     // chroma of this TU; else the parent's chroma with the 4th 4x4 luma block
-    if (!own && blkIdx != 3) return;
-    const int bx = own ? x0 : xBase, by = own ? y0 : yBase;
-    const int l2 = own ? log2C : 2, nTC = 1 << l2;
-    K0_LOOP for (int c = 1; c <= 2; c++) {
-      const int cbf = (f >> (2 * c - 1)) & 3;
-      const int nblk2 = cat == 2 ? 2 : 1;
-      K0_LOOP for (int t = 0; t < nblk2; t++) {
-        const int xB = bx / SubW, yB = by / SubH + t * nTC;
-        const int lx = xB * SubW, ly = yB * SubH;   // mode lookup position of the reference (slice.cc:3760-3763)
-        const int m = p.ipm_c[((lx < p.W - 1 ? lx : p.W - 1) >> 2) + ((ly < p.H - 1 ? ly : p.H - 1) >> 2) * p.w4];
-        uint32_t ro = 0;
-        const bool coded = (cbf >> t) & 1;
-        if (coded) ro = residual_coding(l2, c, m);
-        if (err()) return;
-        emit_blk(c, xB, yB, l2, m, coded, ro);
-      }
+    // chroma of this TU; else the parent's 8x8 chroma with the 4th 4x4 luma block (blkIdx 3: bit 2 of x and y set — a 4x4
+    // TU always has a parent, CUs are at least 8x8)
+    if (!(s.tt_log2 > 2 || cat == 3) && !(s.tt_x & s.tt_y & 4)) return;
+    K0_LOOP for (int k = 0; k < (cat == 2 ? 4 : 2); k++) {
+      int c, xB, yB, l2;
+      bool coded = chroma_block(k, c, xB, yB, l2);
+      const int lx = xB * p.sub_w, ly = yB * p.sub_h;   // mode lookup position of the reference (slice.cc:3760-3763)
+      s.tt_mode = p.ipm_c[((lx < p.W - 1 ? lx : p.W - 1) >> 2) + ((ly < p.H - 1 ? ly : p.H - 1) >> 2) * p.w4];
+      uint32_t ro = 0;
+      if (coded) ro = residual_coding(l2, c, s.tt_mode);
+      if (err()) return;
+      coded = chroma_block(k, c, xB, yB, l2);
+      emit_blk(c, xB, yB, l2, s.tt_mode, coded, ro);
     }
   }
 
-  // ---- 7.3.8.8 transform_tree: the flags are read by one size-independent function, the compile-time recursion
-  // over the block size is a thin shell around it (code size: the parser is instruction-fetch bound) ----
-  // `parent_cbf`: cbf_cb | cbf_cr << 2 of the parent; returns split | cbf_cb << 1 | cbf_cr << 3 | cbf_luma << 5
-  K0_FN int transform_tree_flags(int log2, int depth, int parent_cbf) {
+  // Chroma block k of the transform unit in cs() — Cb, then Cr; with 4:2:2 each as an upper and a lower square: its
+  // component, position and size; returns its cbf. Evaluated again after the block's residual_coding call instead of
+  // being held in registers across it.
+  HC_HD bool chroma_block(int k, int& c, int& xB, int& yB, int& l2) const {
+    const Pic& p = pic();
+    const ChainState& s = cs();
+    const int cat = p.chroma_array_type, log2 = s.tt_log2;
+    const bool own = log2 > 2 || cat == 3;
+    const int t = cat == 2 ? k & 1 : 0;
+    c = cat == 2 ? 1 + (k >> 1) : 1 + k;
+    l2 = cat == 3 ? log2 : (log2 > 2 ? log2 - 1 : 2);
+    xB = (own ? s.tt_x : s.tt_x - 4) / p.sub_w;
+    yB = (own ? s.tt_y : s.tt_y - 4) / p.sub_h + (t << l2);
+    return (s.tt_flags >> (2 * c - 1 + t)) & 1;
+  }
+
+  // ---- 7.3.8.8 transform_tree ----
+  // The flags of one node. `parent_cbf`: cbf_cb | cbf_cr << 2 of the parent; returns
+  // split | cbf_cb << 1 | cbf_cr << 3 | cbf_luma << 5
+  HC_HD int transform_tree_flags(int log2, int depth, int parent_cbf) {
     const Pic& p = pic();
     const Tables& t = tab();
     uint8_t* const ctx = ctxs();
@@ -1084,25 +1099,41 @@ struct Parser {
     return split | (cbf_cb << 1) | (cbf_cr << 3) | (cbf_luma << 5);
   }
 
-  // the transform depth limit and the intra split of the CU are in cs(); `parent_cbf` as for transform_tree_flags
-  template <int LOG2>
-  K0_FN void transform_tree(int x0, int y0, int xBase, int yBase, int depth, int blkIdx, int parent_cbf) {
-    if (err()) return;
-    const int f = transform_tree_flags(LOG2, depth, parent_cbf);
-    if (f & 1) {
-      if (LOG2 > 2) {
-        constexpr int L = LOG2 > 2 ? LOG2 - 1 : 2;
-        constexpr int h = 1 << L;
-        const int cbf = (f >> 1) & 15;
-        transform_tree<L>(x0, y0, x0, y0, depth + 1, 0, cbf);
-        transform_tree<L>(x0 + h, y0, x0, y0, depth + 1, 1, cbf);
-        transform_tree<L>(x0, y0 + h, x0, y0, depth + 1, 2, cbf);
-        transform_tree<L>(x0 + h, y0 + h, x0, y0, depth + 1, 3, cbf);
-      } else {
-        fail(ERR_BITSTREAM);
+  // The transform tree of the current CU (position, size, depth limit and intra split in cs()), walked in z-order by a
+  // loop rather than by recursion, so that a node costs no call and no call frame in local memory: the parser is
+  // instruction-fetch bound. The walk's state is the node (tt_x, tt_y, tt_log2) and the chroma cbfs each open level
+  // hands to its children (tt_cbf); a node's position says which child it is. It lives in cs(), not in registers,
+  // because residual_coding needs nearly all of them.
+  HC_HD void transform_tree() {
+    {
+      ChainState& s = cs();
+      s.tt_x = s.cu_x0; s.tt_y = s.cu_y0; s.tt_log2 = s.cu_log2;
+      s.tt_cbf = 5u << (4 * s.cu_log2);   // the root inherits cbf_cb = cbf_cr = 1
+    }
+    K0_LOOP for (;;) {
+      if (err()) return;
+      ChainState& s = cs();
+      const int log2 = s.tt_log2;
+      const int f = transform_tree_flags(log2, s.cu_log2 - log2, (s.tt_cbf >> (4 * log2)) & 15);
+      if (f & 1) {
+        if (log2 == 2) { fail(ERR_BITSTREAM); return; }
+        s.tt_cbf = (s.tt_cbf & ~(15u << (4 * (log2 - 1)))) | ((uint32_t)((f >> 1) & 15) << (4 * (log2 - 1)));
+        s.tt_log2 = (uint8_t)(log2 - 1);
+        continue;   // first child: same position
       }
-    } else {
-      transform_unit(x0, y0, xBase, yBase, LOG2, blkIdx, f);
+      s.tt_flags = (uint8_t)f;
+      transform_unit();
+      // next node: the next sibling, or up while this node is its parent's 4th child
+      int x = s.tt_x, y = s.tt_y, l = s.tt_log2;
+      const int cu_log2 = s.cu_log2;
+      K0_LOOP for (;;) {
+        if (l == cu_log2) return;
+        const int h = 1 << l;
+        if (!(x & h)) { x += h; break; }           // child 0 -> 1, 2 -> 3
+        if (!(y & h)) { x -= h; y += h; break; }   // child 1 -> 2
+        x -= h; y -= h; l++;
+      }
+      s.tt_x = x; s.tt_y = y; s.tt_log2 = (uint8_t)l;
     }
   }
 
@@ -1113,7 +1144,7 @@ struct Parser {
     const int nCbS = 1 << LOG2;
     {
       ChainState& s = cs();
-      s.cu_x0 = x0; s.cu_y0 = y0; s.cu_log2 = LOG2;
+      s.cu_x0 = x0; s.cu_y0 = y0; s.cu_log2 = (uint8_t)LOG2;
     }
     {
       const int l8 = LOG2 - 3, n8 = nCbS >> 3;     // CUs are at least 8 x 8
@@ -1128,8 +1159,8 @@ struct Parser {
       if (x0 && (x0 & ctbmask) == 0 && !slice().loop_filter_across_slices && slice_addr_of_ctb(ctb_of(x0 - 1, y0)) != slice().slice_addr_rs) filterLeftCbEdge = 0;
       if (y0 && (y0 & ctbmask) == 0 && !slice().loop_filter_across_slices && slice_addr_of_ctb(ctb_of(x0, y0 - 1)) != slice().slice_addr_rs) filterTopCbEdge = 0;
       ChainState& s = cs();
-      s.filterLeftCbEdge = filterLeftCbEdge;
-      s.filterTopCbEdge = filterTopCbEdge;
+      s.filterLeftCbEdge = (uint8_t)filterLeftCbEdge;
+      s.filterTopCbEdge = (uint8_t)filterTopCbEdge;
     }
     derive_qp(x0, y0);
 
@@ -1217,19 +1248,12 @@ struct Parser {
     }
     cabac = cb;
     ChainState& s = cs();
-    s.cu_max_trafo_depth = p.max_th_depth_intra + (nxn ? 1 : 0);
+    s.cu_max_trafo_depth = (uint8_t)(p.max_th_depth_intra + (nxn ? 1 : 0));
     s.cu_intra_split = nxn ? 1 : 0;
   }
 
-  template <int LOG2>
-  HC_HD void coding_unit(int x0, int y0, int depth) {
-    coding_unit_modes(LOG2, x0, y0, depth);
-    if (err()) return;
-    transform_tree<LOG2>(x0, y0, x0, y0, 0, 0, 1 | (1 << 2));
-  }
-
   // ---- 7.3.8.4 coding_quadtree ----
-  K0_FN int coding_quadtree_split(int log2, int x0, int y0, int depth) {
+  HC_HD int coding_quadtree_split(int log2, int x0, int y0, int depth) {
     const Pic& p = pic();
     const int size = 1 << log2;
     int split;
@@ -1245,24 +1269,33 @@ struct Parser {
     return split;
   }
 
-  template <int LOG2>
-  K0_FN void coding_quadtree(int x0, int y0, int depth) {
-    if (err() || cabac.overrun()) { fail(ERR_BITSTREAM); return; }
-    if (coding_quadtree_split(LOG2, x0, y0, depth)) {
-      if (LOG2 > 3) {
-        const Pic& p = pic();
-        constexpr int L = LOG2 > 3 ? LOG2 - 1 : 3;
-        constexpr int h = 1 << L;
-        const int x1 = x0 + h, y1 = y0 + h;
-        coding_quadtree<L>(x0, y0, depth + 1);
-        if (x1 < p.W) coding_quadtree<L>(x1, y0, depth + 1);
-        if (y1 < p.H) coding_quadtree<L>(x0, y1, depth + 1);
-        if (x1 < p.W && y1 < p.H) coding_quadtree<L>(x1, y1, depth + 1);
-      } else {
-        fail(ERR_BITSTREAM);
+  // The coding quadtree of the current CTB, walked in z-order by a loop like transform_tree. Children that lie outside the
+  // picture are skipped: the right ones when x + h >= W, the lower ones when y + h >= H. Every node first checks the
+  // chain's error state and the bitstream position; an error ends the walk. After a CU the walk resumes from the CU's
+  // position in cs(), so that nothing of it is held in registers across the CU's transform tree.
+  HC_HD void coding_quadtree() {
+    int log2 = pic().log2_ctb, x = cs().ctb_x << log2, y = cs().ctb_y << log2;
+    K0_LOOP for (;;) {
+      if (err() || cabac.overrun()) { fail(ERR_BITSTREAM); return; }
+      const int depth = pic().log2_ctb - log2;
+      if (coding_quadtree_split(log2, x, y, depth)) {
+        if (log2 <= 3) { fail(ERR_BITSTREAM); return; }
+        log2--;
+        continue;   // first child: same position, always inside the picture
       }
-    } else {
-      coding_unit<LOG2>(x0, y0, depth);
+      // 7.3.8.5 coding_unit
+      coding_unit_modes(log2, x, y, depth);
+      if (err()) return;
+      transform_tree();
+      const Pic& p = pic();
+      x = cs().cu_x0; y = cs().cu_y0; log2 = cs().cu_log2;
+      K0_LOOP for (;;) {
+        if (log2 == p.log2_ctb) return;
+        const int h = 1 << log2;
+        if (!(x & h) && x + h < p.W) { x += h; break; }             // child 0 -> 1, 2 -> 3
+        if (!(y & h) && y + h < p.H) { x &= ~h; y += h; break; }    // child 0 -> 2 when 1 is outside, 1 -> 2
+        x &= ~h; y &= ~h; log2++;
+      }
     }
   }
 
@@ -1277,13 +1310,7 @@ struct Parser {
       K0_LOOP for (int c = 0; c < 3; c++) { ctu.sao_type[c] = 0; ctu.sao_band_or_class[c] = 0; for (int i = 0; i < 4; i++) ctu.sao_offset[c][i] = 0; }
     }
     if (slice().sao_luma || slice().sao_chroma) read_sao();
-    {
-      const int x0 = cs().ctb_x << p.log2_ctb, y0 = cs().ctb_y << p.log2_ctb;
-      if (p.log2_ctb == 6) coding_quadtree<6>(x0, y0, 0);
-      else if (p.log2_ctb == 5) coding_quadtree<5>(x0, y0, 0);
-      else if (p.log2_ctb == 4) coding_quadtree<4>(x0, y0, 0);
-      else coding_quadtree<3>(x0, y0, 0);
-    }
+    coding_quadtree();
     const ChainState& s = cs();
     const int ctb_rs = s.ctb_rs;
     const uint32_t ntb = s.ntb;
