@@ -152,12 +152,12 @@ def engine():
     e.close()
 
 
-def k0_batch(engine, names, stages):
-    """One batch with every picture of names parsed by K0. Returns {name: planes}."""
+def k0_batch(engine, names, stages, data=ss.data):
+    """One batch with every picture of names parsed by K0; data(name) gives the stream. Returns {name: (planes, pic)}."""
     b = engine.batch()
     items = []
     for name in names:
-        k = hb.K0Picture(ss.data(name), FMT)
+        k = hb.K0Picture(data(name), FMT)
         assert k.eligible, (name, k.why_not)
         p = k.pic
         c = b.add_canvas(p.crop_w, p.crop_h, p.chroma_format, p.bit_depth_y)

@@ -41,7 +41,7 @@ void hc_oracle_residual_block(const hc_pic* pic, const hc_tb* tb, const hc_coeff
                               int32_t* res);
 
 typedef struct hevc_enc_params {
-  int32_t width, height;     // visible size (coded size is rounded up to a multiple of 8)
+  int32_t width, height;     // visible size (coded size is rounded up to a multiple of the min CB size)
   int32_t chroma_format;     // 0..3
   int32_t bit_depth;         // 8..12
   int32_t qp;                // 0..51
@@ -74,6 +74,7 @@ typedef struct hevc_enc_params {
   int32_t chroma_qp_offset_list_len;                    // 0 off, else 1..6 entries with offsets drawn in -12..12
   int32_t diff_cu_chroma_qp_offset_depth;
   int32_t log2_sao_offset_scale_luma, log2_sao_offset_scale_chroma;
+  int32_t log2_min_cb;       // log2 of the min CB size, 3..log2_ctb; 0: 3
   uint32_t seed;
 } hevc_enc_params;
 }
@@ -89,8 +90,9 @@ enum {
 };
 
 // Counters of what the encoder wrote (hevc_enc_encode_ex). X(name, n): n > 1 is an array, named name_0 .. name_<n-1>.
-// Two groups: the syntax extremes of the stress mode, then the range-extension tools (from hevc_enc_rext_stat_first()
-// on), which only streams with those tools switched on reach.
+// Three groups: the syntax extremes of the stress mode, the range-extension tools (from hevc_enc_rext_stat_first()
+// on), which only streams with those tools switched on reach, and the coding-tree geometry (from
+// hevc_enc_tree_stat_first() on).
 #define HEVC_ENC_STATS(X)                                                                                               \
   X(level_min, 1) X(level_max, 1) X(escape_long, 1) X(escape_prefix16, 1) X(rice4, 1)                                  \
   X(sb_16_sig, 1) X(sb_beyond_8, 1) X(sign_hidden_even, 1) X(sign_hidden_odd, 1) X(sign_string_16, 1)                   \
@@ -109,12 +111,23 @@ enum {
   X(cu_chroma_qp_offset_off, 1) X(cu_chroma_qp_offset_idx, 6)                                                            \
   X(sao_offset_scaled_cmax, 1) X(no_edge_flt, 1) X(smoothing_skipped, 1) X(smoothing_skipped_strong, 1)
 
+// cu_log2_<k>, nxn_log2_<k>: CU log2 3 + k. border_split_min_cb_<k>: a split inferred at the picture border at log2 5 + k
+// whose children are min CBs larger than 8 x 8. tu_depth_<k>: transform leaves at trafoDepth k. luma_tb_log2_<k>: luma TBs
+// of log2 2 + k. The rest are single cases of 7.3.8.8 - 7.3.8.10 and 7.4.3.2.1.
+#define HEVC_ENC_TREE_STATS(X)                                                                                          \
+  X(cu_log2, 4) X(nxn_log2, 4) X(border_split_min_cb, 2) X(tu_depth, 5) X(luma_tb_log2, 4)                              \
+  X(split_max_tb_at_depth_limit, 1) X(leaf_at_min_tb_gt4, 1) X(leaf_at_depth_limit, 1) X(chroma4_of_luma8, 1)           \
+  X(cbf422_second_log2_ge4, 1) X(qg_min_cb_gt8, 1) X(conf_offset_ge8, 1)
+
 enum {
 #define HEVC_ENC_STAT_ENUM(name, n) ST_##name, ST_##name##_end_ = ST_##name + (n) - 1,
   HEVC_ENC_STATS(HEVC_ENC_STAT_ENUM)
   ST_REXT_FIRST_,
   ST_REXT_BEFORE_ = ST_REXT_FIRST_ - 1,
   HEVC_ENC_REXT_STATS(HEVC_ENC_STAT_ENUM)
+  ST_TREE_FIRST_,
+  ST_TREE_BEFORE_ = ST_TREE_FIRST_ - 1,
+  HEVC_ENC_TREE_STATS(HEVC_ENC_STAT_ENUM)
 #undef HEVC_ENC_STAT_ENUM
   ST_COUNT
 };
@@ -372,6 +385,7 @@ struct Enc {
   bool cu_bypass = false;
   int cu_x0 = 0, cu_y0 = 0, cu_log2 = 0;
   int log2_min_cu_qp_delta = 6;
+  int log2_min_pcm = 3;         // Log2MinIpcmCbSizeY: Min(MinCbLog2SizeY, 5); the max is Min(CtbLog2SizeY, 5)
   // cu_chroma_qp_offset: the decision of a chroma quantisation group is drawn when the group starts, takes effect at its
   // first TU with a coded chroma block (pass A) and is written there (pass B, in the same order)
   int log2_min_cu_chroma_qp_offset = 6, max_tskip_log2 = 2;
@@ -443,8 +457,10 @@ void Enc::setup() {
   cf = P.chroma_format; bd = P.bit_depth;
   SubW = (cf == 1 || cf == 2) ? 2 : 1;
   SubH = cf == 1 ? 2 : 1;
-  W = (P.width + 7) & ~7;
-  H = (P.height + 7) & ~7;
+  log2_min_cb = P.log2_min_cb ? P.log2_min_cb : 3;
+  const int min_cb = 1 << log2_min_cb;
+  W = (P.width + min_cb - 1) & ~(min_cb - 1);
+  H = (P.height + min_cb - 1) & ~(min_cb - 1);
   log2_ctb = P.log2_ctb; ctb = 1 << log2_ctb;
   ctbs_w = (W + ctb - 1) / ctb; ctbs_h = (H + ctb - 1) / ctb; nctb = ctbs_w * ctbs_h;
   log2_min_tb = P.log2_min_tb; log2_max_tb = std::min(P.log2_max_tb, std::min(5, log2_ctb));
@@ -491,7 +507,8 @@ void Enc::setup() {
   max_tskip_log2 = P.transform_skip ? 2 + P.log2_max_transform_skip_minus2 : 2;
   log2_min_cu_chroma_qp_offset = log2_ctb - P.diff_cu_chroma_qp_offset_depth;
   for (int i = 0; i < P.chroma_qp_offset_list_len; i++) { cqo_cb[i] = rng.below(25) - 12; cqo_cr[i] = rng.below(25) - 12; }
-  log2_min_cu_qp_delta = P.cu_qp_delta ? log2_ctb - std::min(P.cu_qp_delta - 1, log2_ctb - 3) : log2_ctb;
+  log2_min_cu_qp_delta = P.cu_qp_delta ? log2_ctb - std::min(P.cu_qp_delta - 1, log2_ctb - log2_min_cb) : log2_ctb;
+  log2_min_pcm = std::min(log2_min_cb, 5);
 
   // scaling lists
   if (P.scaling_list) {
@@ -590,6 +607,7 @@ void Enc::write_parameter_sets(std::vector<uint8_t>& out) {
     bool crop = W != P.width || H != P.height;
     bw.put(crop, 1);
     if (crop) { bw.ue(0); bw.ue((uint32_t)((W - P.width) / SubW)); bw.ue(0); bw.ue((uint32_t)((H - P.height) / SubH)); }
+    if (W - P.width >= 8 || H - P.height >= 8) stats[ST_conf_offset_ge8]++;
     bw.ue((uint32_t)(bd - 8)); bw.ue((uint32_t)(bd - 8));
     bw.ue(4);  // log2_max_pic_order_cnt_lsb_minus4
     bw.put(1, 1); bw.ue(0); bw.ue(0); bw.ue(0);
@@ -606,7 +624,7 @@ void Enc::write_parameter_sets(std::vector<uint8_t>& out) {
     bw.put(P.pcm ? 1 : 0, 1);
     if (P.pcm) {
       bw.put((uint32_t)(bd - 1), 4); bw.put((uint32_t)(bd - 1), 4);
-      bw.ue(0); bw.ue((uint32_t)(std::min(5, log2_ctb) - 3)); bw.put(0, 1);
+      bw.ue((uint32_t)(log2_min_pcm - 3)); bw.ue((uint32_t)(std::min(5, log2_ctb) - log2_min_pcm)); bw.put(0, 1);
     }
     bw.ue(0);                        // num_short_term_ref_pic_sets
     bw.put(0, 1);                    // long_term_ref_pics_present
@@ -1333,10 +1351,18 @@ void Enc::write_tu(Node& n, const int* luma_modes, const int* chroma_modes) {
 void Enc::write_tree(Node& n, int max_depth, int intra_split, int parent_cbf_cb, int parent_cbf_cr, const int* luma_modes,
                      const int* chroma_modes) {
   const int log2 = n.log2;
-  if (log2 <= log2_max_tb && log2 > log2_min_tb && n.depth < max_depth && !(intra_split && n.depth == 0))
+  if (log2 <= log2_max_tb && log2 > log2_min_tb && n.depth < max_depth && !(intra_split && n.depth == 0)) {
     bin(CTX_SPLIT_TRANSFORM + 5 - log2, n.split);
+  } else if (n.split) {
+    if (log2 > log2_max_tb && n.depth >= max_depth) stats[ST_split_max_tb_at_depth_limit]++;
+  } else if (log2 == log2_min_tb) {
+    if (log2_min_tb > 2) stats[ST_leaf_at_min_tb_gt4]++;
+  } else if (n.depth >= max_depth) {
+    stats[ST_leaf_at_depth_limit]++;
+  }
   int cbf_cb = n.cbf_cb, cbf_cr = n.cbf_cr;
   if ((log2 > 2 && cf != 0) || cf == 3) {
+    if (cf == 2 && !n.split && log2 >= 4) stats[ST_cbf422_second_log2_ge4] += (parent_cbf_cb != 0) + (parent_cbf_cr != 0);
     if (parent_cbf_cb) {
       bin(CTX_CBF_CHROMA + n.depth, cbf_cb & 1);
       if (cf == 2 && (!n.split || log2 == 3)) bin(CTX_CBF_CHROMA + n.depth, (cbf_cb >> 1) & 1);
@@ -1354,6 +1380,9 @@ void Enc::write_tree(Node& n, int max_depth, int intra_split, int parent_cbf_cb,
     // at a split node with a single flag in 4:2:2 the value is "any child"; already aggregated
     for (int i = 0; i < 4; i++) write_tree(*n.child[i], max_depth, intra_split, cbf_cb, cbf_cr, luma_modes, chroma_modes);
   } else {
+    stats[ST_tu_depth + n.depth]++;
+    stats[ST_luma_tb_log2 + log2 - 2]++;
+    if (log2 == 3 && (cf == 1 || cf == 2)) stats[ST_chroma4_of_luma8]++;
     bin(CTX_CBF_LUMA + (n.depth == 0 ? 1 : 0), n.cbf_luma);
     write_tu(n, luma_modes, chroma_modes);
   }
@@ -1366,6 +1395,7 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
   cqo_queue.clear();
   cqo_read = 0;
   if (P.transquant_bypass) bin(CTX_TQ_BYPASS, cu_bypass);
+  stats[ST_cu_log2 + log2 - 3]++;
   {
     int n8 = nCbS >> 3;
     for (int y = 0; y < n8; y++)
@@ -1391,9 +1421,10 @@ void Enc::coding_unit(int x0, int y0, int log2, int depth) {
   if (log2 == log2_min_cb) {
     nxn = log2 > log2_min_tb && (stress(HEVC_ENC_STRESS_MODES) ? rng.chance(50) : variance(x0, y0, nCbS) > 200 ? rng.chance(60) : rng.chance(10));
     bin(CTX_PART_MODE, nxn ? 0 : 1);
+    if (nxn) stats[ST_nxn_log2 + log2 - 3]++;
   }
   bool pcm = false;
-  if (!nxn && P.pcm && log2 >= 3 && log2 <= std::min(5, log2_ctb)) {
+  if (!nxn && P.pcm && log2 >= log2_min_pcm && log2 <= std::min(5, log2_ctb)) {
     pcm = rng.chance(6);
     cabac.terminate(pcm ? 1 : 0);
   }
@@ -1536,8 +1567,10 @@ void Enc::coding_quadtree(int x0, int y0, int log2, int depth) {
     bin(CTX_SPLIT_CU + condL + condA, split);
   } else {
     split = log2 > log2_min_cb;
+    if (split && log2 == log2_min_cb + 1 && log2_min_cb > 3) stats[ST_border_split_min_cb + log2 - 5]++;
   }
   if (P.cu_qp_delta && log2 >= log2_min_cu_qp_delta) {
+    if (log2 == log2_min_cb && log2_min_cb > 3) stats[ST_qg_min_cb_gt8]++;
     IsCuQpDeltaCoded = false;
     CuQpDeltaVal = 0;
     // target QP of this quantisation group (kept within +-6 of the slice QP and the legal range)
@@ -1752,21 +1785,24 @@ extern "C" {
 
 // planes: uint16 samples of the visible picture (width x height, chroma subsampled), tightly
 // packed strides given in samples. Output: 4-byte-length-prefixed NAL units (VPS, SPS, PPS, slices).
-// recon (optional): per component a buffer of the coded size (width and height rounded up to a multiple of 8,
-// chroma subsampled, tightly packed) that receives the encoder's reconstruction before the in-loop filters.
+// recon (optional): per component a buffer of the coded size (width and height rounded up to a multiple of the min CB
+// size, chroma subsampled, tightly packed) that receives the encoder's reconstruction before the in-loop filters.
+// qp (optional): (coded width / 8) x (coded height / 8) bytes that receive QpY of every 8 x 8 luma block.
 // stats (optional): hevc_enc_stat_count() counters of what was written (names: hevc_enc_stat_name; the range-extension
-// group starts at hevc_enc_rext_stat_first()).
+// group starts at hevc_enc_rext_stat_first(), the coding-tree group at hevc_enc_tree_stat_first()).
 int hevc_enc_encode_ex(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
-                       size_t* out_size, uint16_t* const recon[3], uint64_t* stats) {
+                       size_t* out_size, uint16_t* const recon[3], int8_t* qp, uint64_t* stats) {
   if (!params || !planes || !out || !out_size) return -1;
   hevc_enc_params P = *params;
   if (P.width <= 0 || P.height <= 0 || P.chroma_format < 0 || P.chroma_format > 3 || P.bit_depth < 8 || P.bit_depth > 12) return -2;
   if (P.log2_ctb < 4 || P.log2_ctb > 6 || P.log2_min_tb < 2 || P.log2_max_tb > 5 || P.log2_min_tb > P.log2_max_tb) return -2;
-  if (P.log2_min_tb >= 3) return -2;  // min CB is fixed at 8x8 here
+  const int log2_min_cb = P.log2_min_cb ? P.log2_min_cb : 3;
+  if (log2_min_cb < 3 || log2_min_cb > P.log2_ctb || P.log2_min_tb >= log2_min_cb) return -2;
+  if (P.max_th_depth < 0 || P.max_th_depth > P.log2_ctb - P.log2_min_tb) return -2;
   if (P.qp < -6 * (P.bit_depth - 8) || P.qp > 51) return -2;
   if (P.log2_max_transform_skip_minus2 < 0 || P.log2_max_transform_skip_minus2 > 3) return -2;
   if (P.chroma_qp_offset_list_len < 0 || P.chroma_qp_offset_list_len > 6) return -2;
-  if (P.diff_cu_chroma_qp_offset_depth < 0 || P.diff_cu_chroma_qp_offset_depth > P.log2_ctb - 3) return -2;
+  if (P.diff_cu_chroma_qp_offset_depth < 0 || P.diff_cu_chroma_qp_offset_depth > P.log2_ctb - log2_min_cb) return -2;
   const int max_sao_scale = std::max(0, P.bit_depth - 10);
   if (P.log2_sao_offset_scale_luma < 0 || P.log2_sao_offset_scale_luma > max_sao_scale) return -2;
   if (P.log2_sao_offset_scale_chroma < 0 || P.log2_sao_offset_scale_chroma > max_sao_scale) return -2;
@@ -1792,18 +1828,21 @@ int hevc_enc_encode_ex(const hevc_enc_params* params, const uint16_t* const plan
   if (recon)
     for (int c = 0; c < ncomp; c++)
       if (recon[c]) memcpy(recon[c], enc.rec[c].data(), enc.rec[c].size() * sizeof(uint16_t));
+  if (qp) memcpy(qp, enc.qp_y.data(), enc.qp_y.size());
   if (stats) memcpy(stats, enc.stats, sizeof(enc.stats));
   return 0;
 }
 
 int hevc_enc_encode(const hevc_enc_params* params, const uint16_t* const planes[3], const int strides[3], uint8_t** out,
                     size_t* out_size) {
-  return hevc_enc_encode_ex(params, planes, strides, out, out_size, nullptr, nullptr);
+  return hevc_enc_encode_ex(params, planes, strides, out, out_size, nullptr, nullptr, nullptr);
 }
 
 int hevc_enc_stat_count(void) { return ST_COUNT; }
 
 int hevc_enc_rext_stat_first(void) { return ST_REXT_FIRST_; }
+
+int hevc_enc_tree_stat_first(void) { return ST_TREE_FIRST_; }
 
 const char* hevc_enc_stat_name(int i) {
   static const std::vector<std::string> names = [] {
@@ -1812,6 +1851,7 @@ const char* hevc_enc_stat_name(int i) {
   for (int k = 0; k < (n); k++) v.push_back((n) == 1 ? std::string(#name) : std::string(#name) + "_" + std::to_string(k));
     HEVC_ENC_STATS(HEVC_ENC_STAT_NAME)
     HEVC_ENC_REXT_STATS(HEVC_ENC_STAT_NAME)
+    HEVC_ENC_TREE_STATS(HEVC_ENC_STAT_NAME)
 #undef HEVC_ENC_STAT_NAME
     return v;
   }();

@@ -18,7 +18,9 @@ FIELDS = ["width", "height", "chroma_format", "bit_depth", "qp", "log2_ctb", "lo
           "transform_skip_rotation", "transform_skip_context", "implicit_rdpcm", "intra_smoothing_disabled",
           "persistent_rice_adaptation", "extended_precision", "cabac_bypass_alignment", "log2_max_transform_skip_minus2",
           "cross_component_prediction", "chroma_qp_offset_list_len", "diff_cu_chroma_qp_offset_depth",
-          "log2_sao_offset_scale_luma", "log2_sao_offset_scale_chroma"]
+          "log2_sao_offset_scale_luma", "log2_sao_offset_scale_chroma",
+          # coding-tree geometry; 0: min CB 8 x 8
+          "log2_min_cb"]
 
 # stress bits (hevc_enc_params::stress): syntax values at the limits of their legal ranges, for parser tests
 STRESS_LEVELS, STRESS_MODES, STRESS_QP, STRESS_SAO, STRESS_DENSE = 1, 2, 4, 8, 16
@@ -66,16 +68,22 @@ def stat_names():
 
 def rext_stat_names():
     """Counters of the range-extension coding tools (the range-extension fields of the encoder options)."""
-    return _all_stat_names()[lib().hevc_enc_rext_stat_first():]
+    return _all_stat_names()[lib().hevc_enc_rext_stat_first():lib().hevc_enc_tree_stat_first()]
+
+
+def tree_stat_names():
+    """Counters of the coding-tree geometry: CU, PB and TB sizes, transform depths and the inferred splits and leaves."""
+    return _all_stat_names()[lib().hevc_enc_tree_stat_first():]
 
 
 def encode(planes, want=(), **kw):
     """planes: list of 2-D integer arrays (Y[,Cb,Cr]) of the visible picture. Returns bytes:
     4-byte-length-prefixed NAL units (VPS, SPS, PPS, slice segments).
     want: any of "recon" (the encoder's reconstruction before the in-loop filters: uint16 planes of the coded size,
-    width and height rounded up to a multiple of 8) and "stats" ({counter name: count} of what was written: the stress
-    counters under "stats", the range-extension ones under "rext_stats"). With a
-    non-empty want the result is (bytes, {name: value})."""
+    width and height rounded up to a multiple of the min CB size), "qp" (QpY of every 8 x 8 luma block of the coded
+    size, int8) and "stats" ({counter name: count} of what was written: the stress counters under "stats", the
+    range-extension ones under "rext_stats", the coding-tree ones under "tree_stats"). With a non-empty want the result
+    is (bytes, {name: value})."""
     L = lib()
     opts = dict(DEFAULTS)
     opts.update(kw)
@@ -87,16 +95,20 @@ def encode(planes, want=(), **kw):
     pp = (C.c_void_p * 3)(*([a.ctypes.data for a in pl] + [None] * (3 - len(pl))))
     st = (C.c_int * 3)(*([a.shape[1] for a in pl] + [0] * (3 - len(pl))))
     out, size = C.c_void_p(), C.c_size_t()
-    recon = rp = stats = None
+    recon = rp = qp = stats = None
+    m = (1 << (p.log2_min_cb or 3)) - 1
+    cw, ch = (p.width + m) & ~m, (p.height + m) & ~m
     if "recon" in want:
         cf = p.chroma_format
-        w8, h8 = (p.width + 7) & ~7, (p.height + 7) & ~7
         sw, sh = (2 if cf in (1, 2) else 1), (2 if cf == 1 else 1)
-        recon = [np.zeros(d, np.uint16) for d in [(h8, w8)] + ([(h8 // sh, w8 // sw)] * 2 if cf else [])]
+        recon = [np.zeros(d, np.uint16) for d in [(ch, cw)] + ([(ch // sh, cw // sw)] * 2 if cf else [])]
         rp = (C.c_void_p * 3)(*([a.ctypes.data for a in recon] + [None] * (3 - len(recon))))
+    if "qp" in want:
+        qp = np.zeros((ch >> 3, cw >> 3), np.int8)
     if "stats" in want:
         stats = (C.c_uint64 * L.hevc_enc_stat_count())()
-    rc = L.hevc_enc_encode_ex(C.byref(p), pp, st, C.byref(out), C.byref(size), rp, stats)
+    rc = L.hevc_enc_encode_ex(C.byref(p), pp, st, C.byref(out), C.byref(size), rp,
+                              None if qp is None else C.c_void_p(qp.ctypes.data), stats)
     if rc != 0:
         raise RuntimeError("hevc_enc_encode failed: %d" % rc)
     data = C.string_at(out, size.value)
@@ -106,11 +118,13 @@ def encode(planes, want=(), **kw):
     extra = {}
     if recon is not None:
         extra["recon"] = recon
+    if qp is not None:
+        extra["qp"] = qp
     if stats is not None:
-        first = L.hevc_enc_rext_stat_first()
         counts = dict(zip(_all_stat_names(), (int(v) for v in stats)))
-        extra["stats"] = {k: counts[k] for k in _all_stat_names()[:first]}
-        extra["rext_stats"] = {k: counts[k] for k in _all_stat_names()[first:]}
+        extra["stats"] = {k: counts[k] for k in stat_names()}
+        extra["rext_stats"] = {k: counts[k] for k in rext_stat_names()}
+        extra["tree_stats"] = {k: counts[k] for k in tree_stat_names()}
     return data, extra
 
 
