@@ -165,6 +165,26 @@ int hc_heif_grid_tiles(const hc_heif* f, uint32_t id, uint32_t* tiles, int max) 
   for (int i = 0; i < (int)g.tiles.size() && i < max; i++) tiles[i] = g.tiles[i];
   return (int)g.tiles.size();
 }
+int hc_heif_thumbnail_ids(const hc_heif* f, uint32_t id, uint32_t* ids, int max) {
+  std::vector<uint32_t> v = f->file.thumbnails(id);
+  for (int i = 0; i < (int)v.size() && i < max; i++) ids[i] = v[i];
+  return (int)v.size();
+}
+int hc_heif_auxiliary_ids(const hc_heif* f, uint32_t id, int include_alpha, uint32_t* ids, int max) {
+  std::vector<uint32_t> v = f->file.auxiliaries(id, include_alpha != 0);
+  for (int i = 0; i < (int)v.size() && i < max; i++) ids[i] = v[i];
+  return (int)v.size();
+}
+int hc_heif_aux_type(const hc_heif* f, uint32_t id, char* buf, size_t len) {
+  const hc::HeifItem* it = f ? f->file.item(id) : nullptr;
+  if (!it || it->aux_type.empty()) { g_last_error = "hc_heif_aux_type: item " + std::to_string(id) + " has no auxC property"; return HC_ERR_ARGUMENT; }
+  if (buf && len) {
+    const size_t n = std::min(len - 1, it->aux_type.size());
+    memcpy(buf, it->aux_type.data(), n);
+    buf[n] = 0;
+  }
+  return (int)it->aux_type.size();
+}
 int hc_heif_coded_stream(const hc_heif* f, uint32_t id, uint8_t** out, size_t* size) {
   std::vector<uint8_t> v;
   std::string e = f->file.coded_stream(id, v);

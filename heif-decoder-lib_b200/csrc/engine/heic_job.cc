@@ -172,10 +172,11 @@ void hc_heic_job_destroy(hc_heic_job* j) {
 
 }  // extern "C"
 
+// item_ids: image item of each file to decode (NULL, or 0 for an entry: its primary image)
 // band_begin/band_end: tile rows [begin, end) of a grid image to decode (band_end < 0: everything)
 // host_share: percentage of the coded items the host threads parse although the device parser is on (hybrid; < 0: the
 // engine option, where "auto" means none outside hc_heic_decode_stream)
-static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
+static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, const uint32_t* item_ids,
                                     int want_alpha, int threads, int band_begin, int band_end, int host_share_arg) {
   if (!e || nfiles <= 0 || !data || !sizes) {
     hc::set_last_error("hc_heic_job_create: bad argument");
@@ -277,7 +278,15 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
     if (!err.empty()) { hc::set_last_error("file " + std::to_string(f) + ": " + err); return nullptr; }
     hc::HeifFile& hf = *j->files[f];
     ImagePlan& im = j->images[f];
-    const uint32_t id = hf.primary_id();
+    const uint32_t id = item_ids && item_ids[f] ? item_ids[f] : hf.primary_id();
+    if (!hf.is_image_item(id)) {
+      const hc::HeifItem* it = hf.item(id);
+      std::string type;
+      for (int s = 24; it && s >= 0; s -= 8) type.push_back((char)(it->type >> s));
+      hc::set_last_error("file " + std::to_string(f) + ": item " + std::to_string(id) +
+                         (it ? " is of type '" + type + "', not an image item (hvc1, grid, iovl)" : std::string(" does not exist")));
+      return nullptr;
+    }
     if (hf.is_overlay(id)) {
       // 'iovl' (context.cc:2579-2675): every referenced image is decoded like a top-level image, then composed
       if (band_end >= 0) { hc::set_last_error("a tile row band needs a grid image"); return nullptr; }
@@ -629,10 +638,10 @@ static hc_heic_job* job_create_impl(hc_engine* e, int nfiles, const uint8_t* con
 }
 
 // No exception may cross the C ABI: a crafted file can make any allocation of the walk above fail.
-static hc_heic_job* job_create(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
+static hc_heic_job* job_create(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, const uint32_t* item_ids,
                                int want_alpha, int threads, int band_begin, int band_end, int host_share_arg = -1) {
   try {
-    return job_create_impl(e, nfiles, data, sizes, want_alpha, threads, band_begin, band_end, host_share_arg);
+    return job_create_impl(e, nfiles, data, sizes, item_ids, want_alpha, threads, band_begin, band_end, host_share_arg);
   } catch (const std::bad_alloc&) {
     hc::set_last_error("out of memory while preparing the job");
   } catch (const std::exception& ex) {
@@ -645,13 +654,18 @@ extern "C" {
 
 hc_heic_job* hc_heic_job_create(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
                                 int want_alpha, int threads) {
-  return job_create(e, nfiles, data, sizes, want_alpha, threads, 0, -1);
+  return hc_heic_job_create_items(e, nfiles, data, sizes, nullptr, want_alpha, threads);
+}
+
+hc_heic_job* hc_heic_job_create_items(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
+                                      const uint32_t* item_ids, int want_alpha, int threads) {
+  return job_create(e, nfiles, data, sizes, item_ids, want_alpha, threads, 0, -1);
 }
 
 hc_heic_job* hc_heic_job_create_band(hc_engine* e, const uint8_t* data, size_t size, int want_alpha, int threads,
                                      int tile_row_begin, int tile_row_end, int* first_output_row, int* full_height) {
   if (tile_row_end < 0) { hc::set_last_error("hc_heic_job_create_band: bad band"); return nullptr; }
-  hc_heic_job* j = job_create(e, 1, &data, &size, want_alpha, threads, tile_row_begin, tile_row_end);
+  hc_heic_job* j = job_create(e, 1, &data, &size, nullptr, want_alpha, threads, tile_row_begin, tile_row_end);
   if (j && first_output_row) *first_output_row = j->images[0].band_y0;
   if (j && full_height) *full_height = j->images[0].full_height;
   return j;
@@ -726,13 +740,19 @@ int hc_heic_decode_stream(hc_engine* e, int nfiles, const uint8_t* const* data, 
 }
 
 int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, int want_alpha,
-                              int threads, int files_per_batch_arg, const hc_stream_dest* dests, int* file_status, hc_image_callback on_image,
+                              int threads, int files_per_batch, const hc_stream_dest* dests, int* file_status, hc_image_callback on_image,
                               void* user, hc_stream_stats* stats) {
+  return hc_heic_decode_stream_items(e, nfiles, data, sizes, nullptr, want_alpha, threads, files_per_batch, dests, file_status, on_image, user, stats);
+}
+
+int hc_heic_decode_stream_items(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, const uint32_t* item_ids,
+                                int want_alpha, int threads, int files_per_batch_arg, const hc_stream_dest* dests, int* file_status,
+                                hc_image_callback on_image, void* user, hc_stream_stats* stats) {
   int files_per_batch = files_per_batch_arg;
   if (e && nfiles > 0 && data && sizes && files_per_batch == 0) {
     // automatic batch size: the device parser wants some 20,000 substream chains in flight and the kernels behind it stream;
     // measured optimum 64 files of 12 MP (3.6 -> 3.9 GP/s against 32) and 384 of 1080p (1.5 -> 3.2 GP/s against 96), i.e.
-    // about 800 MP of output per batch — taken from the size of the LARGEST primary image among up to 32 files sampled
+    // about 800 MP of output per batch — taken from the size of the LARGEST requested image among up to 32 entries sampled
     // evenly over the list (a batch of the largest must fit)
     double mp = 0.0;
     const int nsample = std::min(nfiles, 32);
@@ -740,7 +760,7 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
       const int k = (int)((long long)q * nfiles / nsample);
       hc::HeifFile hf;
       if (!hf.parse(data[k], sizes[k]).empty()) continue;
-      const hc::HeifItem* it = hf.item(hf.primary_id());
+      const hc::HeifItem* it = hf.item(item_ids && item_ids[k] ? item_ids[k] : hf.primary_id());
       if (it && it->ispe_w > 0 && it->ispe_h > 0) mp = std::max(mp, (double)it->ispe_w * it->ispe_h / 1e6);
     }
     if (mp <= 0.0) mp = 12.0;
@@ -796,20 +816,21 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
     std::lock_guard<std::mutex> one_at_a_time(parse_mu);   // the look-ahead is two batches deep, the thread pool is one
     const auto t0 = clock::now();
     p.share = nbatches > 1 ? share.load() : 0;
-    p.job = job_create(e, n, data + first, sizes + first, want_alpha, threads, 0, -1, p.share);
+    const uint32_t* ids = item_ids ? item_ids + first : nullptr;
+    p.job = job_create(e, n, data + first, sizes + first, ids, want_alpha, threads, 0, -1, p.share);
     p.map.resize(n);
     for (int k = 0; k < n; k++) p.map[k] = k;
     if (!p.job) p.error = hc_last_error();   // thread-local: fetch on the parsing thread
     if (!p.job && file_status) {
       // error isolation: find the files that cannot be decoded (each on its own, headers only unless the device parser
       // cannot take the picture), report them through file_status and go on with the others
-      std::vector<const uint8_t*> gd; std::vector<size_t> gs;
+      std::vector<const uint8_t*> gd; std::vector<size_t> gs; std::vector<uint32_t> gi;
       p.map.clear();
       for (int k = 0; k < n; k++) {
-        hc_heic_job* probe = job_create(e, 1, data + first + k, sizes + first + k, want_alpha, 1, 0, -1, 0);
+        hc_heic_job* probe = job_create(e, 1, data + first + k, sizes + first + k, ids ? ids + k : nullptr, want_alpha, 1, 0, -1, 0);
         if (probe) {
           hc_heic_job_destroy(probe);
-          gd.push_back(data[first + k]); gs.push_back(sizes[first + k]); p.map.push_back(k);
+          gd.push_back(data[first + k]); gs.push_back(sizes[first + k]); gi.push_back(ids ? ids[k] : 0); p.map.push_back(k);
         } else {
           fail_file(first + k, HC_ERR_BITSTREAM, hc_last_error());
         }
@@ -817,7 +838,7 @@ int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* da
       p.error.clear();
       if (!gd.empty() && (int)gd.size() < n) {
         p.share = 0;
-        p.job = job_create(e, (int)gd.size(), gd.data(), gs.data(), want_alpha, threads, 0, -1, 0);
+        p.job = job_create(e, (int)gd.size(), gd.data(), gs.data(), gi.data(), want_alpha, threads, 0, -1, 0);
         if (!p.job) p.error = hc_last_error();
       } else if (!gd.empty()) {
         p.error = "batch failed although every file of it decodes alone";   // e.g. out of memory: not a property of one file

@@ -1,5 +1,6 @@
 // heif_reader.cc — see heif_reader.h.
 #include "heif_reader.h"
+#include <algorithm>
 #include <cstring>
 
 namespace hc {
@@ -55,6 +56,11 @@ bool next_box(Cursor& c, Box& b) {
   b.size = (size_t)(sz - hdr);
   c.pos += b.size;
   return true;
+}
+
+// the auxC types that make an auxiliary image an alpha image
+bool is_alpha_urn(const std::string& urn) {
+  return urn == "urn:mpeg:avc:2015:auxid:1" || urn == "urn:mpeg:hevc:2015:auxid:1" || urn == "urn:mpeg:mpegB:cicp:systems:auxiliary:alpha";
 }
 
 }  // namespace
@@ -375,12 +381,35 @@ uint32_t HeifFile::alpha_item(uint32_t id) const {
     for (uint32_t t : r.to) if (t == id) to_me = true;
     if (!to_me) continue;
     const HeifItem* a = item(r.from);
-    if (!a) continue;
-    if (a->aux_type == "urn:mpeg:avc:2015:auxid:1" || a->aux_type == "urn:mpeg:hevc:2015:auxid:1" ||
-        a->aux_type == "urn:mpeg:mpegB:cicp:systems:auxiliary:alpha")
-      return a->id;
+    if (a && is_alpha_urn(a->aux_type)) return a->id;
   }
   return 0;
+}
+
+bool HeifFile::is_image_item(uint32_t id) const {
+  const HeifItem* it = item(id);
+  return it && (it->type == fourcc("hvc1") || it->type == fourcc("grid") || it->type == fourcc("iovl"));
+}
+
+// the items with a `ref_type` reference to `id`, ascending and each once
+std::vector<uint32_t> HeifFile::referring(uint32_t ref_type, uint32_t id) const {
+  std::vector<uint32_t> out;
+  for (auto& r : refs_) {
+    if (r.type != ref_type || !item(r.from)) continue;
+    for (uint32_t t : r.to)
+      if (t == id) { out.push_back(r.from); break; }
+  }
+  std::sort(out.begin(), out.end());
+  out.erase(std::unique(out.begin(), out.end()), out.end());
+  return out;
+}
+
+std::vector<uint32_t> HeifFile::thumbnails(uint32_t id) const { return referring(fourcc("thmb"), id); }
+
+std::vector<uint32_t> HeifFile::auxiliaries(uint32_t id, bool include_alpha) const {
+  std::vector<uint32_t> out = referring(fourcc("auxl"), id);
+  if (!include_alpha) out.erase(std::remove_if(out.begin(), out.end(), [&](uint32_t a) { return is_alpha_urn(item(a)->aux_type); }), out.end());
+  return out;
 }
 
 std::string HeifFile::coded_stream(uint32_t id, std::vector<uint8_t>& out) const {

@@ -79,8 +79,14 @@ class HeifFile {
   std::string grid(uint32_t id, HeifGrid& g) const;
   bool is_overlay(uint32_t id) const;
   std::string overlay(uint32_t id, HeifOverlay& o) const;
+  // the item types that are decoded as images: 'hvc1', 'grid' and 'iovl'
+  bool is_image_item(uint32_t id) const;
   // alpha auxiliary image item of `id`, or 0
   uint32_t alpha_item(uint32_t id) const;
+  // items with a 'thmb' reference to `id`, in ascending item id
+  std::vector<uint32_t> thumbnails(uint32_t id) const;
+  // items with an 'auxl' reference to `id`, in ascending item id; alpha images only when `include_alpha`
+  std::vector<uint32_t> auxiliaries(uint32_t id, bool include_alpha) const;
   // a 'prem' item reference from the colour image: its samples are stored premultiplied by alpha (context.cc:1150-1161)
   bool premultiplied(uint32_t id) const;
   // hvcC parameter sets followed by the item's coded data, every NAL prefixed by a 4-byte
@@ -90,6 +96,7 @@ class HeifFile {
 
  private:
   std::string read_item_data(const HeifItem& it, std::vector<uint8_t>& out) const;
+  std::vector<uint32_t> referring(uint32_t ref_type, uint32_t id) const;
   const uint8_t* data_ = nullptr;
   size_t size_ = 0;
   uint32_t primary_ = 0;

@@ -108,6 +108,9 @@ SYMBOLS = [
     ("hc_heif_get_image_info", _i, [_vp, _u32, C.POINTER(HeifImageInfo)]),
     ("hc_heif_get_overlay", _i, [_vp, _u32, C.POINTER(HeifOverlayInfo)]),
     ("hc_heif_grid_tiles", _i, [_vp, _u32, C.POINTER(_u32), _i]),
+    ("hc_heif_thumbnail_ids", _i, [_vp, _u32, C.POINTER(_u32), _i]),
+    ("hc_heif_auxiliary_ids", _i, [_vp, _u32, _i, C.POINTER(_u32), _i]),
+    ("hc_heif_aux_type", _i, [_vp, _u32, C.c_char_p, _sz]),
     ("hc_heif_coded_stream", _i, [_vp, _u32, C.POINTER(_vp), C.POINTER(_sz)]),
     ("hc_free", None, [_vp]),
     ("hc_csc_select", _i, [_i, _i, _i, _i, _i, _i, _i, C.POINTER(CscParams)]),
@@ -144,6 +147,7 @@ SYMBOLS = [
     ("hc_batch_launch_count", _i, [_vp]),
     ("hc_batch_upload_bytes", _sz, [_vp]),
     ("hc_heic_job_create", _vp, [_vp, _i, C.POINTER(C.c_char_p), C.POINTER(_sz), _i, _i]),
+    ("hc_heic_job_create_items", _vp, [_vp, _i, C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(_u32), _i, _i]),
     ("hc_heic_job_create_band", _vp, [_vp, C.c_char_p, _sz, _i, _i, _i, _i, C.POINTER(_i), C.POINTER(_i)]),
     ("hc_heic_job_copy_rgb_device", _i, [_vp, _i, _vp, _sz]),
     ("hc_heic_job_set_rgb_target", _i, [_vp, _i, _vp, _i]),
@@ -177,6 +181,8 @@ SYMBOLS = [
                                C.POINTER(StreamStats)]),
     ("hc_heic_decode_stream_ext", _i, [_vp, _i, C.POINTER(C.c_char_p), C.POINTER(_sz), _i, _i, _i, _vp, C.POINTER(_i), IMAGE_CALLBACK,
                                    _vp, C.POINTER(StreamStats)]),
+    ("hc_heic_decode_stream_items", _i, [_vp, _i, C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(_u32), _i, _i, _i, _vp, C.POINTER(_i),
+                                     IMAGE_CALLBACK, _vp, C.POINTER(StreamStats)]),
     ("hc_host_alloc", _vp, [_sz]),
     ("hc_host_free", None, [_vp]),
 ]

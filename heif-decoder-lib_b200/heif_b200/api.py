@@ -116,6 +116,28 @@ class HeifFile:
         n = self._L.hc_heif_top_level_ids(self._h, ids, 64)
         return list(ids[:min(n, 64)])
 
+    def thumbnail_ids(self, item_id):
+        """hc_heif_thumbnail_ids: the items with a 'thmb' reference to image item_id, ascending
+        (heif_image_handle_get_list_of_thumbnail_IDs)"""
+        return self._ids(self._L.hc_heif_thumbnail_ids, item_id)
+
+    def auxiliary_ids(self, item_id, include_alpha=False):
+        """hc_heif_auxiliary_ids: the items with an 'auxl' reference to image item_id, ascending; alpha images only with
+        include_alpha (heif_image_handle_get_list_of_auxiliary_image_IDs)"""
+        return self._ids(lambda h, i, ids, n: self._L.hc_heif_auxiliary_ids(h, i, int(include_alpha), ids, n), item_id)
+
+    def aux_type(self, item_id):
+        """hc_heif_aux_type: the auxC type URN of an auxiliary image (raises for an item without auxC)"""
+        n = check(self._L, self._L.hc_heif_aux_type(self._h, item_id, None, 0), "hc_heif_aux_type")
+        buf = C.create_string_buffer(n + 1)
+        self._L.hc_heif_aux_type(self._h, item_id, buf, n + 1)
+        return buf.value.decode()
+
+    def _ids(self, fn, item_id):
+        n = fn(self._h, item_id, None, 0)
+        ids = (C.c_uint32 * max(n, 1))()
+        return list(ids[:fn(self._h, item_id, ids, n)])
+
     def image_info(self, item_id):
         info = HeifImageInfo()
         check(self._L, self._L.hc_heif_get_image_info(self._h, item_id, C.byref(info)), "hc_heif_get_image_info")
@@ -297,8 +319,9 @@ class Batch:
 
 
 def _place_image(hf, batch, item_id):
-    """Adds one top-level HEIF image (single picture or grid + optional alpha) to a batch.
-    Mirrors HeifContext::decode_image_planar / decode_full_grid_image (context.cc:1729-2404).
+    """Adds one HEIF image (single picture or grid + optional alpha) to a batch, stage by stage: a test helper for
+    placing pictures with the Batch calls (tests/test_scaled_output.py); decode_heic and HeicJob decode through the native
+    job. Mirrors HeifContext::decode_image_planar / decode_full_grid_image (context.cc:1729-2404).
     Returns (canvas, effective nclx tuple (matrix, primaries, full_range), has_alpha, bit_depth, chroma_format)."""
     info = hf.image_info(item_id)
     # this stage-level helper places pictures only; the native job (hc_heic_job, HeicJob) is what applies irot / imir /
@@ -345,37 +368,24 @@ def _place_image(hf, batch, item_id):
 def decode_heic(engine, data, out_format=OUT_RGB, item_id=None):
     """HEIC file bytes -> interleaved RGB rows (numpy uint8 [h, w*bytes_per_pixel]), the Python
     twin of heif_decode_image(handle, &img, heif_colorspace_RGB, heif_chroma_interleaved_*, NULL).
-    The primary image goes through the native job (hc_heic_job: transformations, alpha of any size, every output format);
-    another item of the file (item_id) through the stage-level calls, which refuse what they do not apply."""
-    hf = HeifFile(data)
-    if item_id is None or item_id == hf.primary_id:
-        hf.close()
-        job = HeicJob(engine, [data], out_format=out_format)
-        try:
-            job.upload()
-            job.run()
-            return job.read_rgb(0)
-        finally:
-            job.close()
-    batch = engine.batch()
+    item_id: any image item of the file (a thumbnail, an auxiliary image, another top-level image; None = the primary),
+    decoded through the native job (hc_heic_job_create_items) with its own transformations, alpha and colour properties."""
+    job = HeicJob(engine, [data], out_format=out_format, items=[item_id])
     try:
-        canvas, (matrix, primaries, full_range), has_alpha, bd, cf = _place_image(hf, batch, item_id or hf.primary_id)
-        params = csc_select(matrix, primaries, full_range, cf, bd, has_alpha, out_format)
-        batch.upload()
-        batch.reconstruct(STAGE_ALL)
-        batch.convert(canvas, params)
-        return batch.read_rgb(canvas, out_format)
+        job.upload()
+        job.run()
+        return job.read_rgb(0)
     finally:
-        batch.close()
-        hf.close()
+        job.close()
 
 
 class HeicJob:
     """Many HEIC files -> interleaved RGB through the native batch path (hc_heic_job): host threads
     parse every coded item, the GPU reconstructs all of them as one batch."""
 
-    def __init__(self, engine, files, want_alpha=False, threads=0, out_format=None):
-        """out_format: one of OUT_* for every image whatever its bit depth (HC_OUTPUT_FORMAT), default by bit depth"""
+    def __init__(self, engine, files, want_alpha=False, threads=0, out_format=None, items=None):
+        """out_format: one of OUT_* for every image whatever its bit depth (HC_OUTPUT_FORMAT), default by bit depth.
+        items: per file the image item to decode (0 / None: the primary image), see hc_heic_job_create_items"""
         from ._lib import ImageDesc
         if out_format is not None:
             want_alpha = 0x100 | int(out_format)
@@ -384,7 +394,7 @@ class HeicJob:
         n = len(files)
         ptrs = (C.c_char_p * n)(*[C.cast(b, C.c_char_p) for b in self._bufs])
         sizes = (C.c_size_t * n)(*[len(f) for f in files])
-        self._h = self._L.hc_heic_job_create(engine._h, n, ptrs, sizes, int(want_alpha), threads)
+        self._h = self._L.hc_heic_job_create_items(engine._h, n, ptrs, sizes, _item_ids(items, n), int(want_alpha), threads)
         if not self._h:
             raise HeifCudaError("heic job: " + (self._L.hc_last_error() or b"").decode())
         self.descs = []
@@ -467,15 +477,25 @@ class HeicJob:
         self.close()
 
 
+def _item_ids(items, n):
+    """the item_ids argument of hc_heic_job_create_items / hc_heic_decode_stream_items: NULL, or one id per entry (0 = primary)"""
+    if items is None:
+        return None
+    if len(items) != n:
+        raise ValueError("items: %d ids for %d files" % (len(items), n))
+    return (C.c_uint32 * n)(*[int(i or 0) for i in items])
+
+
 def decode_stream(engine, files, on_image=None, want_alpha=False, threads=0, files_per_batch=8, out_format=None, dests=None,
-                  isolate_errors=False):
+                  isolate_errors=False, items=None):
     """Long file lists (hc_heic_decode_stream): host parse of batch b+1 overlaps upload + kernels + read-back of
     batch b. on_image(file_index, desc, rows) gets every image as a numpy view [h, w*bytes_per_pixel] of PINNED
     host memory that is only valid inside the callback; with out_format=OUT_YCBCR `rows` is instead the list of the image's
     planes (split_planes), views of the same kind. Returns the hc_stream_stats as a dict.
     dests: per file a writable uint8 array or None; [rows, stride] for interleaved output, 1-D (the packed bytes) for OUT_YCBCR.
     isolate_errors: a file that cannot be decoded does not fail the call; the dict gains "file_status" (one HC_* code per
-    file, 0 = delivered) and "first_error" (text)."""
+    file, 0 = delivered) and "first_error" (text).
+    items: per file the image item to decode (0 / None: the primary image); index, dests and file_status are per entry."""
     from ._lib import IMAGE_CALLBACK, StreamStats
     L = engine._L
     if out_format is not None:
@@ -510,8 +530,8 @@ def decode_stream(engine, files, on_image=None, want_alpha=False, threads=0, fil
             if a is not None:
                 xd[k].dst, xd[k].len, xd[k].stride = a.ctypes.data, a.nbytes, a.strides[0] if a.ndim > 1 else 0
     status = (C.c_int * n)() if isolate_errors else None
-    check(L, L.hc_heic_decode_stream_ext(engine._h, n, ptrs, sizes, int(want_alpha), threads, files_per_batch, xd, status, cb, None,
-                                         C.byref(st)), "hc_heic_decode_stream")
+    check(L, L.hc_heic_decode_stream_items(engine._h, n, ptrs, sizes, _item_ids(items, n), int(want_alpha), threads, files_per_batch, xd,
+                                           status, cb, None, C.byref(st)), "hc_heic_decode_stream")
     out = {k: getattr(st, k) for k, _ in StreamStats._fields_}
     if isolate_errors:
         out["file_status"] = list(status)

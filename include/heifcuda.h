@@ -147,6 +147,16 @@ int hc_heif_get_overlay(const hc_heif* f, uint32_t id, hc_heif_overlay_info* inf
 int hc_heif_get_image_info(const hc_heif* f, uint32_t id, hc_heif_image_info* info);
 /* row-major tile item ids of a grid; returns rows*cols or a negative error */
 int hc_heif_grid_tiles(const hc_heif* f, uint32_t id, uint32_t* tiles, int max);
+/* The other images of a file (libheif's heif_image_handle_get_list_of_thumbnail_IDs / ..._auxiliary_image_IDs): the items
+ * with a 'thmb' / 'auxl' reference to image `id`, in ascending item id. Writes up to `max` ids and returns the total count.
+ * include_alpha = 0 leaves out the alpha images (heif_image_handle_get_list_of_auxiliary_image_IDs with
+ * LIBHEIF_AUX_IMAGE_FILTER_OMIT_ALPHA). Any of these items can be decoded by naming it in hc_heic_job_create_items. */
+int hc_heif_thumbnail_ids(const hc_heif* f, uint32_t id, uint32_t* ids, int max);
+int hc_heif_auxiliary_ids(const hc_heif* f, uint32_t id, int include_alpha, uint32_t* ids, int max);
+/* auxC type URN of an auxiliary image (heif_image_handle_get_auxiliary_type), e.g. "urn:mpeg:hevc:2015:auxid:2" for a depth
+ * map: copied NUL-terminated into buf (truncated to len - 1 characters); returns its length, HC_ERR_ARGUMENT for an item
+ * without auxC. */
+int hc_heif_aux_type(const hc_heif* f, uint32_t id, char* buf, size_t len);
 /* hvcC parameter sets + item data as 4-byte-length-prefixed NAL units (what libheif gives
  * heif_decoder_plugin::push_data). *out is malloc'ed; release with hc_free. */
 int hc_heif_coded_stream(const hc_heif* f, uint32_t id, uint8_t** out, size_t* size);
@@ -406,6 +416,15 @@ size_t hc_image_plane_layout(const hc_image_desc* d, size_t offset[4], size_t st
 #define HC_OUTPUT_FORMAT(fmt) (0x100 | (fmt))
 hc_heic_job* hc_heic_job_create(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
                                 int want_alpha, int threads);
+/* Any image item, not only the primary one (heif_context_get_image_handle / heif_image_handle_get_thumbnail /
+ * heif_image_handle_get_auxiliary_image_handle + heif_decode_image): image k of the job is item item_ids[k] of buffer k,
+ * 0 = its primary image; item_ids == NULL is hc_heic_job_create. The same buffer may appear in several entries. The item is
+ * decoded exactly as a primary image would be: its own irot / imir / clap, its own alpha image (an 'auxl' alpha referring to
+ * it, at any size), its own colr, its 'prem' flag, grid and 'iovl' composition. Any 'hvc1', 'grid' or 'iovl' item may be
+ * named: hidden items, thumbnails, auxiliary images (an alpha or depth image decodes as a monochrome image), grid tiles.
+ * Any other item ('Exif', 'mime', 'iden', a missing id) fails the job with a text that names the item. */
+hc_heic_job* hc_heic_job_create_items(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes,
+                                      const uint32_t* item_ids, int want_alpha, int threads);
 /* Multi-GPU decode of ONE huge grid image (BASELINE config C5): every GPU decodes a band of tile rows
  * [tile_row_begin, tile_row_end) of the primary grid image; the job's single output image is that band
  * (desc.height = band height). *first_output_row / *full_height place the band in the whole picture; the
@@ -508,6 +527,14 @@ typedef struct hc_stream_dest {
 int hc_heic_decode_stream_ext(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, int want_alpha,
                               int threads, int files_per_batch, const hc_stream_dest* dests, int* file_status,
                               hc_image_callback on_image, void* user, hc_stream_stats* stats);
+/* hc_heic_decode_stream_ext over entries that name an image item each (see hc_heic_job_create_items): entry k is item
+ * item_ids[k] of buffer k (0 = the primary image), and file_index, file_status[k] and dests[k] refer to entry k; item_ids ==
+ * NULL is hc_heic_decode_stream_ext. The automatic batch size (files_per_batch == 0) follows the size of the named items, so
+ * a list of thumbnails goes in large batches. An entry naming an item that cannot be decoded fails alone under error
+ * isolation. */
+int hc_heic_decode_stream_items(hc_engine* e, int nfiles, const uint8_t* const* data, const size_t* sizes, const uint32_t* item_ids,
+                                int want_alpha, int threads, int files_per_batch, const hc_stream_dest* dests, int* file_status,
+                                hc_image_callback on_image, void* user, hc_stream_stats* stats);
 /* pinned host memory for fast H2D/D2H in the caller (NULL when no CUDA engine) */
 void* hc_host_alloc(size_t bytes);
 void hc_host_free(void* p);
