@@ -816,7 +816,8 @@ int hc_batch_upload(hc_batch* b) {
     uint8_t* kst_out = H + o_kstatic;
     hc::k0::Sub* ksub_out = (hc::k0::Sub*)(H + o_ksubs);
     size_t is = 0, ic = 0, isub = 0, ib = 0;
-    std::vector<std::pair<int, hc::k0::Chain>> chains;   // (row of the first substream, chain)
+    struct ChainKey { int row; uint64_t bytes; hc::k0::Chain chain; };   // row of the first substream, slice data bytes
+    std::vector<ChainKey> chains;
     for (int q = 0; q < nk0; q++) {
       const int i = b->k0_pic_of[q];
       const hc::K0HostPicture& k = *b->pics[i].k0;
@@ -850,14 +851,27 @@ int hc_batch_upload(hc_batch* b) {
       memcpy(kst_out + 4 * ic, k.ctu_static.data(), k.ctu_static.size());
       k0_copies.push_back({H + o_kbytes + ib, k.bytes.data(), k.bytes.size()});
       for (size_t t = 0; t < k.subs.size(); t++) { ksub_out[isub + t] = k.subs[t]; ksub_out[isub + t].pic = (uint32_t)q; }
-      for (const hc::k0::Chain& c : k.chains) chains.push_back({k.subs[c.first_sub].first_ctb / k.pic.ctbs_w, {(uint32_t)(isub + c.first_sub), c.nsubs}});
+      for (const hc::k0::Chain& c : k.chains) {
+        // a substream ends at the next one's entry point or at the end of its slice segment's data
+        uint64_t bytes = 0;
+        for (uint32_t t = c.first_sub; t < c.first_sub + c.nsubs; t++) {
+          const hc::k0::Sub& sub = k.subs[t];
+          const bool entry_next = t + 1 < k.subs.size() && k.subs[t + 1].slice == sub.slice;
+          const uint32_t end = entry_next ? k.subs[t + 1].byte_begin : k.slices[sub.slice].data_end;
+          bytes += end > sub.byte_begin ? end - sub.byte_begin : 0;
+        }
+        chains.push_back({k.subs[c.first_sub].first_ctb / k.pic.ctbs_w, bytes, {(uint32_t)(isub + c.first_sub), c.nsubs}});
+      }
       is += k.slices.size(); ic += k.ctb_slice.size(); isub += k.subs.size(); ib += align_up(k.bytes.size(), 16);
     }
     memset(H + o_kbytes + ib, 0, 64);
-    // rows of all pictures interleaved: a chain only ever waits for a chain with a smaller index
-    std::stable_sort(chains.begin(), chains.end(), [](const std::pair<int, hc::k0::Chain>& a, const std::pair<int, hc::k0::Chain>& c) { return a.first < c.first; });
+    // rows of all pictures interleaved: a chain only ever waits for a chain with a smaller index. Within a row the chain
+    // with the most slice data comes first: the four chains of a K0 CTA, which holds its slot until the slowest one
+    // ends, then take about the same time, and the longest chains do not start last. The key (row, -bytes, position) is
+    // total, so the order is deterministic.
+    std::stable_sort(chains.begin(), chains.end(), [](const ChainKey& a, const ChainKey& c) { return a.row != c.row ? a.row < c.row : a.bytes > c.bytes; });
     hc::k0::Chain* kch_out = (hc::k0::Chain*)(H + o_kchains);
-    for (size_t t = 0; t < chains.size(); t++) kch_out[t] = chains[t].second;
+    for (size_t t = 0; t < chains.size(); t++) kch_out[t] = chains[t].chain;
     b->d_k0_pics = (const hc::k0::Pic*)(Dk + o_kpics);
     b->d_k0_subs = (const hc::k0::Sub*)(Dk + o_ksubs);
     b->d_k0_chains = (const hc::k0::Chain*)(Dk + o_kchains);

@@ -3,17 +3,19 @@
 // CABAC is serial inside a substream, so the parallelism is across substreams: the CTB rows of WPP pictures
 // (wavefront-synchronised with the row above, kernels/k0_core.cuh) and across the pictures / grid tiles / files of a
 // batch — a 12 MP iPhone-style grid image is 48 tiles x 8 rows = 384 chains; a batch of 8 such files keeps 3072
-// chains in flight. Chains are ordered row-major across all pictures so that a chain only ever waits for a chain
-// with a smaller index (scheduled no later than itself). Tables, context states and the picture / slice descriptors
-// of a chain live in shared memory (k0_core.cuh: Scratch).
+// chains in flight. Chains are ordered row-major across all pictures, the longest first within a row, so that a chain
+// only ever waits for a chain with a smaller index (scheduled no later than itself). Tables, context states and the
+// picture / slice descriptors of a chain live in shared memory (k0_core.cuh: Scratch).
 #include "launch.h"
 #include "k0_core.cuh"
 
 namespace hc {
 
 // Chains per CTA: the warps of a CTA share one shared-memory copy of the parser tables; each warp owns a Scratch
-// (context states, picture / slice descriptors, K1 list staging). Consecutive chains are the same CTB row of
-// consecutive pictures, so the warps of a CTA run for about the same time.
+// (context states, picture / slice descriptors, K1 list staging). A CTA frees its slot when its slowest chain ends;
+// consecutive chains are the same CTB row with about the same amount of slice data (engine.cu sorts them so), so the
+// warps of a CTA run for about the same time. Warps that claim chains one by one from a counter instead were measured
+// slower (DESIGN.md §3a, v10).
 constexpr int K0_WARPS = 4;
 
 // K0_MIN_CTAS: CTAs per SM the register allocation must allow (5 -> 96 registers, 6 -> 80, 8 -> 64). A chain uses one

@@ -81,7 +81,7 @@ struct PackBatch {
 void launch_k8_batch(const PackBatch& b, cudaStream_t stream);
 
 namespace k0 { struct Tables; struct Pic; struct Sub; struct Chain; }
-// K0: device CABAC parse of the pictures added as bitstreams (one CTA per substream chain)
+// K0: device CABAC parse of the pictures added as bitstreams (one warp per substream chain, four chains per CTA)
 void launch_k0(const k0::Tables* tables, const k0::Pic* pics, const k0::Sub* subs, const k0::Chain* chains, int nchains,
                cudaStream_t stream);
 void launch_k0_finish(const k0::Pic* pics, int npics, int max_ctbs, cudaStream_t stream);
